@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py - BN254 pairings/sec and BLS verifies/sec on N B200s, beside the host-core CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 20] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1]): a batch of 2^20 independent optimal-ate pairings on random
 G1 x G2 points per GPU (weak scaling: every rank runs its own contiguous 2^20 slice, no data-path
@@ -69,7 +69,15 @@ def parse():
     ap.add_argument("--groth-log2n", type=int, default=18)
     ap.add_argument("--mul-log2n", type=int, default=22)
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="budget of each cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of rank 0's last-step pairings to DIR as .npy "
+                         "(inputs are seeded, so two builds run with the same arguments can be compared)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -232,6 +240,24 @@ def roofline_block(kernel: str, label: str, n_items: int, fp_mul_per_item: float
     return blk
 
 
+DUMP_ROWS = 1 << 15  # sampled pairings: 32768 x 96 limbs x 8 bytes = 24 MiB
+
+
+def dump_pairing_outputs(out_dir: str, d_out) -> None:
+    """Writes a fixed, seeded sample of the rows of d_out: pairing_batch.npy holds the Gt values as float64
+    (rows, 12, 8) - 12 Fp coefficients of 8 little-endian 32-bit limbs each, every limb exact in float64 - and
+    pairing_batch_rows.npy the batch indices of those rows."""
+    import numpy as np
+    import torch
+
+    n = d_out.shape[0]
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    sample = d_out[torch.from_numpy(rows).to(d_out.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pairing_batch.npy"), sample.view("<u4").reshape(len(rows), 12, 8).astype(np.float64))
+    np.save(os.path.join(out_dir, "pairing_batch_rows.npy"), rows.astype(np.float64))
+
+
 def main():
     args = parse()
     if args.impl == "reference":
@@ -344,6 +370,8 @@ def main():
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:  # before the legs below overwrite d_out
+        dump_pairing_outputs(args.dump_outputs, d_out)
     value = world * n * K / (ms_total * 1e-3)
     analytic = sms * 32.0 * (clocks["sm_mhz"] or 1965.0) * 1e6
 
