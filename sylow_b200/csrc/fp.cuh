@@ -525,9 +525,8 @@ __device__ __forceinline__ void redc_round(uint32_t* X, uint32_t* Y) {
       : "r"(m));
 }
 
-// r = T * R^-1 mod p, fully reduced, for T < p * R.  The 8 rounds work on the low half only:
-// (T_lo + M p) / R <= p, and the high half (< p) is added at the end.
-__device__ __forceinline__ Fp fp_redc_wide(const uint32_t* T) {
+// W = (T_lo + M p) / R <= p for the low half T_lo = T[0..7] (8 reduce-only CIOS rounds): W = T_lo * R^-1 mod p.
+__device__ __forceinline__ Fp redc_low(const uint32_t* T) {
   uint32_t ev[8], od[8];
 #pragma unroll
   for (int i = 0; i < 8; i++) ev[i] = T[i];
@@ -539,8 +538,8 @@ __device__ __forceinline__ Fp fp_redc_wide(const uint32_t* T) {
   redc_round<false>(od, ev);
   redc_round<false>(ev, od);
   redc_round<false>(od, ev);
-  // last round: X = od, Y = ev  ->  W = ev + (od >> 32); r = W + T_hi
-  Fp w, r;
+  // last round: X = od, Y = ev  ->  W = ev + (od >> 32)
+  Fp w;
   asm("add.cc.u32 %0, %8, %16;\n\t"
       "addc.cc.u32 %1, %9, %17;\n\t"
       "addc.cc.u32 %2, %10, %18;\n\t"
@@ -552,6 +551,12 @@ __device__ __forceinline__ Fp fp_redc_wide(const uint32_t* T) {
       : "=r"(w.l[0]), "=r"(w.l[1]), "=r"(w.l[2]), "=r"(w.l[3]), "=r"(w.l[4]), "=r"(w.l[5]), "=r"(w.l[6]), "=r"(w.l[7])
       : "r"(ev[0]), "r"(ev[1]), "r"(ev[2]), "r"(ev[3]), "r"(ev[4]), "r"(ev[5]), "r"(ev[6]), "r"(ev[7]),
         "r"(od[1]), "r"(od[2]), "r"(od[3]), "r"(od[4]), "r"(od[5]), "r"(od[6]), "r"(od[7]));
+  return w;
+}
+
+// r = T * R^-1 mod p, fully reduced, for T < p * R: W + T_hi with W <= p, T_hi < p.
+__device__ __forceinline__ Fp fp_redc_wide(const uint32_t* T) {
+  Fp w = redc_low(T), r;
   asm("add.cc.u32 %0, %8, %16;\n\t"
       "addc.cc.u32 %1, %9, %17;\n\t"
       "addc.cc.u32 %2, %10, %18;\n\t"
@@ -641,6 +646,150 @@ __device__ __forceinline__ void wide_dbl(uint32_t* a) {
   for (int i = 15; i > 0; i--) a[i] = __funnelshift_l(a[i - 1], a[i], 1);
   a[0] <<= 1;
 }
+
+// ---- 17-limb accumulators: a signed combination of 512-bit products, reduced once ---------------------------------
+// A = sum k_i T_i + L p R with small integers k_i and a lift L p R (a multiple of p, so the residue is unchanged) that
+// makes the sum non-negative.  The limbs are exact mod 2^544, so only the FINAL value has to lie in [0, 2^544); the
+// callers state their bounds.  Each helper is one carry chain (acc_madd: two chains of 8 IMAD.WIDE).
+// The top limb is materialised at the end of every helper: ptxas otherwise defers its final carry addition to the
+// reduction, keeps that carry in a predicate register across the next products and spills predicates into a bit mask.
+#define SY_ACC_TOP(A) asm volatile("" : "+r"((A)[16]))
+// A = L p R - T for T < L p R; the 8 limbs of L p (< 2^256) are Lp.  A[16] = 0.
+__device__ __forceinline__ void acc_lift_sub(uint32_t* A, const uint32_t* Lp, const uint32_t* T) {
+  asm("sub.cc.u32 %0, 0, %17;\n\t"
+      "subc.cc.u32 %1, 0, %18;\n\t"
+      "subc.cc.u32 %2, 0, %19;\n\t"
+      "subc.cc.u32 %3, 0, %20;\n\t"
+      "subc.cc.u32 %4, 0, %21;\n\t"
+      "subc.cc.u32 %5, 0, %22;\n\t"
+      "subc.cc.u32 %6, 0, %23;\n\t"
+      "subc.cc.u32 %7, 0, %24;\n\t"
+      "subc.cc.u32 %8, %33, %25;\n\t"
+      "subc.cc.u32 %9, %34, %26;\n\t"
+      "subc.cc.u32 %10, %35, %27;\n\t"
+      "subc.cc.u32 %11, %36, %28;\n\t"
+      "subc.cc.u32 %12, %37, %29;\n\t"
+      "subc.cc.u32 %13, %38, %30;\n\t"
+      "subc.cc.u32 %14, %39, %31;\n\t"
+      "subc.u32 %15, %40, %32;\n\t"
+      "mov.u32 %16, 0;"
+      : "=r"(A[0]), "=r"(A[1]), "=r"(A[2]), "=r"(A[3]), "=r"(A[4]), "=r"(A[5]), "=r"(A[6]), "=r"(A[7]), "=r"(A[8]),
+        "=r"(A[9]), "=r"(A[10]), "=r"(A[11]), "=r"(A[12]), "=r"(A[13]), "=r"(A[14]), "=r"(A[15]), "=r"(A[16])
+      : "r"(T[0]), "r"(T[1]), "r"(T[2]), "r"(T[3]), "r"(T[4]), "r"(T[5]), "r"(T[6]), "r"(T[7]), "r"(T[8]), "r"(T[9]),
+        "r"(T[10]), "r"(T[11]), "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]), "r"(Lp[0]), "r"(Lp[1]), "r"(Lp[2]),
+        "r"(Lp[3]), "r"(Lp[4]), "r"(Lp[5]), "r"(Lp[6]), "r"(Lp[7]));
+}
+// A += T
+__device__ __forceinline__ void acc_add(uint32_t* A, const uint32_t* T) {
+  asm("add.cc.u32 %0, %0, %17;\n\t"
+      "addc.cc.u32 %1, %1, %18;\n\t"
+      "addc.cc.u32 %2, %2, %19;\n\t"
+      "addc.cc.u32 %3, %3, %20;\n\t"
+      "addc.cc.u32 %4, %4, %21;\n\t"
+      "addc.cc.u32 %5, %5, %22;\n\t"
+      "addc.cc.u32 %6, %6, %23;\n\t"
+      "addc.cc.u32 %7, %7, %24;\n\t"
+      "addc.cc.u32 %8, %8, %25;\n\t"
+      "addc.cc.u32 %9, %9, %26;\n\t"
+      "addc.cc.u32 %10, %10, %27;\n\t"
+      "addc.cc.u32 %11, %11, %28;\n\t"
+      "addc.cc.u32 %12, %12, %29;\n\t"
+      "addc.cc.u32 %13, %13, %30;\n\t"
+      "addc.cc.u32 %14, %14, %31;\n\t"
+      "addc.cc.u32 %15, %15, %32;\n\t"
+      "addc.u32 %16, %16, 0;"
+      : "+r"(A[0]), "+r"(A[1]), "+r"(A[2]), "+r"(A[3]), "+r"(A[4]), "+r"(A[5]), "+r"(A[6]), "+r"(A[7]), "+r"(A[8]),
+        "+r"(A[9]), "+r"(A[10]), "+r"(A[11]), "+r"(A[12]), "+r"(A[13]), "+r"(A[14]), "+r"(A[15]), "+r"(A[16])
+      : "r"(T[0]), "r"(T[1]), "r"(T[2]), "r"(T[3]), "r"(T[4]), "r"(T[5]), "r"(T[6]), "r"(T[7]), "r"(T[8]), "r"(T[9]),
+        "r"(T[10]), "r"(T[11]), "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]));
+  SY_ACC_TOP(A);
+}
+// A -= T
+__device__ __forceinline__ void acc_sub(uint32_t* A, const uint32_t* T) {
+  asm("sub.cc.u32 %0, %0, %17;\n\t"
+      "subc.cc.u32 %1, %1, %18;\n\t"
+      "subc.cc.u32 %2, %2, %19;\n\t"
+      "subc.cc.u32 %3, %3, %20;\n\t"
+      "subc.cc.u32 %4, %4, %21;\n\t"
+      "subc.cc.u32 %5, %5, %22;\n\t"
+      "subc.cc.u32 %6, %6, %23;\n\t"
+      "subc.cc.u32 %7, %7, %24;\n\t"
+      "subc.cc.u32 %8, %8, %25;\n\t"
+      "subc.cc.u32 %9, %9, %26;\n\t"
+      "subc.cc.u32 %10, %10, %27;\n\t"
+      "subc.cc.u32 %11, %11, %28;\n\t"
+      "subc.cc.u32 %12, %12, %29;\n\t"
+      "subc.cc.u32 %13, %13, %30;\n\t"
+      "subc.cc.u32 %14, %14, %31;\n\t"
+      "subc.cc.u32 %15, %15, %32;\n\t"
+      "subc.u32 %16, %16, 0;"
+      : "+r"(A[0]), "+r"(A[1]), "+r"(A[2]), "+r"(A[3]), "+r"(A[4]), "+r"(A[5]), "+r"(A[6]), "+r"(A[7]), "+r"(A[8]),
+        "+r"(A[9]), "+r"(A[10]), "+r"(A[11]), "+r"(A[12]), "+r"(A[13]), "+r"(A[14]), "+r"(A[15]), "+r"(A[16])
+      : "r"(T[0]), "r"(T[1]), "r"(T[2]), "r"(T[3]), "r"(T[4]), "r"(T[5]), "r"(T[6]), "r"(T[7]), "r"(T[8]), "r"(T[9]),
+        "r"(T[10]), "r"(T[11]), "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]));
+  SY_ACC_TOP(A);
+}
+// A += K T: the even limbs of T in one chain over A[0..16], the odd limbs in a second one over A[1..16]
+template <uint32_t K>
+__device__ __forceinline__ void acc_madd(uint32_t* A, const uint32_t* T) {
+  asm("mad.lo.cc.u32 %0, %17, %25, %0;\n\t"
+      "madc.hi.cc.u32 %1, %17, %25, %1;\n\t"
+      "madc.lo.cc.u32 %2, %18, %25, %2;\n\t"
+      "madc.hi.cc.u32 %3, %18, %25, %3;\n\t"
+      "madc.lo.cc.u32 %4, %19, %25, %4;\n\t"
+      "madc.hi.cc.u32 %5, %19, %25, %5;\n\t"
+      "madc.lo.cc.u32 %6, %20, %25, %6;\n\t"
+      "madc.hi.cc.u32 %7, %20, %25, %7;\n\t"
+      "madc.lo.cc.u32 %8, %21, %25, %8;\n\t"
+      "madc.hi.cc.u32 %9, %21, %25, %9;\n\t"
+      "madc.lo.cc.u32 %10, %22, %25, %10;\n\t"
+      "madc.hi.cc.u32 %11, %22, %25, %11;\n\t"
+      "madc.lo.cc.u32 %12, %23, %25, %12;\n\t"
+      "madc.hi.cc.u32 %13, %23, %25, %13;\n\t"
+      "madc.lo.cc.u32 %14, %24, %25, %14;\n\t"
+      "madc.hi.cc.u32 %15, %24, %25, %15;\n\t"
+      "addc.u32 %16, %16, 0;"
+      : "+r"(A[0]), "+r"(A[1]), "+r"(A[2]), "+r"(A[3]), "+r"(A[4]), "+r"(A[5]), "+r"(A[6]), "+r"(A[7]), "+r"(A[8]),
+        "+r"(A[9]), "+r"(A[10]), "+r"(A[11]), "+r"(A[12]), "+r"(A[13]), "+r"(A[14]), "+r"(A[15]), "+r"(A[16])
+      : "r"(T[0]), "r"(T[2]), "r"(T[4]), "r"(T[6]), "r"(T[8]), "r"(T[10]), "r"(T[12]), "r"(T[14]), "n"(K));
+  asm("mad.lo.cc.u32 %0, %16, %24, %0;\n\t"
+      "madc.hi.cc.u32 %1, %16, %24, %1;\n\t"
+      "madc.lo.cc.u32 %2, %17, %24, %2;\n\t"
+      "madc.hi.cc.u32 %3, %17, %24, %3;\n\t"
+      "madc.lo.cc.u32 %4, %18, %24, %4;\n\t"
+      "madc.hi.cc.u32 %5, %18, %24, %5;\n\t"
+      "madc.lo.cc.u32 %6, %19, %24, %6;\n\t"
+      "madc.hi.cc.u32 %7, %19, %24, %7;\n\t"
+      "madc.lo.cc.u32 %8, %20, %24, %8;\n\t"
+      "madc.hi.cc.u32 %9, %20, %24, %9;\n\t"
+      "madc.lo.cc.u32 %10, %21, %24, %10;\n\t"
+      "madc.hi.cc.u32 %11, %21, %24, %11;\n\t"
+      "madc.lo.cc.u32 %12, %22, %24, %12;\n\t"
+      "madc.hi.cc.u32 %13, %22, %24, %13;\n\t"
+      "madc.lo.cc.u32 %14, %23, %24, %14;\n\t"
+      "madc.hi.u32 %15, %23, %24, %15;"
+      : "+r"(A[1]), "+r"(A[2]), "+r"(A[3]), "+r"(A[4]), "+r"(A[5]), "+r"(A[6]), "+r"(A[7]), "+r"(A[8]), "+r"(A[9]),
+        "+r"(A[10]), "+r"(A[11]), "+r"(A[12]), "+r"(A[13]), "+r"(A[14]), "+r"(A[15]), "+r"(A[16])
+      : "r"(T[1]), "r"(T[3]), "r"(T[5]), "r"(T[7]), "r"(T[9]), "r"(T[11]), "r"(T[13]), "r"(T[15]), "n"(K));
+  SY_ACC_TOP(A);
+}
+// V = A * R^-1 mod p, not reduced: V = W + A_hi with W <= p (redc_low) and A_hi = floor(A / R).  9 limbs, the caller
+// keeps A small enough for lin9_reduce (V < 2^262).
+__device__ __forceinline__ void fp_redc_acc(uint32_t* V, const uint32_t* A) {
+  Fp w = redc_low(A);
+  asm("add.cc.u32 %0, %9, %17;\n\t"
+      "addc.cc.u32 %1, %10, %18;\n\t"
+      "addc.cc.u32 %2, %11, %19;\n\t"
+      "addc.cc.u32 %3, %12, %20;\n\t"
+      "addc.cc.u32 %4, %13, %21;\n\t"
+      "addc.cc.u32 %5, %14, %22;\n\t"
+      "addc.cc.u32 %6, %15, %23;\n\t"
+      "addc.cc.u32 %7, %16, %24;\n\t"
+      "addc.u32 %8, %25, 0;"
+      : "=r"(V[0]), "=r"(V[1]), "=r"(V[2]), "=r"(V[3]), "=r"(V[4]), "=r"(V[5]), "=r"(V[6]), "=r"(V[7]), "=r"(V[8])
+      : "r"(w.l[0]), "r"(w.l[1]), "r"(w.l[2]), "r"(w.l[3]), "r"(w.l[4]), "r"(w.l[5]), "r"(w.l[6]), "r"(w.l[7]),
+        "r"(A[8]), "r"(A[9]), "r"(A[10]), "r"(A[11]), "r"(A[12]), "r"(A[13]), "r"(A[14]), "r"(A[15]), "r"(A[16]));
+}
 #else
 // host simulation only: same contracts with 64-bit temporaries
 inline void fp_sub_nr(uint32_t* r, const uint32_t* a, const uint32_t* b) {
@@ -715,14 +864,81 @@ inline void fp_add_nr(uint32_t* r, const uint32_t* a, const uint32_t* b) {
     c >>= 32;
   }
 }
+inline void acc_lift_sub(uint32_t* A, const uint32_t* Lp, const uint32_t* T) {
+  int64_t bw = 0;
+  for (int i = 0; i < 16; i++) {
+    int64_t d = (int64_t)(i < 8 ? 0u : Lp[i - 8]) - (int64_t)T[i] + bw;
+    A[i] = (uint32_t)d;
+    bw = d >> 32;
+  }
+  A[16] = 0;
+}
+inline void acc_add(uint32_t* A, const uint32_t* T) {
+  uint64_t c = 0;
+  for (int i = 0; i < 17; i++) {
+    c += (uint64_t)A[i] + (i < 16 ? T[i] : 0u);
+    A[i] = (uint32_t)c;
+    c >>= 32;
+  }
+}
+inline void acc_sub(uint32_t* A, const uint32_t* T) {
+  int64_t bw = 0;
+  for (int i = 0; i < 17; i++) {
+    int64_t d = (int64_t)A[i] - (int64_t)(i < 16 ? T[i] : 0u) + bw;
+    A[i] = (uint32_t)d;
+    bw = d >> 32;
+  }
+}
+template <uint32_t K>
+inline void acc_madd(uint32_t* A, const uint32_t* T) {
+  uint64_t c = 0;
+  for (int i = 0; i < 17; i++) {
+    c += (uint64_t)A[i] + (i < 16 ? (uint64_t)K * T[i] : 0u);
+    A[i] = (uint32_t)c;
+    c >>= 32;
+  }
+}
+inline void fp_redc_acc(uint32_t* V, const uint32_t* A) {
+  uint32_t t[17] = {0};
+  for (int i = 0; i < 8; i++) t[i] = A[i];
+  for (int i = 0; i < 8; i++) {  // W = (A_lo + M p) / R, as the device's redc_low
+    uint32_t m = t[i] * SY_INV;
+    uint64_t c = 0;
+    for (int j = 0; j < 8; j++) {
+      c += (uint64_t)m * kP_h[j] + t[i + j];
+      t[i + j] = (uint32_t)c;
+      c >>= 32;
+    }
+    for (int j = i + 8; j < 17 && c; j++) {
+      c += t[j];
+      t[j] = (uint32_t)c;
+      c >>= 32;
+    }
+  }
+  uint64_t c = 0;
+  for (int i = 0; i < 9; i++) {
+    c += (uint64_t)(i < 8 ? t[8 + i] : 0u) + A[8 + i];
+    V[i] = (uint32_t)c;
+    c >>= 32;
+  }
+#if defined(SYLOW_HOSTSIM)
+  if (t[16] != 0 || c != 0) {
+    fprintf(stderr, "fp_redc_acc: W > p or V >= 2^288\n");
+    abort();
+  }
+#endif
+}
 #endif
 
 SY_DEFINE_TABLE(uint32_t, kP2, 8, 0xb0f9fa8eu, 0x7841182du, 0xd0e3951au, 0x2f02d522u, 0x0302b0bbu, 0x70a08b6du, 0xc2634053u, 0x60c89ce5u)  // 2p
+SY_DEFINE_TABLE(uint32_t, kP4, 8, 0x61f3f51cu, 0xf082305bu, 0xa1c72a34u, 0x5e05aa45u, 0x06056176u, 0xe14116dau, 0x84c680a6u, 0xc19139cbu)  // 4p
 
 // ---- 9 x + y + t mod p in one pass (the multiplications by xi = 9 + u, tower.cuh) --------------------------------
-// x, y, t < p, so T = 9x + y + t < 11p needs 9 limbs.  The quotient is estimated from the top 32 bits,
-// q = floor(floor(T / 2^226) * 21 / 2^32) in {floor(T/p) - 1, floor(T/p)} (2^34 / 21 is 0.76 % above p / 2^224), and
-// T - q p in [0, 2p) is formed mod 2^256 as T + q (2^256 - p) with one multiplier row, then one conditional subtraction.
+// x, y, t < p, so T = 9x + y + t < 11p needs 9 limbs.  lin9_reduce takes any 9-limb T < 2^262 (338 p; the wide
+// accumulators of the cyclotomic squaring end there, fp_redc_acc).  The quotient is estimated from the top 32 bits,
+// q = floor(floor(T / 2^230) * 338 / 2^32): 338 / 2^262 is below 1 / p (2^262 / p = 338.57), so q never exceeds T / p,
+// and it falls short by less than 338.57 * (1 - 338 / 338.57) + 1 < 2.  T - q p in [0, 2p) is formed mod 2^256 as
+// T + q (2^256 - p) with one multiplier row, then one conditional subtraction.
 // 8 IMAD.WIDE + about 60 ALU instructions instead of the 120 of three doublings, two additions and their reductions.
 #define SY_NP0 0x278302b9
 #define SY_NP1 0xc3df73e9
@@ -758,12 +974,12 @@ SY_HD void lin9_acc(uint32_t* T, const uint32_t* a) {
   T[8] += (uint32_t)c;
 #endif
 }
-// T (9 limbs, < 11p) -> canonical residue
+// T (9 limbs, < 2^262) -> canonical residue
 SY_HD Fp lin9_reduce(const uint32_t* T) {
-  uint32_t h = (T[8] << 30) | (T[7] >> 2);
+  uint32_t h = (T[8] << 26) | (T[7] >> 6);
   Fp r;
 #if defined(__CUDA_ARCH__)
-  uint32_t q = __umulhi(h, 21u);
+  uint32_t q = __umulhi(h, 338u);
   uint32_t e[8], o[8];
   asm("mad.lo.cc.u32 %0, %8, " SY_STR(SY_NP0) ", %9;\n\t"
       "madc.hi.cc.u32 %1, %8, " SY_STR(SY_NP0) ", %10;\n\t"
@@ -793,7 +1009,13 @@ SY_HD Fp lin9_reduce(const uint32_t* T) {
       : "r"(e[1]), "r"(e[2]), "r"(e[3]), "r"(e[4]), "r"(e[5]), "r"(e[6]), "r"(e[7]), "r"(o[1]), "r"(o[2]), "r"(o[3]),
         "r"(o[4]), "r"(o[5]), "r"(o[6]), "r"(o[7]));
 #else
-  uint32_t q = (uint32_t)(((uint64_t)h * 21u) >> 32);
+#if defined(SYLOW_HOSTSIM)
+  if (T[8] >> 6) {
+    fprintf(stderr, "lin9_reduce: input >= 2^262\n");
+    abort();
+  }
+#endif
+  uint32_t q = (uint32_t)(((uint64_t)h * 338u) >> 32);
   uint64_t c = 0;
   for (int i = 0; i < 8; i++) {  // T + q (2^256 - p) mod 2^256
     c += (uint64_t)T[i] + (uint64_t)q * SY_TAB(kNegP)[i];
@@ -849,6 +1071,45 @@ SY_HD Fp fp_neg_nr(const Fp& z) {
   for (int i = 0; i < 8; i++) pp.l[i] = SY_TAB(kP)[i];
   fp_sub_nr(r.l, pp.l, z.l);
   return r;
+}
+
+// ---- 9-limb combinations of fp_redc_acc outputs, finished by lin9_reduce ---------------------------------------------
+// r = a + (b << s)   (9 limbs, s < 32 a compile-time constant; the caller guarantees no overflow)
+SY_HD void u9_add_shl(uint32_t* r, const uint32_t* a, const uint32_t* b, int s) {
+  uint32_t t[9];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+  for (int i = 8; i > 0; i--) t[i] = s ? __funnelshift_l(b[i - 1], b[i], s) : b[i];
+  t[0] = b[0] << s;
+  asm("add.cc.u32 %0, %9, %18;\n\t"
+      "addc.cc.u32 %1, %10, %19;\n\t"
+      "addc.cc.u32 %2, %11, %20;\n\t"
+      "addc.cc.u32 %3, %12, %21;\n\t"
+      "addc.cc.u32 %4, %13, %22;\n\t"
+      "addc.cc.u32 %5, %14, %23;\n\t"
+      "addc.cc.u32 %6, %15, %24;\n\t"
+      "addc.cc.u32 %7, %16, %25;\n\t"
+      "addc.u32 %8, %17, %26;"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(a[4]), "r"(a[5]), "r"(a[6]), "r"(a[7]), "r"(a[8]),
+        "r"(t[0]), "r"(t[1]), "r"(t[2]), "r"(t[3]), "r"(t[4]), "r"(t[5]), "r"(t[6]), "r"(t[7]), "r"(t[8]));
+#else
+  for (int i = 8; i > 0; i--) t[i] = s ? (b[i] << s) | (b[i - 1] >> (32 - s)) : b[i];
+  t[0] = b[0] << s;
+  uint64_t c = 0;
+  for (int i = 0; i < 9; i++) {
+    c += (uint64_t)a[i] + t[i];
+    r[i] = (uint32_t)c;
+    c >>= 32;
+  }
+#endif
+}
+// 3 V + y mod p for a 9-limb V and y < 2^256 (3 V + y < 2^262)
+SY_HD Fp fp_lin3(const uint32_t* V, const Fp& y) {
+  uint32_t T[9];
+  u9_add_shl(T, V, V, 1);
+  lin9_acc(T, y.l);
+  return lin9_reduce(T);
 }
 
 SY_HD Fp fp_sqr(const Fp& a) { return fp_mul(a, a); }

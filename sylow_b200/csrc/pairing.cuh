@@ -198,32 +198,132 @@ SY_HD Fp12 fp12_frobenius(const Fp12& a, int e) {
   return r;
 }
 
-// pairing.rs:274-289
-SY_HD void fp4_square(const Fp2& a, const Fp2& b, Fp2& c0, Fp2& c1) {
-  Fp2 t0 = fp2_sqr(a);
-  Fp2 t1 = fp2_sqr(b);
-  c0 = fp2_mul_xi_add(t1, t0);
-  c1 = fp2_sub(fp2_sub(fp2_sqr(fp2_add(a, b)), t0), t1);
+// One Fp4 squaring of Granger-Scott (pairing.rs:274-289 and the update of its two outputs, :309-346) with lazy reduction:
+//   A = a^2 + xi b^2,  B = 2 a b = (a + b)^2 - a^2 - b^2,  x <- 3 A - 2 x,  y <- 3 B + 2 y  (3 xi B + 2 y when xi is set)
+// Every coefficient of A and B is ONE signed combination of 512-bit products in a 17-limb accumulator (fp.cuh: acc_*),
+// reduced once; the factor 3, the +-2 x / y term and the multiplication by xi = 9 + u act on the 9-limb values after
+// that reduction (fp_lin3).  With u^2 = -1, and all inputs canonical (< p):
+//   S_a = (a0 + a1)(a0 + p - a1) = a0^2 - a1^2 (mod p)  < 4 p^2      Q_a = 2 a0 a1 < 2 p^2     (S_b, Q_b alike)
+//   S_c, Q_c the same for c = a + b (c0, c1 < 2p, not reduced):  S_c < 16 p^2,  Q_c < 8 p^2
+//   A0 = S_a + 9 S_b - Q_b + p R        < 45.3 p^2       A1 = Q_a + S_b + 9 Q_b         < 24 p^2
+//   B0 = S_c - S_a - S_b + 2 p R        < 26.6 p^2       B1 = Q_c - Q_a - Q_b + p R     < 13.3 p^2
+// (p R = 5.29 p^2; every lift exceeds what it covers, so each value is non-negative, and all are below 2^513).  After
+// fp_redc_acc, V = W + floor(acc / R) with W <= p: V_A0 < 9.57 p, V_A1 < 5.54 p, V_B0 < 6.03 p, V_B1 < 3.52 p, and
+// the reduced inputs of lin9_reduce are at most 3 * 9.57 p + 2 p (x), 3 * 6.03 p + 2 p (y) or, with xi,
+// 3 (9 V_B0 + 4 p - V_B1) + 2 p < 177 p and 3 (V_B0 + 9 V_B1) + 2 p < 116 p: all below its 338 p.
+// Six 512-bit products and four Montgomery reductions instead of three Fp2 squarings (nine reductions) and about thirty
+// modular additions.  a and x, b and y may alias (the outputs are written after the last read of the inputs).
+SY_HD_NOINLINE void gs_fp4_square(const Fp2& a_, const Fp2& b_, Fp2& x, Fp2& y, bool xi) {
+  const Fp2 a = fp2_ldv(a_), b = fp2_ldv(b_);
+  uint32_t pp[8], T[16], s[8], d[8], A0[17], A1[17], B0[17], B1[17];
+#pragma unroll
+  for (int i = 0; i < 8; i++) pp[i] = SY_TAB(kP)[i];
+  // Q_b: B1 = p R - Q_b, A0 = p R - Q_b, A1 = 9 Q_b
+  fp_add_nr(s, b.c0.l, b.c0.l);
+  fp_mul_wide(T, s, b.c1.l);
+  acc_lift_sub(B1, pp, T);
+  SY_AFTER(T[0], B1[15]);
+  acc_lift_sub(A0, pp, T);
+#pragma unroll
+  for (int i = 0; i < 17; i++) A1[i] = 0;
+  SY_AFTER(A1[0], A0[15]);
+  acc_madd<9>(A1, T);
+  // Q_a
+  fp_add_nr(s, a.c0.l, a.c0.l);
+  SY_AFTER8(s, A1[16]);
+  fp_mul_wide(T, s, a.c1.l);
+  acc_add(A1, T);
+  SY_AFTER(B1[0], A1[16]);
+  acc_sub(B1, T);
+  // S_b: B0 = 2 p R - S_b
+  fp_add_nr(s, b.c0.l, b.c1.l);
+  fp_add_nr(d, b.c0.l, pp);
+  fp_sub_nr(d, d, b.c1.l);
+  SY_AFTER8(s, B1[16]);
+  SY_AFTER8(d, B1[16]);
+  fp_mul_wide(T, s, d);
+  acc_madd<9>(A0, T);
+  SY_AFTER(A1[0], A0[16]);
+  acc_add(A1, T);
+  SY_AFTER(T[0], A1[16]);
+  acc_lift_sub(B0, SY_TAB(kP2), T);
+  // S_a
+  fp_add_nr(s, a.c0.l, a.c1.l);
+  fp_add_nr(d, a.c0.l, pp);
+  fp_sub_nr(d, d, a.c1.l);
+  SY_AFTER8(s, B0[15]);
+  SY_AFTER8(d, B0[15]);
+  fp_mul_wide(T, s, d);
+  acc_add(A0, T);
+  SY_AFTER(B0[0], A0[16]);
+  acc_sub(B0, T);
+  // c = a + b; from here on only c and the accumulators are live
+  Fp2 c;
+  fp_add_nr(c.c0.l, a.c0.l, b.c0.l);
+  fp_add_nr(c.c1.l, a.c1.l, b.c1.l);
+  // x <- 3 A - 2 x
+  uint32_t V[9];
+  Fp2 r;
+  const Fp2 xo = fp2_ldv(x);
+  SY_AFTER(A0[0], B0[16]);
+  fp_redc_acc(V, A0);
+  fp_sub_nr(s, pp, xo.c0.l);  // 2 (p - x0) <= 2p
+  fp_add_nr(s, s, s);
+  r.c0 = fp_lin3(V, Fp{{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7]}});
+  SY_AFTER(A1[0], r.c0.l[7]);
+  fp_redc_acc(V, A1);
+  fp_sub_nr(s, pp, xo.c1.l);
+  fp_add_nr(s, s, s);
+  r.c1 = fp_lin3(V, Fp{{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7]}});
+  x = r;
+  // S_c, Q_c
+  fp_add_nr(s, c.c0.l, c.c1.l);  // < 4p
+#pragma unroll
+  for (int i = 0; i < 8; i++) d[i] = SY_TAB(kP2)[i];
+  fp_add_nr(d, c.c0.l, d);
+  fp_sub_nr(d, d, c.c1.l);       // c0 + 2p - c1 in (0, 4p)
+  SY_AFTER8(s, r.c1.l[7]);
+  SY_AFTER8(d, r.c1.l[7]);
+  fp_mul_wide(T, s, d);
+  acc_add(B0, T);
+  uint32_t VB0[9], VB1[9];
+  SY_AFTER(B0[0], T[15]);
+  fp_redc_acc(VB0, B0);
+  fp_add_nr(s, c.c0.l, c.c0.l);  // 2 c0 < 4p
+  SY_AFTER8(s, VB0[8]);
+  fp_mul_wide(T, s, c.c1.l);
+  acc_add(B1, T);
+  SY_AFTER(B1[0], T[15]);
+  fp_redc_acc(VB1, B1);
+  // y <- 3 B + 2 y, or 3 xi B + 2 y with xi B = (9 B0 - B1) + (B0 + 9 B1) u
+  const Fp2 yo = fp2_ldv(y);
+  if (xi) {
+#pragma unroll
+    for (int i = 0; i < 8; i++) d[i] = SY_TAB(kP4)[i];
+    fp_sub_nr(V, d, VB1);  // V_B1 < 3.52 p < 2^256: 4p - V_B1 > 0 in 8 limbs
+    V[8] = 0;
+    u9_add_shl(V, V, VB0, 3);
+    u9_add_shl(V, V, VB0, 0);     // 9 V_B0 + 4p - V_B1
+    u9_add_shl(VB1, VB1, VB1, 3);
+    u9_add_shl(VB1, VB1, VB0, 0);  // V_B0 + 9 V_B1
+#pragma unroll
+    for (int i = 0; i < 9; i++) VB0[i] = V[i];
+  }
+  fp_add_nr(s, yo.c0.l, yo.c0.l);
+  r.c0 = fp_lin3(VB0, Fp{{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7]}});
+  fp_add_nr(s, yo.c1.l, yo.c1.l);
+  r.c1 = fp_lin3(VB1, Fp{{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7]}});
+  y = r;
 }
 
-// Granger-Scott (pairing.rs:309-346)
-// In place, pair by pair: no copies of the six coefficients and no assembled result (the three Fp4 squarings read
-// disjoint pairs, and each pair's outputs only need that pair's - or, for the third, the second pair's - old values).
-// The form that copied z0..z5 into locals and assigned a result record cost 104 scalar spill stores, 105 reloads and 48
-// vector copies per call at 168 registers: k_final_exp 173.9 -> 160.5 ms per 2^20 (profiles/r02s_kbench_inplace.jsonl).
+// Granger-Scott (pairing.rs:309-346), in place: (z0, z1) -> (z0, z1), (z2, z3) -> (z4, z5), (z4, z5) -> (z3, z2).
+// The second pair's outputs overwrite the third pair's inputs, so those two coefficients are copied first.
 SY_HD_NOINLINE void cyclotomic_square_assign(Fp12& f) {
   Fp2 &z0 = f.c0.c0, &z4 = f.c0.c1, &z3 = f.c0.c2, &z2 = f.c1.c0, &z1 = f.c1.c1, &z5 = f.c1.c2;
-  Fp2 t0, t1, t2, t3;
-  fp4_square(z0, z1, t0, t1);
-  z0 = fp2_add(fp2_dbl(fp2_sub(t0, z0)), t0);
-  z1 = fp2_add(fp2_dbl(fp2_add(t1, z1)), t1);
-  fp4_square(z2, z3, t0, t1);
-  fp4_square(z4, z5, t2, t3);
-  z4 = fp2_add(fp2_dbl(fp2_sub(t0, z4)), t0);
-  z5 = fp2_add(fp2_dbl(fp2_add(t1, z5)), t1);
-  t0 = fp2_mul_xi(t3);
-  z2 = fp2_add(fp2_dbl(fp2_add(t0, z2)), t0);
-  z3 = fp2_add(fp2_dbl(fp2_sub(t2, z3)), t2);
+  gs_fp4_square(z0, z1, z0, z1, false);
+  const Fp2 t4 = z4, t5 = z5;
+  gs_fp4_square(z2, z3, z4, z5, false);
+  gs_fp4_square(t4, t5, z3, z2, true);
 }
 SY_HD Fp12 cyclotomic_squared(const Fp12& f) {
   Fp12 r = f;
