@@ -337,7 +337,7 @@ int sylow_b200_batch_weights(sylow_b200_ctx* ctx, const uint8_t* weight_seed /* 
  * mad.wide.u32; 11: independent 32-bit mad.lo.u32; 12: mad.lo.cc/madc.hi.cc carry chains (the
  * IMAD.WIDE.U32.X form fp_mul uses); 13: independent fma.rn.f64 (the FP64 pipe, for comparison) - *ops_out =
  * multiply-add instructions issued per thread x threads.
- * *ms_out = device time of the second of two launches. */
+ * *ms_out = device time of the second of two launches.  Any other variant returns SYLOW_B200_ERR_ARG. */
 int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int threads, int iters, float* ms_out,
                           double* ops_out);
 

@@ -35,21 +35,13 @@
   __device__ __constant__ const type name##_d[n] = {__VA_ARGS__}; \
   static const type name##_h[n] = {__VA_ARGS__};
 
-// Optional block-wide re-convergence inside the long loops: keeps the warps of a block in the same
-// region of the (large) instruction stream so instruction-cache lines fetched by one warp are hit by
-// the others.  Only legal when every thread of the block runs the loop (the kernels guarantee it).
-#ifndef SY_BLOCK_SYNC
-#define SY_BLOCK_SYNC 1
-#endif
-#if defined(__CUDA_ARCH__) && SY_BLOCK_SYNC >= 1
+// Block-wide re-convergence inside the long loops: keeps the warps of a block in the same region of
+// the (large) instruction stream so instruction-cache lines fetched by one warp are hit by the others.
+// Only legal when every thread of the block runs the loop (the kernels guarantee it).
+#if defined(__CUDA_ARCH__)
 #define SY_LOOP_SYNC() __syncthreads()
 #else
 #define SY_LOOP_SYNC() ((void)0)
-#endif
-#if defined(__CUDA_ARCH__) && SY_BLOCK_SYNC >= 2
-#define SY_STEP_SYNC() __syncthreads()
-#else
-#define SY_STEP_SYNC() ((void)0)
 #endif
 
 namespace sylow {
@@ -250,12 +242,8 @@ SY_HD Fp fp_dbl(const Fp& a) { return fp_add(a, a); }
 
 // Four 32x32->64 products with no addend, one IMAD.WIDE each: (X[2k], X[2k+1]) = a_k * b.  Written as mul.wide.u32
 // because ptxas does not fuse a mul.lo / mul.hi pair (it emits IMAD + IMAD.HI, two multiplier-pipe instructions).
-#ifndef SY_MULWIDE
-#define SY_MULWIDE 1
-#endif
 #if defined(__CUDA_ARCH__)
 __device__ __forceinline__ void mul_row4(uint32_t* X, uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b) {
-#if SY_MULWIDE
   asm("{\n\t"
       ".reg .u64 t0, t1, t2, t3;\n\t"
       "mul.wide.u32 t0, %8, %12;\n\t"
@@ -269,14 +257,6 @@ __device__ __forceinline__ void mul_row4(uint32_t* X, uint32_t a0, uint32_t a1, 
       "}"
       : "=r"(X[0]), "=r"(X[1]), "=r"(X[2]), "=r"(X[3]), "=r"(X[4]), "=r"(X[5]), "=r"(X[6]), "=r"(X[7])
       : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b));
-#else
-  asm("mul.lo.u32 %0, %8, %12; mul.hi.u32 %1, %8, %12;\n\t"
-      "mul.lo.u32 %2, %9, %12; mul.hi.u32 %3, %9, %12;\n\t"
-      "mul.lo.u32 %4, %10, %12; mul.hi.u32 %5, %10, %12;\n\t"
-      "mul.lo.u32 %6, %11, %12; mul.hi.u32 %7, %11, %12;"
-      : "=r"(X[0]), "=r"(X[1]), "=r"(X[2]), "=r"(X[3]), "=r"(X[4]), "=r"(X[5]), "=r"(X[6]), "=r"(X[7])
-      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b));
-#endif
 }
 #endif
 

@@ -5,27 +5,15 @@
 #include "wire.cuh"
 #include "pairing_lanes.cuh"
 
-#ifndef SY_MILLER_THREADS
 #define SY_MILLER_THREADS 128
-#endif
 // Three 128-thread blocks per SM at 168 registers run one plain launch of 2^20 pairs 1 % faster (164.4 against 166.2 ms,
 // profiles/r02h_kbench.jsonl) but lose it again in the library, where the wave remainders run at low occupancy
 // (2^20: 167.6 against 166.0 ms, 2^17: 22.3 against 21.6 ms, profiles/r02i_policy_sweep_m128x3.jsonl): two blocks stay.
-#ifndef SY_MILLER_MINB
 #define SY_MILLER_MINB 2
-#endif
-#ifndef SY_GLUED_THREADS
 #define SY_GLUED_THREADS 128
-#endif
-#ifndef SY_GLUED_MINB
 #define SY_GLUED_MINB 2
-#endif
-#ifndef SY_FEXP_THREADS
 #define SY_FEXP_THREADS 384
-#endif
-#ifndef SY_FEXP_MINB
 #define SY_FEXP_MINB 1
-#endif
 
 // Shared-memory slot of one thread's hot Fp12 accumulator: 384 bytes padded to 400, so that the eight lanes of a
 // 128-bit shared-memory access phase fall into different banks (100 words x lane = 4 x lane mod 32).
@@ -33,29 +21,19 @@
 // 166.1 ms (and no register spills left); the Miller loop's G2 point in shared memory as well: slower (169.6).  The final
 // exponentiation's running value in shared memory made no difference while the Granger-Scott squaring still copied it
 // (174.6 / 174.7 ms); with the in-place squaring it does: 160.6 -> 158.1 ms (profiles/r02v_kbench_fexp_smem.jsonl).
-#ifndef SY_MILLER_SMEM
-#define SY_MILLER_SMEM 1
-#endif
-#ifndef SY_FEXP_SMEM
-#define SY_FEXP_SMEM 1
-#endif
 #define SY_ACC_STRIDE 400
 // Two lanes per Miller loop (pairing_lanes.cuh): one PairSlot (1 024 bytes) per lane pair, padded to 1 040 so that
 // consecutive slots start four banks apart (the eight lanes of a 128-bit access phase are four pairs).
-#ifndef SY_LANES_THREADS
 #define SY_LANES_THREADS 128
-#endif
-#ifndef SY_LANES_MINB
 #define SY_LANES_MINB 2
-#endif
 #define SY_SLOT_STRIDE 1040
 #define SY_LANES_SMEM_BYTES(threads) ((size_t)((threads) / 2) * SY_SLOT_STRIDE)
 // two lanes per final exponentiation: FexpHot (768 bytes) per lane pair, padded the same way; FexpCold in global scratch
 #define SY_FHOT_STRIDE 784
 #define SY_FLANES_SMEM_BYTES(threads) ((size_t)((threads) / 2) * SY_FHOT_STRIDE)
 #define SY_FLANES_SCRATCH_BYTES(pairs) ((size_t)(pairs) * sizeof(sylow::FexpCold))
-#define SY_MILLER_SMEM_BYTES(threads) (SY_MILLER_SMEM ? (size_t)(threads) * SY_ACC_STRIDE : (size_t)0)
-#define SY_FEXP_SMEM_BYTES(threads) (SY_FEXP_SMEM ? (size_t)(threads) * SY_ACC_STRIDE : (size_t)0)
+#define SY_MILLER_SMEM_BYTES(threads) ((size_t)(threads) * SY_ACC_STRIDE)
+#define SY_FEXP_SMEM_BYTES(threads) ((size_t)(threads) * SY_ACC_STRIDE)
 
 namespace sylow_kernels {
 using namespace sylow;
@@ -76,7 +54,7 @@ k_miller(const uint8_t* __restrict__ g1, const uint8_t* __restrict__ g1_inf, con
   bool inf = (g1_inf && g1_inf[i]) || (g2_inf && g2_inf[j]);
   const uint8_t* p = g1 + i * 64;
   const uint8_t* q = g2 + j * 128;
-  Fp12 f = miller_loop(fp_load(p), fp_load(p + 32), fp2_load(q), fp2_load(q + 64), SY_MILLER_SMEM ? acc_slot() : nullptr);
+  Fp12 f = miller_loop(fp_load(p), fp_load(p + 32), fp2_load(q), fp2_load(q + 64), acc_slot());
   if (i0 >= n) return;
   if (inf) f = fp12_one();
   if (raw_out)
@@ -119,7 +97,7 @@ k_final_exp(const uint8_t* f_in, int raw_in, size_t n, uint8_t* gt_out) {
   size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t i = i0 < n ? i0 : n - 1;  // all threads run the loops (SY_LOOP_SYNC); the surplus is discarded
   Fp12 f = raw_in ? fp12_load_raw(f_in + i * 384) : fp12_load(f_in + i * 384);
-  final_exponentiation_assign(f, SY_FEXP_SMEM ? acc_slot() : nullptr);
+  final_exponentiation_assign(f, acc_slot());
   if (i0 >= n) return;
   fp12_store(gt_out + i * 384, f);
 }

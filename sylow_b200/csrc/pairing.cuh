@@ -67,15 +67,11 @@ SY_HD_NOINLINE Fp12 miller_loop(const Fp& xp, const Fp& yp, const Fp2& qx, const
   for (int i = 0; i < 64; i++) {
     SY_LOOP_SYNC();
     Ell l = g2_doubling_step(r);
-    SY_STEP_SYNC();
     if (i != 0) fp12_sqr_assign(f);  // 1^2 = 1 (SURVEY Q6)
-    SY_STEP_SYNC();
     miller_mul_line(f, l, xp, yp);
     int digit = SY_TAB(kAteNaf)[i];
     if (digit != 0) {
-      SY_STEP_SYNC();
       l = g2_addition_step(r, qx, digit > 0 ? qy : nqy);
-      SY_STEP_SYNC();
       miller_mul_line(f, l, xp, yp);
     }
   }
@@ -331,9 +327,6 @@ SY_HD Fp12 cyclotomic_squared(const Fp12& f) {
   return r;
 }
 
-#ifndef SY_FEXP_SYNC_EVERY
-#define SY_FEXP_SYNC_EVERY 2
-#endif
 // f <- conj(f^x) with x = BLS_X (pairing.rs:366-392), in place.  The reference walks 256 exponent bits one at a time;
 // the value f^x is the same for any addition chain, so this uses the width-4 NAF of x (63 digits, 14 of them non-zero,
 // digits +-1 .. +-7): 62 + 1 cyclotomic squarings and 13 + 3 multiplications instead of 62 + 27.  A negative digit
@@ -357,7 +350,7 @@ SY_HD_NOINLINE void exp_by_neg_z_assign(Fp12& f, Fp12* acc = nullptr) {
   for (int i = 1; i < SY_XWNAF4_LEN; i++) {
     // the block re-converges every SECOND digit: 177.0 -> 174.4 ms per 2^20 against a barrier per digit (every third or
     // fourth digit, or only after the digits that multiply, are slower again: profiles/r02p_kbench_sync.jsonl)
-    if (i % SY_FEXP_SYNC_EVERY == 0) SY_LOOP_SYNC();
+    if (i % 2 == 0) SY_LOOP_SYNC();
     cyclotomic_square_assign(res);
     int d = SY_TAB(kXWnaf4)[i];
     if (d != 0) {

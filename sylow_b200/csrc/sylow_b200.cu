@@ -21,35 +21,13 @@ using namespace sylow;
 // kernels.  One item (pair / point / message / check) per thread; control flow is uniform across
 // a warp except for the infinity early-outs and the message-length loops of the hash.
 // ------------------------------------------------------------------------------------------------
-// Scalar multiplication ladder: GLV (curve.cuh) by default; -DSY_GLV=0 restores the plain 4-bit window ladder.
-#ifndef SY_GLV
-#define SY_GLV 1
-#endif
-// G2 additionally has the 4-dimensional GLS split (psi); -DSY_GLS=0 falls back to SY_SCALAR_MUL
-#ifndef SY_GLS
-#define SY_GLS 1
-#endif
-#if SY_GLV
-#define SY_SCALAR_MUL proj_scalar_mul_glv
-#else
-#define SY_SCALAR_MUL proj_scalar_mul
-#endif
 #define SY_MUL_THREADS 256
-#ifndef SY_G2_THREADS
 #define SY_G2_THREADS 256
-#endif
-#ifndef SY_G2_MINB
 #define SY_G2_MINB 2
-#endif
 #define SY_HASH_THREADS 256
-#ifndef SY_G1_MINB
 #define SY_G1_MINB 2  // resident 256-thread blocks per SM for the Fp-only kernels (G1 ladder, hash-to-curve)
-#endif
 #define SY_SMALL_THREADS 128
 
-#ifndef SY_VERIFY_GLUE
-#define SY_VERIFY_GLUE 0  // signatures per thread in verify_batch's Miller stage: 0 = by batch size, or 1, 2, 4; SYLOW_B200_VERIFY_GLUE overrides
-#endif
 struct DstPrime {
   uint8_t b[256];
   uint32_t len;
@@ -126,9 +104,8 @@ k_glued(const uint8_t* __restrict__ g1v, size_t sv, const uint8_t* __restrict__ 
     p[NV + t].skip = g1f_inf && g1f_inf[i * sf + t];
   }
   // the accumulator's shared-memory slot sits behind the NF tables (16-byte aligned: 87 * 192 is a multiple of 16)
-  Fp12* acc = SY_MILLER_SMEM ? reinterpret_cast<Fp12*>(reinterpret_cast<char*>(sy_smem) + (size_t)NF * 87 * 192 +
-                                                       (size_t)threadIdx.x * SY_ACC_STRIDE)
-                             : nullptr;
+  Fp12* acc = reinterpret_cast<Fp12*>(reinterpret_cast<char*>(sy_smem) + (size_t)NF * 87 * 192 +
+                                      (size_t)threadIdx.x * SY_ACC_STRIDE);
   Fp12 f = glued_miller_loop<NV, NF>(p, qx, qy, tabs, acc);
   if (i0 >= n) return;
   fp12_store_raw(f_out + i * 384, f);
@@ -169,7 +146,7 @@ k_check_products(const uint8_t* f_raw, size_t k, size_t n_checks, uint8_t* ok) {
     Fp12 v = fp12_load_raw(f_raw + (c * k + j) * 384);
     acc = j == 0 ? v : fp12_mul(acc, v);
   }
-  final_exponentiation_assign(acc, SY_FEXP_SMEM ? acc_slot() : nullptr);
+  final_exponentiation_assign(acc, acc_slot());
   bool one = fp12_eq(acc, fp12_one());
   if (c0 >= n_checks) return;
   ok[c] = one ? 1 : 0;
@@ -271,7 +248,7 @@ k_g1_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf,
   size_t i = i0 < n ? i0 : n - 1;  // all threads run the (block-synchronised) loops; surplus is discarded
   G1Aff a{fp_load(pts + i * 64), fp_load(pts + i * 64 + 32), pts_inf && pts_inf[i]};
   Fp k = fp_load_raw(scalars + i * 32);
-  G1Proj q = SY_SCALAR_MUL(affine_to_proj(a), k.l);
+  G1Proj q = proj_scalar_mul_glv(affine_to_proj(a), k.l);
   if (proj_out) {  // large batches: k_g1_batch_affine shares one inversion between eight points
     if (i0 < n) g1_store_proj(proj_out + i * 96, q);
     return;
@@ -307,11 +284,7 @@ k_g2_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf,
   size_t i = i0 < n ? i0 : n - 1;
   G2Aff a{fp2_load(pts + i * 128), fp2_load(pts + i * 128 + 64), pts_inf && pts_inf[i]};
   Fp k = fp_load_raw(scalars + i * 32);
-#if SY_GLS
   G2Proj q = g2_scalar_mul_gls(affine_to_proj(a), k.l);
-#else
-  G2Proj q = SY_SCALAR_MUL(affine_to_proj(a), k.l);
-#endif
   if (proj_out) {
     if (i0 < n) {
       fp2_store_raw(proj_out + i * 192, q.x);
@@ -632,7 +605,7 @@ k_lagrange_mul(const uint64_t* __restrict__ ids, const uint8_t* __restrict__ sig
   uint32_t w[8];
   fr_to_words(w, lam);
   G1Aff a{fp_load(sigs + g * 64), fp_load(sigs + g * 64 + 32), sigs_inf && sigs_inf[g]};
-  G1Proj r = SY_SCALAR_MUL(affine_to_proj(a), w);
+  G1Proj r = proj_scalar_mul_glv(affine_to_proj(a), w);
   if (g0 != g) return;
   fp_store_raw(out + g * 96, r.x);
   fp_store_raw(out + g * 96 + 32, r.y);
@@ -894,112 +867,6 @@ __global__ void k_imad_probe(int iters, const uint32_t* src, uint32_t* sink) {
   if (acc == 0x12345678u) sink[0] = acc;  // practically never true; keeps the loop alive
 }
 
-// Instruction-fetch probe: the same dependent Montgomery multiplications as k_imad_probe<1>, but UNROLL copies of
-// the multiplication in the loop body (UNROLL * ~3 KB of straight-line code per iteration), to see how the
-// achieved rate depends on the instruction footprint that has to stream through the instruction caches.
-template <int UNROLL>
-__global__ void k_ifetch_probe(int iters, const uint32_t* src, uint32_t* sink) {
-  Fp x = fp_one(), y;
-  for (int i = 0; i < 8; i++) y.l[i] = src[i];
-  x.l[0] += threadIdx.x;
-  for (int it = 0; it < iters; it++) {
-#pragma unroll
-    for (int c = 0; c < UNROLL; c++) x = fp_mul(x, y);
-  }
-  uint32_t acc = 0;
-  for (int i = 0; i < 8; i++) acc ^= x.l[i];
-  if (acc == 0x12345678u) sink[0] = acc;
-}
-
-// Tower-level throughput probe: `iters` dependent applications of one tower operation per thread on
-// thread-private operands, launched like the pairing kernels (256 threads, one block per SM), to see at
-// which level of the tower the limb-product rate falls below the back-to-back fp_mul rate.
-template <int OP>
-__global__ void __launch_bounds__(256, 1) k_tower_probe(int iters, const uint32_t* src, uint32_t* sink) {
-  Fp12 a, b;
-  Fp* pa = reinterpret_cast<Fp*>(&a);
-  Fp* pb = reinterpret_cast<Fp*>(&b);
-  for (int j = 0; j < 12; j++)
-    for (int i = 0; i < 8; i++) {
-      pa[j].l[i] = (src[i] + threadIdx.x * 977u + j) & (i == 7 ? 0x1FFFFFFFu : 0xFFFFFFFFu);
-      pb[j].l[i] = (src[8 + i] + threadIdx.x * 131u + j * 7u) & (i == 7 ? 0x1FFFFFFFu : 0xFFFFFFFFu);
-    }
-  G2Proj r{a.c0.c0, a.c0.c1, a.c0.c2};
-  for (int it = 0; it < iters; it++) {
-    if (OP == 0) a.c0.c0 = fp2_mul(a.c0.c0, b.c0.c0);
-    if (OP == 1) a.c0.c0 = fp2_sqr(a.c0.c0);
-    if (OP == 2) a.c0 = fp6_mul(a.c0, b.c0);
-    if (OP == 3) a = fp12_mul(a, b);
-    if (OP == 4) a = fp12_sqr(a);
-    if (OP == 5) a = fp12_sparse_mul(a, b.c0.c0, b.c0.c1, b.c0.c2);
-    if (OP == 6) a = cyclotomic_squared(a);
-    if (OP == 7) {
-      Ell e = g2_doubling_step(r);
-      a.c0.c0 = fp2_add(a.c0.c0, e.c0);
-      a.c0.c1 = fp2_add(a.c0.c1, e.c1);
-      a.c0.c2 = fp2_add(a.c0.c2, e.c2);
-    }
-    if (OP == 8) a.c0.c0 = fp2_add(fp2_sub(a.c0.c0, b.c0.c0), a.c0.c1);
-    if (OP == 9) a.c0.c0.c0 = fp_add(fp_sub(a.c0.c0.c0, b.c0.c0.c0), a.c0.c0.c1);
-  }
-  uint32_t acc = 0;
-  for (int j = 0; j < 12; j++)
-    for (int i = 0; i < 8; i++) acc ^= pa[j].l[i];
-  acc ^= r.x.c0.l[0] ^ r.y.c0.l[1] ^ r.z.c1.l[2];
-  if (acc == 0x12345678u) sink[0] = acc;
-}
-
-// Pipe-overlap probe: one fp_mul (IMAD.WIDE pipe) and eight fp additions (ALU pipe) per iteration.
-//   MODE 0: the additions are independent of the product (same basic block: the scheduler may interleave them)
-//   MODE 1: strictly alternating phases (the additions consume the product, the next product consumes the sum)
-//   MODE 2: MODE 1 with the odd warps skewed by one addition phase
-//   MODE 3: MODE 1 with the odd warps skewed by half a multiplication
-template <int MODE>
-__global__ void __launch_bounds__(1024, 1) k_overlap_probe(int iters, const uint32_t* src, uint32_t* sink) {
-  Fp x = fp_one(), y, u, v;
-  for (int i = 0; i < 8; i++) {
-    y.l[i] = src[i] & (i == 7 ? 0x1FFFFFFFu : 0xFFFFFFFFu);
-    u.l[i] = (src[8 + i] + threadIdx.x) & (i == 7 ? 0x0FFFFFFFu : 0xFFFFFFFFu);
-    v.l[i] = (src[16 + i] ^ threadIdx.x) & (i == 7 ? 0x0FFFFFFFu : 0xFFFFFFFFu);
-  }
-  x.l[0] += threadIdx.x;
-  if (MODE == 2 && ((threadIdx.x >> 5) & 1)) {
-#pragma unroll 1
-    for (int k = 0; k < 4; k++) {
-      u = fp_add(fp_sub(u, v), y);
-      v = fp_sub(fp_add(v, u), y);
-    }
-  }
-  if (MODE == 3 && ((threadIdx.x >> 5) & 1)) {
-    uint32_t t = 0;
-#pragma unroll 1
-    for (int k = 0; k < 40; k++) t = t * x.l[1] + u.l[k & 7];
-    u.l[0] ^= t & 1u;
-  }
-#pragma unroll 1
-  for (int it = 0; it < iters; it++) {
-    if (MODE == 0) {
-      x = fp_mul(x, y);
-#pragma unroll
-      for (int k = 0; k < 2; k++) {
-        u = fp_add(fp_sub(u, v), y);
-        v = fp_sub(fp_add(v, u), y);
-      }
-    } else {
-      x = fp_mul(u, y);
-      u = fp_add(fp_sub(x, v), y);
-      v = fp_sub(fp_add(v, u), y);
-      u = fp_add(fp_sub(u, v), y);
-      v = fp_sub(fp_add(v, u), x);
-      u = fp_add(u, v);
-      u.l[7] &= 0x1FFFFFFFu;
-    }
-  }
-  uint32_t acc = 0;
-  for (int i = 0; i < 8; i++) acc ^= x.l[i] ^ u.l[i] ^ v.l[i];
-  if (acc == 0x12345678u) sink[0] = acc;
-}
-
 // Raw pipe probes.  MODE 0: independent mad.wide.u32 (IMAD.WIDE.U32); MODE 1: independent 32-bit
 // mad.lo.u32 (IMAD); MODE 2: mad.lo.cc/madc.hi.cc carry chains of 4 pairs (IMAD.WIDE.U32.X with
 // predicate carries, the exact instruction form fp_mul uses).  64 multiply-adds per loop iteration.
@@ -1081,7 +948,7 @@ struct sylow_b200_ctx {
   cudaStream_t stream = nullptr;
   cudaStream_t copy_in = nullptr, copy_out = nullptr;  // host<->device copies of the chunked host-pointer calls
   cudaStream_t stream2 = nullptr;                      // second compute stream: odd chunks (their tails overlap)
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;    // fork/join of the chunk-interleaved device paths
+  cudaEvent_t ev_fork = nullptr;                       // copy_in -> compute stream hand-off of verify_batch_partial
   int sms = 148;
   int last_cuda = 0;
   uint64_t launches = 0;
@@ -1164,9 +1031,7 @@ static WaveSplit wave_split(const sylow_b200_ctx* ctx, size_t n, int threads, in
   WaveSplit w{n, 0, 0, 0};
   const size_t wave = (size_t)ctx->sms * threads * blocks_per_sm;
   const size_t r = n % wave;
-  const char* v = getenv("SYLOW_B200_TAIL_SPLIT");  // 0 disables (measurement)
-  const int mode = v ? atoi(v) : 1;
-  if (!mode || r == 0 || r * 10 >= wave * 6) return w;
+  if (r == 0 || r * 10 >= wave * 6) return w;
   const size_t slots = (size_t)ctx->sms * blocks_per_sm;
   unsigned t = (unsigned)(((r + slots - 1) / slots + 31) / 32 * 32);
   if (t > (unsigned)threads) t = threads;
@@ -1312,10 +1177,9 @@ int sylow_b200_create(sylow_b200_ctx** out, int device_id) {
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming);
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&ctx->sms, cudaDevAttrMultiProcessorCount, device_id);
   // opt-in for more than 48 KB of dynamic shared memory (the Miller loop's accumulators); per device
-  if (e == cudaSuccess && SY_MILLER_SMEM)
+  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(k_miller, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)SY_MILLER_SMEM_BYTES(SY_MILLER_THREADS));
   if (e == cudaSuccess)
@@ -1324,10 +1188,10 @@ int sylow_b200_create(sylow_b200_ctx** out, int device_id) {
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(k_final_exp_lanes, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)SY_FLANES_SMEM_BYTES(SY_LANES_THREADS));
-  if (e == cudaSuccess && SY_FEXP_SMEM)
+  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(k_final_exp, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS));
-  if (e == cudaSuccess && SY_FEXP_SMEM)
+  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(k_check_products, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS));
   if (e == cudaSuccess) e = cudaMalloc(&ctx->d_fail, sizeof(int));
@@ -1368,7 +1232,6 @@ int sylow_b200_destroy(sylow_b200_ctx* ctx) {
   if (ctx->copy_out) cudaStreamDestroy(ctx->copy_out);
   if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
   if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-  if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   delete ctx;
   return 0;
 }
@@ -1452,27 +1315,15 @@ int sylow_b200_final_exp_batch_dev(sylow_b200_ctx* ctx, const uint8_t* f, size_t
   return launch_final_exp(ctx, f, 0, n, gt_out, pick(ctx, stream));
 }
 
-// Miller loops then final exponentiations of one slice on one stream.  The Miller values (Montgomery form) are staged
-// in gt_out itself; the final exponentiation is in place.
+// Miller loops then final exponentiations of one batch on one stream.  The Miller values (Montgomery form) are staged
+// in gt_out itself; the final exponentiation is in place.  (Slicing the batch over two streams was measured and only
+// adds wave tails: a k_final_exp block needs a whole SM's registers and a k_miller block half of them, so the partly
+// filled last wave of one kernel never usefully overlaps the other stream's kernels, profiles/r02_pair_chunk_sweep.jsonl.
+// The low-occupancy tail launches of launch_miller / launch_final_exp handle the tails instead.)
 static int pairing_dev_single(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                               const uint8_t* g2_inf, size_t n, uint8_t* gt_out, cudaStream_t s) {
   CKS(launch_miller(ctx, g1, g1_inf, g2, g2_inf, n, gt_out, 1, s));
   return launch_final_exp(ctx, gt_out, 1, n, gt_out, s);
-}
-
-// Optional slicing of the device path over the caller's stream and the context's second stream (SYLOW_B200_PAIR_CHUNK =
-// slice size in pairs).  Measured (profiles/r02_pair_chunk_sweep.jsonl): the partly filled last wave of one kernel does
-// NOT usefully overlap the other stream's kernels - a k_final_exp block needs a whole SM's registers and a k_miller
-// block half of them, so the two never share an SM - and slicing only adds wave tails.  Off by default; the tails are
-// handled by the low-occupancy tail launches above instead.
-static size_t pairing_chunk(const sylow_b200_ctx* ctx, size_t n) {
-  static const long env = [] {
-    const char* v = getenv("SYLOW_B200_PAIR_CHUNK");
-    return v ? atol(v) : 0L;
-  }();
-  if (env > 0) return (size_t)env;
-  (void)ctx;
-  return n;  // default: no slicing (the tail launches of launch_miller / launch_final_exp do the work; see below)
 }
 
 int sylow_b200_pairing_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
@@ -1480,21 +1331,7 @@ int sylow_b200_pairing_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, const u
   ENTER_DEV(ctx);
   if (!ctx || (n && (!g1 || !g2 || !gt_out))) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  cudaStream_t s = pick(ctx, stream);
-  const size_t chunk = pairing_chunk(ctx, n);
-  if (n <= chunk + chunk / 2 || s == ctx->stream2) return pairing_dev_single(ctx, g1, g1_inf, g2, g2_inf, n, gt_out, s);
-  CK(cudaEventRecord(ctx->ev_fork, s));
-  CK(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
-  size_t c = 0;
-  for (size_t off = 0; off < n; c++) {
-    size_t m = n - off <= chunk + chunk / 2 ? n - off : chunk;
-    CKS(pairing_dev_single(ctx, g1 + off * 64, g1_inf ? g1_inf + off : nullptr, g2 + off * 128,
-                           g2_inf ? g2_inf + off : nullptr, m, gt_out + off * 384, (c & 1) ? ctx->stream2 : s));
-    off += m;
-  }
-  CK(cudaEventRecord(ctx->ev_join, ctx->stream2));
-  CK(cudaStreamWaitEvent(s, ctx->ev_join, 0));
-  return 0;
+  return pairing_dev_single(ctx, g1, g1_inf, g2, g2_inf, n, gt_out, pick(ctx, stream));
 }
 
 // reduce n Montgomery-form Fp12 values at `buf` (clobbered, with `tmp` as ping-pong space of at least
@@ -1814,20 +1651,16 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
     LAUNCHED(ctx);
     CKS(g1_batch_affine(ctx, ctx->proj.p, n, 0, d_hm, d_hm_inf, s));
   }
-  // The n Miller loops (-r_i H(m_i), pk_i) only ever meet as a product, so SY_VERIFY_GLUE signatures share one thread
+  // The n Miller loops (-r_i H(m_i), pk_i) only ever meet as a product, so 1, 2 or 4 signatures share one thread
   // and ONE Fp12 squaring per loop digit - what glued_miller_loop does for the whole batch in the reference
   // (pairing.rs:970-1022).  A thread's 2 / 4 pairs save 63 x 36 of the 8 444 multiplications of every pair after its
   // first.  The n % GLUE leftover pairs go through k_miller.
-  static const int glue_env = [] {
-    const char* v = getenv("SYLOW_B200_VERIFY_GLUE");
-    int g = v ? atoi(v) : SY_VERIFY_GLUE;
-    return g == 1 || g == 2 || g == 4 ? g : 0;
-  }();
-  int glue = glue_env;
-  if (!glue) {
-    // fewest wave-times: whole waves of n / g threads (256 resident per SM) times the multiplications of g glued pairs.
-    // Measured at 2^20 signatures (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 / 163.3 ms for 1 / 2 / 4; at 2^13 the
-    // order reverses (9.3 / 12.4 / 18.4 ms: a quarter of the threads, each four times as long).
+  // The glue is the one of fewest wave-times: whole waves of n / g threads (256 resident per SM) times the
+  // multiplications of g glued pairs.  Measured at 2^20 signatures (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 /
+  // 163.3 ms for 1 / 2 / 4; at 2^13 the order reverses (9.3 / 12.4 / 18.4 ms: a quarter of the threads, each four times
+  // as long).
+  int glue = 0;
+  {
     const size_t wave = (size_t)ctx->sms * SY_GLUED_THREADS * SY_GLUED_MINB;
     const size_t cost[3] = {8444, 2 * 8444 - 2268, 4 * 8444 - 3 * 2268};
     size_t best = ~(size_t)0;
@@ -2931,24 +2764,6 @@ int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int thre
       case 11: k_pipe_probe<1><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 64; break;
       case 12: k_pipe_probe<2><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 64; break;
       case 13: k_dfma_probe<<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 64; break;
-      case 20: k_ifetch_probe<4><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 4; break;
-      case 21: k_ifetch_probe<16><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 16; break;
-      case 22: k_ifetch_probe<64><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 64; break;
-      case 23: k_ifetch_probe<256><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 256; break;
-      case 30: k_tower_probe<0><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 3; break;
-      case 31: k_tower_probe<1><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 2; break;
-      case 32: k_tower_probe<2><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 18; break;
-      case 33: k_tower_probe<3><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 54; break;
-      case 34: k_tower_probe<4><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 36; break;
-      case 35: k_tower_probe<5><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 39; break;
-      case 36: k_tower_probe<6><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 18; break;
-      case 37: k_tower_probe<7><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 26; break;
-      case 38: k_tower_probe<8><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 4; break;
-      case 39: k_tower_probe<9><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 2; break;
-      case 40: k_overlap_probe<0><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 1; break;
-      case 41: k_overlap_probe<1><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 1; break;
-      case 42: k_overlap_probe<2><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 1; break;
-      case 43: k_overlap_probe<3><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 1; break;
       default: return SYLOW_B200_ERR_ARG;
     }
     LAUNCHED(ctx);

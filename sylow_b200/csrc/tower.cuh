@@ -76,16 +76,10 @@ SY_HD_ADD Fp2 fp2_sub_mul_xi(const Fp2& t, const Fp2& a) {
 #define SY_AFTER(x, y) ((void)0)
 #define SY_AFTER8(v, y) ((void)0)
 #endif
-#ifndef SY_FENCE_ALL
-#define SY_FENCE_ALL 1
-#endif
-#ifndef SY_VEC_LOAD
-#define SY_VEC_LOAD 1
-#endif
 // An Fp2 operand arrives by reference (generic pointer into the caller's frame); ptxas loads it limb by limb unless
 // told that the 64 bytes are four aligned 128-bit words (Fp is alignas(16)).
 SY_HD Fp2 fp2_ldv(const Fp2& a) {
-#if defined(__CUDA_ARCH__) && SY_VEC_LOAD
+#if defined(__CUDA_ARCH__)
   const uint4* p = reinterpret_cast<const uint4*>(&a);
   uint4 w0 = p[0], w1 = p[1], w2 = p[2], w3 = p[3];
   Fp2 r;
@@ -104,19 +98,11 @@ SY_HD_MUL2 Fp2 fp2_mul(const Fp2& a_, const Fp2& b_) {
   fp_mul_wide(t0, a.c0.l, b.c0.l);
 #pragma unroll
   for (int i = 0; i < 8; i++) a1[i] = a.c1.l[i];
-#if SY_FENCE_ALL
   SY_AFTER8(a1, t0[15]);
-#else
-  SY_AFTER(a1[0], t0[15]);
-#endif
   fp_mul_wide(t1, a1, b.c1.l);
   fp_add_nr(sa, a.c0.l, a1);
   fp_add_nr(sb, b.c0.l, b.c1.l);
-#if SY_FENCE_ALL
   SY_AFTER8(sa, t1[15]);
-#else
-  SY_AFTER(sa[0], t1[15]);
-#endif
   fp_mul_wide(t2, sa, sb);
   wide_sub(t2, t0);
   wide_sub(t2, t1);

@@ -1,8 +1,9 @@
 // Stand-alone timing + checksum harness for the two pairing kernels (k_miller, k_final_exp), compiled from the SAME
-// header as the library (csrc/kernels_pairing.cuh).  Used to compare build variants (-D switches) on the GPU box
-// without the 3-minute full-library build: every variant prints its kernel times and a checksum of the outputs on
-// fixed pseudo-random inputs, so a variant that changes a single bit of any result is caught in the same run.
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -DSY_VARIANT='"name"' [-D...] \
+// header as the library (csrc/kernels_pairing.cuh).  Used to compare the kernels of two checkouts (tools/kbench_build.sh
+// name:tree ...) on the GPU without the 3-minute full-library build: every variant prints its kernel times and a
+// checksum of the outputs on fixed pseudo-random inputs, so a variant that changes a single bit of any result is caught
+// in the same run.
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -DSY_VARIANT='"name"' \
 //        -o build/kbench/name tools/kbench.cu
 //   build/kbench/name [log2n=18] [reps=3] [n=2^log2n] [miller block threads] [lanes block threads]
 // The two-lane Miller kernel (k_miller_lanes) runs on the same inputs and must give the same checksum as k_miller.

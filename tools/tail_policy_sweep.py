@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Time the Miller-loop and final-exponentiation launches of one GPU for batch sizes around the wave boundaries under
-the launch policies of sylow_b200.cu (read per call from the environment):
-  SYLOW_B200_LANES      0 one thread per item only, 1 automatic, 2 two lanes per item always
-  SYLOW_B200_TAIL_SPLIT 0 plain launches, 1 low-occupancy launch of the remainder, (2 = last 1 + r waves as two equal rounds: measured in r02g, not better, removed)
+the lane policies of sylow_b200.cu (SYLOW_B200_LANES, read per call from the environment): 0 one thread per item only,
+1 automatic, 2 two lanes per item always.
+  tools/tail_policy_sweep.py [sizes, comma-separated] [policies, comma-separated, e.g. 0,1]
 Prints one JSON line per policy: ms per call of miller_loop_batch_dev / final_exp_batch_dev / pairing_batch_dev."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -13,8 +13,7 @@ eng = sylow_b200.Engine(0)
 dev = torch.device("cuda", 0)
 sizes = [int(x) for x in sys.argv[1].split(",")] if len(sys.argv) > 1 else \
     [1, 64, 1024, 4096, 9472, 14000, 18944, 25000, 1 << 15, 1 << 16, 80776, 113664, 1 << 17, 1 << 18, 257328]
-policies = [tuple(p.split(":")) for p in sys.argv[2].split(",")] if len(sys.argv) > 2 else \
-    [("0", "1"), ("1", "1"), ("0", "2"), ("1", "2"), ("2", "1")]
+policies = sys.argv[2].split(",") if len(sys.argv) > 2 else ["0", "1", "2"]
 nmax = max(sizes)
 g1 = torch.randint(0, 255, (nmax, 64), dtype=torch.uint8, device=dev)
 g2 = torch.randint(0, 255, (nmax, 128), dtype=torch.uint8, device=dev)
@@ -37,12 +36,9 @@ def timed(fn, reps):
     return round(a.elapsed_time(b) / reps, 4)
 
 
-for lanes, tail in policies:
-    if lanes == "2" and nmax > (1 << 17):
-        pass
+for lanes in policies:
     os.environ["SYLOW_B200_LANES"] = lanes
-    os.environ["SYLOW_B200_TAIL_SPLIT"] = tail
-    out = {"lanes": lanes, "tail_split": tail, "miller_ms": {}, "fexp_ms": {}, "pairing_ms": {}, "same_bits": True}
+    out = {"lanes": lanes, "miller_ms": {}, "fexp_ms": {}, "pairing_ms": {}, "same_bits": True}
     for n in sizes:
         reps = 2 if n > (1 << 17) else 5
         a1, a2, af, ag = g1[:n], g2[:n], f[:n], gt[:n]
