@@ -8,7 +8,7 @@
 //! ```ignore
 //! mod batch;
 //! pub use crate::batch::{final_exponentiation_batch, g1_mul_batch, g2_mul_batch, glued_miller_loop_batch,
-//!                        glued_pairing_batch, pairing_batch, pairing_check_batch, sign_batch,
+//!                        glued_miller_loop_precomputed_batch, glued_pairing_batch, pairing_batch, pairing_check_batch, sign_batch,
 //!                        threshold_aggregate_batch, verify_batch, verify_each, BatchError, Engine};
 //! ```
 //!
@@ -28,7 +28,7 @@ use crate::groups::g1::{G1Affine, G1Projective};
 use crate::groups::g2::{G2Affine, G2Projective};
 use crate::groups::group::GroupError;
 use crate::groups::gt::Gt;
-use crate::pairing::MillerLoopResult;
+use crate::pairing::{G2PreComputed, MillerLoopResult};
 use crypto_bigint::U256;
 use subtle::Choice;
 use sylow_cuda_sys as sys;
@@ -205,6 +205,33 @@ pub fn glued_miller_loop_batch(e: &mut Engine, p: &[G1Projective], q: &[G2Projec
     let mut out = [0u8; 384];
     e.check(unsafe {
         sys::sylow_b200_miller_product(e.ctx, g1.as_ptr(), g1i.as_ptr(), g2.as_ptr(), g2i.as_ptr(), n, out.as_mut_ptr())
+    })?;
+    Ok(MillerLoopResult(get_fp12(&out)))
+}
+
+/// `glued_miller_loop(&[G2PreComputed], &[G1Affine])` itself (src/pairing.rs:970-1022): the 87 `Ell` triples of every
+/// table go over canonically, one table per pair.  Pairs with an infinite G1 point, or a table of the identity,
+/// contribute 1.  This moves 16.7 KB per pair to the device; keep hot tables resident with
+/// `sylow_b200_g2_precompute_dev` + `sylow_b200_miller_product_precomputed_dev` instead.
+pub fn glued_miller_loop_precomputed_batch(e: &mut Engine, q: &[G2PreComputed], p: &[G1Affine]) -> Result<MillerLoopResult, BatchError> {
+    let n = p.len().min(q.len()); // zip truncation, like the reference (:975)
+    let (mut coeffs, mut g1, mut g1i) = (Vec::with_capacity(n * 16704), Vec::with_capacity(n * 64), Vec::with_capacity(n));
+    for (pc, a) in q[..n].iter().zip(&p[..n]) {
+        if pc.coeffs.len() != 87 {
+            return Err(BatchError::InvalidArgument);
+        }
+        for (c0, c1, c2) in pc.coeffs.iter() {
+            for c in [c0.0[0], c0.0[1], c1.0[0], c1.0[1], c2.0[0], c2.0[1]] {
+                put_fp(&mut coeffs, &c);
+            }
+        }
+        put_fp(&mut g1, &a.x);
+        put_fp(&mut g1, &a.y);
+        g1i.push((a.is_zero() || pc.q.is_zero()) as u8);
+    }
+    let mut out = [0u8; 384];
+    e.check(unsafe {
+        sys::sylow_b200_miller_product_precomputed(e.ctx, coeffs.as_ptr(), g1.as_ptr(), g1i.as_ptr(), n, out.as_mut_ptr())
     })?;
     Ok(MillerLoopResult(get_fp12(&out)))
 }

@@ -135,6 +135,20 @@ int sylow_b200_pairing_check_fixed_batch(sylow_b200_ctx* ctx, const uint8_t* g1,
                                          const uint8_t* g2_var, const uint8_t* g2_var_inf, size_t k_var,
                                          const uint8_t* coeffs_fixed, size_t k_fixed, size_t n_checks, uint8_t* ok_out);
 
+/* One table PER PAIR (sylow_b200_miller_loop_precomputed uses one table for all pairs): pair i is g1[i] against the
+ * canonical table coeffs[i*16704 ..] (sylow_b200_g2_precompute output).  A table has no infinity form: drop such pairs
+ * or flag them on the G1 side.  These two host entry points move 16.7 KB per pair over the host link; they are there
+ * for API parity and moderate batches.  The throughput path keeps the tables resident in device memory
+ * (sylow_b200_g2_precompute_dev + sylow_b200_miller_product_precomputed_dev).
+ * _batch: f_out[i] = G2PreComputed::miller_loop(g1[i]) (pairing.rs:590-619), canonical; infinite G1 gives 1.
+ * product: glued_miller_loop(&[G2PreComputed], &[G1Affine]) (pairing.rs:970-1022), bit-identical to
+ *   sylow_b200_miller_product on the same points; infinite G1 pairs are skipped, n = 0 gives 1. */
+int sylow_b200_miller_loop_precomputed_batch(sylow_b200_ctx* ctx, const uint8_t* coeffs /* n*16704 */,
+                                             const uint8_t* g1, const uint8_t* g1_inf, size_t n,
+                                             uint8_t* f_out /* n*384 */);
+int sylow_b200_miller_product_precomputed(sylow_b200_ctx* ctx, const uint8_t* coeffs /* n*16704 */, const uint8_t* g1,
+                                          const uint8_t* g1_inf, size_t n, uint8_t f_out[384]);
+
 /* ---- input validation (untrusted batches: precompile calldata, aggregated signatures) ------------- */
 
 /* status_out[i] = 0 if g1[i] is a valid point, SYLOW_B200_ERR_DECODE if a coordinate is >= p
@@ -300,6 +314,19 @@ int sylow_b200_pairing_check_fixed_batch_dev(sylow_b200_ctx* ctx, const uint8_t*
 /* Converts k canonical host tables (sylow_b200_g2_precompute output) to the device form at d_tables_out
  * (k*16704 B of device memory). */
 int sylow_b200_tables_to_device(sylow_b200_ctx* ctx, const uint8_t* coeffs, size_t k, uint8_t* d_tables_out, void* stream);
+/* G2Affine::precompute of n device-resident points straight into caller-owned device memory, in the device form
+ * (d_tables_out: n*16704 B).  No host round trip and no staging buffer: 2^20 tables take 17.5 GB once. */
+int sylow_b200_g2_precompute_dev(sylow_b200_ctx* ctx, const uint8_t* d_g2, size_t n, uint8_t* d_tables_out,
+                                 void* stream);
+/* d_f_out (384 B, canonical) = the Miller product over n pairs, pair i = d_g1[i] against device-form table
+ * d_table_idx[i] of d_tables (n_tables tables).  d_table_idx NULL: pair i uses table i, and n > n_tables is
+ * SYLOW_B200_ERR_ARG.  An index >= n_tables makes the product the Fp12 zero (its final exponentiation is zero, never
+ * the identity, so a check built on it fails closed); nothing is read out of bounds.  Infinite G1 pairs are skipped,
+ * n = 0 gives 1.  1, 2 or 4 pairs share one thread's Fp12 squarings, by the fewest-wave-times rule. */
+int sylow_b200_miller_product_precomputed_dev(sylow_b200_ctx* ctx, const uint8_t* d_tables, size_t n_tables,
+                                              const uint32_t* d_table_idx, const uint8_t* d_g1,
+                                              const uint8_t* d_g1_inf, size_t n, uint8_t* d_f_out /* 384 */,
+                                              void* stream);
 int sylow_b200_g1_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_pts, const uint8_t* d_pts_inf,
                                 const uint8_t* d_scalars, size_t n, uint8_t* d_out, uint8_t* d_out_inf, void* stream);
 int sylow_b200_g2_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_pts, const uint8_t* d_pts_inf,

@@ -38,6 +38,10 @@ _SIGNATURES = {
     "sylow_b200_pairing_check_fixed_batch": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_size_t, _P]),
     "sylow_b200_pairing_check_fixed_batch_dev": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_size_t, _P, _P]),
     "sylow_b200_tables_to_device": (c_int, [_P, _P, c_size_t, _P, _P]),
+    "sylow_b200_miller_loop_precomputed_batch": (c_int, [_P, _P, _P, _P, c_size_t, _P]),
+    "sylow_b200_miller_product_precomputed": (c_int, [_P, _P, _P, _P, c_size_t, _P]),
+    "sylow_b200_g2_precompute_dev": (c_int, [_P, _P, c_size_t, _P, _P]),
+    "sylow_b200_miller_product_precomputed_dev": (c_int, [_P, _P, c_size_t, _P, _P, _P, c_size_t, _P, _P]),
     "sylow_b200_g1_validate_batch": (c_int, [_P, _P, _P, c_size_t, _P]),
     "sylow_b200_g2_validate_batch": (c_int, [_P, _P, _P, c_size_t, _P]),
     "sylow_b200_g1_from_be_bytes_batch": (c_int, [_P, _P, c_size_t, c_int, _P, _P, _P]),

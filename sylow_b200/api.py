@@ -153,6 +153,31 @@ class Engine:
                                                               _ptr(out)), "miller_loop_precomputed")
         return out
 
+    def _table_pairs(self, coeffs, g1, g1_inf):
+        g1 = _u8(g1, 64, "g1")
+        n = g1.shape[0]
+        coeffs = np.ascontiguousarray(coeffs, dtype=np.uint8).reshape(-1, 87 * 192)
+        if coeffs.shape[0] != n:
+            raise ValueError("one table per pair: %d tables for %d G1 points" % (coeffs.shape[0], n))
+        g1_inf = None if g1_inf is None else np.ascontiguousarray(g1_inf, dtype=np.uint8).reshape(n)
+        return coeffs, g1, g1_inf, n
+
+    def miller_loop_precomputed_batch(self, coeffs, g1, g1_inf=None) -> np.ndarray:
+        """G2PreComputed::miller_loop with one canonical table per pair: coeffs (n, 16704), g1 (n, 64) -> (n, 384)."""
+        coeffs, g1, g1_inf, n = self._table_pairs(coeffs, g1, g1_inf)
+        out = np.empty((n, 384), dtype=np.uint8)
+        self._ck(self._lib.sylow_b200_miller_loop_precomputed_batch(self._h, _ptr(coeffs), _ptr(g1), _ptr(g1_inf), n,
+                                                                    _ptr(out)), "miller_loop_precomputed_batch")
+        return out
+
+    def miller_product_precomputed(self, coeffs, g1, g1_inf=None) -> np.ndarray:
+        """glued_miller_loop(&[G2PreComputed], &[G1Affine]): one canonical table per pair; infinite G1 pairs skipped."""
+        coeffs, g1, g1_inf, n = self._table_pairs(coeffs, g1, g1_inf)
+        out = np.empty(384, dtype=np.uint8)
+        self._ck(self._lib.sylow_b200_miller_product_precomputed(self._h, _ptr(coeffs), _ptr(g1), _ptr(g1_inf), n,
+                                                                 _ptr(out)), "miller_product_precomputed")
+        return out
+
     def pairing_check_fixed_batch(self, g1, g2_var, coeffs_fixed, k_var: int, k_fixed: int, g1_inf=None,
                                   g2_var_inf=None) -> np.ndarray:
         g1 = _u8(g1, 64, "g1")
@@ -523,6 +548,23 @@ class Engine:
         self._ck(self._lib.sylow_b200_miller_product_dev(self._h, self._tp(d_g1), self._tp(d_g1_inf), self._tp(d_g2),
                                                          self._tp(d_g2_inf), n, self._tp(d_out), self._stream()),
                  "miller_product_dev")
+
+    def g2_precompute_dev(self, d_g2, d_tables):
+        """Device-form tables of the (n, 128) points d_g2 into d_tables (n * 16704 bytes of device memory)."""
+        self._ck(self._lib.sylow_b200_g2_precompute_dev(self._h, self._tp(d_g2), d_g2.shape[0], self._tp(d_tables),
+                                                        self._stream()), "g2_precompute_dev")
+
+    def miller_product_precomputed_dev(self, d_tables, d_g1, d_out, d_table_idx=None, d_g1_inf=None):
+        """Miller product over resident device-form tables: pair i is d_g1[i] against table d_table_idx[i] (int32 or
+        uint32 tensor; None: table i).  An index past the last table makes the product zero."""
+        if d_table_idx is not None and d_table_idx.element_size() != 4:
+            raise ValueError("d_table_idx must hold 32-bit indices")
+        n_tables = d_tables.numel() // (87 * 192)
+        self._ck(self._lib.sylow_b200_miller_product_precomputed_dev(self._h, self._tp(d_tables), n_tables,
+                                                                     self._tp(d_table_idx), self._tp(d_g1),
+                                                                     self._tp(d_g1_inf), d_g1.shape[0], self._tp(d_out),
+                                                                     self._stream()),
+                 "miller_product_precomputed_dev")
 
     def final_exp_batch_dev(self, d_f, d_out):
         self._ck(self._lib.sylow_b200_final_exp_batch_dev(self._h, self._tp(d_f), d_f.shape[0], self._tp(d_out),

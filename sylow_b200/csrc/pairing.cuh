@@ -124,7 +124,10 @@ SY_HD void glued_mul_line(Fp12& f, const Ell& l, const MillerG1& p) {
 // Montgomery form; on the device they sit in shared memory and every thread reads the same triple).
 // One shared Fp12 squaring per digit for all NV + NF pairs.  The product equals the reference's
 // (multiplication order differs; Fp12 multiplication is exact and commutative).
-template <int NV, int NF>
+// COPY only names a separate compiled copy: ptxas builds one body of a noinline function for all its callers, so a new
+// kernel calling an existing instantiation would change the register allocation of the kernels that already call it.
+// The loops over per-pair tables in global memory (miller_tables.cuh) use COPY = 1.
+template <int NV, int NF, int COPY = 0>
 SY_HD_NOINLINE Fp12 glued_miller_loop(const MillerG1* p /* NV + NF */, const Fp2* qx, const Fp2* qy /* NV */,
                                       const Ell* const* tables /* NF */, Fp12* acc = nullptr) {
   G2Proj r[NV > 0 ? NV : 1];

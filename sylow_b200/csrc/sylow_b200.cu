@@ -14,6 +14,7 @@
 #include "fr.cuh"
 #include "wire.cuh"
 #include "kernels_pairing.cuh"
+#include "miller_tables.cuh"
 
 using namespace sylow;
 
@@ -109,6 +110,24 @@ k_glued(const uint8_t* __restrict__ g1v, size_t sv, const uint8_t* __restrict__ 
   Fp12 f = glued_miller_loop<NV, NF>(p, qx, qy, tabs, acc);
   if (i0 >= n) return;
   fp12_store_raw(f_out + i * 384, f);
+}
+
+// f_out[i] = the glued Miller loop of pairs [i M, i M + M), each against its own table in global memory
+// (miller_tables_item), Montgomery form if raw_out, else canonical.  The accumulator lives in the thread's shared-memory
+// slot like k_miller's; every thread runs the loop (SY_LOOP_SYNC) and surplus threads redo the last item.
+template <int M>
+__global__ void __launch_bounds__(SY_GLUED_THREADS, SY_GLUED_MINB)
+k_miller_tables(const uint8_t* __restrict__ tables, size_t n_tables, const uint32_t* __restrict__ table_idx,
+                const uint8_t* __restrict__ g1, const uint8_t* __restrict__ g1_inf, size_t n_items,
+                uint8_t* __restrict__ f_out, int raw_out) {
+  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t i = i0 < n_items ? i0 : n_items - 1;
+  Fp12 f = miller_tables_item<M>(tables, n_tables, table_idx, g1, g1_inf, i, acc_slot());
+  if (i0 >= n_items) return;
+  if (raw_out)
+    fp12_store_raw(f_out + i * 384, f);
+  else
+    fp12_store(f_out + i * 384, f);
 }
 
 // out[t] = in[t] * in[t + T] * in[t + 2T] * ...   (Montgomery form in and out)
@@ -1157,6 +1176,25 @@ static int launch_check_products(sylow_b200_ctx* ctx, const uint8_t* f, size_t k
   return 0;
 }
 
+// Pairs per thread (1, 2 or 4) for n >= 1 pairs whose Miller loops only meet as a product, glued into one loop per
+// thread (k_glued<M, 0>, k_miller_tables<M>): the glue of fewest wave-times, i.e. whole waves of n / g threads (256
+// resident per SM) times the Fp multiplications of g glued pairs.  pair_cost is one pair's count (8 444 fused, 6 045
+// from a table); every pair after the first saves its Fp12 squarings, 63 x 36 multiplications.
+static int glue_pairs(const sylow_b200_ctx* ctx, size_t n, size_t pair_cost) {
+  const size_t wave = (size_t)ctx->sms * SY_GLUED_THREADS * SY_GLUED_MINB, save = 63 * 36;
+  const size_t cost[3] = {pair_cost, 2 * pair_cost - save, 4 * pair_cost - 3 * save};
+  int glue = 0;
+  size_t best = ~(size_t)0;
+  for (int j = 0; j < 3; j++) {
+    const size_t g = (size_t)1 << j, waves = (n / g + wave - 1) / wave;
+    if (n >= g && waves * cost[j] < best) {
+      best = waves * cost[j];
+      glue = (int)g;
+    }
+  }
+  return glue;
+}
+
 // defined further down (needs the table constants): one glued loop of NV fused + NF table pairs per item
 template <int NV, int NF>
 static int launch_glued(sylow_b200_ctx* ctx, const uint8_t* g1v, size_t sv, const uint8_t* g1v_inf, const uint8_t* g2v,
@@ -1194,6 +1232,15 @@ int sylow_b200_create(sylow_b200_ctx** out, int device_id) {
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(k_check_products, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS));
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(k_miller_tables<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(k_miller_tables<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(k_miller_tables<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
   if (e == cudaSuccess) e = cudaMalloc(&ctx->d_fail, sizeof(int));
   if (e == cudaSuccess) e = cudaMemset(ctx->d_fail, 0, sizeof(int));
   if (e != cudaSuccess) {
@@ -1516,8 +1563,6 @@ static const uint64_t kG2GenWords[16] = {
     5541340697920699818ull,  16416156555105522555ull, 5380518976772849807ull,  1353435754470862315ull,
     6173549831154472795ull,  13567992399387660019ull, 17050234209342075797ull, 650358724130500725ull};
 
-#define SY_TABLE_BYTES (87 * 192)
-
 }  // extern "C" (templates need C++ linkage)
 
 template <int NV, int NF>
@@ -1655,23 +1700,10 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
   // and ONE Fp12 squaring per loop digit - what glued_miller_loop does for the whole batch in the reference
   // (pairing.rs:970-1022).  A thread's 2 / 4 pairs save 63 x 36 of the 8 444 multiplications of every pair after its
   // first.  The n % GLUE leftover pairs go through k_miller.
-  // The glue is the one of fewest wave-times: whole waves of n / g threads (256 resident per SM) times the
-  // multiplications of g glued pairs.  Measured at 2^20 signatures (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 /
-  // 163.3 ms for 1 / 2 / 4; at 2^13 the order reverses (9.3 / 12.4 / 18.4 ms: a quarter of the threads, each four times
-  // as long).
-  int glue = 0;
-  {
-    const size_t wave = (size_t)ctx->sms * SY_GLUED_THREADS * SY_GLUED_MINB;
-    const size_t cost[3] = {8444, 2 * 8444 - 2268, 4 * 8444 - 3 * 2268};
-    size_t best = ~(size_t)0;
-    for (int j = 0; j < 3; j++) {
-      const size_t g = (size_t)1 << j, waves = (n / g + wave - 1) / wave;
-      if (n >= g && waves * cost[j] < best) {
-        best = waves * cost[j];
-        glue = (int)g;
-      }
-    }
-  }
+  // The glue is the one of fewest wave-times (glue_pairs).  Measured at 2^20 signatures
+  // (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 / 163.3 ms for 1 / 2 / 4; at 2^13 the order reverses (9.3 / 12.4 /
+  // 18.4 ms: a quarter of the threads, each four times as long).
+  const int glue = glue_pairs(ctx, n, 8444);
   size_t n_f = n;  // Miller values in scratch0 before the signature pair's value is appended
   if (glue > 1 && n >= (size_t)glue) {
     const size_t items = n / glue, done = items * glue;
@@ -2281,6 +2313,115 @@ int sylow_b200_pairing_check_fixed_batch(sylow_b200_ctx* ctx, const uint8_t* g1,
                                                nullptr));
   CK(cudaMemcpyAsync(ok_out, ctx->out.p, n_checks, cudaMemcpyDeviceToHost, ctx->stream));
   return finish(ctx);
+}
+
+// n_items items of m pairs each (k_miller_tables<m>) -> f_out, one Fp12 per item
+static int launch_miller_tables(sylow_b200_ctx* ctx, int m, const uint8_t* tables, size_t n_tables, const uint32_t* idx,
+                                const uint8_t* g1, const uint8_t* g1_inf, size_t n_items, uint8_t* f_out, int raw_out,
+                                cudaStream_t s) {
+  const unsigned blocks = nblocks(n_items, SY_GLUED_THREADS);
+  const size_t smem = SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS);
+  if (m == 4)
+    k_miller_tables<4><<<blocks, SY_GLUED_THREADS, smem, s>>>(tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
+  else if (m == 2)
+    k_miller_tables<2><<<blocks, SY_GLUED_THREADS, smem, s>>>(tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
+  else
+    k_miller_tables<1><<<blocks, SY_GLUED_THREADS, smem, s>>>(tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
+  LAUNCHED(ctx);
+  return 0;
+}
+
+// d_out (canonical) = prod over n >= 1 pairs of the Miller loop of g1[k] against table idx[k] (k if idx is null):
+// glue_pairs' choice of pairs per thread, the n % glue leftover pairs one per thread, then product_reduce.
+static int miller_product_tables(sylow_b200_ctx* ctx, const uint8_t* tables, size_t n_tables, const uint32_t* idx,
+                                 const uint8_t* g1, const uint8_t* g1_inf, size_t n, uint8_t* d_out, cudaStream_t s) {
+  const int glue = glue_pairs(ctx, n, 6045);
+  const size_t items = n / glue, done = items * glue;
+  CKS(reserve(ctx, ctx->scratch0, n * 384));
+  CKS(reserve(ctx, ctx->scratch1, (n / 4 + 1) * 384));
+  CKS(launch_miller_tables(ctx, glue, tables, n_tables, idx, g1, g1_inf, items, ctx->scratch0.p, 1, s));
+  if (done < n) {
+    // without an index pair k uses table k: the leftover pairs start at table `done`
+    const uint8_t* t = idx ? tables : tables + done * SY_TABLE_BYTES;
+    CKS(launch_miller_tables(ctx, 1, t, idx ? n_tables : n_tables - done, idx ? idx + done : nullptr, g1 + done * 64,
+                             adv(g1_inf, done), n - done, ctx->scratch0.p + items * 384, 1, s));
+  }
+  return product_reduce(ctx, ctx->scratch0.p, ctx->scratch1.p, items + (n - done), d_out, 0, s);
+}
+
+int sylow_b200_miller_loop_precomputed_batch(sylow_b200_ctx* ctx, const uint8_t* coeffs, const uint8_t* g1,
+                                             const uint8_t* g1_inf, size_t n, uint8_t* f_out) {
+  if (is_multi(ctx) && coeffs && g1 && f_out)
+    return multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t, size_t off, size_t m) {
+      return sylow_b200_miller_loop_precomputed_batch(c, coeffs + off * SY_TABLE_BYTES, g1 + off * 64, adv(g1_inf, off),
+                                                      m, f_out + off * 384);
+    });
+  ENTER(ctx);
+  if (n && (!coeffs || !g1 || !f_out)) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  const uint8_t *d1, *d1i;
+  CKS(tables_to_dev(ctx, coeffs, n));
+  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
+  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
+  CKS(reserve(ctx, ctx->out, n * 384));
+  CKS(launch_miller_tables(ctx, 1, ctx->tables.p, n, nullptr, d1, d1i, n, ctx->out.p, 0, ctx->stream));
+  CK(cudaMemcpyAsync(f_out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
+  return finish(ctx);
+}
+
+int sylow_b200_miller_product_precomputed(sylow_b200_ctx* ctx, const uint8_t* coeffs, const uint8_t* g1,
+                                          const uint8_t* g1_inf, size_t n, uint8_t f_out[384]) {
+  if (is_multi(ctx) && coeffs && g1 && f_out && n) {
+    const size_t G = ctx->children.size();
+    std::vector<uint8_t> part(G * 384, 0);
+    for (size_t g = 0; g < G; g++) part[g * 384] = 1;  // empty slices contribute 1
+    uint8_t* pp = part.data();
+    CKS(multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t g, size_t off, size_t m) {
+      return sylow_b200_miller_product_precomputed(c, coeffs + off * SY_TABLE_BYTES, g1 + off * 64, adv(g1_inf, off), m,
+                                                   pp + g * 384);
+    }));
+    return sylow_b200_fp12_product(ctx->children[0], pp, G, f_out);
+  }
+  ENTER(ctx);
+  if (!f_out || (n && (!coeffs || !g1))) return SYLOW_B200_ERR_ARG;
+  if (!n) {
+    memcpy(f_out, kOneCanonical, 384);
+    return 0;
+  }
+  const uint8_t *d1, *d1i;
+  CKS(tables_to_dev(ctx, coeffs, n));
+  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
+  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
+  CKS(reserve(ctx, ctx->out, 384));
+  CKS(miller_product_tables(ctx, ctx->tables.p, n, nullptr, d1, d1i, n, ctx->out.p, ctx->stream));
+  CK(cudaMemcpyAsync(f_out, ctx->out.p, 384, cudaMemcpyDeviceToHost, ctx->stream));
+  return finish(ctx);
+}
+
+int sylow_b200_g2_precompute_dev(sylow_b200_ctx* ctx, const uint8_t* d_g2, size_t n, uint8_t* d_tables_out,
+                                 void* stream) {
+  ENTER_DEV(ctx);
+  if (!ctx || (n && (!d_g2 || !d_tables_out))) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  CK(cudaSetDevice(ctx->device));
+  k_g2_precompute<<<nblocks(n, SY_GLUED_THREADS), SY_GLUED_THREADS, 0, pick(ctx, stream)>>>(d_g2, n, d_tables_out, 1);
+  LAUNCHED(ctx);
+  return 0;
+}
+
+int sylow_b200_miller_product_precomputed_dev(sylow_b200_ctx* ctx, const uint8_t* d_tables, size_t n_tables,
+                                              const uint32_t* d_table_idx, const uint8_t* d_g1, const uint8_t* d_g1_inf,
+                                              size_t n, uint8_t* d_f_out, void* stream) {
+  ENTER_DEV(ctx);
+  if (!ctx || !d_f_out || (n && (!d_tables || !d_g1 || !n_tables || (!d_table_idx && n > n_tables))))
+    return SYLOW_B200_ERR_ARG;
+  CK(cudaSetDevice(ctx->device));
+  cudaStream_t s = pick(ctx, stream);
+  if (!n) {
+    CK(cudaMemcpyAsync(d_f_out, kOneCanonical, 384, cudaMemcpyHostToDevice, s));
+    return 0;
+  }
+  return miller_product_tables(ctx, d_tables, n_tables, d_table_idx, d_g1, d_g1_inf, n, d_f_out, s);
 }
 
 // ------------------------------------------------------------------------------- validation

@@ -264,11 +264,21 @@ def pairing(p: G1Affine, q: G2Affine) -> Gt:
     return _gt_from(out[0])
 
 
-def glued_miller_loop(g2s: Sequence[G2Affine], g1s: Sequence[G1Affine]) -> MillerLoopResult:
-    """pairing.rs:970-1022 (takes the G2 points; the engine fuses the precomputation)."""
+def glued_miller_loop(g2s: Sequence, g1s: Sequence[G1Affine]) -> MillerLoopResult:
+    """pairing.rs:970-1022.  g2s holds `G2PreComputed` values (the reference's signature: the engine runs the loop
+    from their tables) or `G2Affine` points (the engine fuses the precomputation).  Pairs with an infinite point are
+    skipped."""
     n = min(len(g1s), len(g2s))
     if n == 0:
         return MillerLoopResult(Gt.identity().c)
+    if all(isinstance(q, G2PreComputed) for q in g2s[:n]):
+        coeffs = np.stack([np.ascontiguousarray(q.coeffs, dtype=np.uint8).reshape(87 * 192) for q in g2s[:n]])
+        g1 = _arr(b"".join(p._b() for p in g1s[:n]), 64)
+        skip = [int(p.infinity or q.q.infinity) for p, q in zip(g1s[:n], g2s[:n])]  # a table has no infinity form
+        row = engine().miller_product_precomputed(coeffs, g1, skip)
+        return MillerLoopResult(_gt_from(row).c)
+    if any(isinstance(q, G2PreComputed) for q in g2s[:n]):
+        raise TypeError("g2s mixes G2PreComputed and G2Affine values")
     g1 = _arr(b"".join(p._b() for p in g1s[:n]), 64)
     g2 = _arr(b"".join(q._b() for q in g2s[:n]), 128)
     row = engine().miller_product(g1, g2, [int(p.infinity) for p in g1s[:n]], [int(q.infinity) for q in g2s[:n]])
