@@ -15,6 +15,7 @@
 #include "wire.cuh"
 #include "kernels_pairing.cuh"
 #include "miller_tables.cuh"
+#include "launch_plan.h"
 
 using namespace sylow;
 
@@ -957,9 +958,16 @@ __global__ void k_dfma_probe(int iters, const uint32_t* src, uint32_t* sink) {
 // ------------------------------------------------------------------------------------------------
 // context
 // ------------------------------------------------------------------------------------------------
+// device memory of one context, freed with it (the context's device is current when its destructor runs)
 struct DevBuf {
   uint8_t* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
 };
 
 struct sylow_b200_ctx {
@@ -977,9 +985,21 @@ struct sylow_b200_ctx {
   DevBuf tables, sum0, sum1, proj, msm;
   DevBuf check_stage[2];  // group products / Gt values of launch_check_products' two-lane path, per compute stream
   DevBuf fexp_lanes[2];  // FexpCold records of k_final_exp_lanes, one buffer per compute stream (stream, stream2)
-  unsigned glued_attr_mask = 0;
   // multi-device parent (sylow_b200_create_multi): owns one single-device context per GPU and nothing else
   std::vector<sylow_b200_ctx*> children;
+
+  // releases whatever was created, so it also undoes a partly finished sylow_b200_create (hidden: the library exports
+  // its C ABI, not C++ members)
+  __attribute__((visibility("hidden"))) ~sylow_b200_ctx() {
+    for (sylow_b200_ctx* c : children) delete c;
+    if (!children.empty()) return;
+    cudaSetDevice(device);  // the DevBuf members are freed after this body, on the same device
+    if (d_fail) cudaFree(d_fail);
+    if (d_gen_table) cudaFree(d_gen_table);
+    for (cudaStream_t s : {stream, copy_in, copy_out, stream2})
+      if (s) cudaStreamDestroy(s);
+    if (ev_fork) cudaEventDestroy(ev_fork);
+  }
 };
 
 static int fail_cuda(sylow_b200_ctx* ctx, cudaError_t e) {
@@ -1001,9 +1021,11 @@ static int fail_cuda(sylow_b200_ctx* ctx, cudaError_t e) {
   if (!(ctx)) return SYLOW_B200_ERR_ARG;                    \
   if (!(ctx)->children.empty()) (ctx) = (ctx)->children[0]; \
   CK(cudaSetDevice((ctx)->device));
-// `_dev` entry points work on one device's memory: they need a single-device context (sylow_b200_device_ctx)
-#define ENTER_DEV(ctx) \
-  if ((ctx) && !(ctx)->children.empty()) return SYLOW_B200_ERR_ARG;
+// `_dev` entry points work on one device's memory: they need a single-device context (sylow_b200_device_ctx), and run
+// on its device whatever device the calling thread has current
+#define ENTER_DEV(ctx)                                                   \
+  if (!(ctx) || !(ctx)->children.empty()) return SYLOW_B200_ERR_ARG; \
+  CK(cudaSetDevice((ctx)->device));
 
 static int reserve(sylow_b200_ctx* ctx, DevBuf& b, size_t bytes) {
   if (bytes <= b.cap) return 0;
@@ -1022,7 +1044,6 @@ static int reserve(sylow_b200_ctx* ctx, DevBuf& b, size_t bytes) {
 
 static constexpr size_t sy_gcd(size_t a, size_t b) { return b ? sy_gcd(b, a % b) : a; }
 static constexpr size_t sy_lcm(size_t a, size_t b) { return a / sy_gcd(a, b) * b; }
-static inline unsigned nblocks(size_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 static inline cudaStream_t pick(sylow_b200_ctx* ctx, void* stream) {
   return stream ? (cudaStream_t)stream : ctx->stream;
 }
@@ -1032,174 +1053,120 @@ static inline cudaStream_t pick(sylow_b200_ctx* ctx, void* stream) {
     CK(cudaGetLastError());  \
   } while (0)
 
-// Launch shapes that do not waste the last wave.  Both pairing kernels run one item per thread for several
-// milliseconds, so a batch that is not a whole number of waves (k_miller keeps 256 threads resident per SM,
-// k_final_exp 384) ends with a partly filled wave that takes as long as a full one - at 2^17 items per GPU (a 2^20
-// batch sharded over 8) that is 3.46 and 2.31 waves.  The whole waves are launched as usual; a remainder of less than
-// 0.6 wave is launched separately as one (k_final_exp) or two (k_miller) SMALL blocks per SM, so that every SM works
-// on it at low occupancy - a lone warp per scheduler runs 1.5x (Miller) to 2x (final exponentiation) faster than one of
-// two or three co-resident warps (profiles/r01_overlap_probe.md), and the remainder finishes in that much less time.
-struct WaveSplit {
-  size_t n_main;       // items in whole waves (launched with the kernel's normal block size)
-  size_t n_tail;       // remainder
-  unsigned tail_threads, tail_blocks;
-};
-// (Cutting the last 1 + r waves into two rounds of equal, reduced occupancy instead was measured and is not better:
-// profiles/r02g_policy_sweep.jsonl, tail_split 2.)
-static WaveSplit wave_split(const sylow_b200_ctx* ctx, size_t n, int threads, int blocks_per_sm) {
-  WaveSplit w{n, 0, 0, 0};
-  const size_t wave = (size_t)ctx->sms * threads * blocks_per_sm;
-  const size_t r = n % wave;
-  if (r == 0 || r * 10 >= wave * 6) return w;
-  const size_t slots = (size_t)ctx->sms * blocks_per_sm;
-  unsigned t = (unsigned)(((r + slots - 1) / slots + 31) / 32 * 32);
-  if (t > (unsigned)threads) t = threads;
-  w.n_main = n - r;
-  w.n_tail = r;
-  w.tail_threads = t;
-  w.tail_blocks = (unsigned)((r + t - 1) / t);
-  return w;
-}
-// Two lanes per item (k_miller_lanes, k_final_exp_lanes, csrc/pairing_lanes.cuh): the same values in 0.55-0.6 of the
-// time per item when the items alone cannot fill the GPU, 0.88 of the one-thread kernels' throughput when they can
-// (profiles/r02f_lanes_kbench.jsonl, r02g_policy_sweep.jsonl).  Used for batches of at most one two-lane wave
-// (148 x 128 items) and for the remainder of a larger batch after its whole one-thread waves when that remainder fits one
-// two-lane wave: 1 .. 9 472 pairings 8.5 -> 5.0 ms, 2^17 pairings (a 2^20 batch over 8 GPUs) 46.3 -> 44.3 ms.
-// SYLOW_B200_LANES: 0 never, 1 automatic (default), 2 always (measurement and the parity tests).
+static inline const uint8_t* adv(const uint8_t* p, size_t bytes) { return p ? p + bytes : nullptr; }
+static inline uint8_t* adv(uint8_t* p, size_t bytes) { return p ? p + bytes : nullptr; }
+
+// block shapes of the batch kernels (kernels_pairing.cuh), for the launch policy of launch_plan.h
+static constexpr BlockShape kMillerShape{SY_MILLER_THREADS, SY_MILLER_MINB}, kFexpShape{SY_FEXP_THREADS, SY_FEXP_MINB},
+    kLanesShape{SY_LANES_THREADS, SY_LANES_MINB}, kGluedShape{SY_GLUED_THREADS, SY_GLUED_MINB};
+
+// SYLOW_B200_LANES: 0 never, 1 automatic (default), 2 always (measurement and the parity tests); see batch_plan.
 static int lanes_mode() {  // read on every call (the tests flip it inside one process)
   const char* v = getenv("SYLOW_B200_LANES");
   return v ? atoi(v) : 1;
 }
-static int launch_miller_lanes(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
-                               const uint8_t* g2_inf, size_t n, uint8_t* f_out, int raw_out, cudaStream_t s) {
-  // spread a small batch over every SM: pairs per block = n / (2 blocks x SMs), in whole warps (16 pairs), at most 64
-  const size_t slots = (size_t)ctx->sms * SY_LANES_MINB;
-  size_t pairs = ((n + slots - 1) / slots + 15) / 16 * 16;
-  if (pairs > SY_LANES_THREADS / 2) pairs = SY_LANES_THREADS / 2;
-  const unsigned threads = (unsigned)pairs * 2;
-  k_miller_lanes<<<nblocks(n, (int)pairs), threads, SY_LANES_SMEM_BYTES(threads), s>>>(g1, g1_inf, g2, g2_inf, n, f_out,
-                                                                                      raw_out);
-  LAUNCHED(ctx);
-  return 0;
-}
 static int launch_miller(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                          const uint8_t* g2_inf, size_t n, uint8_t* f_out, int raw_out, cudaStream_t s) {
-  const int lanes = lanes_mode();
-  const size_t lane_wave = (size_t)ctx->sms * (SY_LANES_THREADS / 2) * SY_LANES_MINB;
-  if (lanes == 2 || (lanes == 1 && n <= lane_wave))
-    return launch_miller_lanes(ctx, g1, g1_inf, g2, g2_inf, n, f_out, raw_out, s);
-  WaveSplit w = wave_split(ctx, n, SY_MILLER_THREADS, SY_MILLER_MINB);
-  const size_t wave1 = (size_t)ctx->sms * SY_MILLER_THREADS * SY_MILLER_MINB;
-  if (lanes == 1 && n % wave1 && n % wave1 <= lane_wave) {
-    const size_t r = n % wave1, o = n - r;
-    k_miller<<<nblocks(o, SY_MILLER_THREADS), SY_MILLER_THREADS, SY_MILLER_SMEM_BYTES(SY_MILLER_THREADS), s>>>(
-        g1, g1_inf, g2, g2_inf, 1, o, f_out, raw_out);
-    LAUNCHED(ctx);
-    return launch_miller_lanes(ctx, g1 + o * 64, g1_inf ? g1_inf + o : nullptr, g2 + o * 128,
-                               g2_inf ? g2_inf + o : nullptr, r, f_out + o * 384, raw_out, s);
-  }
-  if (w.n_main) {
-    k_miller<<<nblocks(w.n_main, SY_MILLER_THREADS), SY_MILLER_THREADS, SY_MILLER_SMEM_BYTES(SY_MILLER_THREADS), s>>>(
-        g1, g1_inf, g2, g2_inf, 1, w.n_main, f_out, raw_out);
-    LAUNCHED(ctx);
-  }
-  if (w.n_tail) {
-    const size_t o = w.n_main;
-    k_miller<<<w.tail_blocks, w.tail_threads, SY_MILLER_SMEM_BYTES(w.tail_threads), s>>>(
-        g1 + o * 64, g1_inf ? g1_inf + o : nullptr, g2 + o * 128, g2_inf ? g2_inf + o : nullptr, 1, w.n_tail,
-        f_out + o * 384, raw_out);
+  for (const Segment& g : batch_plan(ctx->sms, n, kMillerShape, kLanesShape, lanes_mode())) {
+    const size_t o = g.first;
+    if (g.lanes)
+      k_miller_lanes<<<g.blocks, g.threads, SY_LANES_SMEM_BYTES(g.threads), s>>>(
+          g1 + o * 64, adv(g1_inf, o), g2 + o * 128, adv(g2_inf, o), g.count, f_out + o * 384, raw_out);
+    else
+      k_miller<<<g.blocks, g.threads, SY_MILLER_SMEM_BYTES(g.threads), s>>>(
+          g1 + o * 64, adv(g1_inf, o), g2 + o * 128, adv(g2_inf, o), 1, g.count, f_out + o * 384, raw_out);
     LAUNCHED(ctx);
   }
   return 0;
 }
-static int launch_final_exp_lanes(sylow_b200_ctx* ctx, const uint8_t* f, int raw_in, size_t n, uint8_t* gt_out,
+// k_final_exp_lanes over the items of g; its FexpCold scratch is kept per compute stream
+static int launch_final_exp_lanes(sylow_b200_ctx* ctx, const Segment& g, const uint8_t* f, int raw_in, uint8_t* gt_out,
                                   cudaStream_t s) {
-  const size_t slots = (size_t)ctx->sms * SY_LANES_MINB;
-  size_t pairs = ((n + slots - 1) / slots + 15) / 16 * 16;
-  if (pairs > SY_LANES_THREADS / 2) pairs = SY_LANES_THREADS / 2;
-  const unsigned threads = (unsigned)pairs * 2, blocks = nblocks(n, (int)pairs);
   DevBuf& scratch = ctx->fexp_lanes[s == ctx->stream2 ? 1 : 0];
-  CKS(reserve(ctx, scratch, SY_FLANES_SCRATCH_BYTES((size_t)blocks * pairs)));
-  k_final_exp_lanes<<<blocks, threads, SY_FLANES_SMEM_BYTES(threads), s>>>(f, raw_in, n, gt_out, scratch.p);
+  CKS(reserve(ctx, scratch, SY_FLANES_SCRATCH_BYTES((size_t)g.blocks * (g.threads / 2))));
+  k_final_exp_lanes<<<g.blocks, g.threads, SY_FLANES_SMEM_BYTES(g.threads), s>>>(f + g.first * 384, raw_in, g.count,
+                                                                                 gt_out + g.first * 384, scratch.p);
   LAUNCHED(ctx);
   return 0;
 }
 static int launch_final_exp(sylow_b200_ctx* ctx, const uint8_t* f, int raw_in, size_t n, uint8_t* gt_out, cudaStream_t s) {
-  const int lanes = lanes_mode();
-  const size_t lane_wave = (size_t)ctx->sms * (SY_LANES_THREADS / 2) * SY_LANES_MINB;
-  if (lanes == 2 || (lanes == 1 && n <= lane_wave)) return launch_final_exp_lanes(ctx, f, raw_in, n, gt_out, s);
-  const size_t wave1 = (size_t)ctx->sms * SY_FEXP_THREADS * SY_FEXP_MINB;
-  if (lanes == 1 && n % wave1 && n % wave1 <= lane_wave) {
-    const size_t r = n % wave1, o = n - r;
-    k_final_exp<<<nblocks(o, SY_FEXP_THREADS), SY_FEXP_THREADS, SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS), s>>>(f, raw_in, o,
-                                                                                                       gt_out);
-    LAUNCHED(ctx);
-    return launch_final_exp_lanes(ctx, f + o * 384, raw_in, r, gt_out + o * 384, s);
-  }
-  const WaveSplit w = wave_split(ctx, n, SY_FEXP_THREADS, SY_FEXP_MINB);
-  if (w.n_main) {
-    k_final_exp<<<nblocks(w.n_main, SY_FEXP_THREADS), SY_FEXP_THREADS, SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS), s>>>(
-        f, raw_in, w.n_main, gt_out);
-    LAUNCHED(ctx);
-  }
-  if (w.n_tail) {
-    const size_t o = w.n_main;
-    k_final_exp<<<w.tail_blocks, w.tail_threads, SY_FEXP_SMEM_BYTES(w.tail_threads), s>>>(f + o * 384, raw_in, w.n_tail,
-                                                                                         gt_out + o * 384);
+  for (const Segment& g : batch_plan(ctx->sms, n, kFexpShape, kLanesShape, lanes_mode())) {
+    if (g.lanes) {
+      CKS(launch_final_exp_lanes(ctx, g, f, raw_in, gt_out, s));
+      continue;
+    }
+    k_final_exp<<<g.blocks, g.threads, SY_FEXP_SMEM_BYTES(g.threads), s>>>(f + g.first * 384, raw_in, g.count,
+                                                                           gt_out + g.first * 384);
     LAUNCHED(ctx);
   }
   return 0;
 }
 
-// ok[c] = final_exp(prod_{j<k} f[c*k + j]) == 1 for the Montgomery-form Miller values at f.  Batches that fit one
-// two-lane wave go through k_final_exp_lanes (group products, exponentiation, comparison as three launches: about half
-// the latency); larger ones through the fused one-thread kernel, in blocks small enough to reach every SM.
+// ok[c] = final_exp(prod_{j<k} f[c*k + j]) == 1 for the Montgomery-form Miller values at f (check_products_segment)
 static int launch_check_products(sylow_b200_ctx* ctx, const uint8_t* f, size_t k, size_t n_checks, uint8_t* ok,
                                  cudaStream_t s) {
-  const size_t lane_wave = (size_t)ctx->sms * (SY_LANES_THREADS / 2) * SY_LANES_MINB;
-  if (lanes_mode() != 0 && n_checks <= lane_wave) {
+  const Segment g = check_products_segment(ctx->sms, n_checks, kFexpShape, kLanesShape, lanes_mode());
+  if (g.lanes) {
     DevBuf& stage = ctx->check_stage[s == ctx->stream2 ? 1 : 0];
     CKS(reserve(ctx, stage, n_checks * 384));
     if (k > 1) {
       k_group_products<<<nblocks(n_checks, 32), 32, 0, s>>>(f, k, n_checks, stage.p);
       LAUNCHED(ctx);
     }
-    CKS(launch_final_exp_lanes(ctx, k > 1 ? stage.p : f, 1, n_checks, stage.p, s));
+    CKS(launch_final_exp_lanes(ctx, g, k > 1 ? stage.p : f, 1, stage.p, s));
     k_gt_is_one<<<nblocks(n_checks, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(stage.p, n_checks, ok);
     LAUNCHED(ctx);
     return 0;
   }
-  unsigned t = (unsigned)(((n_checks + ctx->sms - 1) / ctx->sms + 31) / 32 * 32);
-  if (t > SY_FEXP_THREADS) t = SY_FEXP_THREADS;
-  k_check_products<<<nblocks(n_checks, (int)t), t, SY_FEXP_SMEM_BYTES(t), s>>>(f, k, n_checks, ok);
+  k_check_products<<<g.blocks, g.threads, SY_FEXP_SMEM_BYTES(g.threads), s>>>(f, k, n_checks, ok);
   LAUNCHED(ctx);
   return 0;
 }
 
-// Pairs per thread (1, 2 or 4) for n >= 1 pairs whose Miller loops only meet as a product, glued into one loop per
-// thread (k_glued<M, 0>, k_miller_tables<M>): the glue of fewest wave-times, i.e. whole waves of n / g threads (256
-// resident per SM) times the Fp multiplications of g glued pairs.  pair_cost is one pair's count (8 444 fused, 6 045
-// from a table); every pair after the first saves its Fp12 squarings, 63 x 36 multiplications.
-static int glue_pairs(const sylow_b200_ctx* ctx, size_t n, size_t pair_cost) {
-  const size_t wave = (size_t)ctx->sms * SY_GLUED_THREADS * SY_GLUED_MINB, save = 63 * 36;
-  const size_t cost[3] = {pair_cost, 2 * pair_cost - save, 4 * pair_cost - 3 * save};
-  int glue = 0;
-  size_t best = ~(size_t)0;
-  for (int j = 0; j < 3; j++) {
-    const size_t g = (size_t)1 << j, waves = (n / g + wave - 1) / wave;
-    if (n >= g && waves * cost[j] < best) {
-      best = waves * cost[j];
-      glue = (int)g;
-    }
+// The compiled glued-loop shapes k_glued<NV, NF>: NV fused pairs and NF pairs against fixed tables per item.
+static const struct {
+  size_t nv, nf;
+  decltype(&k_glued<0, 1>) kernel;
+} kGlued[] = {{2, 0, k_glued<2, 0>}, {4, 0, k_glued<4, 0>}, {1, 1, k_glued<1, 1>}, {0, 1, k_glued<0, 1>}, {1, 3, k_glued<1, 3>}};
+// the NF tables, then the accumulators
+static size_t glued_smem(size_t nf) { return nf * SY_TABLE_BYTES + SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS); }
+static bool glued_shape_ok(size_t nv, size_t nf) {
+  for (const auto& v : kGlued)
+    if (v.nv == nv && v.nf == nf) return true;
+  return false;
+}
+// one glued loop of nv fused + nf table pairs per item; SYLOW_B200_ERR_ARG for a shape that is not compiled
+static int launch_glued(sylow_b200_ctx* ctx, size_t nv, size_t nf, const uint8_t* g1v, size_t sv, const uint8_t* g1v_inf,
+                        const uint8_t* g2v, const uint8_t* g2v_inf, const uint8_t* g1f, size_t sf, const uint8_t* g1f_inf,
+                        const uint8_t* tables, size_t n, uint8_t* f_out, cudaStream_t s) {
+  for (const auto& v : kGlued) {
+    if (v.nv != nv || v.nf != nf) continue;
+    v.kernel<<<nblocks(n, SY_GLUED_THREADS), SY_GLUED_THREADS, glued_smem(nf), s>>>(g1v, sv, g1v_inf, g2v, g2v_inf, g1f, sf,
+                                                                                   g1f_inf, tables, n, f_out);
+    LAUNCHED(ctx);
+    return 0;
   }
-  return glue;
+  return SYLOW_B200_ERR_ARG;
 }
 
-// defined further down (needs the table constants): one glued loop of NV fused + NF table pairs per item
-template <int NV, int NF>
-static int launch_glued(sylow_b200_ctx* ctx, const uint8_t* g1v, size_t sv, const uint8_t* g1v_inf, const uint8_t* g2v,
-                        const uint8_t* g2v_inf, const uint8_t* g1f, size_t sf, const uint8_t* g1f_inf,
-                        const uint8_t* tables, size_t n, uint8_t* f_out, cudaStream_t s);
+// The compiled k_miller_tables<M>: M pairs per item, each against its own table.
+static const struct {
+  int m;
+  decltype(&k_miller_tables<1>) kernel;
+} kMillerTables[] = {{1, k_miller_tables<1>}, {2, k_miller_tables<2>}, {4, k_miller_tables<4>}};
+// n_items items of m pairs each -> f_out, one Fp12 per item; SYLOW_B200_ERR_ARG for an m that is not compiled
+static int launch_miller_tables(sylow_b200_ctx* ctx, int m, const uint8_t* tables, size_t n_tables, const uint32_t* idx,
+                                const uint8_t* g1, const uint8_t* g1_inf, size_t n_items, uint8_t* f_out, int raw_out,
+                                cudaStream_t s) {
+  for (const auto& v : kMillerTables) {
+    if (v.m != m) continue;
+    v.kernel<<<nblocks(n_items, SY_GLUED_THREADS), SY_GLUED_THREADS, SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS), s>>>(
+        tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
+    LAUNCHED(ctx);
+    return 0;
+  }
+  return SYLOW_B200_ERR_ARG;
+}
 
 extern "C" {
 
@@ -1216,31 +1183,22 @@ int sylow_b200_create(sylow_b200_ctx** out, int device_id) {
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&ctx->stream2, cudaStreamNonBlocking);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&ctx->sms, cudaDevAttrMultiProcessorCount, device_id);
-  // opt-in for more than 48 KB of dynamic shared memory (the Miller loop's accumulators); per device
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_miller, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_MILLER_SMEM_BYTES(SY_MILLER_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_miller_lanes, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_LANES_SMEM_BYTES(SY_LANES_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_final_exp_lanes, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_FLANES_SMEM_BYTES(SY_LANES_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_final_exp, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_check_products, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_miller_tables<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_miller_tables<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(k_miller_tables<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
+  // opt-ins for more than 48 KB of dynamic shared memory (the accumulators, the glued loops' tables); per device
+  const struct {
+    const void* kernel;
+    size_t bytes;
+  } smem[] = {{(const void*)k_miller, SY_MILLER_SMEM_BYTES(SY_MILLER_THREADS)},
+              {(const void*)k_miller_lanes, SY_LANES_SMEM_BYTES(SY_LANES_THREADS)},
+              {(const void*)k_final_exp_lanes, SY_FLANES_SMEM_BYTES(SY_LANES_THREADS)},
+              {(const void*)k_final_exp, SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS)},
+              {(const void*)k_check_products, SY_FEXP_SMEM_BYTES(SY_FEXP_THREADS)}};
+  const cudaFuncAttribute max_smem = cudaFuncAttributeMaxDynamicSharedMemorySize;
+  for (const auto& k : smem)
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k.kernel, max_smem, (int)k.bytes);
+  for (const auto& v : kMillerTables)
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(v.kernel, max_smem, (int)SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS));
+  for (const auto& v : kGlued)
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(v.kernel, max_smem, (int)glued_smem(v.nf));
   if (e == cudaSuccess) e = cudaMalloc(&ctx->d_fail, sizeof(int));
   if (e == cudaSuccess) e = cudaMemset(ctx->d_fail, 0, sizeof(int));
   if (e != cudaSuccess) {
@@ -1253,32 +1211,6 @@ int sylow_b200_create(sylow_b200_ctx** out, int device_id) {
 
 int sylow_b200_destroy(sylow_b200_ctx* ctx) {
   if (!ctx) return SYLOW_B200_ERR_ARG;
-  if (!ctx->children.empty()) {
-    for (sylow_b200_ctx* c : ctx->children) sylow_b200_destroy(c);
-    delete ctx;
-    return 0;
-  }
-  cudaSetDevice(ctx->device);
-  DevBuf* bufs[] = {&ctx->in_a, &ctx->in_b, &ctx->in_c, &ctx->in_d, &ctx->flag_a,
-                    &ctx->flag_b, &ctx->out, &ctx->scratch0, &ctx->scratch1, &ctx->scratch2};
-  for (DevBuf* b : bufs)
-    if (b->p) cudaFree(b->p);
-  if (ctx->d_fail) cudaFree(ctx->d_fail);
-  if (ctx->d_gen_table) cudaFree(ctx->d_gen_table);
-  if (ctx->tables.p) cudaFree(ctx->tables.p);
-  if (ctx->sum0.p) cudaFree(ctx->sum0.p);
-  if (ctx->sum1.p) cudaFree(ctx->sum1.p);
-  if (ctx->proj.p) cudaFree(ctx->proj.p);
-  if (ctx->msm.p) cudaFree(ctx->msm.p);
-  for (DevBuf& b : ctx->fexp_lanes)
-    if (b.p) cudaFree(b.p);
-  for (DevBuf& b : ctx->check_stage)
-    if (b.p) cudaFree(b.p);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  if (ctx->copy_in) cudaStreamDestroy(ctx->copy_in);
-  if (ctx->copy_out) cudaStreamDestroy(ctx->copy_out);
-  if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
-  if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
   delete ctx;
   return 0;
 }
@@ -1297,12 +1229,11 @@ int sylow_b200_create_multi(sylow_b200_ctx** out, const int* device_ids, int n_d
       try {
         parent->children.push_back(c);
       } catch (...) {
-        sylow_b200_destroy(c);
+        delete c;
         st = SYLOW_B200_ERR_NOMEM;
       }
     }
     if (st != 0) {
-      for (sylow_b200_ctx* d : parent->children) sylow_b200_destroy(d);
       delete parent;
       return st;
     }
@@ -1350,14 +1281,14 @@ uint64_t sylow_b200_launch_count(const sylow_b200_ctx* ctx) {
 int sylow_b200_miller_loop_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                                      const uint8_t* g2_inf, size_t n, uint8_t* f_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!g1 || !g2 || !f_out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!g1 || !g2 || !f_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   return launch_miller(ctx, g1, g1_inf, g2, g2_inf, n, f_out, 0, pick(ctx, stream));
 }
 
 int sylow_b200_final_exp_batch_dev(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, uint8_t* gt_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!f || !gt_out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!f || !gt_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   return launch_final_exp(ctx, f, 0, n, gt_out, pick(ctx, stream));
 }
@@ -1376,7 +1307,7 @@ static int pairing_dev_single(sylow_b200_ctx* ctx, const uint8_t* g1, const uint
 int sylow_b200_pairing_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                                  const uint8_t* g2_inf, size_t n, uint8_t* gt_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!g1 || !g2 || !gt_out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!g1 || !g2 || !gt_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   return pairing_dev_single(ctx, g1, g1_inf, g2, g2_inf, n, gt_out, pick(ctx, stream));
 }
@@ -1412,7 +1343,7 @@ static const uint8_t kOneCanonical[384] = {1};
 int sylow_b200_miller_product_dev(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                                   const uint8_t* g2_inf, size_t n, uint8_t* f_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || !f_out || (n && (!g1 || !g2))) return SYLOW_B200_ERR_ARG;
+  if (!f_out || (n && (!g1 || !g2))) return SYLOW_B200_ERR_ARG;
   cudaStream_t s = pick(ctx, stream);
   if (!n) {
     CK(cudaMemcpyAsync(f_out, kOneCanonical, 384, cudaMemcpyHostToDevice, s));
@@ -1428,7 +1359,7 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
                                        const uint8_t* g2, const uint8_t* g2_inf, size_t k, size_t n_checks,
                                        uint8_t* ok_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n_checks && !ok_out)) return SYLOW_B200_ERR_ARG;
+  if (n_checks && !ok_out) return SYLOW_B200_ERR_ARG;
   if (!n_checks) return 0;
   size_t n = k * n_checks;
   if (n && (!g1 || !g2)) return SYLOW_B200_ERR_ARG;
@@ -1438,12 +1369,9 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
     CKS(reserve(ctx, ctx->scratch0, n * 384));
     // 2- and 4-pair checks (ecPairing, Groth16 without fixed tables) as ONE glued loop per check: one Fp12 squaring per
     // digit for all pairs of the check, like glued_miller_loop (pairing.rs:970-1022); needs enough checks to fill the GPU
-    const size_t wave = (size_t)ctx->sms * SY_GLUED_THREADS * SY_GLUED_MINB;
-    if (k == 2 && n_checks >= wave) {
-      CKS((launch_glued<2, 0>(ctx, g1, 2, g1_inf, g2, g2_inf, nullptr, 0, nullptr, nullptr, n_checks, ctx->scratch0.p, s)));
-      k_prod = 1;
-    } else if (k == 4 && n_checks >= wave / 2) {
-      CKS((launch_glued<4, 0>(ctx, g1, 4, g1_inf, g2, g2_inf, nullptr, 0, nullptr, nullptr, n_checks, ctx->scratch0.p, s)));
+    const size_t wave = wave_items(ctx->sms, kGluedShape);
+    if ((k == 2 && n_checks >= wave) || (k == 4 && n_checks >= wave / 2)) {
+      CKS(launch_glued(ctx, k, 0, g1, k, g1_inf, g2, g2_inf, nullptr, 0, nullptr, nullptr, n_checks, ctx->scratch0.p, s));
       k_prod = 1;
     } else {
       CKS(launch_miller(ctx, g1, g1_inf, g2, g2_inf, n, ctx->scratch0.p, 1, s));
@@ -1452,12 +1380,25 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
   return launch_check_products(ctx, ctx->scratch0.p, k_prod, n_checks, ok_out, s);
 }
 
-// batches from this size on convert to affine coordinates with one inversion per eight points
+// Batches from SY_AFF_MIN_BATCH points on leave their results in projective form (proj_bytes per point, Montgomery form) in
+// ctx->proj and convert them to affine coordinates afterwards, with one inversion per SY_AFF_K points (affine_tail);
+// smaller ones convert each point in the kernel (*proj = null).
 #define SY_AFF_MIN_BATCH 32768
-static int g1_batch_affine(sylow_b200_ctx* ctx, const uint8_t* d_proj, size_t n, int negate, uint8_t* d_out,
-                           uint8_t* d_out_inf, cudaStream_t s) {
-  size_t T = (n + SY_AFF_K - 1) / SY_AFF_K;
-  k_g1_batch_affine<<<nblocks(T, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_proj, n, negate, d_out, d_out_inf);
+static int affine_stage(sylow_b200_ctx* ctx, size_t n, size_t proj_bytes, uint8_t** proj) {
+  *proj = nullptr;
+  if (n < SY_AFF_MIN_BATCH) return 0;
+  CKS(reserve(ctx, ctx->proj, n * proj_bytes));
+  *proj = ctx->proj.p;
+  return 0;
+}
+// n projective points at d_proj -> affine wire format + infinity flags; G1 points optionally negated
+static int affine_tail(sylow_b200_ctx* ctx, bool g2, const uint8_t* d_proj, size_t n, int negate, uint8_t* d_out,
+                       uint8_t* d_out_inf, cudaStream_t s) {
+  const unsigned blocks = nblocks((n + SY_AFF_K - 1) / SY_AFF_K, SY_MUL_THREADS);
+  if (g2)
+    k_g2_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(d_proj, n, d_out, d_out_inf);
+  else
+    k_g1_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(d_proj, n, negate, d_out, d_out_inf);
   LAUNCHED(ctx);
   return 0;
 }
@@ -1465,37 +1406,27 @@ static int g1_batch_affine(sylow_b200_ctx* ctx, const uint8_t* d_proj, size_t n,
 int sylow_b200_g1_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf,
                                 const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!pts || !scalars || !out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!pts || !scalars || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  uint8_t* proj = nullptr;
-  if (n >= SY_AFF_MIN_BATCH) {
-    CKS(reserve(ctx, ctx->proj, n * 96));
-    proj = ctx->proj.p;
-  }
-  k_g1_mul<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, pick(ctx, stream)>>>(pts, pts_inf, scalars, n,
-                                                                                        out, out_inf, proj);
+  cudaStream_t s = pick(ctx, stream);
+  uint8_t* proj;
+  CKS(affine_stage(ctx, n, 96, &proj));
+  k_g1_mul<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(pts, pts_inf, scalars, n, out, out_inf, proj);
   LAUNCHED(ctx);
-  if (proj) CKS(g1_batch_affine(ctx, proj, n, 0, out, out_inf, pick(ctx, stream)));
+  if (proj) CKS(affine_tail(ctx, false, proj, n, 0, out, out_inf, s));
   return 0;
 }
 int sylow_b200_g2_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf,
                                 const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!pts || !scalars || !out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!pts || !scalars || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  uint8_t* proj = nullptr;
-  if (n >= SY_AFF_MIN_BATCH) {
-    CKS(reserve(ctx, ctx->proj, n * 192));
-    proj = ctx->proj.p;
-  }
-  k_g2_mul<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, pick(ctx, stream)>>>(pts, pts_inf, scalars,
-                                                                                          n, out, out_inf, proj);
+  cudaStream_t s = pick(ctx, stream);
+  uint8_t* proj;
+  CKS(affine_stage(ctx, n, 192, &proj));
+  k_g2_mul<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(pts, pts_inf, scalars, n, out, out_inf, proj);
   LAUNCHED(ctx);
-  if (proj) {
-    size_t T = (n + SY_AFF_K - 1) / SY_AFF_K;
-    k_g2_batch_affine<<<nblocks(T, SY_MUL_THREADS), SY_MUL_THREADS, 0, pick(ctx, stream)>>>(proj, n, out, out_inf);
-    LAUNCHED(ctx);
-  }
+  if (proj) CKS(affine_tail(ctx, true, proj, n, 0, out, out_inf, s));
   return 0;
 }
 
@@ -1531,16 +1462,13 @@ static int make_dst_prime(sylow_b200_ctx* ctx, const uint8_t* dst, size_t dst_le
 
 static int hash_launch(sylow_b200_ctx* ctx, const uint8_t* d_msgs, const uint64_t* d_offsets, size_t n,
                        const DstPrime& dp, int negate, uint8_t* d_out, uint8_t* d_out_inf, cudaStream_t s) {
-  uint8_t* proj = nullptr;
-  if (n >= SY_AFF_MIN_BATCH) {
-    CKS(reserve(ctx, ctx->proj, n * 96));
-    proj = ctx->proj.p;
-  }
+  uint8_t* proj;
+  CKS(affine_stage(ctx, n, 96, &proj));
   CK(cudaMemsetAsync(ctx->d_fail, 0, sizeof(int), s));  // the flag reports THIS call's hashes only
   k_hash_to_g1<<<nblocks(n, SY_HASH_THREADS), SY_HASH_THREADS, 0, s>>>(d_msgs, d_offsets, n, dp, negate, d_out,
                                                                      d_out_inf, ctx->d_fail, proj);
   LAUNCHED(ctx);
-  if (proj) CKS(g1_batch_affine(ctx, proj, n, negate, d_out, d_out_inf, s));
+  if (proj) CKS(affine_tail(ctx, false, proj, n, negate, d_out, d_out_inf, s));
   return 0;
 }
 
@@ -1548,7 +1476,7 @@ int sylow_b200_hash_to_g1_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_msgs, 
                                     const uint8_t* dst, size_t dst_len, int hash_id, uint8_t* d_out,
                                     uint8_t* d_out_inf, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!d_offsets || !d_out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!d_offsets || !d_out)) return SYLOW_B200_ERR_ARG;
   DstPrime dp;
   CKS(make_dst_prime(ctx, dst, dst_len, hash_id, dp));
   if (!n) return 0;
@@ -1562,27 +1490,6 @@ static const uint64_t kG2GenWords[16] = {
     10945020018377822914ull, 17413811393473931026ull, 8241798111626485029ull,  1841571559660931130ull,
     5541340697920699818ull,  16416156555105522555ull, 5380518976772849807ull,  1353435754470862315ull,
     6173549831154472795ull,  13567992399387660019ull, 17050234209342075797ull, 650358724130500725ull};
-
-}  // extern "C" (templates need C++ linkage)
-
-template <int NV, int NF>
-static int launch_glued(sylow_b200_ctx* ctx, const uint8_t* g1v, size_t sv, const uint8_t* g1v_inf, const uint8_t* g2v,
-                        const uint8_t* g2v_inf, const uint8_t* g1f, size_t sf, const uint8_t* g1f_inf,
-                        const uint8_t* tables, size_t n, uint8_t* f_out, cudaStream_t s) {
-  // the opt-in for > 48 KB of dynamic shared memory is per device: remember it per context
-  size_t smem = (size_t)NF * SY_TABLE_BYTES + SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS);
-  unsigned bit = 1u << (NV * 4 + NF);
-  if (!(ctx->glued_attr_mask & bit)) {
-    CK(cudaFuncSetAttribute(k_glued<NV, NF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ctx->glued_attr_mask |= bit;
-  }
-  k_glued<NV, NF><<<nblocks(n, SY_GLUED_THREADS), SY_GLUED_THREADS, smem, s>>>(g1v, sv, g1v_inf, g2v, g2v_inf, g1f, sf,
-                                                                              g1f_inf, tables, n, f_out);
-  LAUNCHED(ctx);
-  return 0;
-}
-
-extern "C" {
 
 // G2PreComputed of the generator, computed on the device once per context
 static int ensure_gen_table(sylow_b200_ctx* ctx, cudaStream_t s) {
@@ -1620,8 +1527,8 @@ static int verify_miller_values(sylow_b200_ctx* ctx, const uint8_t* d_pks, const
   uint8_t* d_hm = ctx->scratch2.p;
   uint8_t* d_hm_inf = d_hm + n * 64;
   CKS(hash_launch(ctx, d_msgs, d_offsets, n, dp, 1, d_hm, d_hm_inf, s));
-  return launch_glued<1, 1>(ctx, d_hm, 1, d_hm_inf, d_pks, d_pks_inf, d_sigs, 1, d_sigs_inf, ctx->d_gen_table, n,
-                            ctx->scratch0.p, s);
+  return launch_glued(ctx, 1, 1, d_hm, 1, d_hm_inf, d_pks, d_pks_inf, d_sigs, 1, d_sigs_inf, ctx->d_gen_table, n,
+                      ctx->scratch0.p, s);
 }
 
 // sum of n affine G1 points (wire format, optional infinity flags) -> one affine point + flag at d_out / d_out_inf
@@ -1694,7 +1601,7 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
     CKS(reserve(ctx, ctx->proj, n * 96));
     k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_hm, d_hm_inf, ws, first_index, n, ctx->proj.p);
     LAUNCHED(ctx);
-    CKS(g1_batch_affine(ctx, ctx->proj.p, n, 0, d_hm, d_hm_inf, s));
+    CKS(affine_tail(ctx, false, ctx->proj.p, n, 0, d_hm, d_hm_inf, s));
   }
   // The n Miller loops (-r_i H(m_i), pk_i) only ever meet as a product, so 1, 2 or 4 signatures share one thread
   // and ONE Fp12 squaring per loop digit - what glued_miller_loop does for the whole batch in the reference
@@ -1703,14 +1610,12 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
   // The glue is the one of fewest wave-times (glue_pairs).  Measured at 2^20 signatures
   // (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 / 163.3 ms for 1 / 2 / 4; at 2^13 the order reverses (9.3 / 12.4 /
   // 18.4 ms: a quarter of the threads, each four times as long).
-  const int glue = glue_pairs(ctx, n, 8444);
+  const int glue = glue_pairs(ctx->sms, n, 8444, kGluedShape);
   size_t n_f = n;  // Miller values in scratch0 before the signature pair's value is appended
   if (glue > 1 && n >= (size_t)glue) {
     const size_t items = n / glue, done = items * glue;
-    if (glue == 2)
-      CKS((launch_glued<2, 0>(ctx, d_hm, 2, d_hm_inf, d_pks, d_pks_inf, nullptr, 0, nullptr, nullptr, items, ctx->scratch0.p, s)));
-    else
-      CKS((launch_glued<4, 0>(ctx, d_hm, 4, d_hm_inf, d_pks, d_pks_inf, nullptr, 0, nullptr, nullptr, items, ctx->scratch0.p, s)));
+    CKS(launch_glued(ctx, glue, 0, d_hm, glue, d_hm_inf, d_pks, d_pks_inf, nullptr, 0, nullptr, nullptr, items,
+                     ctx->scratch0.p, s));
     if (done < n)
       CKS(launch_miller(ctx, d_hm + done * 64, d_hm_inf + done, d_pks + done * 128, d_pks_inf ? d_pks_inf + done : nullptr,
                         n - done, ctx->scratch0.p + items * 384, 1, s));
@@ -1726,8 +1631,8 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
   } else {
     CKS(g1_sum_reduce(ctx, d_sigs, d_sigs_inf, n, 0, d_sum, d_sum_inf, s));
   }
-  CKS((launch_glued<0, 1>(ctx, nullptr, 0, nullptr, nullptr, nullptr, d_sum, 1, d_sum_inf, ctx->d_gen_table, 1,
-                          ctx->scratch0.p + n_f * 384, s)));
+  CKS(launch_glued(ctx, 0, 1, nullptr, 0, nullptr, nullptr, nullptr, d_sum, 1, d_sum_inf, ctx->d_gen_table, 1,
+                   ctx->scratch0.p + n_f * 384, s));
   return product_reduce(ctx, ctx->scratch0.p, ctx->scratch1.p, n_f + 1, d_f_out, 0, s);
 }
 
@@ -1745,8 +1650,7 @@ int sylow_b200_verify_batch_partial_dev(sylow_b200_ctx* ctx, const uint8_t* d_pk
 // check (GroupError::CannotHashToGroup); synchronises the stream and clears the flag.
 int sylow_b200_hash_failed_dev(sylow_b200_ctx* ctx, void* stream, int* failed) {
   ENTER_DEV(ctx);
-  if (!ctx || !failed) return SYLOW_B200_ERR_ARG;
-  CK(cudaSetDevice(ctx->device));
+  if (!failed) return SYLOW_B200_ERR_ARG;
   cudaStream_t s = pick(ctx, stream);
   int f = 0;
   CK(cudaMemcpyAsync(&f, ctx->d_fail, sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -1866,9 +1770,18 @@ static int multi_slices(sylow_b200_ctx* ctx, size_t n, Fn fn) {
     if (r) return r;
   return 0;
 }
+// Product forms: fn(child, off, m, partial) writes the canonical product of its slice to `partial` (an empty slice
+// contributes 1), and the first device multiplies the G partials into f_out.
+template <class Fn>
+static int multi_product(sylow_b200_ctx* ctx, size_t n, Fn fn, uint8_t* f_out) {
+  const size_t G = ctx->children.size();
+  std::vector<uint8_t> part(G * 384, 0);
+  for (size_t g = 0; g < G; g++) part[g * 384] = 1;
+  uint8_t* pp = part.data();
+  CKS(multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t g, size_t off, size_t m) { return fn(c, off, m, pp + g * 384); }));
+  return sylow_b200_fp12_product(ctx->children[0], pp, G, f_out);
+}
 static inline bool is_multi(const sylow_b200_ctx* ctx) { return ctx && ctx->children.size() > 1; }
-static inline const uint8_t* adv(const uint8_t* p, size_t bytes) { return p ? p + bytes : nullptr; }
-static inline uint8_t* adv(uint8_t* p, size_t bytes) { return p ? p + bytes : nullptr; }
 // messages of the slice [off, off + m): the byte range and offsets rebased to 0
 struct MsgSlice {
   const uint8_t* msgs;
@@ -1908,17 +1821,10 @@ int sylow_b200_miller_loop_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const u
 
 int sylow_b200_miller_product(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                               const uint8_t* g2_inf, size_t n, uint8_t f_out[384]) {
-  if (is_multi(ctx) && g1 && g2 && f_out && n) {
-    const size_t G = ctx->children.size();
-    std::vector<uint8_t> part(G * 384, 0);
-    for (size_t g = 0; g < G; g++) part[g * 384] = 1;  // empty slices contribute 1
-    uint8_t* pp = part.data();
-    CKS(multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t g, size_t off, size_t m) {
-      return sylow_b200_miller_product(c, g1 + off * 64, adv(g1_inf, off), g2 + off * 128, adv(g2_inf, off), m,
-                                       pp + g * 384);
-    }));
-    return sylow_b200_fp12_product(ctx->children[0], pp, G, f_out);
-  }
+  if (is_multi(ctx) && g1 && g2 && f_out && n)
+    return multi_product(ctx, n, [=](sylow_b200_ctx* c, size_t off, size_t m, uint8_t* part) {
+      return sylow_b200_miller_product(c, g1 + off * 64, adv(g1_inf, off), g2 + off * 128, adv(g2_inf, off), m, part);
+    }, f_out);
   ENTER(ctx);
   if (!f_out || (n && (!g1 || !g2))) return SYLOW_B200_ERR_ARG;
   const uint8_t *d1, *d1i, *d2, *d2i;
@@ -2114,19 +2020,13 @@ int sylow_b200_verify_batch_partial(sylow_b200_ctx* ctx, const uint8_t* pks, con
                                     const uint64_t* offsets, const uint8_t* sigs, const uint8_t* sigs_inf, size_t n,
                                     const uint8_t* dst, size_t dst_len, int hash_id, const uint8_t* weight_seed,
                                     uint64_t first_index, uint8_t f_out[384]) {
-  if (is_multi(ctx) && offsets && pks && sigs && f_out && n) {
-    const size_t G = ctx->children.size();
-    std::vector<uint8_t> part(G * 384, 0);
-    for (size_t g = 0; g < G; g++) part[g * 384] = 1;
-    uint8_t* pp = part.data();
-    CKS(multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t g, size_t off, size_t m) {
+  if (is_multi(ctx) && offsets && pks && sigs && f_out && n)
+    return multi_product(ctx, n, [=](sylow_b200_ctx* c, size_t off, size_t m, uint8_t* part) {
       MsgSlice ms(msgs, offsets, off, m);
       return sylow_b200_verify_batch_partial(c, pks + off * 128, adv(pks_inf, off), ms.msgs, ms.offs.data(),
                                              sigs + off * 64, adv(sigs_inf, off), m, dst, dst_len, hash_id,
-                                             weight_seed, first_index + off, pp + g * 384);
-    }));
-    return sylow_b200_fp12_product(ctx->children[0], pp, G, f_out);
-  }
+                                             weight_seed, first_index + off, part);
+    }, f_out);
   ENTER(ctx);
   if (!f_out) return SYLOW_B200_ERR_ARG;
   DstPrime dp;
@@ -2250,8 +2150,8 @@ int sylow_b200_miller_loop_precomputed(sylow_b200_ctx* ctx, const uint8_t* coeff
   CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
   CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
   CKS(reserve(ctx, ctx->out, n * 384));
-  CKS((launch_glued<0, 1>(ctx, nullptr, 0, nullptr, nullptr, nullptr, d1, 1, d1i, ctx->tables.p, n, ctx->out.p,
-                          ctx->stream)));
+  CKS(launch_glued(ctx, 0, 1, nullptr, 0, nullptr, nullptr, nullptr, d1, 1, d1i, ctx->tables.p, n, ctx->out.p,
+                   ctx->stream));
   k_fp12_convert<<<nblocks(n, 128), 128, 0, ctx->stream>>>(ctx->out.p, n, ctx->out.p, 0);
   LAUNCHED(ctx);
   CK(cudaMemcpyAsync(f_out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2263,30 +2163,22 @@ int sylow_b200_pairing_check_fixed_batch_dev(sylow_b200_ctx* ctx, const uint8_t*
                                              const uint8_t* d_tables, size_t k_fixed, size_t n_checks,
                                              uint8_t* d_ok_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n_checks && (!d_g1 || !d_ok_out || !d_tables || (k_var && !d_g2_var)))) return SYLOW_B200_ERR_ARG;
+  if (n_checks && (!d_g1 || !d_ok_out || !d_tables || (k_var && !d_g2_var))) return SYLOW_B200_ERR_ARG;
   if (!n_checks) return 0;
   cudaStream_t s = pick(ctx, stream);
   size_t k = k_var + k_fixed;
   CKS(reserve(ctx, ctx->scratch0, n_checks * 384));
   const uint8_t* g1f = d_g1 + k_var * 64;
   const uint8_t* g1f_inf = d_g1_inf ? d_g1_inf + k_var : nullptr;
-  int st;
-  if (k_var == 1 && k_fixed == 1)
-    st = launch_glued<1, 1>(ctx, d_g1, k, d_g1_inf, d_g2_var, d_g2_var_inf, g1f, k, g1f_inf, d_tables, n_checks, ctx->scratch0.p, s);
-  else if (k_var == 1 && k_fixed == 3)
-    st = launch_glued<1, 3>(ctx, d_g1, k, d_g1_inf, d_g2_var, d_g2_var_inf, g1f, k, g1f_inf, d_tables, n_checks, ctx->scratch0.p, s);
-  else if (k_var == 0 && k_fixed == 1)
-    st = launch_glued<0, 1>(ctx, d_g1, k, d_g1_inf, d_g2_var, d_g2_var_inf, g1f, k, g1f_inf, d_tables, n_checks, ctx->scratch0.p, s);
-  else
-    return SYLOW_B200_ERR_ARG;  // other shapes: use sylow_b200_pairing_check_batch
-  CKS(st);
+  if (!k_fixed) return SYLOW_B200_ERR_ARG;  // other shapes: use sylow_b200_pairing_check_batch
+  CKS(launch_glued(ctx, k_var, k_fixed, d_g1, k, d_g1_inf, d_g2_var, d_g2_var_inf, g1f, k, g1f_inf, d_tables, n_checks,
+                   ctx->scratch0.p, s));
   return launch_check_products(ctx, ctx->scratch0.p, 1, n_checks, d_ok_out, s);
 }
 
 int sylow_b200_tables_to_device(sylow_b200_ctx* ctx, const uint8_t* coeffs, size_t k, uint8_t* d_tables_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || !coeffs || !d_tables_out || !k) return SYLOW_B200_ERR_ARG;
-  CK(cudaSetDevice(ctx->device));
+  if (!coeffs || !d_tables_out || !k) return SYLOW_B200_ERR_ARG;
   CKS(tables_to_dev(ctx, coeffs, k));
   CK(cudaStreamSynchronize(ctx->stream));
   CK(cudaMemcpyAsync(d_tables_out, ctx->tables.p, k * SY_TABLE_BYTES, cudaMemcpyDeviceToDevice, pick(ctx, stream)));
@@ -2299,7 +2191,7 @@ int sylow_b200_pairing_check_fixed_batch(sylow_b200_ctx* ctx, const uint8_t* g1,
                                          const uint8_t* coeffs_fixed, size_t k_fixed, size_t n_checks, uint8_t* ok_out) {
   ENTER(ctx);
   if (n_checks && (!g1 || !ok_out || !coeffs_fixed || (k_var && !g2_var))) return SYLOW_B200_ERR_ARG;
-  if (!((k_var == 1 && (k_fixed == 1 || k_fixed == 3)) || (k_var == 0 && k_fixed == 1))) return SYLOW_B200_ERR_ARG;
+  if (!k_fixed || !glued_shape_ok(k_var, k_fixed)) return SYLOW_B200_ERR_ARG;
   if (!n_checks) return 0;
   size_t k = k_var + k_fixed;
   const uint8_t *d1, *d1i, *d2, *d2i;
@@ -2315,27 +2207,11 @@ int sylow_b200_pairing_check_fixed_batch(sylow_b200_ctx* ctx, const uint8_t* g1,
   return finish(ctx);
 }
 
-// n_items items of m pairs each (k_miller_tables<m>) -> f_out, one Fp12 per item
-static int launch_miller_tables(sylow_b200_ctx* ctx, int m, const uint8_t* tables, size_t n_tables, const uint32_t* idx,
-                                const uint8_t* g1, const uint8_t* g1_inf, size_t n_items, uint8_t* f_out, int raw_out,
-                                cudaStream_t s) {
-  const unsigned blocks = nblocks(n_items, SY_GLUED_THREADS);
-  const size_t smem = SY_MILLER_SMEM_BYTES(SY_GLUED_THREADS);
-  if (m == 4)
-    k_miller_tables<4><<<blocks, SY_GLUED_THREADS, smem, s>>>(tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
-  else if (m == 2)
-    k_miller_tables<2><<<blocks, SY_GLUED_THREADS, smem, s>>>(tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
-  else
-    k_miller_tables<1><<<blocks, SY_GLUED_THREADS, smem, s>>>(tables, n_tables, idx, g1, g1_inf, n_items, f_out, raw_out);
-  LAUNCHED(ctx);
-  return 0;
-}
-
 // d_out (canonical) = prod over n >= 1 pairs of the Miller loop of g1[k] against table idx[k] (k if idx is null):
 // glue_pairs' choice of pairs per thread, the n % glue leftover pairs one per thread, then product_reduce.
 static int miller_product_tables(sylow_b200_ctx* ctx, const uint8_t* tables, size_t n_tables, const uint32_t* idx,
                                  const uint8_t* g1, const uint8_t* g1_inf, size_t n, uint8_t* d_out, cudaStream_t s) {
-  const int glue = glue_pairs(ctx, n, 6045);
+  const int glue = glue_pairs(ctx->sms, n, 6045, kGluedShape);
   const size_t items = n / glue, done = items * glue;
   CKS(reserve(ctx, ctx->scratch0, n * 384));
   CKS(reserve(ctx, ctx->scratch1, (n / 4 + 1) * 384));
@@ -2371,17 +2247,11 @@ int sylow_b200_miller_loop_precomputed_batch(sylow_b200_ctx* ctx, const uint8_t*
 
 int sylow_b200_miller_product_precomputed(sylow_b200_ctx* ctx, const uint8_t* coeffs, const uint8_t* g1,
                                           const uint8_t* g1_inf, size_t n, uint8_t f_out[384]) {
-  if (is_multi(ctx) && coeffs && g1 && f_out && n) {
-    const size_t G = ctx->children.size();
-    std::vector<uint8_t> part(G * 384, 0);
-    for (size_t g = 0; g < G; g++) part[g * 384] = 1;  // empty slices contribute 1
-    uint8_t* pp = part.data();
-    CKS(multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t g, size_t off, size_t m) {
+  if (is_multi(ctx) && coeffs && g1 && f_out && n)
+    return multi_product(ctx, n, [=](sylow_b200_ctx* c, size_t off, size_t m, uint8_t* part) {
       return sylow_b200_miller_product_precomputed(c, coeffs + off * SY_TABLE_BYTES, g1 + off * 64, adv(g1_inf, off), m,
-                                                   pp + g * 384);
-    }));
-    return sylow_b200_fp12_product(ctx->children[0], pp, G, f_out);
-  }
+                                                   part);
+    }, f_out);
   ENTER(ctx);
   if (!f_out || (n && (!coeffs || !g1))) return SYLOW_B200_ERR_ARG;
   if (!n) {
@@ -2401,9 +2271,8 @@ int sylow_b200_miller_product_precomputed(sylow_b200_ctx* ctx, const uint8_t* co
 int sylow_b200_g2_precompute_dev(sylow_b200_ctx* ctx, const uint8_t* d_g2, size_t n, uint8_t* d_tables_out,
                                  void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || (n && (!d_g2 || !d_tables_out))) return SYLOW_B200_ERR_ARG;
+  if (n && (!d_g2 || !d_tables_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  CK(cudaSetDevice(ctx->device));
   k_g2_precompute<<<nblocks(n, SY_GLUED_THREADS), SY_GLUED_THREADS, 0, pick(ctx, stream)>>>(d_g2, n, d_tables_out, 1);
   LAUNCHED(ctx);
   return 0;
@@ -2413,9 +2282,8 @@ int sylow_b200_miller_product_precomputed_dev(sylow_b200_ctx* ctx, const uint8_t
                                               const uint32_t* d_table_idx, const uint8_t* d_g1, const uint8_t* d_g1_inf,
                                               size_t n, uint8_t* d_f_out, void* stream) {
   ENTER_DEV(ctx);
-  if (!ctx || !d_f_out || (n && (!d_tables || !d_g1 || !n_tables || (!d_table_idx && n > n_tables))))
+  if (!d_f_out || (n && (!d_tables || !d_g1 || !n_tables || (!d_table_idx && n > n_tables))))
     return SYLOW_B200_ERR_ARG;
-  CK(cudaSetDevice(ctx->device));
   cudaStream_t s = pick(ctx, stream);
   if (!n) {
     CK(cudaMemcpyAsync(d_f_out, kOneCanonical, 384, cudaMemcpyHostToDevice, s));
@@ -2889,14 +2757,19 @@ int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int thre
   if (!ms_out || !ops_out || blocks <= 0 || threads <= 0 || threads > 1024 || iters <= 0) return SYLOW_B200_ERR_ARG;
   CKS(reserve(ctx, ctx->out, 256));
   CK(cudaMemsetAsync(ctx->out.p, 0x5a, 256, ctx->stream));
-  cudaEvent_t e0, e1;
-  CK(cudaEventCreate(&e0));
-  CK(cudaEventCreate(&e1));
+  struct Event {
+    cudaEvent_t e = nullptr;
+    ~Event() {
+      if (e) cudaEventDestroy(e);
+    }
+  } e0, e1;  // released on every return
+  CK(cudaEventCreate(&e0.e));
+  CK(cudaEventCreate(&e1.e));
   const uint32_t* src = reinterpret_cast<const uint32_t*>(ctx->out.p);
   uint32_t* sink = reinterpret_cast<uint32_t*>(ctx->out.p) + 32;
   double per_thread_iter = 0;
   for (int rep = 0; rep < 2; rep++) {  // the first pass warms up
-    CK(cudaEventRecord(e0, ctx->stream));
+    CK(cudaEventRecord(e0.e, ctx->stream));
     switch (variant) {
       case 0: k_imad_probe<1><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 1; break;
       case 1: k_imad_probe<2><<<blocks, threads, 0, ctx->stream>>>(iters, src, sink); per_thread_iter = 2; break;
@@ -2908,13 +2781,11 @@ int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int thre
       default: return SYLOW_B200_ERR_ARG;
     }
     LAUNCHED(ctx);
-    CK(cudaEventRecord(e1, ctx->stream));
-    CK(cudaEventSynchronize(e1));
+    CK(cudaEventRecord(e1.e, ctx->stream));
+    CK(cudaEventSynchronize(e1.e));
   }
-  CK(cudaEventElapsedTime(ms_out, e0, e1));
+  CK(cudaEventElapsedTime(ms_out, e0.e, e1.e));
   *ops_out = (double)blocks * threads * (double)iters * per_thread_iter;
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
   return 0;
 }
 

@@ -34,7 +34,7 @@ def power_limit() -> str:
 
 
 def glue(n: int, sms: int, pair_cost: int) -> int:
-    """Pairs per thread the library picks (glue_pairs in sylow_b200/csrc/sylow_b200.cu), for the report."""
+    """Pairs per thread the library picks (glue_pairs in sylow_b200/csrc/launch_plan.h), for the report."""
     wave, save = sms * 256, 63 * 36
     best, g_best = None, 1
     for g, c in ((1, pair_cost), (2, 2 * pair_cost - save), (4, 4 * pair_cost - 3 * save)):
