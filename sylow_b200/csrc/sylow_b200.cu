@@ -979,7 +979,8 @@ struct sylow_b200_ctx {
   int sms = 148;
   int last_cuda = 0;
   uint64_t launches = 0;
-  DevBuf in_a, in_b, in_c, in_d, flag_a, flag_b, out, scratch0, scratch1, scratch2;
+  DevBuf stage[7];  // staging slots of the host-pointer calls (Staging); seven is the most one call takes
+  DevBuf scratch0, scratch1, scratch2;
   int* d_fail = nullptr;
   uint8_t* d_gen_table = nullptr;  // G2PreComputed of the G2 generator, Montgomery form (16704 B)
   DevBuf tables, sum0, sum1, proj, msm;
@@ -1041,6 +1042,52 @@ static int reserve(sylow_b200_ctx* ctx, DevBuf& b, size_t bytes) {
   b.cap = cap;
   return 0;
 }
+
+// Staging of one host-pointer call: the context's staging slots, handed out in the order they are asked for, so two
+// areas of one call never overlap (and no host form calls another while its staging is live).  `_dev` forms and the
+// static helpers they call never touch the staging slots: that is what lets a host form's staged inputs survive the
+// device form it calls.  A slot keeps the largest area ever asked of it, so calls ask for their large areas first.
+// The first error sticks (later requests give null and queue nothing) and finish() returns it.  A call that returns
+// without finishing waits for ctx->stream and ctx->copy_in in the destructor: whatever the status, no copy from or into
+// caller memory runs on after a host entry point returns.
+namespace {
+struct Staging {
+  sylow_b200_ctx* const ctx;
+  int err = 0, used = 0;
+  bool finished = false;
+  explicit Staging(sylow_b200_ctx* c) : ctx(c) {}
+  ~Staging() {
+    if (finished) return;
+    cudaStreamSynchronize(ctx->stream);
+    cudaStreamSynchronize(ctx->copy_in);
+  }
+  // a device-only area for outputs and intermediates; null, and no slot, for 0 bytes; ERR_NOMEM past the last slot
+  uint8_t* area(size_t bytes) {
+    if (err || !bytes) return nullptr;
+    err = used < (int)std::size(ctx->stage) ? reserve(ctx, ctx->stage[used], bytes) : SYLOW_B200_ERR_NOMEM;
+    return err ? nullptr : ctx->stage[used++].p;
+  }
+  // a device copy of `bytes` of host memory at h, queued on ctx->stream; null for a null h or 0 bytes
+  const uint8_t* up(const void* h, size_t bytes) {
+    uint8_t* d = area(h ? bytes : 0);
+    if (d) check(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    return err ? nullptr : d;
+  }
+  // queues the copy of `bytes` at device address d back to host memory at h
+  void down(void* h, const void* d, size_t bytes) {
+    if (!err) check(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  // waits for ctx->stream; the first error of the call, or 0
+  int finish() {
+    if (!err) check(cudaStreamSynchronize(ctx->stream));
+    finished = !err;
+    return err;
+  }
+  void check(cudaError_t e) {
+    if (e != cudaSuccess) err = fail_cuda(ctx, e);
+  }
+};
+}  // namespace
 
 static constexpr size_t sy_gcd(size_t a, size_t b) { return b ? sy_gcd(b, a % b) : a; }
 static constexpr size_t sy_lcm(size_t a, size_t b) { return a / sy_gcd(a, b) * b; }
@@ -1661,32 +1708,16 @@ int sylow_b200_hash_failed_dev(sylow_b200_ctx* ctx, void* stream, int* failed) {
 }
 
 // ------------------------------------------------------------------------------- host variants
-static int to_dev(sylow_b200_ctx* ctx, DevBuf& b, const void* h, size_t bytes, const uint8_t** d) {
-  *d = nullptr;
-  if (!h || !bytes) return 0;
-  CKS(reserve(ctx, b, bytes));
-  CK(cudaMemcpyAsync(b.p, h, bytes, cudaMemcpyHostToDevice, ctx->stream));
-  *d = b.p;
-  return 0;
-}
-static int finish(sylow_b200_ctx* ctx) {
-  CK(cudaStreamSynchronize(ctx->stream));
-  return 0;
-}
-
-
 // Host-pointer pairing / Miller-loop batch.  Large batches are cut into chunks of whole waves of both kernels (SMs x
 // 1536 pairs: six Miller-loop waves, four final-exponentiation waves) and pipelined over three streams: the
 // host->device copy of chunk c+1 and the device->host copy of chunk c-1 run under the kernels of chunk c, so the
 // PCIe time of the 576 bytes per pairing disappears from the call.
 static int pairing_host(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                         const uint8_t* g2_inf, size_t n, uint8_t* out, bool final_exp) {
-  const uint8_t *d1i, *d2i;
-  CKS(reserve(ctx, ctx->in_a, n * 64));
-  CKS(reserve(ctx, ctx->in_b, n * 128));
-  CKS(reserve(ctx, ctx->out, n * 384));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(to_dev(ctx, ctx->flag_b, g2_inf, n, &d2i));
+  Staging io(ctx);
+  uint8_t *d_out = io.area(n * 384), *d2 = io.area(n * 128), *d1 = io.area(n * 64);
+  const uint8_t *d1i = io.up(g1_inf, n), *d2i = io.up(g2_inf, n);
+  CKS(io.err);
   if (d1i || d2i) CK(cudaStreamSynchronize(ctx->stream));  // the flags are read from both compute streams
   // whole waves of both kernels: a multiple of the threads each of them keeps resident per SM
   const size_t chunk =
@@ -1701,25 +1732,22 @@ static int pairing_host(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g
     size_t off = c * step, m = off + step < n ? step : n - off;
     cudaError_t r = cudaStreamWaitEvent(ctx->copy_out, ev[2 * c + 1], 0);
     if (r == cudaSuccess)
-      r = cudaMemcpyAsync(out + off * 384, ctx->out.p + off * 384, m * 384, cudaMemcpyDeviceToHost, ctx->copy_out);
+      r = cudaMemcpyAsync(out + off * 384, d_out + off * 384, m * 384, cudaMemcpyDeviceToHost, ctx->copy_out);
     return r;
   };
   for (size_t c = 0; c < n_chunks && e == cudaSuccess && rc == 0; c++) {
     size_t off = c * step, m = off + step < n ? step : n - off;
-    e = cudaMemcpyAsync(ctx->in_a.p + off * 64, g1 + off * 64, m * 64, cudaMemcpyHostToDevice, ctx->copy_in);
-    if (e == cudaSuccess)
-      e = cudaMemcpyAsync(ctx->in_b.p + off * 128, g2 + off * 128, m * 128, cudaMemcpyHostToDevice, ctx->copy_in);
+    e = cudaMemcpyAsync(d1 + off * 64, g1 + off * 64, m * 64, cudaMemcpyHostToDevice, ctx->copy_in);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d2 + off * 128, g2 + off * 128, m * 128, cudaMemcpyHostToDevice, ctx->copy_in);
     if (e == cudaSuccess) e = cudaEventRecord(ev[2 * c], ctx->copy_in);
     cudaStream_t cs = (c & 1) ? ctx->stream2 : ctx->stream;
     if (e == cudaSuccess) e = cudaStreamWaitEvent(cs, ev[2 * c], 0);
     if (e != cudaSuccess) break;
-    const uint8_t* f1 = d1i ? d1i + off : nullptr;
-    const uint8_t* f2 = d2i ? d2i + off : nullptr;
-    uint8_t* o = ctx->out.p + off * 384;
+    uint8_t* o = d_out + off * 384;
     if (final_exp)
-      rc = pairing_dev_single(ctx, ctx->in_a.p + off * 64, f1, ctx->in_b.p + off * 128, f2, m, o, cs);
+      rc = pairing_dev_single(ctx, d1 + off * 64, adv(d1i, off), d2 + off * 128, adv(d2i, off), m, o, cs);
     else
-      rc = sylow_b200_miller_loop_batch_dev(ctx, ctx->in_a.p + off * 64, f1, ctx->in_b.p + off * 128, f2, m, o, cs);
+      rc = sylow_b200_miller_loop_batch_dev(ctx, d1 + off * 64, adv(d1i, off), d2 + off * 128, adv(d2i, off), m, o, cs);
     if (rc) break;
     e = cudaEventRecord(ev[2 * c + 1], cs);
     // the device->host copy of the PREVIOUS chunk is issued after this chunk's kernels are queued: with pageable
@@ -1739,7 +1767,7 @@ static int pairing_host(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g
   if (e == cudaSuccess) e = e4;
   if (e == cudaSuccess) e = e5;
   if (e != cudaSuccess) return fail_cuda(ctx, e);
-  return 0;
+  return io.finish();
 }
 
 }  // extern "C" (templates need C++ linkage)
@@ -1827,15 +1855,13 @@ int sylow_b200_miller_product(sylow_b200_ctx* ctx, const uint8_t* g1, const uint
     }, f_out);
   ENTER(ctx);
   if (!f_out || (n && (!g1 || !g2))) return SYLOW_B200_ERR_ARG;
-  const uint8_t *d1, *d1i, *d2, *d2i;
-  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(to_dev(ctx, ctx->in_b, g2, n * 128, &d2));
-  CKS(to_dev(ctx, ctx->flag_b, g2_inf, n, &d2i));
-  CKS(reserve(ctx, ctx->out, 384));
-  CKS(sylow_b200_miller_product_dev(ctx, d1, d1i, d2, d2i, n, ctx->out.p, nullptr));
-  CK(cudaMemcpyAsync(f_out, ctx->out.p, 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  const uint8_t *d2 = io.up(g2, n * 128), *d1 = io.up(g1, n * 64), *d1i = io.up(g1_inf, n), *d2i = io.up(g2_inf, n);
+  uint8_t* d_f = io.area(384);
+  CKS(io.err);
+  CKS(sylow_b200_miller_product_dev(ctx, d1, d1i, d2, d2i, n, d_f, nullptr));
+  io.down(f_out, d_f, 384);
+  return io.finish();
 }
 
 int sylow_b200_final_exp_batch(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, uint8_t* gt_out) {
@@ -1846,12 +1872,13 @@ int sylow_b200_final_exp_batch(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, 
   ENTER(ctx);
   if (n && (!f || !gt_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t* df;
-  CKS(to_dev(ctx, ctx->in_a, f, n * 384, &df));
-  CKS(reserve(ctx, ctx->out, n * 384));
-  CKS(sylow_b200_final_exp_batch_dev(ctx, df, n, ctx->out.p, nullptr));
-  CK(cudaMemcpyAsync(gt_out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  const uint8_t* df = io.up(f, n * 384);
+  uint8_t* d_gt = io.area(n * 384);
+  CKS(io.err);
+  CKS(sylow_b200_final_exp_batch_dev(ctx, df, n, d_gt, nullptr));
+  io.down(gt_out, d_gt, n * 384);
+  return io.finish();
 }
 
 int sylow_b200_fp12_product(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, uint8_t out[384]) {
@@ -1861,16 +1888,17 @@ int sylow_b200_fp12_product(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, uin
     memcpy(out, kOneCanonical, 384);
     return 0;
   }
-  const uint8_t* df;
-  CKS(to_dev(ctx, ctx->in_a, f, n * 384, &df));
+  Staging io(ctx);
+  const uint8_t* df = io.up(f, n * 384);
+  uint8_t* d_prod = io.area(384);
+  CKS(io.err);
   CKS(reserve(ctx, ctx->scratch0, n * 384));
   CKS(reserve(ctx, ctx->scratch1, (n / 4 + 1) * 384));
-  CKS(reserve(ctx, ctx->out, 384));
   k_fp12_convert<<<nblocks(n, 128), 128, 0, ctx->stream>>>(df, n, ctx->scratch0.p, 1);
   LAUNCHED(ctx);
-  CKS(product_reduce(ctx, ctx->scratch0.p, ctx->scratch1.p, n, ctx->out.p, 0, ctx->stream));
-  CK(cudaMemcpyAsync(out, ctx->out.p, 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  CKS(product_reduce(ctx, ctx->scratch0.p, ctx->scratch1.p, n, d_prod, 0, ctx->stream));
+  io.down(out, d_prod, 384);
+  return io.finish();
 }
 
 int sylow_b200_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
@@ -1885,15 +1913,13 @@ int sylow_b200_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const
   if (!n_checks) return 0;
   size_t n = k * n_checks;
   if (n && (!g1 || !g2)) return SYLOW_B200_ERR_ARG;
-  const uint8_t *d1, *d1i, *d2, *d2i;
-  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(to_dev(ctx, ctx->in_b, g2, n * 128, &d2));
-  CKS(to_dev(ctx, ctx->flag_b, g2_inf, n, &d2i));
-  CKS(reserve(ctx, ctx->out, n_checks));
-  CKS(sylow_b200_pairing_check_batch_dev(ctx, d1, d1i, d2, d2i, k, n_checks, ctx->out.p, nullptr));
-  CK(cudaMemcpyAsync(ok_out, ctx->out.p, n_checks, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  const uint8_t *d2 = io.up(g2, n * 128), *d1 = io.up(g1, n * 64), *d1i = io.up(g1_inf, n), *d2i = io.up(g2_inf, n);
+  uint8_t* d_ok = io.area(n_checks);
+  CKS(io.err);
+  CKS(sylow_b200_pairing_check_batch_dev(ctx, d1, d1i, d2, d2i, k, n_checks, d_ok, nullptr));
+  io.down(ok_out, d_ok, n_checks);
+  return io.finish();
 }
 
 static int mul_host(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
@@ -1908,19 +1934,18 @@ static int mul_host(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8
   if (n && (!pts || !scalars || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   size_t pb = g2 ? 128 : 64;
-  const uint8_t *dp, *dpi, *dk;
-  CKS(to_dev(ctx, ctx->in_a, pts, n * pb, &dp));
-  CKS(to_dev(ctx, ctx->flag_a, pts_inf, n, &dpi));
-  CKS(to_dev(ctx, ctx->in_b, scalars, n * 32, &dk));
-  CKS(reserve(ctx, ctx->out, n * pb));
-  CKS(reserve(ctx, ctx->flag_b, n));
+  Staging io(ctx);
+  uint8_t* d_out = io.area(n * pb);
+  const uint8_t *dp = io.up(pts, n * pb), *dk = io.up(scalars, n * 32), *dpi = io.up(pts_inf, n);
+  uint8_t* d_out_inf = io.area(n);
+  CKS(io.err);
   if (g2)
-    CKS(sylow_b200_g2_mul_batch_dev(ctx, dp, dpi, dk, n, ctx->out.p, ctx->flag_b.p, nullptr));
+    CKS(sylow_b200_g2_mul_batch_dev(ctx, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
   else
-    CKS(sylow_b200_g1_mul_batch_dev(ctx, dp, dpi, dk, n, ctx->out.p, ctx->flag_b.p, nullptr));
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * pb, cudaMemcpyDeviceToHost, ctx->stream));
-  if (out_inf) CK(cudaMemcpyAsync(out_inf, ctx->flag_b.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+    CKS(sylow_b200_g1_mul_batch_dev(ctx, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
+  io.down(out, d_out, n * pb);
+  if (out_inf) io.down(out_inf, d_out_inf, n);
+  return io.finish();
 }
 int sylow_b200_g1_mul_batch(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
                             size_t n, uint8_t* out, uint8_t* out_inf) {
@@ -1931,10 +1956,12 @@ int sylow_b200_g2_mul_batch(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8
   return mul_host(ctx, 1, pts, pts_inf, scalars, n, out, out_inf);
 }
 
-static int check_hash_fail(sylow_b200_ctx* ctx) {
+// the end of a hashing host form: finishes with the hash-to-curve failure flag, then CannotHashToGroup if it is set
+static int check_hash_fail(Staging& io) {
+  sylow_b200_ctx* ctx = io.ctx;
   int f = 0;
-  CK(cudaMemcpyAsync(&f, ctx->d_fail, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
+  io.down(&f, ctx->d_fail, sizeof(int));
+  CKS(io.finish());
   if (f) {
     CK(cudaMemsetAsync(ctx->d_fail, 0, sizeof(int), ctx->stream));
     return SYLOW_B200_ERR_CANNOT_HASH;
@@ -1942,25 +1969,21 @@ static int check_hash_fail(sylow_b200_ctx* ctx) {
   return 0;
 }
 
-static int msgs_to_dev(sylow_b200_ctx* ctx, const uint8_t* msgs, const uint64_t* offsets, size_t n,
-                       const uint8_t** d_msgs, const uint64_t** d_off) {
-  if (!offsets) return SYLOW_B200_ERR_ARG;
-  if (offsets[0] != 0) return SYLOW_B200_ERR_ARG;
-  for (size_t i = 0; i < n; i++)
-    if (offsets[i + 1] < offsets[i]) return SYLOW_B200_ERR_ARG;
-  size_t total = (size_t)offsets[n];
-  if (total && !msgs) return SYLOW_B200_ERR_ARG;
-  const uint8_t* dm;
-  const uint8_t* dof;
-  CKS(to_dev(ctx, ctx->in_c, msgs, total, &dm));
-  if (!dm) {  // all messages empty: still need a valid pointer
-    CKS(reserve(ctx, ctx->in_c, 16));
-    dm = ctx->in_c.p;
+// n messages and their offsets, staged; malformed offsets or a missing message buffer fail the call with ERR_ARG
+struct DevMsgs {
+  const uint8_t* msgs;
+  const uint64_t* offsets;
+};
+static DevMsgs msgs_to_dev(Staging& io, const uint8_t* msgs, const uint64_t* offsets, size_t n) {
+  bool ok = offsets && offsets[0] == 0;
+  for (size_t i = 0; ok && i < n; i++) ok = offsets[i + 1] >= offsets[i];
+  const size_t total = ok ? (size_t)offsets[n] : 0;
+  if (!ok || (total && !msgs)) {
+    if (!io.err) io.err = SYLOW_B200_ERR_ARG;
+    return {};
   }
-  CKS(to_dev(ctx, ctx->in_d, offsets, (n + 1) * sizeof(uint64_t), &dof));
-  *d_msgs = dm;
-  *d_off = reinterpret_cast<const uint64_t*>(dof);
-  return 0;
+  const uint8_t* dm = total ? io.up(msgs, total) : io.area(16);  // all messages empty: still a valid pointer
+  return {dm, reinterpret_cast<const uint64_t*>(io.up(offsets, (n + 1) * sizeof(uint64_t)))};
 }
 
 int sylow_b200_hash_to_g1_batch(sylow_b200_ctx* ctx, const uint8_t* msgs, const uint64_t* offsets, size_t n,
@@ -1976,15 +1999,15 @@ int sylow_b200_hash_to_g1_batch(sylow_b200_ctx* ctx, const uint8_t* msgs, const 
   CKS(make_dst_prime(ctx, dst, dst_len, hash_id, dp));
   if (!n) return 0;
   if (!out) return SYLOW_B200_ERR_ARG;
-  const uint8_t* dm;
-  const uint64_t* dof;
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(reserve(ctx, ctx->out, n * 64));
-  CKS(reserve(ctx, ctx->flag_b, n));
-  CKS(hash_launch(ctx, dm, dof, n, dp, 0, ctx->out.p, ctx->flag_b.p, ctx->stream));
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 64, cudaMemcpyDeviceToHost, ctx->stream));
-  if (out_inf) CK(cudaMemcpyAsync(out_inf, ctx->flag_b.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return check_hash_fail(ctx);
+  Staging io(ctx);
+  uint8_t* d_out = io.area(n * 64);
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  uint8_t* d_out_inf = io.area(n);
+  CKS(io.err);
+  CKS(hash_launch(ctx, m.msgs, m.offsets, n, dp, 0, d_out, d_out_inf, ctx->stream));
+  io.down(out, d_out, n * 64);
+  if (out_inf) io.down(out_inf, d_out_inf, n);
+  return check_hash_fail(io);
 }
 
 int sylow_b200_sign_batch(sylow_b200_ctx* ctx, const uint8_t* sks, const uint8_t* msgs, const uint64_t* offsets,
@@ -2001,19 +2024,17 @@ int sylow_b200_sign_batch(sylow_b200_ctx* ctx, const uint8_t* sks, const uint8_t
   CKS(make_dst_prime(ctx, dst, dst_len, hash_id, dp));
   if (!n) return 0;
   if (!sks || !sigs_out) return SYLOW_B200_ERR_ARG;
-  const uint8_t *dm, *dk;
-  const uint64_t* dof;
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(to_dev(ctx, ctx->in_b, sks, n * 32, &dk));
-  CKS(reserve(ctx, ctx->scratch2, n * 65));
-  CKS(reserve(ctx, ctx->out, n * 64));
-  CKS(reserve(ctx, ctx->flag_b, n));
-  CKS(hash_launch(ctx, dm, dof, n, dp, 0, ctx->scratch2.p, ctx->scratch2.p + n * 64, ctx->stream));
-  CKS(sylow_b200_g1_mul_batch_dev(ctx, ctx->scratch2.p, ctx->scratch2.p + n * 64, dk, n, ctx->out.p, ctx->flag_b.p,
-                                  nullptr));
-  CK(cudaMemcpyAsync(sigs_out, ctx->out.p, n * 64, cudaMemcpyDeviceToHost, ctx->stream));
-  if (sigs_out_inf) CK(cudaMemcpyAsync(sigs_out_inf, ctx->flag_b.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return check_hash_fail(ctx);
+  Staging io(ctx);
+  uint8_t *d_hm = io.area(n * 65), *d_sig = io.area(n * 64);  // H(m_i), then their flags; the signatures
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  const uint8_t* dk = io.up(sks, n * 32);
+  uint8_t* d_sig_inf = io.area(n);
+  CKS(io.err);
+  CKS(hash_launch(ctx, m.msgs, m.offsets, n, dp, 0, d_hm, d_hm + n * 64, ctx->stream));
+  CKS(sylow_b200_g1_mul_batch_dev(ctx, d_hm, d_hm + n * 64, dk, n, d_sig, d_sig_inf, nullptr));
+  io.down(sigs_out, d_sig, n * 64);
+  if (sigs_out_inf) io.down(sigs_out_inf, d_sig_inf, n);
+  return check_hash_fail(io);
 }
 
 int sylow_b200_verify_batch_partial(sylow_b200_ctx* ctx, const uint8_t* pks, const uint8_t* pks_inf, const uint8_t* msgs,
@@ -2036,35 +2057,22 @@ int sylow_b200_verify_batch_partial(sylow_b200_ctx* ctx, const uint8_t* pks, con
     return 0;
   }
   if (!pks || !sigs) return SYLOW_B200_ERR_ARG;
-  const uint8_t *dm, *dpk, *dsg, *dpki, *dsgi;
-  const uint64_t* dof;
+  Staging io(ctx);
+  uint8_t *dpk = io.area(n * 128), *dsg = io.area(n * 64);
   // messages first, on the compute stream: the hash-to-curve kernel starts as soon as they are there, while the keys
   // and signatures (six times the bytes) still travel on the copy stream
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(reserve(ctx, ctx->in_a, n * 128));
-  CKS(reserve(ctx, ctx->in_b, n * 64));
-  if (pks_inf) CKS(reserve(ctx, ctx->flag_a, n));
-  if (sigs_inf) CKS(reserve(ctx, ctx->flag_b, n));
-  CKS(reserve(ctx, ctx->out, 384));
-  dpk = ctx->in_a.p;
-  dsg = ctx->in_b.p;
-  dpki = pks_inf ? ctx->flag_a.p : nullptr;
-  dsgi = sigs_inf ? ctx->flag_b.p : nullptr;
-  cudaError_t e = cudaMemcpyAsync(ctx->in_a.p, pks, n * 128, cudaMemcpyHostToDevice, ctx->copy_in);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->in_b.p, sigs, n * 64, cudaMemcpyHostToDevice, ctx->copy_in);
-  if (e == cudaSuccess && pks_inf) e = cudaMemcpyAsync(ctx->flag_a.p, pks_inf, n, cudaMemcpyHostToDevice, ctx->copy_in);
-  if (e == cudaSuccess && sigs_inf) e = cudaMemcpyAsync(ctx->flag_b.p, sigs_inf, n, cudaMemcpyHostToDevice, ctx->copy_in);
-  if (e == cudaSuccess) e = cudaEventRecord(ctx->ev_fork, ctx->copy_in);
-  int st_core = e == cudaSuccess ? verify_partial_core(ctx, dpk, dpki, dm, dof, dsg, dsgi, n, dst, dst_len, hash_id,
-                                                       weight_seed, first_index, ctx->out.p, nullptr, ctx->ev_fork)
-                                 : fail_cuda(ctx, e);
-  if (st_core) {
-    cudaStreamSynchronize(ctx->copy_in);  // the caller's buffers must not be in flight when we return
-    cudaStreamSynchronize(ctx->stream);
-    return st_core;
-  }
-  CK(cudaMemcpyAsync(f_out, ctx->out.p, 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return check_hash_fail(ctx);
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  uint8_t *dpki = io.area(pks_inf ? n : 0), *dsgi = io.area(sigs_inf ? n : 0), *d_f = io.area(384);
+  CKS(io.err);
+  CK(cudaMemcpyAsync(dpk, pks, n * 128, cudaMemcpyHostToDevice, ctx->copy_in));
+  CK(cudaMemcpyAsync(dsg, sigs, n * 64, cudaMemcpyHostToDevice, ctx->copy_in));
+  if (pks_inf) CK(cudaMemcpyAsync(dpki, pks_inf, n, cudaMemcpyHostToDevice, ctx->copy_in));
+  if (sigs_inf) CK(cudaMemcpyAsync(dsgi, sigs_inf, n, cudaMemcpyHostToDevice, ctx->copy_in));
+  CK(cudaEventRecord(ctx->ev_fork, ctx->copy_in));
+  CKS(verify_partial_core(ctx, dpk, dpki, m.msgs, m.offsets, dsg, dsgi, n, dst, dst_len, hash_id, weight_seed,
+                          first_index, d_f, nullptr, ctx->ev_fork));
+  io.down(f_out, d_f, 384);
+  return check_hash_fail(io);
 }
 
 int sylow_b200_verify_batch_finish(sylow_b200_ctx* ctx, const uint8_t* partials, size_t n_partials, int* ok) {
@@ -2101,18 +2109,16 @@ int sylow_b200_verify_each(sylow_b200_ctx* ctx, const uint8_t* pks, const uint8_
   CKS(make_dst_prime(ctx, dst, dst_len, hash_id, dp));
   if (!n) return 0;
   if (!pks || !sigs || !ok_out) return SYLOW_B200_ERR_ARG;
-  const uint8_t *dm, *dpk, *dsg, *dpki, *dsgi;
-  const uint64_t* dof;
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(to_dev(ctx, ctx->in_a, pks, n * 128, &dpk));
-  CKS(to_dev(ctx, ctx->in_b, sigs, n * 64, &dsg));
-  CKS(to_dev(ctx, ctx->flag_a, pks_inf, n, &dpki));
-  CKS(to_dev(ctx, ctx->flag_b, sigs_inf, n, &dsgi));
-  CKS(verify_miller_values(ctx, dpk, dpki, dm, dof, dsg, dsgi, n, dp, ctx->stream));
-  CKS(reserve(ctx, ctx->out, n));
-  CKS(launch_check_products(ctx, ctx->scratch0.p, 1, n, ctx->out.p, ctx->stream));
-  CK(cudaMemcpyAsync(ok_out, ctx->out.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return check_hash_fail(ctx);
+  Staging io(ctx);
+  const uint8_t *dpk = io.up(pks, n * 128), *dsg = io.up(sigs, n * 64);
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  const uint8_t *dpki = io.up(pks_inf, n), *dsgi = io.up(sigs_inf, n);
+  uint8_t* d_ok = io.area(n);
+  CKS(io.err);
+  CKS(verify_miller_values(ctx, dpk, dpki, m.msgs, m.offsets, dsg, dsgi, n, dp, ctx->stream));
+  CKS(launch_check_products(ctx, ctx->scratch0.p, 1, n, d_ok, ctx->stream));
+  io.down(ok_out, d_ok, n);
+  return check_hash_fail(io);
 }
 
 // ------------------------------------------------------------------------------- precomputed G2
@@ -2120,19 +2126,21 @@ int sylow_b200_g2_precompute(sylow_b200_ctx* ctx, const uint8_t* g2, size_t n, u
   ENTER(ctx);
   if (n && (!g2 || !coeffs_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t* d2;
-  CKS(to_dev(ctx, ctx->in_b, g2, n * 128, &d2));
-  CKS(reserve(ctx, ctx->out, n * SY_TABLE_BYTES));
-  k_g2_precompute<<<nblocks(n, SY_GLUED_THREADS), SY_GLUED_THREADS, 0, ctx->stream>>>(d2, n, ctx->out.p, 0);
+  Staging io(ctx);
+  uint8_t* d_tab = io.area(n * SY_TABLE_BYTES);
+  const uint8_t* d2 = io.up(g2, n * 128);
+  CKS(io.err);
+  k_g2_precompute<<<nblocks(n, SY_GLUED_THREADS), SY_GLUED_THREADS, 0, ctx->stream>>>(d2, n, d_tab, 0);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(coeffs_out, ctx->out.p, n * SY_TABLE_BYTES, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(coeffs_out, d_tab, n * SY_TABLE_BYTES);
+  return io.finish();
 }
 
 // uploads k canonical tables and converts them to Montgomery form in ctx->tables
-static int tables_to_dev(sylow_b200_ctx* ctx, const uint8_t* coeffs, size_t k) {
-  const uint8_t* dc;
-  CKS(to_dev(ctx, ctx->in_d, coeffs, k * SY_TABLE_BYTES, &dc));
+static int tables_to_dev(Staging& io, const uint8_t* coeffs, size_t k) {
+  sylow_b200_ctx* ctx = io.ctx;
+  const uint8_t* dc = io.up(coeffs, k * SY_TABLE_BYTES);
+  CKS(io.err);
   CKS(reserve(ctx, ctx->tables, k * SY_TABLE_BYTES));
   size_t nfp = k * SY_TABLE_BYTES / 32;
   k_fp_convert<<<nblocks(nfp, 128), 128, 0, ctx->stream>>>(dc, nfp, ctx->tables.p, 1);
@@ -2145,17 +2153,16 @@ int sylow_b200_miller_loop_precomputed(sylow_b200_ctx* ctx, const uint8_t* coeff
   ENTER(ctx);
   if (!coeffs || (n && (!g1 || !f_out))) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *d1, *d1i;
-  CKS(tables_to_dev(ctx, coeffs, 1));
-  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(reserve(ctx, ctx->out, n * 384));
-  CKS(launch_glued(ctx, 0, 1, nullptr, 0, nullptr, nullptr, nullptr, d1, 1, d1i, ctx->tables.p, n, ctx->out.p,
-                   ctx->stream));
-  k_fp12_convert<<<nblocks(n, 128), 128, 0, ctx->stream>>>(ctx->out.p, n, ctx->out.p, 0);
+  Staging io(ctx);
+  CKS(tables_to_dev(io, coeffs, 1));
+  uint8_t* d_f = io.area(n * 384);
+  const uint8_t *d1 = io.up(g1, n * 64), *d1i = io.up(g1_inf, n);
+  CKS(io.err);
+  CKS(launch_glued(ctx, 0, 1, nullptr, 0, nullptr, nullptr, nullptr, d1, 1, d1i, ctx->tables.p, n, d_f, ctx->stream));
+  k_fp12_convert<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d_f, n, d_f, 0);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(f_out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(f_out, d_f, n * 384);
+  return io.finish();
 }
 
 int sylow_b200_pairing_check_fixed_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_g1, const uint8_t* d_g1_inf,
@@ -2179,8 +2186,9 @@ int sylow_b200_pairing_check_fixed_batch_dev(sylow_b200_ctx* ctx, const uint8_t*
 int sylow_b200_tables_to_device(sylow_b200_ctx* ctx, const uint8_t* coeffs, size_t k, uint8_t* d_tables_out, void* stream) {
   ENTER_DEV(ctx);
   if (!coeffs || !d_tables_out || !k) return SYLOW_B200_ERR_ARG;
-  CKS(tables_to_dev(ctx, coeffs, k));
-  CK(cudaStreamSynchronize(ctx->stream));
+  Staging io(ctx);
+  CKS(tables_to_dev(io, coeffs, k));
+  CKS(io.finish());
   CK(cudaMemcpyAsync(d_tables_out, ctx->tables.p, k * SY_TABLE_BYTES, cudaMemcpyDeviceToDevice, pick(ctx, stream)));
   CK(cudaStreamSynchronize(pick(ctx, stream)));  // ctx->tables is reused by the next call
   return 0;
@@ -2194,17 +2202,16 @@ int sylow_b200_pairing_check_fixed_batch(sylow_b200_ctx* ctx, const uint8_t* g1,
   if (!k_fixed || !glued_shape_ok(k_var, k_fixed)) return SYLOW_B200_ERR_ARG;
   if (!n_checks) return 0;
   size_t k = k_var + k_fixed;
-  const uint8_t *d1, *d1i, *d2, *d2i;
-  CKS(tables_to_dev(ctx, coeffs_fixed, k_fixed));
-  CKS(to_dev(ctx, ctx->in_a, g1, n_checks * k * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n_checks * k, &d1i));
-  CKS(to_dev(ctx, ctx->in_b, g2_var, n_checks * k_var * 128, &d2));
-  CKS(to_dev(ctx, ctx->flag_b, g2_var_inf, n_checks * k_var, &d2i));
-  CKS(reserve(ctx, ctx->out, n_checks));
-  CKS(sylow_b200_pairing_check_fixed_batch_dev(ctx, d1, d1i, d2, d2i, k_var, ctx->tables.p, k_fixed, n_checks, ctx->out.p,
+  Staging io(ctx);
+  CKS(tables_to_dev(io, coeffs_fixed, k_fixed));
+  const uint8_t *d2 = io.up(g2_var, n_checks * k_var * 128), *d1 = io.up(g1, n_checks * k * 64);
+  const uint8_t *d1i = io.up(g1_inf, n_checks * k), *d2i = io.up(g2_var_inf, n_checks * k_var);
+  uint8_t* d_ok = io.area(n_checks);
+  CKS(io.err);
+  CKS(sylow_b200_pairing_check_fixed_batch_dev(ctx, d1, d1i, d2, d2i, k_var, ctx->tables.p, k_fixed, n_checks, d_ok,
                                                nullptr));
-  CK(cudaMemcpyAsync(ok_out, ctx->out.p, n_checks, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(ok_out, d_ok, n_checks);
+  return io.finish();
 }
 
 // d_out (canonical) = prod over n >= 1 pairs of the Miller loop of g1[k] against table idx[k] (k if idx is null):
@@ -2235,14 +2242,14 @@ int sylow_b200_miller_loop_precomputed_batch(sylow_b200_ctx* ctx, const uint8_t*
   ENTER(ctx);
   if (n && (!coeffs || !g1 || !f_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *d1, *d1i;
-  CKS(tables_to_dev(ctx, coeffs, n));
-  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(reserve(ctx, ctx->out, n * 384));
-  CKS(launch_miller_tables(ctx, 1, ctx->tables.p, n, nullptr, d1, d1i, n, ctx->out.p, 0, ctx->stream));
-  CK(cudaMemcpyAsync(f_out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  CKS(tables_to_dev(io, coeffs, n));
+  uint8_t* d_f = io.area(n * 384);
+  const uint8_t *d1 = io.up(g1, n * 64), *d1i = io.up(g1_inf, n);
+  CKS(io.err);
+  CKS(launch_miller_tables(ctx, 1, ctx->tables.p, n, nullptr, d1, d1i, n, d_f, 0, ctx->stream));
+  io.down(f_out, d_f, n * 384);
+  return io.finish();
 }
 
 int sylow_b200_miller_product_precomputed(sylow_b200_ctx* ctx, const uint8_t* coeffs, const uint8_t* g1,
@@ -2258,14 +2265,14 @@ int sylow_b200_miller_product_precomputed(sylow_b200_ctx* ctx, const uint8_t* co
     memcpy(f_out, kOneCanonical, 384);
     return 0;
   }
-  const uint8_t *d1, *d1i;
-  CKS(tables_to_dev(ctx, coeffs, n));
-  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(reserve(ctx, ctx->out, 384));
-  CKS(miller_product_tables(ctx, ctx->tables.p, n, nullptr, d1, d1i, n, ctx->out.p, ctx->stream));
-  CK(cudaMemcpyAsync(f_out, ctx->out.p, 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  CKS(tables_to_dev(io, coeffs, n));
+  const uint8_t *d1 = io.up(g1, n * 64), *d1i = io.up(g1_inf, n);
+  uint8_t* d_f = io.area(384);
+  CKS(io.err);
+  CKS(miller_product_tables(ctx, ctx->tables.p, n, nullptr, d1, d1i, n, d_f, ctx->stream));
+  io.down(f_out, d_f, 384);
+  return io.finish();
 }
 
 int sylow_b200_g2_precompute_dev(sylow_b200_ctx* ctx, const uint8_t* d_g2, size_t n, uint8_t* d_tables_out,
@@ -2298,14 +2305,14 @@ int sylow_b200_g1_validate_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const u
   ENTER(ctx);
   if (n && (!g1 || !status_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *d1, *d1i;
-  CKS(to_dev(ctx, ctx->in_a, g1, n * 64, &d1));
-  CKS(to_dev(ctx, ctx->flag_a, g1_inf, n, &d1i));
-  CKS(reserve(ctx, ctx->out, n));
-  k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d1, d1i, n, reinterpret_cast<int8_t*>(ctx->out.p), 0);
+  Staging io(ctx);
+  const uint8_t *d1 = io.up(g1, n * 64), *d1i = io.up(g1_inf, n);
+  int8_t* d_st = reinterpret_cast<int8_t*>(io.area(n));
+  CKS(io.err);
+  k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d1, d1i, n, d_st, 0);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(status_out, ctx->out.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(status_out, d_st, n);
+  return io.finish();
 }
 
 int sylow_b200_g2_validate_batch(sylow_b200_ctx* ctx, const uint8_t* g2, const uint8_t* g2_inf, size_t n,
@@ -2317,15 +2324,14 @@ int sylow_b200_g2_validate_batch(sylow_b200_ctx* ctx, const uint8_t* g2, const u
   ENTER(ctx);
   if (n && (!g2 || !status_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *d2, *d2i;
-  CKS(to_dev(ctx, ctx->in_b, g2, n * 128, &d2));
-  CKS(to_dev(ctx, ctx->flag_b, g2_inf, n, &d2i));
-  CKS(reserve(ctx, ctx->out, n));
-  k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(d2, d2i, n,
-                                                                               reinterpret_cast<int8_t*>(ctx->out.p), 0);
+  Staging io(ctx);
+  const uint8_t *d2 = io.up(g2, n * 128), *d2i = io.up(g2_inf, n);
+  int8_t* d_st = reinterpret_cast<int8_t*>(io.area(n));
+  CKS(io.err);
+  k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(d2, d2i, n, d_st, 0);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(status_out, ctx->out.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(status_out, d_st, n);
+  return io.finish();
 }
 
 // ------------------------------------------------------------------------------- big-endian codecs
@@ -2335,31 +2341,30 @@ static int from_be(sylow_b200_ctx* ctx, int g2, const uint8_t* be, size_t n, int
   if (n && (!be || !out || !inf_out || !status_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   size_t w = g2 ? 128 : 64;
-  const uint8_t* dbe;
-  CKS(to_dev(ctx, ctx->in_c, be, n * w, &dbe));
-  CKS(reserve(ctx, ctx->in_a, n * w));
-  CKS(reserve(ctx, ctx->flag_a, n));
-  CKS(reserve(ctx, ctx->out, n));
-  int8_t* st = reinterpret_cast<int8_t*>(ctx->out.p);
+  Staging io(ctx);
+  const uint8_t* dbe = io.up(be, n * w);
+  uint8_t *d_pts = io.area(n * w), *d_inf = io.area(n);
+  int8_t* st = reinterpret_cast<int8_t*>(io.area(n));
+  CKS(io.err);
   if (g2) {
-    k_decode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dbe, 128, n, mode, ctx->in_a.p, ctx->flag_a.p, st);
+    k_decode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dbe, 128, n, mode, d_pts, d_inf, st);
     LAUNCHED(ctx);
     if (validate) {
-      k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(ctx->in_a.p, ctx->flag_a.p, n, st, 1);
+      k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(d_pts, d_inf, n, st, 1);
       LAUNCHED(ctx);
     }
   } else {
-    k_decode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dbe, 64, n, mode, ctx->in_a.p, ctx->flag_a.p, st);
+    k_decode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dbe, 64, n, mode, d_pts, d_inf, st);
     LAUNCHED(ctx);
     if (validate) {
-      k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(ctx->in_a.p, ctx->flag_a.p, n, st, 1);
+      k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d_pts, d_inf, n, st, 1);
       LAUNCHED(ctx);
     }
   }
-  CK(cudaMemcpyAsync(out, ctx->in_a.p, n * w, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(inf_out, ctx->flag_a.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(status_out, st, n, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_pts, n * w);
+  io.down(inf_out, d_inf, n);
+  io.down(status_out, st, n);
+  return io.finish();
 }
 int sylow_b200_g1_from_be_bytes_batch(sylow_b200_ctx* ctx, const uint8_t* be, size_t n, int eip_mode, uint8_t* g1_out,
                                       uint8_t* inf_out, int8_t* status_out) {
@@ -2374,17 +2379,17 @@ static int to_be(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8_t*
   if (n && (!pts || !be_out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   size_t w = g2 ? 128 : 64;
-  const uint8_t *dp, *di;
-  CKS(to_dev(ctx, ctx->in_a, pts, n * w, &dp));
-  CKS(to_dev(ctx, ctx->flag_a, inf, n, &di));
-  CKS(reserve(ctx, ctx->out, n * w));
+  Staging io(ctx);
+  const uint8_t *dp = io.up(pts, n * w), *di = io.up(inf, n);
+  uint8_t* d_be = io.area(n * w);
+  CKS(io.err);
   if (g2)
-    k_encode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dp, di, n, scrub, ctx->out.p);
+    k_encode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dp, di, n, scrub, d_be);
   else
-    k_encode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dp, di, n, scrub, ctx->out.p);
+    k_encode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(dp, di, n, scrub, d_be);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(be_out, ctx->out.p, n * w, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(be_out, d_be, n * w);
+  return io.finish();
 }
 int sylow_b200_g1_to_be_bytes_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, size_t n, int scrubbed,
                                     uint8_t* be_out) {
@@ -2401,52 +2406,47 @@ int sylow_b200_eip197_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* in
   if (n_checks && (!ok_out || !status_out || (k && !input))) return SYLOW_B200_ERR_ARG;
   if (!n_checks) return 0;
   size_t n = k * n_checks;
-  CKS(reserve(ctx, ctx->out, 2 * n_checks + 64));
-  uint8_t* d_ok = ctx->out.p;
-  int8_t* d_st = reinterpret_cast<int8_t*>(ctx->out.p + ((n_checks + 15) / 16) * 16);
+  Staging io(ctx);
+  const uint8_t* din = io.up(input, n * 192);
+  uint8_t *d2 = io.area(n * 128), *d1 = io.area(n * 64), *d1i = io.area(n), *d2i = io.area(n);
+  int8_t* st1 = reinterpret_cast<int8_t*>(io.area(2 * n));  // per-pair decode status of G1, then of G2
+  int8_t* st2 = st1 + n;
+  uint8_t* d_ok = io.area(2 * n_checks + 64);
+  CKS(io.err);
+  int8_t* d_st = reinterpret_cast<int8_t*>(d_ok + ((n_checks + 15) / 16) * 16);
   if (n) {
-    const uint8_t* din;
-    CKS(to_dev(ctx, ctx->in_c, input, n * 192, &din));
-    CKS(reserve(ctx, ctx->in_a, n * 64));
-    CKS(reserve(ctx, ctx->in_b, n * 128));
-    CKS(reserve(ctx, ctx->flag_a, n));
-    CKS(reserve(ctx, ctx->flag_b, n));
-    CKS(reserve(ctx, ctx->scratch2, 2 * n + 64));
-    int8_t* st1 = reinterpret_cast<int8_t*>(ctx->scratch2.p);
-    int8_t* st2 = st1 + n;
-    k_decode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(din, 192, n, 1, ctx->in_a.p, ctx->flag_a.p, st1);
+    k_decode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(din, 192, n, 1, d1, d1i, st1);
     LAUNCHED(ctx);
-    k_decode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(din + 64, 192, n, 1, ctx->in_b.p, ctx->flag_b.p, st2);
+    k_decode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(din + 64, 192, n, 1, d2, d2i, st2);
     LAUNCHED(ctx);
-    k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(ctx->in_a.p, ctx->flag_a.p, n, st1, 1);
+    k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d1, d1i, n, st1, 1);
     LAUNCHED(ctx);
-    k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(ctx->in_b.p, ctx->flag_b.p, n, st2, 1);
+    k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(d2, d2i, n, st2, 1);
     LAUNCHED(ctx);
-    CKS(sylow_b200_pairing_check_batch_dev(ctx, ctx->in_a.p, ctx->flag_a.p, ctx->in_b.p, ctx->flag_b.p, k, n_checks, d_ok,
-                                           nullptr));
+    CKS(sylow_b200_pairing_check_batch_dev(ctx, d1, d1i, d2, d2i, k, n_checks, d_ok, nullptr));
     k_fold_status<<<nblocks(n_checks, 128), 128, 0, ctx->stream>>>(st1, st2, k, n_checks, d_ok, d_st);
     LAUNCHED(ctx);
   } else {
     CK(cudaMemsetAsync(d_ok, 1, n_checks, ctx->stream));  // empty input: success (reth_bn128.rs:173-175)
     CK(cudaMemsetAsync(d_st, 0, n_checks, ctx->stream));
   }
-  CK(cudaMemcpyAsync(ok_out, d_ok, n_checks, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(status_out, d_st, n_checks, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(ok_out, d_ok, n_checks);
+  io.down(status_out, d_st, n_checks);
+  return io.finish();
 }
 
 int sylow_b200_gt_mul_batch(sylow_b200_ctx* ctx, const uint8_t* gt, const uint8_t* scalars, size_t n, uint8_t* out) {
   ENTER(ctx);
   if (n && (!gt || !scalars || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *dg, *dk;
-  CKS(to_dev(ctx, ctx->in_a, gt, n * 384, &dg));
-  CKS(to_dev(ctx, ctx->in_b, scalars, n * 32, &dk));
-  CKS(reserve(ctx, ctx->out, n * 384));
-  k_gt_pow<<<nblocks(n, SY_FEXP_THREADS), SY_FEXP_THREADS, 0, ctx->stream>>>(dg, dk, n, ctx->out.p);
+  Staging io(ctx);
+  uint8_t* d_out = io.area(n * 384);
+  const uint8_t *dg = io.up(gt, n * 384), *dk = io.up(scalars, n * 32);
+  CKS(io.err);
+  k_gt_pow<<<nblocks(n, SY_FEXP_THREADS), SY_FEXP_THREADS, 0, ctx->stream>>>(dg, dk, n, d_out);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_out, n * 384);
+  return io.finish();
 }
 
 // ------------------------------------------------------------------------------- Expander trait
@@ -2460,14 +2460,14 @@ int sylow_b200_expand_message_batch(sylow_b200_ctx* ctx, const uint8_t* msgs, co
   if (hash_id != SYLOW_B200_HASH_SHAKE128 && (len_in_bytes + 31) / 32 > 255) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   if (!out) return SYLOW_B200_ERR_ARG;
-  const uint8_t* dm;
-  const uint64_t* dof;
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(reserve(ctx, ctx->out, n * len_in_bytes));
-  k_expand_message<<<nblocks(n, 128), 128, 0, ctx->stream>>>(dm, dof, n, dp, (uint32_t)len_in_bytes, ctx->out.p);
+  Staging io(ctx);
+  uint8_t* d_out = io.area(n * len_in_bytes);
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  CKS(io.err);
+  k_expand_message<<<nblocks(n, 128), 128, 0, ctx->stream>>>(m.msgs, m.offsets, n, dp, (uint32_t)len_in_bytes, d_out);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * len_in_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_out, n * len_in_bytes);
+  return io.finish();
 }
 
 int sylow_b200_hash_to_field_batch(sylow_b200_ctx* ctx, const uint8_t* msgs, const uint64_t* offsets, size_t n,
@@ -2477,14 +2477,14 @@ int sylow_b200_hash_to_field_batch(sylow_b200_ctx* ctx, const uint8_t* msgs, con
   CKS(make_dst_prime(ctx, dst, dst_len, hash_id, dp));
   if (!n) return 0;
   if (!out) return SYLOW_B200_ERR_ARG;
-  const uint8_t* dm;
-  const uint64_t* dof;
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(reserve(ctx, ctx->out, n * 64));
-  k_hash_to_field<<<nblocks(n, 128), 128, 0, ctx->stream>>>(dm, dof, n, dp, ctx->out.p);
+  Staging io(ctx);
+  uint8_t* d_out = io.area(n * 64);
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  CKS(io.err);
+  k_hash_to_field<<<nblocks(n, 128), 128, 0, ctx->stream>>>(m.msgs, m.offsets, n, dp, d_out);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 64, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_out, n * 64);
+  return io.finish();
 }
 
 // ------------------------------------------------------------------------------- sums / same-signer batches
@@ -2498,14 +2498,14 @@ int sylow_b200_g1_sum(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pt
     *out_inf = 1;
     return 0;
   }
-  const uint8_t *dp, *di;
-  CKS(to_dev(ctx, ctx->in_a, pts, n * 64, &dp));
-  CKS(to_dev(ctx, ctx->flag_a, pts_inf, n, &di));
-  CKS(reserve(ctx, ctx->out, 128));
-  CKS(g1_sum_reduce(ctx, dp, di, n, 0, ctx->out.p, ctx->out.p + 64, ctx->stream));
-  CK(cudaMemcpyAsync(out, ctx->out.p, 64, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(out_inf, ctx->out.p + 64, 1, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  const uint8_t *dp = io.up(pts, n * 64), *di = io.up(pts_inf, n);
+  uint8_t* d_sum = io.area(128);  // point, then its flag
+  CKS(io.err);
+  CKS(g1_sum_reduce(ctx, dp, di, n, 0, d_sum, d_sum + 64, ctx->stream));
+  io.down(out, d_sum, 64);
+  io.down(out_inf, d_sum + 64, 1);
+  return io.finish();
 }
 
 #define SY_MSM_BUCKET_MIN 131072
@@ -2572,15 +2572,14 @@ int sylow_b200_g1_msm_bucket(sylow_b200_ctx* ctx, const uint8_t* pts, const uint
   if (!out || !out_inf || (n && (!pts || !scalars)) || window_bits < 0 || window_bits > 16) return SYLOW_B200_ERR_ARG;
   if (!n) return sylow_b200_g1_sum(ctx, nullptr, nullptr, 0, out, out_inf);
   if (n >= ((size_t)1 << 31)) return SYLOW_B200_ERR_ARG;
-  const uint8_t *dp, *di, *dk;
-  CKS(to_dev(ctx, ctx->in_a, pts, n * 64, &dp));
-  CKS(to_dev(ctx, ctx->flag_a, pts_inf, n, &di));
-  CKS(to_dev(ctx, ctx->in_b, scalars, n * 32, &dk));
-  CKS(reserve(ctx, ctx->out, 128));
-  CKS(g1_msm_bucket_dev(ctx, dp, di, dk, n, window_bits, ctx->out.p, ctx->out.p + 64, ctx->stream));
-  CK(cudaMemcpyAsync(out, ctx->out.p, 64, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(out_inf, ctx->out.p + 64, 1, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  const uint8_t *dp = io.up(pts, n * 64), *dk = io.up(scalars, n * 32), *di = io.up(pts_inf, n);
+  uint8_t* d_sum = io.area(128);  // point, then its flag
+  CKS(io.err);
+  CKS(g1_msm_bucket_dev(ctx, dp, di, dk, n, window_bits, d_sum, d_sum + 64, ctx->stream));
+  io.down(out, d_sum, 64);
+  io.down(out_inf, d_sum + 64, 1);
+  return io.finish();
 }
 
 int sylow_b200_g1_msm(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars, size_t n,
@@ -2591,17 +2590,16 @@ int sylow_b200_g1_msm(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pt
   // from 2^17 points on the bucket method beats n GLV ladders + tree sum (tools/msm_time.py)
   if (n >= SY_MSM_BUCKET_MIN && n < ((size_t)1 << 31))
     return sylow_b200_g1_msm_bucket(ctx, pts, pts_inf, scalars, n, 0, out, out_inf);
-  const uint8_t *dp, *di, *dk;
-  CKS(to_dev(ctx, ctx->in_a, pts, n * 64, &dp));
-  CKS(to_dev(ctx, ctx->flag_a, pts_inf, n, &di));
-  CKS(to_dev(ctx, ctx->in_b, scalars, n * 32, &dk));
-  CKS(reserve(ctx, ctx->scratch2, n * 65));
-  CKS(reserve(ctx, ctx->out, 128));
-  CKS(sylow_b200_g1_mul_batch_dev(ctx, dp, di, dk, n, ctx->scratch2.p, ctx->scratch2.p + n * 64, nullptr));
-  CKS(g1_sum_reduce(ctx, ctx->scratch2.p, ctx->scratch2.p + n * 64, n, 0, ctx->out.p, ctx->out.p + 64, ctx->stream));
-  CK(cudaMemcpyAsync(out, ctx->out.p, 64, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(out_inf, ctx->out.p + 64, 1, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  Staging io(ctx);
+  uint8_t* d_kp = io.area(n * 65);  // k_i P_i, then their flags
+  const uint8_t *dp = io.up(pts, n * 64), *dk = io.up(scalars, n * 32), *di = io.up(pts_inf, n);
+  uint8_t* d_sum = io.area(128);
+  CKS(io.err);
+  CKS(sylow_b200_g1_mul_batch_dev(ctx, dp, di, dk, n, d_kp, d_kp + n * 64, nullptr));
+  CKS(g1_sum_reduce(ctx, d_kp, d_kp + n * 64, n, 0, d_sum, d_sum + 64, ctx->stream));
+  io.down(out, d_sum, 64);
+  io.down(out_inf, d_sum + 64, 1);
+  return io.finish();
 }
 
 int sylow_b200_lagrange_coefficients_batch(sylow_b200_ctx* ctx, const uint64_t* ids, size_t n_sets, size_t t,
@@ -2610,13 +2608,14 @@ int sylow_b200_lagrange_coefficients_batch(sylow_b200_ctx* ctx, const uint64_t* 
   if ((n_sets && t) && (!ids || !out)) return SYLOW_B200_ERR_ARG;
   size_t n = n_sets * t;
   if (!n) return 0;
-  const uint8_t* d_ids;
-  CKS(to_dev(ctx, ctx->in_a, reinterpret_cast<const uint8_t*>(ids), n * 8, &d_ids));
-  CKS(reserve(ctx, ctx->out, n * 32));
-  k_lagrange<<<nblocks(n, 128), 128, 0, ctx->stream>>>(reinterpret_cast<const uint64_t*>(d_ids), n_sets, t, ctx->out.p);
+  Staging io(ctx);
+  uint8_t* d_lam = io.area(n * 32);
+  const uint64_t* d_ids = reinterpret_cast<const uint64_t*>(io.up(ids, n * 8));
+  CKS(io.err);
+  k_lagrange<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d_ids, n_sets, t, d_lam);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 32, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_lam, n * 32);
+  return io.finish();
 }
 
 int sylow_b200_threshold_aggregate_batch(sylow_b200_ctx* ctx, const uint64_t* ids, const uint8_t* sigs,
@@ -2634,21 +2633,19 @@ int sylow_b200_threshold_aggregate_batch(sylow_b200_ctx* ctx, const uint64_t* id
     return 0;
   }
   size_t n = n_sets * t;
-  const uint8_t *d_ids, *d_sigs, *d_inf;
-  CKS(to_dev(ctx, ctx->in_b, reinterpret_cast<const uint8_t*>(ids), n * 8, &d_ids));
-  CKS(to_dev(ctx, ctx->in_a, sigs, n * 64, &d_sigs));
-  CKS(to_dev(ctx, ctx->flag_a, sigs_inf, n, &d_inf));
-  CKS(reserve(ctx, ctx->scratch2, n * 96));
-  CKS(reserve(ctx, ctx->out, n_sets * 65));
+  Staging io(ctx);
+  uint8_t* d_shares = io.area(n * 96);  // lambda_i sig_i, projective
+  const uint8_t *d_sigs = io.up(sigs, n * 64), *d_ids = io.up(ids, n * 8), *d_inf = io.up(sigs_inf, n);
+  uint8_t* d_agg = io.area(n_sets * 65);  // the n_sets points, then their flags
+  CKS(io.err);
   k_lagrange_mul<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(
-      reinterpret_cast<const uint64_t*>(d_ids), d_sigs, d_inf, n_sets, t, ctx->scratch2.p);
+      reinterpret_cast<const uint64_t*>(d_ids), d_sigs, d_inf, n_sets, t, d_shares);
   LAUNCHED(ctx);
-  k_g1_segment_sum<<<nblocks(n_sets, 4), 128, 0, ctx->stream>>>(ctx->scratch2.p, n_sets, t, ctx->out.p,
-                                                               ctx->out.p + n_sets * 64);
+  k_g1_segment_sum<<<nblocks(n_sets, 4), 128, 0, ctx->stream>>>(d_shares, n_sets, t, d_agg, d_agg + n_sets * 64);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n_sets * 64, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaMemcpyAsync(out_inf, ctx->out.p + n_sets * 64, n_sets, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_agg, n_sets * 64);
+  io.down(out_inf, d_agg + n_sets * 64, n_sets);
+  return io.finish();
 }
 
 int sylow_b200_verify_batch_same_signer(sylow_b200_ctx* ctx, const uint8_t* pk, int pk_inf, const uint8_t* msgs,
@@ -2666,23 +2663,21 @@ int sylow_b200_verify_batch_same_signer(sylow_b200_ctx* ctx, const uint8_t* pk, 
   if (!pk || !sigs) return SYLOW_B200_ERR_ARG;
   WeightSeed ws;
   const bool weighted = load_seed(weight_seed, ws);
-  const uint8_t *dm, *dpk, *dsg, *dsgi;
-  const uint64_t* dof;
-  CKS(msgs_to_dev(ctx, msgs, offsets, n, &dm, &dof));
-  CKS(to_dev(ctx, ctx->in_a, pk, 128, &dpk));
-  CKS(to_dev(ctx, ctx->in_b, sigs, n * 64, &dsg));
-  CKS(to_dev(ctx, ctx->flag_b, sigs_inf, n, &dsgi));
+  uint8_t h_ok = 0;
+  Staging io(ctx);
+  uint8_t* d_hm = io.area(n * 65);  // H(m_i), then their flags
+  const uint8_t* dsg = io.up(sigs, n * 64);
+  const DevMsgs m = msgs_to_dev(io, msgs, offsets, n);
+  const uint8_t *dsgi = io.up(sigs_inf, n), *dpk = io.up(pk, 128);
   // e(sum r_i sig_i, G2gen) * e(-sum r_i H(m_i), pk) == 1 (r_i = 1 without a seed): two Miller loops for the whole batch
-  CKS(reserve(ctx, ctx->scratch2, n * 65 + 64));
-  CKS(reserve(ctx, ctx->out, 1024));
-  uint8_t* d_pairs = ctx->out.p;        // two G1 points (128 B) + two flags at +128 + the G2 pair at +256
-  uint8_t* d_flags = ctx->out.p + 128;
-  uint8_t* d_g2 = ctx->out.p + 256;     // G2gen || pk
-  uint8_t* d_g2_inf = ctx->out.p + 520; // 0, pk_inf
-  uint8_t* d_ok = ctx->out.p + 512;
-  uint8_t* d_hm = ctx->scratch2.p;
+  uint8_t* d_pairs = io.area(1024);     // two G1 points (128 B) + two flags at +128 + the G2 pair at +256
+  CKS(io.err);
+  uint8_t* d_flags = d_pairs + 128;
+  uint8_t* d_g2 = d_pairs + 256;        // G2gen || pk
+  uint8_t* d_g2_inf = d_pairs + 520;    // 0, pk_inf
+  uint8_t* d_ok = d_pairs + 512;
   cudaStream_t st_ = ctx->stream;
-  CKS(hash_launch(ctx, dm, dof, n, dp, 0, d_hm, d_hm + n * 64, st_));
+  CKS(hash_launch(ctx, m.msgs, m.offsets, n, dp, 0, d_hm, d_hm + n * 64, st_));
   if (weighted) {
     CKS(reserve(ctx, ctx->proj, n * 96));
     k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, st_>>>(dsg, dsgi, ws, 0, n, ctx->proj.p);
@@ -2700,9 +2695,8 @@ int sylow_b200_verify_batch_same_signer(sylow_b200_ctx* ctx, const uint8_t* pk, 
   CK(cudaMemcpyAsync(d_g2 + 128, dpk, 128, cudaMemcpyDeviceToDevice, st_));
   CK(cudaMemcpyAsync(d_g2_inf, h_g2_inf, 2, cudaMemcpyHostToDevice, st_));
   CKS(sylow_b200_pairing_check_batch_dev(ctx, d_pairs, d_flags, d_g2, d_g2_inf, 2, 1, d_ok, nullptr));
-  uint8_t h_ok = 0;
-  CK(cudaMemcpyAsync(&h_ok, d_ok, 1, cudaMemcpyDeviceToHost, st_));
-  int st = check_hash_fail(ctx);
+  io.down(&h_ok, d_ok, 1);
+  int st = check_hash_fail(io);
   *ok = h_ok;
   return st;
 }
@@ -2715,39 +2709,41 @@ int sylow_b200_batch_weights(sylow_b200_ctx* ctx, const uint8_t* weight_seed, ui
   if (!n) return 0;
   WeightSeed ws;
   load_seed(weight_seed, ws);
-  CKS(reserve(ctx, ctx->out, n * 8));
-  k_batch_weights<<<nblocks(n, 128), 128, 0, ctx->stream>>>(ws, first_index, n, reinterpret_cast<uint64_t*>(ctx->out.p));
+  Staging io(ctx);
+  uint64_t* d_w = reinterpret_cast<uint64_t*>(io.area(n * 8));
+  CKS(io.err);
+  k_batch_weights<<<nblocks(n, 128), 128, 0, ctx->stream>>>(ws, first_index, n, d_w);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_w, n * 8);
+  return io.finish();
 }
 
 int sylow_b200_fp_op_batch(sylow_b200_ctx* ctx, int op, const uint8_t* a, const uint8_t* b, size_t n, uint8_t* out) {
   ENTER(ctx);
   if (n && (!a || !b || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *da, *db;
-  CKS(to_dev(ctx, ctx->in_a, a, n * 32, &da));
-  CKS(to_dev(ctx, ctx->in_b, b, n * 32, &db));
-  CKS(reserve(ctx, ctx->out, n * 32));
-  k_fp_op<<<nblocks(n, 128), 128, 0, ctx->stream>>>(op, da, db, n, ctx->out.p);
+  Staging io(ctx);
+  const uint8_t *da = io.up(a, n * 32), *db = io.up(b, n * 32);
+  uint8_t* d_out = io.area(n * 32);
+  CKS(io.err);
+  k_fp_op<<<nblocks(n, 128), 128, 0, ctx->stream>>>(op, da, db, n, d_out);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 32, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_out, n * 32);
+  return io.finish();
 }
 
 int sylow_b200_fp12_op_batch(sylow_b200_ctx* ctx, int op, const uint8_t* a, const uint8_t* b, size_t n, uint8_t* out) {
   ENTER(ctx);
   if (n && (!a || !b || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
-  const uint8_t *da, *db;
-  CKS(to_dev(ctx, ctx->in_a, a, n * 384, &da));
-  CKS(to_dev(ctx, ctx->in_b, b, n * 384, &db));
-  CKS(reserve(ctx, ctx->out, n * 384));
-  k_fp12_op<<<nblocks(n, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, ctx->stream>>>(op, da, db, n, ctx->out.p);
+  Staging io(ctx);
+  const uint8_t *da = io.up(a, n * 384), *db = io.up(b, n * 384);
+  uint8_t* d_out = io.area(n * 384);
+  CKS(io.err);
+  k_fp12_op<<<nblocks(n, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, ctx->stream>>>(op, da, db, n, d_out);
   LAUNCHED(ctx);
-  CK(cudaMemcpyAsync(out, ctx->out.p, n * 384, cudaMemcpyDeviceToHost, ctx->stream));
-  return finish(ctx);
+  io.down(out, d_out, n * 384);
+  return io.finish();
 }
 
 
@@ -2755,8 +2751,10 @@ int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int thre
                           double* ops_out) {
   ENTER(ctx);
   if (!ms_out || !ops_out || blocks <= 0 || threads <= 0 || threads > 1024 || iters <= 0) return SYLOW_B200_ERR_ARG;
-  CKS(reserve(ctx, ctx->out, 256));
-  CK(cudaMemsetAsync(ctx->out.p, 0x5a, 256, ctx->stream));
+  Staging io(ctx);
+  uint8_t* d_words = io.area(256);
+  CKS(io.err);
+  CK(cudaMemsetAsync(d_words, 0x5a, 256, ctx->stream));
   struct Event {
     cudaEvent_t e = nullptr;
     ~Event() {
@@ -2765,8 +2763,8 @@ int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int thre
   } e0, e1;  // released on every return
   CK(cudaEventCreate(&e0.e));
   CK(cudaEventCreate(&e1.e));
-  const uint32_t* src = reinterpret_cast<const uint32_t*>(ctx->out.p);
-  uint32_t* sink = reinterpret_cast<uint32_t*>(ctx->out.p) + 32;
+  const uint32_t* src = reinterpret_cast<const uint32_t*>(d_words);
+  uint32_t* sink = reinterpret_cast<uint32_t*>(d_words) + 32;
   double per_thread_iter = 0;
   for (int rep = 0; rep < 2; rep++) {  // the first pass warms up
     CK(cudaEventRecord(e0.e, ctx->stream));
@@ -2786,7 +2784,7 @@ int sylow_b200_imad_probe(sylow_b200_ctx* ctx, int variant, int blocks, int thre
   }
   CK(cudaEventElapsedTime(ms_out, e0.e, e1.e));
   *ops_out = (double)blocks * threads * (double)iters * per_thread_iter;
-  return 0;
+  return io.finish();
 }
 
 }  // extern "C"
