@@ -1,89 +1,34 @@
-"""ctypes binding of libsylow_b200.so (include/sylow_b200.h).  Fails loudly if the CUDA library is
-missing or no CUDA device is usable - there is no CPU fallback."""
+"""ctypes binding of libsylow_b200.so.  Prototypes and constants are read from include/sylow_b200.h when this module
+is imported, so the header is the one declaration of the C ABI.  Fails loudly if the CUDA library is missing or no
+CUDA device is usable - there is no CPU fallback."""
 from __future__ import annotations
 
 import ctypes
 import os
 from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_size_t, c_uint64, c_void_p
 
+from . import _header
 from .build import LIB_PATH
 
 _lib = None
 
-OK = 0
-ERR_ARG, ERR_CUDA, ERR_NOT_ON_CURVE, ERR_NOT_IN_SUBGROUP, ERR_CANNOT_HASH, ERR_DECODE, ERR_NOMEM = range(-1, -8, -1)
-HASH_KECCAK256 = 0
-HASH_SHA256 = 1
-HASH_SHAKE128 = 2
+_CONSTS, _FUNCS = _header.parse()
+# the header's SYLOW_B200_* constants without the prefix: OK, ERR_ARG ... ERR_NOMEM, HASH_KECCAK256, HASH_SHA256,
+# HASH_SHAKE128
+globals().update({name[len("SYLOW_B200_"):]: int(value) for name, value in _CONSTS})
 
-# every symbol include/sylow_b200.h declares (tests/test_capi_symbols.py checks the header against this)
-_P = c_void_p
-_SIGNATURES = {
-    "sylow_b200_create": (c_int, [POINTER(c_void_p), c_int]),
-    "sylow_b200_create_multi": (c_int, [POINTER(c_void_p), POINTER(c_int), c_int]),
-    "sylow_b200_device_count": (c_int, [_P]),
-    "sylow_b200_device_ctx": (c_void_p, [_P, c_int]),
-    "sylow_b200_destroy": (c_int, [_P]),
-    "sylow_b200_strerror": (c_char_p, [c_int]),
-    "sylow_b200_last_cuda_error": (c_int, [_P]),
-    "sylow_b200_launch_count": (c_uint64, [_P]),
-    "sylow_b200_pairing_batch": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P]),
-    "sylow_b200_miller_loop_batch": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P]),
-    "sylow_b200_miller_product": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P]),
-    "sylow_b200_final_exp_batch": (c_int, [_P, _P, c_size_t, _P]),
-    "sylow_b200_fp12_product": (c_int, [_P, _P, c_size_t, _P]),
-    "sylow_b200_pairing_check_batch": (c_int, [_P, _P, _P, _P, _P, c_size_t, c_size_t, _P]),
-    "sylow_b200_g2_precompute": (c_int, [_P, _P, c_size_t, _P]),
-    "sylow_b200_miller_loop_precomputed": (c_int, [_P, _P, _P, _P, c_size_t, _P]),
-    "sylow_b200_pairing_check_fixed_batch": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_size_t, _P]),
-    "sylow_b200_pairing_check_fixed_batch_dev": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_size_t, _P, _P]),
-    "sylow_b200_tables_to_device": (c_int, [_P, _P, c_size_t, _P, _P]),
-    "sylow_b200_miller_loop_precomputed_batch": (c_int, [_P, _P, _P, _P, c_size_t, _P]),
-    "sylow_b200_miller_product_precomputed": (c_int, [_P, _P, _P, _P, c_size_t, _P]),
-    "sylow_b200_g2_precompute_dev": (c_int, [_P, _P, c_size_t, _P, _P]),
-    "sylow_b200_miller_product_precomputed_dev": (c_int, [_P, _P, c_size_t, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_g1_validate_batch": (c_int, [_P, _P, _P, c_size_t, _P]),
-    "sylow_b200_g2_validate_batch": (c_int, [_P, _P, _P, c_size_t, _P]),
-    "sylow_b200_g1_from_be_bytes_batch": (c_int, [_P, _P, c_size_t, c_int, _P, _P, _P]),
-    "sylow_b200_g2_from_be_bytes_batch": (c_int, [_P, _P, c_size_t, c_int, _P, _P, _P]),
-    "sylow_b200_g1_to_be_bytes_batch": (c_int, [_P, _P, _P, c_size_t, c_int, _P]),
-    "sylow_b200_g2_to_be_bytes_batch": (c_int, [_P, _P, _P, c_size_t, c_int, _P]),
-    "sylow_b200_eip197_pairing_check_batch": (c_int, [_P, _P, c_size_t, c_size_t, _P, _P]),
-    "sylow_b200_gt_mul_batch": (c_int, [_P, _P, _P, c_size_t, _P]),
-    "sylow_b200_g1_mul_batch": (c_int, [_P, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_g2_mul_batch": (c_int, [_P, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_hash_to_g1_batch": (c_int, [_P, _P, _P, c_size_t, _P, c_size_t, c_int, _P, _P]),
-    "sylow_b200_g1_sum": (c_int, [_P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_g1_msm": (c_int, [_P, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_g1_msm_bucket": (c_int, [_P, _P, _P, _P, c_size_t, c_int, _P, _P]),
-    "sylow_b200_lagrange_coefficients_batch": (c_int, [_P, _P, c_size_t, c_size_t, _P]),
-    "sylow_b200_threshold_aggregate_batch": (c_int, [_P, _P, _P, _P, c_size_t, c_size_t, _P, _P]),
-    "sylow_b200_verify_batch_same_signer": (c_int, [_P, _P, c_int, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_int, _P,
-                                                    POINTER(c_int)]),
-    "sylow_b200_expand_message_batch": (c_int, [_P, _P, _P, c_size_t, _P, c_size_t, c_int, c_size_t, _P]),
-    "sylow_b200_hash_to_field_batch": (c_int, [_P, _P, _P, c_size_t, _P, c_size_t, c_int, _P]),
-    "sylow_b200_sign_batch": (c_int, [_P, _P, _P, _P, c_size_t, _P, c_size_t, c_int, _P, _P]),
-    "sylow_b200_verify_each": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_int, _P]),
-    "sylow_b200_verify_batch_partial": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_int, _P, c_uint64,
-                                                _P]),
-    "sylow_b200_verify_batch_finish": (c_int, [_P, _P, c_size_t, POINTER(c_int)]),
-    "sylow_b200_verify_batch": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_int, _P, POINTER(c_int)]),
-    "sylow_b200_hash_failed_dev": (c_int, [_P, _P, POINTER(c_int)]),
-    "sylow_b200_batch_weights": (c_int, [_P, _P, c_uint64, c_size_t, _P]),
-    "sylow_b200_pairing_batch_dev": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_miller_loop_batch_dev": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_miller_product_dev": (c_int, [_P, _P, _P, _P, _P, c_size_t, _P, _P]),
-    "sylow_b200_final_exp_batch_dev": (c_int, [_P, _P, c_size_t, _P, _P]),
-    "sylow_b200_pairing_check_batch_dev": (c_int, [_P, _P, _P, _P, _P, c_size_t, c_size_t, _P, _P]),
-    "sylow_b200_g1_mul_batch_dev": (c_int, [_P, _P, _P, _P, c_size_t, _P, _P, _P]),
-    "sylow_b200_g2_mul_batch_dev": (c_int, [_P, _P, _P, _P, c_size_t, _P, _P, _P]),
-    "sylow_b200_hash_to_g1_batch_dev": (c_int, [_P, _P, _P, c_size_t, _P, c_size_t, c_int, _P, _P, _P]),
-    "sylow_b200_verify_batch_partial_dev": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_size_t, _P, c_size_t, c_int, _P,
-                                                    c_uint64, _P, _P]),
-    "sylow_b200_fp_op_batch": (c_int, [_P, c_int, _P, _P, c_size_t, _P]),
-    "sylow_b200_fp12_op_batch": (c_int, [_P, c_int, _P, _P, c_size_t, _P]),
-    "sylow_b200_imad_probe": (c_int, [_P, c_int, c_int, c_int, c_int, POINTER(c_float), POINTER(c_double)]),
-}
+# A pointer is a c_void_p unless the binding reads or writes through it as a ctypes object.  An integer type missing
+# from _INTS fails the import: a narrower ctypes type would truncate the argument, so it has to be mapped by hand.
+_INTS = {"int": c_int, "size_t": c_size_t, "uint64_t": c_uint64}
+_POINTERS = {("int", 1): POINTER(c_int), ("float", 1): POINTER(c_float), ("double", 1): POINTER(c_double),
+             ("sylow_b200_ctx", 2): POINTER(c_void_p), ("char", 1): c_char_p}
+
+
+def _ctypes_type(t: _header.CType):
+    return _POINTERS.get((t.base, t.stars), c_void_p) if t.stars else _INTS[t.base]
+
+
+_PROTOTYPES = {name: (_ctypes_type(ret), [_ctypes_type(t) for _, t in params]) for name, params, ret in _FUNCS}
 
 
 class SylowB200Error(RuntimeError):
@@ -107,7 +52,7 @@ def load():
             "libsylow_b200.so is not built (%s). Run `python -c 'import __graft_entry__ as g; g.build()'` "
             "or `python -m sylow_b200.build`. There is no CPU fallback." % LIB_PATH)
     lib = ctypes.CDLL(path)
-    for name, (res, args) in _SIGNATURES.items():
+    for name, (res, args) in _PROTOTYPES.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype = res
         fn.argtypes = args
@@ -116,4 +61,4 @@ def load():
 
 
 def exported_symbols():
-    return sorted(_SIGNATURES)
+    return sorted(_PROTOTYPES)

@@ -36,6 +36,28 @@ def test_header_symbols_are_exported(lib):
     assert set(declared) <= exported, set(declared) - exported
 
 
+def test_ctypes_prototypes_from_the_header(lib):
+    """_lib.py derives argtypes/restype from the header.  Pin the entry points whose types are not plain data pointers,
+    and the three bench.py calls through Engine._lib with c_void_p / None pointers."""
+    from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_size_t, c_uint64, c_void_p as P
+
+    pins = {
+        "sylow_b200_create": (c_int, [POINTER(P), c_int]),
+        "sylow_b200_create_multi": (c_int, [POINTER(P), POINTER(c_int), c_int]),
+        "sylow_b200_strerror": (c_char_p, [c_int]),
+        "sylow_b200_device_ctx": (P, [P, c_int]),
+        "sylow_b200_launch_count": (c_uint64, [P]),
+        "sylow_b200_imad_probe": (c_int, [P, c_int, c_int, c_int, c_int, POINTER(c_float), POINTER(c_double)]),
+        "sylow_b200_hash_failed_dev": (c_int, [P, P, POINTER(c_int)]),
+        "sylow_b200_pairing_batch": (c_int, [P, P, P, P, P, c_size_t, P]),
+        "sylow_b200_verify_batch": (c_int, [P, P, P, P, P, P, P, c_size_t, P, c_size_t, c_int, P, POINTER(c_int)]),
+        "sylow_b200_verify_batch_partial": (c_int, [P, P, P, P, P, P, P, c_size_t, P, c_size_t, c_int, P, c_uint64, P]),
+    }
+    for name, (res, args) in pins.items():
+        fn = getattr(lib, name)
+        assert (fn.restype, list(fn.argtypes)) == (res, args), name
+
+
 def test_strerror_and_arg_checks(lib):
     assert lib.sylow_b200_strerror(0) == b"ok"
     assert b"argument" in lib.sylow_b200_strerror(-1)
