@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import bn254_py as o
+from tests import bound_cases as bc
 from tests import wire as w
 
 pytestmark = pytest.mark.gpu
@@ -101,24 +102,8 @@ def test_fp12_ops(eng):
 
 def test_fp12_edge_coefficients(eng):
     """Carry-propagation extremes of the lazy-reduction Fp2 arithmetic: every coefficient drawn from
-    {0, 1, 2, p-1, p-2, (p-1)/2, (p+1)/2, 2^32-1, 2^224, R mod p, ...}."""
-    rng = random.Random(29)
-    edge = [0, 1, 2, o.P - 1, o.P - 2, (o.P - 1) // 2, (o.P + 1) // 2, (1 << 32) - 1, 1 << 224, (1 << 253) + 1,
-            (1 << 256) % o.P, o.P - ((1 << 256) % o.P), 0xFFFFFFFF00000000FFFFFFFF00000000FFFFFFFF00000000 % o.P]
-    # the lazy-reduction bounds are on the MONTGOMERY representatives: -1/R mod p is stored as p - 1
-    top = o.P - pow(1 << 256, -1, o.P)
-    edge += [top, (o.P - 2) * pow(1 << 256, -1, o.P) % o.P]
-    n = 200
-    a = [o.fp12_from_list([rng.choice(edge) for _ in range(12)]) for _ in range(n)]
-    b = [o.fp12_from_list([rng.choice(edge) for _ in range(12)]) for _ in range(n)]
-    a[0] = o.fp12_from_list([o.P - 1] * 12)
-    b[0] = o.fp12_from_list([o.P - 1] * 12)
-    a[1], b[1] = o.fp12_from_list([top] * 12), o.fp12_from_list([top] * 12)
-    a[2], b[2] = o.fp12_from_list([top, 0] * 6), o.fp12_from_list([0, top] * 6)
-    a[3], b[3] = o.fp12_from_list([top] * 6 + [0] * 6), o.fp12_from_list([0] * 6 + [top] * 6)
-    for i in range(4, 64):
-        a[i] = o.fp12_from_list([rng.choice([0, top]) for _ in range(12)])
-        b[i] = o.fp12_from_list([rng.choice([0, top]) for _ in range(12)])
+    {0, 1, 2, p-1, p-2, (p-1)/2, (p+1)/2, 2^32-1, 2^224, R mod p, ...} (tests/bound_cases.py: fp12_edge_pairs)."""
+    a, b = bc.fp12_edge_pairs()
     A, B = arr([w.fp12_b(x) for x in a]), arr([w.fp12_b(x) for x in b])
     dec = lambda out: [w.b_fp12(bytes(r)) for r in out]
     assert dec(eng.fp12_op_batch(0, A, B)) == [o.fp12_mul(x, y) for x, y in zip(a, b)]
