@@ -7,7 +7,8 @@
 //!
 //! ```ignore
 //! mod batch;
-//! pub use crate::batch::{final_exponentiation_batch, g1_mul_batch, g2_mul_batch, glued_miller_loop_batch,
+//! pub use crate::batch::{final_exponentiation_batch, g1_generator_mul_batch, g1_mul_batch, g2_generator_mul_batch,
+//!                        g2_mul_batch, glued_miller_loop_batch,
 //!                        glued_miller_loop_precomputed_batch, glued_pairing_batch, pairing_batch, pairing_check_batch, sign_batch,
 //!                        threshold_aggregate_batch, verify_batch, verify_each, BatchError, Engine};
 //! ```
@@ -290,6 +291,25 @@ pub fn g2_mul_batch(e: &mut Engine, pts: &[G2Projective], scalars: &[Fp]) -> Res
     e.check(unsafe {
         sys::sylow_b200_g2_mul_batch(e.ctx, g2.as_ptr(), g2i.as_ptr(), ks.as_ptr(), n, out.as_mut_ptr(), inf.as_mut_ptr())
     })?;
+    Ok(out.chunks_exact(128).zip(&inf).map(|(b, &i)| get_g2(b, i)).collect())
+}
+
+/// `G1Projective::generator() * &scalars[i]`, returned affine: the values of `g1_mul_batch` on the repeated generator,
+/// from a fixed-base table of the generator.
+pub fn g1_generator_mul_batch(e: &mut Engine, scalars: &[Fp]) -> Result<Vec<G1Affine>, BatchError> {
+    let n = scalars.len();
+    let ks = marshal_scalars(scalars);
+    let (mut out, mut inf) = (vec![0u8; n * 64], vec![0u8; n]);
+    e.check(unsafe { sys::sylow_b200_g1_mul_generator_batch(e.ctx, ks.as_ptr(), n, out.as_mut_ptr(), inf.as_mut_ptr()) })?;
+    Ok(out.chunks_exact(64).zip(&inf).map(|(b, &i)| get_g1(b, i)).collect())
+}
+
+/// The same on the twist: `KeyPair::generate`'s public keys (src/lib.rs:105-137).
+pub fn g2_generator_mul_batch(e: &mut Engine, scalars: &[Fp]) -> Result<Vec<G2Affine>, BatchError> {
+    let n = scalars.len();
+    let ks = marshal_scalars(scalars);
+    let (mut out, mut inf) = (vec![0u8; n * 128], vec![0u8; n]);
+    e.check(unsafe { sys::sylow_b200_g2_mul_generator_batch(e.ctx, ks.as_ptr(), n, out.as_mut_ptr(), inf.as_mut_ptr()) })?;
     Ok(out.chunks_exact(128).zip(&inf).map(|(b, &i)| get_g2(b, i)).collect())
 }
 

@@ -192,6 +192,14 @@ int sylow_b200_g1_mul_batch(sylow_b200_ctx* ctx, const uint8_t* pts /* n*64 */, 
 int sylow_b200_g2_mul_batch(sylow_b200_ctx* ctx, const uint8_t* pts /* n*128 */, const uint8_t* pts_inf,
                             const uint8_t* scalars /* n*32 */, size_t n, uint8_t* out /* n*128 */, uint8_t* out_inf);
 
+/* out[i] = affine(scalars[i] * G) for the G1 / G2 generator: the same bytes as g1_mul_batch / g2_mul_batch on the
+ * repeated generator (`G1Projective::generator() * &k`; KeyPair::generate's pk, lib.rs:105-137).  A fixed-base table
+ * of the generator, built on the device on a context's first such call, replaces the ladder.  out_inf may be NULL. */
+int sylow_b200_g1_mul_generator_batch(sylow_b200_ctx* ctx, const uint8_t* scalars /* n*32 */, size_t n,
+                                      uint8_t* out /* n*64 */, uint8_t* out_inf);
+int sylow_b200_g2_mul_generator_batch(sylow_b200_ctx* ctx, const uint8_t* scalars /* n*32 */, size_t n,
+                                      uint8_t* out /* n*128 */, uint8_t* out_inf);
+
 /* out[i] = gt[i] * scalars[i] in sylow's additive notation, i.e. gt[i]^scalars[i] in Fp12  (`&Gt * &Fr`,
  * groups/gt.rs:188-215).  gt[i] must be a Gt value (a final-exponentiation output: cyclotomic subgroup). */
 int sylow_b200_gt_mul_batch(sylow_b200_ctx* ctx, const uint8_t* gt /* n*384 */, const uint8_t* scalars /* n*32 */,
@@ -331,6 +339,10 @@ int sylow_b200_g1_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_pts, const
                                 const uint8_t* d_scalars, size_t n, uint8_t* d_out, uint8_t* d_out_inf, void* stream);
 int sylow_b200_g2_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_pts, const uint8_t* d_pts_inf,
                                 const uint8_t* d_scalars, size_t n, uint8_t* d_out, uint8_t* d_out_inf, void* stream);
+int sylow_b200_g1_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
+                                          uint8_t* d_out_inf, void* stream);
+int sylow_b200_g2_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
+                                          uint8_t* d_out_inf, void* stream);
 int sylow_b200_hash_to_g1_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_msgs, const uint64_t* d_offsets, size_t n,
                                     const uint8_t* dst, size_t dst_len /* host */, int hash_id, uint8_t* d_out,
                                     uint8_t* d_out_inf, void* stream);

@@ -135,6 +135,25 @@ class Engine {
     return r;
   }
 
+  // G1Projective::generator() * &k[i] and G2Projective::generator() * &k[i] (KeyPair::generate's pk, lib.rs:105-137):
+  // the values of g1_mul_batch / g2_mul_batch on the repeated generator, from a fixed-base table
+  std::vector<G1Affine> g1_mul_generator_batch(const std::vector<Fp>& k) {
+    std::vector<std::uint8_t> out(k.size() * 64), inf(k.size());
+    ck(sylow_b200_g1_mul_generator_batch(ctx_, reinterpret_cast<const std::uint8_t*>(k.data()), k.size(), out.data(),
+                                         inf.data()), "g1_mul_generator_batch");
+    std::vector<G1Affine> r(k.size());
+    for (size_t i = 0; i < k.size(); i++) { std::memcpy(&r[i].x, &out[64 * i], 64); r[i].infinity = inf[i]; }
+    return r;
+  }
+  std::vector<G2Affine> g2_mul_generator_batch(const std::vector<Fp>& k) {
+    std::vector<std::uint8_t> out(k.size() * 128), inf(k.size());
+    ck(sylow_b200_g2_mul_generator_batch(ctx_, reinterpret_cast<const std::uint8_t*>(k.data()), k.size(), out.data(),
+                                         inf.data()), "g2_mul_generator_batch");
+    std::vector<G2Affine> r(k.size());
+    for (size_t i = 0; i < k.size(); i++) { std::memcpy(&r[i].x, &out[128 * i], 128); r[i].infinity = inf[i]; }
+    return r;
+  }
+
   // G1Projective::hash_to_curve(&XMDExpander::<Keccak256>::new(dst, 128), msg) (g1.rs:307-331)
   std::vector<G1Affine> hash_to_g1_batch(const std::vector<std::string>& msgs, const std::string& dst = DST()) {
     Msgs m(msgs);

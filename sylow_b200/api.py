@@ -325,6 +325,22 @@ class Engine:
     def g2_mul_batch(self, pts, scalars, pts_inf=None):
         return self._mul("sylow_b200_g2_mul_batch", 128, pts, scalars, pts_inf)
 
+    def _mul_generator(self, symbol, width, scalars):
+        scalars = _rows(scalars, 32, "scalars")
+        n = scalars.shape[0]
+        out = np.empty((n, width), dtype=np.uint8)
+        out_inf = np.empty(n, dtype=np.uint8)
+        self._call(symbol, scalars, n, out, out_inf)
+        return out, out_inf
+
+    def g1_mul_generator_batch(self, scalars):
+        """scalars[i] * G1 generator: the values of g1_mul_batch on the repeated generator, from a fixed-base table."""
+        return self._mul_generator("sylow_b200_g1_mul_generator_batch", 64, scalars)
+
+    def g2_mul_generator_batch(self, scalars):
+        """scalars[i] * G2 generator (KeyPair::generate's public key), like g1_mul_generator_batch."""
+        return self._mul_generator("sylow_b200_g2_mul_generator_batch", 128, scalars)
+
     def gt_mul_batch(self, gt, scalars) -> np.ndarray:
         """`Gt * Fr`: gt[i]^scalars[i] (gt must be final-exponentiation outputs)."""
         gt = _rows(gt, 384, "gt")
@@ -522,6 +538,14 @@ class Engine:
 
     def g2_mul_batch_dev(self, d_pts, d_scalars, d_out, d_out_inf=None, d_pts_inf=None):
         self._call("sylow_b200_g2_mul_batch_dev", d_pts, d_pts_inf, d_scalars, d_pts.shape[0], d_out, d_out_inf,
+                   self._stream())
+
+    def g1_mul_generator_batch_dev(self, d_scalars, d_out, d_out_inf=None):
+        self._call("sylow_b200_g1_mul_generator_batch_dev", d_scalars, d_scalars.shape[0], d_out, d_out_inf,
+                   self._stream())
+
+    def g2_mul_generator_batch_dev(self, d_scalars, d_out, d_out_inf=None):
+        self._call("sylow_b200_g2_mul_generator_batch_dev", d_scalars, d_scalars.shape[0], d_out, d_out_inf,
                    self._stream())
 
     def hash_to_g1_batch_dev(self, d_msgs, d_offsets, d_out, d_out_inf=None, dst: bytes = DST):

@@ -391,6 +391,120 @@ SY_HD_NOINLINE G2Proj g2_scalar_mul_gls(const G2Proj& p, const uint32_t* k) {
   return acc;
 }
 
+// ---- fixed-base multiplication by a generator -------------------------------------------------------------
+// k G with a table of affine multiples of G: T[w][j] = (j + 1) 2^(C w) G, j < 2^(C-1), Montgomery form, x || y.
+// k mod r is recoded into W = ceil(254 / C) signed C-bit digits, least significant first, and the selected entries are
+// added up: W mixed additions and no doublings.  The table is built on the device from the variable-base ladder
+// (sylow_b200.cu: ensure_mul_table), so its entries are the ladder's own affine points.
+#define SY_GEN_C 8
+#define SY_GEN_W ((254 + SY_GEN_C - 1) / SY_GEN_C)
+#define SY_GEN_E (1 << (SY_GEN_C - 1))  // entries per window
+static_assert(SY_GEN_C >= 6 && SY_GEN_C <= 8, "the top digit bound below is shown for C = 6, 7, 8");
+
+SY_HD Fp f_select(bool c, const Fp& a, const Fp& b) { return fp_select(c, a, b); }
+SY_HD Fp2 f_select(bool c, const Fp2& a, const Fp2& b) { return fp2_select(c, a, b); }
+
+// Renes-Costello-Batina Alg. 8 (a = 0): a + (b.x : b.y : 1), 11M + 2 m_3b.  Complete for every projective a, b.inf
+// ignored (the caller never adds the point at infinity): a = O gives b, a = -b gives O, a = b doubles.
+template <class F>
+SY_HD_NOINLINE Proj<F> proj_add_mixed(const Proj<F>& a, const Affine<F>& b) {
+  F t0 = f_mul(a.x, b.x);
+  F t1 = f_mul(a.y, b.y);
+  F t3 = f_mul(f_add(b.x, b.y), f_add(a.x, a.y));
+  t3 = f_sub(t3, f_add(t0, t1));
+  F t4 = f_add(f_mul(b.y, a.z), a.y);
+  F y3 = f_add(f_mul(b.x, a.z), a.x);
+  F x3 = f_add(t0, t0);
+  t0 = f_add(x3, t0);
+  F t2 = f_mul_b3(a.z);
+  F z3 = f_add(t1, t2);
+  t1 = f_sub(t1, t2);
+  y3 = f_mul_b3(y3);
+  x3 = f_mul(t4, y3);
+  t2 = f_mul(t3, t1);
+  x3 = f_sub(t2, x3);
+  y3 = f_mul(y3, t0);
+  t1 = f_mul(t1, z3);
+  y3 = f_add(t1, y3);
+  t0 = f_mul(t0, t3);
+  z3 = f_mul(z3, t4);
+  z3 = f_add(z3, t0);
+  return Proj<F>{x3, y3, z3};
+}
+
+// k mod r in place for any 256-bit k: 2^256 < 6 r, so five conditional subtractions leave k < r < 2^254
+SY_HD void scalar_reduce_r(uint32_t* k) {
+  for (int s = 0; s < 5; s++) {
+    uint32_t d[8], borrow = 0;
+    for (int i = 0; i < 8; i++) {
+      uint64_t v = (uint64_t)k[i] - SY_TAB(kFrMod)[i] - borrow;
+      d[i] = (uint32_t)v;
+      borrow = (uint32_t)(v >> 63);
+    }
+    for (int i = 0; i < 8; i++) k[i] = borrow ? k[i] : d[i];
+  }
+}
+// bits [pos, pos + C) of the 256-bit k (pos + C may pass bit 255: those bits read as 0)
+template <int C>
+SY_HD uint32_t scalar_window(const uint32_t* k, int pos) {
+  const int i = pos >> 5, s = pos & 31;
+  uint64_t v = k[i];
+  if (i < 7) v |= (uint64_t)k[i + 1] << 32;
+  return (uint32_t)(v >> s) & ((1u << C) - 1);
+}
+// Signed digit of window w of k < 2^254, and the carry into window w + 1: d in [-2^(C-1) + 1, 2^(C-1)].  The top
+// window holds at most 254 - C (W - 1) <= C - 2 bits, so its digit plus carry stays below 2^(C-1) and never carries.
+template <int C>
+SY_HD int scalar_digit(const uint32_t* k, int w, int& carry) {
+  int d = (int)scalar_window<C>(k, C * w) + carry;
+  carry = d > (1 << (C - 1));
+  return d - (carry << C);
+}
+
+SY_HD uint4 ld_nc(const uint8_t* p) {
+#if defined(__CUDA_ARCH__)
+  return __ldg(reinterpret_cast<const uint4*>(p));  // ld.global.nc: the table is read-only while a kernel reads it
+#else
+  return *reinterpret_cast<const uint4*>(p);
+#endif
+}
+SY_HD void gen_entry_load(const uint8_t* p, Affine<Fp>& e) {
+  uint4 v[4] = {ld_nc(p), ld_nc(p + 16), ld_nc(p + 32), ld_nc(p + 48)};
+  e.x = Fp{{v[0].x, v[0].y, v[0].z, v[0].w, v[1].x, v[1].y, v[1].z, v[1].w}};
+  e.y = Fp{{v[2].x, v[2].y, v[2].z, v[2].w, v[3].x, v[3].y, v[3].z, v[3].w}};
+}
+SY_HD void gen_entry_load(const uint8_t* p, Affine<Fp2>& e) {
+  Affine<Fp> a, b;
+  gen_entry_load(p, a);
+  gen_entry_load(p + 64, b);
+  e.x = Fp2{a.x, a.y};
+  e.y = Fp2{b.x, b.y};
+}
+
+// k G over the table `tab` of G (SY_GEN_W x SY_GEN_E entries of 2 sizeof(F) bytes): the digit only selects an entry
+// and the sign of its y, a zero digit keeps the accumulator; no data-dependent branches.
+template <class F>
+SY_HD_NOINLINE Proj<F> gen_scalar_mul(const uint8_t* __restrict__ tab, const uint32_t* k_in) {
+  uint32_t k[8];
+  for (int i = 0; i < 8; i++) k[i] = k_in[i];
+  scalar_reduce_r(k);
+  Proj<F> acc = proj_zero<F>();
+  int carry = 0;
+#pragma unroll
+  for (int w = 0; w < SY_GEN_W; w++) {
+    const int d = scalar_digit<SY_GEN_C>(k, w, carry);
+    const int m = d < 0 ? -d : d;
+    Affine<F> e;
+    gen_entry_load(tab + ((size_t)w * SY_GEN_E + (m ? m - 1 : 0)) * 2 * sizeof(F), e);
+    e.y = f_select(d < 0, f_neg(e.y), e.y);
+    Proj<F> s = proj_add_mixed(acc, e);
+    acc.x = f_select(m != 0, s.x, acc.x);
+    acc.y = f_select(m != 0, s.y, acc.y);
+    acc.z = f_select(m != 0, s.z, acc.z);
+  }
+  return acc;
+}
+
 // y^2 == x^3 + b
 SY_HD bool g1_on_curve(const Fp& x, const Fp& y) {
   Fp rhs = fp_add(fp_mul(fp_sqr(x), x), SY_TAB(kFpThree)[0]);

@@ -207,8 +207,8 @@ SY_HD Fp f_load_raw(const uint8_t* p, const Fp*) { return fp_load_raw(p); }
 SY_HD Fp2 f_load_raw(const uint8_t* p, const Fp2*) { return fp2_load_raw(p); }
 SY_HD void f_store(uint8_t* p, const Fp& v) { fp_store(p, v); }
 SY_HD void f_store(uint8_t* p, const Fp2& v) { fp2_store(p, v); }
-SY_HD Fp f_select(bool c, const Fp& a, const Fp& b) { return fp_select(c, a, b); }
-SY_HD Fp2 f_select(bool c, const Fp2& a, const Fp2& b) { return fp2_select(c, a, b); }
+SY_HD void f_store_raw(uint8_t* p, const Fp& v) { fp_store_raw(p, v); }
+SY_HD void f_store_raw(uint8_t* p, const Fp2& v) { fp2_store_raw(p, v); }
 template <class F>
 __device__ __forceinline__ void batch_affine(const uint8_t* __restrict__ proj, size_t n, int negate,
                                              uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf) {
@@ -318,6 +318,41 @@ k_g2_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf,
   fp2_store(out + i * 128, r.x);
   fp2_store(out + i * 128 + 64, r.y);
   if (out_inf) out_inf[i] = r.inf;
+}
+
+// out[i] = affine(scalars[i] * G) for the generator G of `table` (gen_scalar_mul; ensure_mul_table), any 256-bit
+// scalar; large batches leave projective points in proj_out for affine_tail, like k_g1_mul / k_g2_mul
+template <class F>
+__device__ __forceinline__ void mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n,
+                                        uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
+                                        uint8_t* __restrict__ proj_out) {
+  constexpr size_t W = sizeof(F);
+  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t i = i0 < n ? i0 : n - 1;  // the inversion of proj_to_affine is block-synchronised: every thread runs it
+  Fp k = fp_load_raw(scalars + i * 32);
+  Proj<F> q = gen_scalar_mul<F>(table, k.l);
+  if (proj_out) {
+    if (i0 >= n) return;
+    f_store_raw(proj_out + i * 3 * W, q.x);
+    f_store_raw(proj_out + i * 3 * W + W, q.y);
+    f_store_raw(proj_out + i * 3 * W + 2 * W, q.z);
+    return;
+  }
+  Affine<F> r = proj_to_affine(q);
+  if (i0 >= n) return;
+  f_store(out + i * 2 * W, r.x);
+  f_store(out + i * 2 * W + W, r.y);
+  if (out_inf) out_inf[i] = r.inf;
+}
+__global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
+k_g1_mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
+             uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  mul_gen<Fp>(table, scalars, n, out, out_inf, proj_out);
+}
+__global__ void __launch_bounds__(SY_G2_THREADS, SY_G2_MINB)
+k_g2_mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
+             uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  mul_gen<Fp2>(table, scalars, n, out, out_inf, proj_out);
 }
 
 // out[i] = affine(+-hash_to_curve(msg_i)); status[i] = 1 if the SvdW sqrt check failed
@@ -983,6 +1018,7 @@ struct sylow_b200_ctx {
   DevBuf scratch0, scratch1, scratch2;
   int* d_fail = nullptr;
   uint8_t* d_gen_table = nullptr;  // G2PreComputed of the G2 generator, Montgomery form (16704 B)
+  uint8_t* d_mul_table[2] = {};    // fixed-base tables of the G1 and G2 generators (ensure_mul_table)
   DevBuf tables, sum0, sum1, proj, msm;
   DevBuf check_stage[2];  // group products / Gt values of launch_check_products' two-lane path, per compute stream
   DevBuf fexp_lanes[2];  // FexpCold records of k_final_exp_lanes, one buffer per compute stream (stream, stream2)
@@ -997,6 +1033,8 @@ struct sylow_b200_ctx {
     cudaSetDevice(device);  // the DevBuf members are freed after this body, on the same device
     if (d_fail) cudaFree(d_fail);
     if (d_gen_table) cudaFree(d_gen_table);
+    for (uint8_t* t : d_mul_table)
+      if (t) cudaFree(t);
     for (cudaStream_t s : {stream, copy_in, copy_out, stream2})
       if (s) cudaStreamDestroy(s);
     if (ev_fork) cudaEventDestroy(ev_fork);
@@ -1562,6 +1600,76 @@ static int ensure_gen_table(sylow_b200_ctx* ctx, cudaStream_t s) {
   return 0;
 }
 
+// Fixed-base table of the G1 (g2 = 0) or G2 generator for gen_scalar_mul (curve.cuh), built on the device once per
+// context: the ladder of g1/g2_mul_batch_dev multiplies the generator by (j + 1) 2^(C w) mod r, and k_fp_convert takes
+// the affine results to Montgomery form, so every entry is the ladder's own point.  The field is set only after the
+// build has finished, like ensure_gen_table's.
+static int ensure_mul_table(sylow_b200_ctx* ctx, int g2, cudaStream_t s) {
+  if (ctx->d_mul_table[g2]) return 0;
+  const size_t n = (size_t)SY_GEN_W * SY_GEN_E, pb = g2 ? 128 : 64, in_bytes = n * (32 + pb);
+  std::vector<uint8_t> in(in_bytes);  // n scalars, then the generator n times
+  Fr step{{1}};                       // 2^(C w) mod r
+  for (int w = 0; w < SY_GEN_W; w++) {
+    Fr m = step;
+    for (int j = 0; j < SY_GEN_E; j++, m = fr_add(m, step)) memcpy(&in[((size_t)w * SY_GEN_E + j) * 32], m.l, 32);
+    for (int b = 0; b < SY_GEN_C; b++) step = fr_add(step, step);
+  }
+  static const uint64_t kG1GenWords[8] = {1, 0, 0, 0, 2, 0, 0, 0};  // (1, 2)
+  for (size_t i = 0; i < n; i++) memcpy(&in[n * 32 + i * pb], g2 ? (const void*)kG2GenWords : kG1GenWords, pb);
+  uint8_t *d_in = nullptr, *d_tab = nullptr;
+  cudaError_t e = cudaMalloc(&d_in, in_bytes + n * pb);  // inputs, then the canonical affine points
+  if (e == cudaSuccess) e = cudaMalloc(&d_tab, n * pb);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_in, in.data(), in_bytes, cudaMemcpyHostToDevice, s);
+  int st = e == cudaSuccess ? 0 : fail_cuda(ctx, e);
+  uint8_t* d_aff = d_in + in_bytes;
+  if (!st)
+    st = (g2 ? sylow_b200_g2_mul_batch_dev : sylow_b200_g1_mul_batch_dev)(ctx, d_in + n * 32, nullptr, d_in, n, d_aff,
+                                                                           nullptr, s);
+  if (!st) {
+    k_fp_convert<<<nblocks(n * pb / 32, 128), 128, 0, s>>>(d_aff, n * pb / 32, d_tab, 1);
+    ctx->launches++;
+    e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) st = fail_cuda(ctx, e);
+  }
+  if (d_in) cudaFree(d_in);
+  if (st) {
+    if (d_tab) cudaFree(d_tab);
+    return st;
+  }
+  ctx->d_mul_table[g2] = d_tab;
+  return 0;
+}
+
+// out[i] = affine(scalars[i] * G) for the G1 (g2 = 0) or G2 generator: the form of g1/g2_mul_batch_dev with the
+// fixed-base table in place of the ladder
+static int mul_gen_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf,
+                       void* stream) {
+  ENTER_DEV(ctx);
+  if (n && (!scalars || !out)) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  cudaStream_t s = pick(ctx, stream);
+  CKS(ensure_mul_table(ctx, g2, s));
+  uint8_t* proj;
+  CKS(affine_stage(ctx, n, g2 ? 192 : 96, &proj));
+  if (g2)
+    k_g2_mul_gen<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(ctx->d_mul_table[1], scalars, n, out, out_inf, proj);
+  else
+    k_g1_mul_gen<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(ctx->d_mul_table[0], scalars, n, out, out_inf,
+                                                                        proj);
+  LAUNCHED(ctx);
+  if (proj) CKS(affine_tail(ctx, g2, proj, n, 0, out, out_inf, s));
+  return 0;
+}
+int sylow_b200_g1_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
+                                          uint8_t* d_out_inf, void* stream) {
+  return mul_gen_dev(ctx, 0, d_scalars, n, d_out, d_out_inf, stream);
+}
+int sylow_b200_g2_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
+                                          uint8_t* d_out_inf, void* stream) {
+  return mul_gen_dev(ctx, 1, d_scalars, n, d_out, d_out_inf, stream);
+}
+
 // f[i] = miller(sig_i, G2gen) * miller(-H(m_i), pk_i) for every signature, Montgomery form, in scratch0:
 // one 2-pair glued loop per thread (shared squaring; the generator's lines come from shared memory).  An infinite
 // signature or key makes its pair contribute 1, like pairing() does (pairing.rs:876-886).
@@ -1922,16 +2030,18 @@ int sylow_b200_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const
   return io.finish();
 }
 
+// pts == nullptr: the generator of the group (g1/g2_mul_generator_batch)
 static int mul_host(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
                     size_t n, uint8_t* out, uint8_t* out_inf) {
-  if (is_multi(ctx) && pts && scalars && out) {
+  if (is_multi(ctx) && scalars && out) {
     const size_t pb = g2 ? 128 : 64;
     return multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t, size_t off, size_t m) {
-      return mul_host(c, g2, pts + off * pb, adv(pts_inf, off), scalars + off * 32, m, out + off * pb, adv(out_inf, off));
+      return mul_host(c, g2, adv(pts, off * pb), adv(pts_inf, off), scalars + off * 32, m, out + off * pb,
+                      adv(out_inf, off));
     });
   }
   ENTER(ctx);
-  if (n && (!pts || !scalars || !out)) return SYLOW_B200_ERR_ARG;
+  if (n && (!scalars || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   size_t pb = g2 ? 128 : 64;
   Staging io(ctx);
@@ -1939,7 +2049,9 @@ static int mul_host(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8
   const uint8_t *dp = io.up(pts, n * pb), *dk = io.up(scalars, n * 32), *dpi = io.up(pts_inf, n);
   uint8_t* d_out_inf = io.area(n);
   CKS(io.err);
-  if (g2)
+  if (!pts)
+    CKS(mul_gen_dev(ctx, g2, dk, n, d_out, d_out_inf, nullptr));
+  else if (g2)
     CKS(sylow_b200_g2_mul_batch_dev(ctx, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
   else
     CKS(sylow_b200_g1_mul_batch_dev(ctx, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
@@ -1949,11 +2061,21 @@ static int mul_host(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8
 }
 int sylow_b200_g1_mul_batch(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
                             size_t n, uint8_t* out, uint8_t* out_inf) {
+  if (n && !pts) return SYLOW_B200_ERR_ARG;
   return mul_host(ctx, 0, pts, pts_inf, scalars, n, out, out_inf);
 }
 int sylow_b200_g2_mul_batch(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
                             size_t n, uint8_t* out, uint8_t* out_inf) {
+  if (n && !pts) return SYLOW_B200_ERR_ARG;
   return mul_host(ctx, 1, pts, pts_inf, scalars, n, out, out_inf);
+}
+int sylow_b200_g1_mul_generator_batch(sylow_b200_ctx* ctx, const uint8_t* scalars, size_t n, uint8_t* out,
+                                      uint8_t* out_inf) {
+  return mul_host(ctx, 0, nullptr, nullptr, scalars, n, out, out_inf);
+}
+int sylow_b200_g2_mul_generator_batch(sylow_b200_ctx* ctx, const uint8_t* scalars, size_t n, uint8_t* out,
+                                      uint8_t* out_inf) {
+  return mul_host(ctx, 1, nullptr, nullptr, scalars, n, out, out_inf);
 }
 
 // the end of a hashing host form: finishes with the hash-to-curve failure flag, then CannotHashToGroup if it is set

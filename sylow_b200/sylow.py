@@ -328,7 +328,8 @@ class KeyPair:
     @classmethod
     def generate(cls) -> "KeyPair":
         sk = int(Fr.rand())
-        return cls(sk, G2Affine.generator() * sk)
+        out, inf = engine().g2_mul_generator_batch(_arr(_fp(sk), 32))
+        return cls(sk, _g2_from(out[0], inf[0]))
 
 
 def sign(k: int, msg: bytes) -> G1Affine:
