@@ -7,8 +7,8 @@
 //!
 //! ```ignore
 //! mod batch;
-//! pub use crate::batch::{final_exponentiation_batch, g1_generator_mul_batch, g1_mul_batch, g2_generator_mul_batch,
-//!                        g2_mul_batch, glued_miller_loop_batch,
+//! pub use crate::batch::{final_exponentiation_batch, g1_add_batch, g1_generator_mul_batch, g1_mul_batch, g2_add_batch,
+//!                        g2_generator_mul_batch, g2_mul_batch, glued_miller_loop_batch,
 //!                        glued_miller_loop_precomputed_batch, glued_pairing_batch, pairing_batch, pairing_check_batch, sign_batch,
 //!                        threshold_aggregate_batch, verify_batch, verify_each, BatchError, Engine};
 //! ```
@@ -280,6 +280,30 @@ pub fn g1_mul_batch(e: &mut Engine, pts: &[G1Projective], scalars: &[Fp]) -> Res
         sys::sylow_b200_g1_mul_batch(e.ctx, g1.as_ptr(), g1i.as_ptr(), ks.as_ptr(), n, out.as_mut_ptr(), inf.as_mut_ptr())
     })?;
     Ok(out.chunks_exact(64).zip(&inf).map(|(b, &i)| get_g1(b, i)).collect())
+}
+
+/// `&a[i] + &b[i]`, or `&a[i] - &b[i]` when `subtract` (src/groups/group.rs:528-624), followed by the affine conversion.
+pub fn g1_add_batch(e: &mut Engine, a: &[G1Projective], b: &[G1Projective], subtract: bool) -> Result<Vec<G1Affine>, BatchError> {
+    let n = same_len(a.len(), b.len())?;
+    let ((pa, ia), (pb, ib)) = (marshal_g1(a), marshal_g1(b));
+    let (mut out, mut inf) = (vec![0u8; n * 64], vec![0u8; n]);
+    e.check(unsafe {
+        sys::sylow_b200_g1_add_batch(e.ctx, pa.as_ptr(), ia.as_ptr(), pb.as_ptr(), ib.as_ptr(), n, subtract as i32,
+                                     out.as_mut_ptr(), inf.as_mut_ptr())
+    })?;
+    Ok(out.chunks_exact(64).zip(&inf).map(|(b, &i)| get_g1(b, i)).collect())
+}
+
+/// The same on the twist.
+pub fn g2_add_batch(e: &mut Engine, a: &[G2Projective], b: &[G2Projective], subtract: bool) -> Result<Vec<G2Affine>, BatchError> {
+    let n = same_len(a.len(), b.len())?;
+    let ((pa, ia), (pb, ib)) = (marshal_g2(a), marshal_g2(b));
+    let (mut out, mut inf) = (vec![0u8; n * 128], vec![0u8; n]);
+    e.check(unsafe {
+        sys::sylow_b200_g2_add_batch(e.ctx, pa.as_ptr(), ia.as_ptr(), pb.as_ptr(), ib.as_ptr(), n, subtract as i32,
+                                     out.as_mut_ptr(), inf.as_mut_ptr())
+    })?;
+    Ok(out.chunks_exact(128).zip(&inf).map(|(b, &i)| get_g2(b, i)).collect())
 }
 
 /// The same on the twist.

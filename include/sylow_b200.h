@@ -183,6 +183,28 @@ int sylow_b200_g2_to_be_bytes_batch(sylow_b200_ctx* ctx, const uint8_t* g2, cons
 int sylow_b200_eip197_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* input, size_t k, size_t n_checks,
                                           uint8_t* ok_out, int8_t* status_out);
 
+/* The EIP-196 precompile bodies (examples/reth_bn128.rs, the adapter ahead of the ecPairing body at :156-217) over
+ * n fixed-size inputs.  The caller zero-pads short calldata and truncates long calldata, as the EVM does.
+ * add: input i = x1 || y1 || x2 || y2 (128 B big-endian);  mul: input i = x || y || s (96 B; s any 256-bit integer).
+ * out[i] = 64 B big-endian result; the point at infinity is all-zero (input and output).
+ * status_out[i] = 0, SYLOW_B200_ERR_DECODE (a coordinate >= p) or SYLOW_B200_ERR_NOT_ON_CURVE;
+ * a failed input gives out[i] = 64 zero bytes.  The call itself returns 0. */
+int sylow_b200_eip196_add_batch(sylow_b200_ctx* ctx, const uint8_t* input /* n*128 */, size_t n, uint8_t* out /* n*64 */,
+                                int8_t* status_out);
+int sylow_b200_eip196_mul_batch(sylow_b200_ctx* ctx, const uint8_t* input /* n*96 */, size_t n, uint8_t* out /* n*64 */,
+                                int8_t* status_out);
+
+/* ---- group law --------------------------------------------------------------------------------- */
+
+/* out[i] = affine(a[i] + b[i]), or affine(a[i] - b[i]) when subtract != 0 (group.rs:528-624, :475-495).
+ * Complete: equal, opposite and infinite operands are ordinary inputs.  a_inf, b_inf and out_inf may be NULL. */
+int sylow_b200_g1_add_batch(sylow_b200_ctx* ctx, const uint8_t* a /* n*64 */, const uint8_t* a_inf,
+                            const uint8_t* b /* n*64 */, const uint8_t* b_inf, size_t n, int subtract,
+                            uint8_t* out /* n*64 */, uint8_t* out_inf);
+int sylow_b200_g2_add_batch(sylow_b200_ctx* ctx, const uint8_t* a /* n*128 */, const uint8_t* a_inf,
+                            const uint8_t* b /* n*128 */, const uint8_t* b_inf, size_t n, int subtract,
+                            uint8_t* out /* n*128 */, uint8_t* out_inf);
+
 /* ---- scalar multiplication --------------------------------------------------------------------- */
 
 /* out[i] = affine(scalars[i] * pts[i]);  replaces `&G1Projective * &Fp` + GroupAffine::from
@@ -339,6 +361,12 @@ int sylow_b200_g1_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_pts, const
                                 const uint8_t* d_scalars, size_t n, uint8_t* d_out, uint8_t* d_out_inf, void* stream);
 int sylow_b200_g2_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_pts, const uint8_t* d_pts_inf,
                                 const uint8_t* d_scalars, size_t n, uint8_t* d_out, uint8_t* d_out_inf, void* stream);
+int sylow_b200_g1_add_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_a, const uint8_t* d_a_inf, const uint8_t* d_b,
+                                const uint8_t* d_b_inf, size_t n, int subtract, uint8_t* d_out, uint8_t* d_out_inf,
+                                void* stream);
+int sylow_b200_g2_add_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_a, const uint8_t* d_a_inf, const uint8_t* d_b,
+                                const uint8_t* d_b_inf, size_t n, int subtract, uint8_t* d_out, uint8_t* d_out_inf,
+                                void* stream);
 int sylow_b200_g1_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
                                           uint8_t* d_out_inf, void* stream);
 int sylow_b200_g2_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,

@@ -109,6 +109,29 @@ class Engine {
     for (size_t i = 0; i < n; i++) { std::memcpy(&r[i].x, &out[64 * i], 64); r[i].infinity = inf[i]; }
     return r;
   }
+  // &a[i] + &b[i], or &a[i] - &b[i] when subtract (group.rs:528-624), + GroupAffine::from (:475-495)
+  std::vector<G1Affine> g1_add_batch(const std::vector<G1Affine>& a, const std::vector<G1Affine>& b,
+                                     bool subtract = false) {
+    size_t n = same(a.size(), b.size());
+    Packed pa = pack(a), pb = pack(b);
+    std::vector<std::uint8_t> out(n * 64), inf(n);
+    ck(sylow_b200_g1_add_batch(ctx_, pa.pts.data(), pa.inf.data(), pb.pts.data(), pb.inf.data(), n, subtract ? 1 : 0,
+                               out.data(), inf.data()), "g1_add_batch");
+    std::vector<G1Affine> r(n);
+    for (size_t i = 0; i < n; i++) { std::memcpy(&r[i].x, &out[64 * i], 64); r[i].infinity = inf[i]; }
+    return r;
+  }
+  std::vector<G2Affine> g2_add_batch(const std::vector<G2Affine>& a, const std::vector<G2Affine>& b,
+                                     bool subtract = false) {
+    size_t n = same(a.size(), b.size());
+    Packed pa = pack(a), pb = pack(b);
+    std::vector<std::uint8_t> out(n * 128), inf(n);
+    ck(sylow_b200_g2_add_batch(ctx_, pa.pts.data(), pa.inf.data(), pb.pts.data(), pb.inf.data(), n, subtract ? 1 : 0,
+                               out.data(), inf.data()), "g2_add_batch");
+    std::vector<G2Affine> r(n);
+    for (size_t i = 0; i < n; i++) { std::memcpy(&r[i].x, &out[128 * i], 128); r[i].infinity = inf[i]; }
+    return r;
+  }
   // Threshold aggregation: `n_sets` sets of `t` shares; ids[s*t + i] is the participant id of share i of set s.
   // out[s] = sum_i lambda_i * sigs[s*t + i] with the Lagrange coefficients at 0 (examples/dkg.rs:190-226).
   std::vector<G1Affine> threshold_aggregate_batch(const std::vector<std::uint64_t>& ids,

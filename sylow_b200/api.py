@@ -310,6 +310,43 @@ class Engine:
         self._call("sylow_b200_eip197_pairing_check_batch", inputs, k, n, ok, st)
         return ok.astype(bool), st
 
+    def _eip196(self, symbol, width, inputs):
+        inputs = _rows(inputs, width, "inputs")
+        n = inputs.shape[0]
+        out = np.empty((n, 64), dtype=np.uint8)
+        st = np.empty(n, dtype=np.int8)
+        self._call(symbol, inputs, n, out, st)
+        return out, st
+
+    def eip196_add_batch(self, inputs):
+        """EIP-196 ecAdd bodies: inputs (n, 128) big-endian x1 || y1 || x2 || y2 (the caller pads or truncates calldata
+        to 128 bytes); returns (out (n, 64) big-endian, all zero for infinity and for a failed input; int8 status: 0,
+        ERR_DECODE or ERR_NOT_ON_CURVE)."""
+        return self._eip196("sylow_b200_eip196_add_batch", 128, inputs)
+
+    def eip196_mul_batch(self, inputs):
+        """EIP-196 ecMul bodies: inputs (n, 96) big-endian x || y || s, s any 256-bit integer; returns like
+        eip196_add_batch."""
+        return self._eip196("sylow_b200_eip196_mul_batch", 96, inputs)
+
+    # ------------------------------------------------------------------ group law
+    def _add(self, symbol, width, a, b, a_inf, b_inf, subtract):
+        a = _rows(a, width, "a")
+        n = a.shape[0]
+        out = np.empty((n, width), dtype=np.uint8)
+        out_inf = np.empty(n, dtype=np.uint8)
+        self._call(symbol, a, _flags(a_inf, n, "a_inf"), _rows(b, width, "b", n), _flags(b_inf, n, "b_inf"), n,
+                   int(bool(subtract)), out, out_inf)
+        return out, out_inf
+
+    def g1_add_batch(self, a, b, a_inf=None, b_inf=None, subtract=False):
+        """a[i] + b[i] (a[i] - b[i] with subtract) in G1, affine: (out (n, 64), out_inf (n,))."""
+        return self._add("sylow_b200_g1_add_batch", 64, a, b, a_inf, b_inf, subtract)
+
+    def g2_add_batch(self, a, b, a_inf=None, b_inf=None, subtract=False):
+        """a[i] + b[i] (a[i] - b[i] with subtract) in G2, affine: (out (n, 128), out_inf (n,))."""
+        return self._add("sylow_b200_g2_add_batch", 128, a, b, a_inf, b_inf, subtract)
+
     # ------------------------------------------------------------------ scalar multiplication
     def _mul(self, symbol, width, pts, scalars, pts_inf):
         pts = _rows(pts, width, "pts")
@@ -539,6 +576,14 @@ class Engine:
     def g2_mul_batch_dev(self, d_pts, d_scalars, d_out, d_out_inf=None, d_pts_inf=None):
         self._call("sylow_b200_g2_mul_batch_dev", d_pts, d_pts_inf, d_scalars, d_pts.shape[0], d_out, d_out_inf,
                    self._stream())
+
+    def g1_add_batch_dev(self, d_a, d_b, d_out, d_out_inf=None, d_a_inf=None, d_b_inf=None, subtract=False):
+        self._call("sylow_b200_g1_add_batch_dev", d_a, d_a_inf, d_b, d_b_inf, d_a.shape[0], int(bool(subtract)), d_out,
+                   d_out_inf, self._stream())
+
+    def g2_add_batch_dev(self, d_a, d_b, d_out, d_out_inf=None, d_a_inf=None, d_b_inf=None, subtract=False):
+        self._call("sylow_b200_g2_add_batch_dev", d_a, d_a_inf, d_b, d_b_inf, d_a.shape[0], int(bool(subtract)), d_out,
+                   d_out_inf, self._stream())
 
     def g1_mul_generator_batch_dev(self, d_scalars, d_out, d_out_inf=None):
         self._call("sylow_b200_g1_mul_generator_batch_dev", d_scalars, d_scalars.shape[0], d_out, d_out_inf,

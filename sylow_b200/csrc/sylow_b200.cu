@@ -15,6 +15,7 @@
 #include "wire.cuh"
 #include "kernels_pairing.cuh"
 #include "miller_tables.cuh"
+#include "group_law.cuh"
 #include "launch_plan.h"
 
 using namespace sylow;
@@ -355,6 +356,43 @@ k_g2_mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scal
   mul_gen<Fp2>(table, scalars, n, out, out_inf, proj_out);
 }
 
+// out[i] = affine(a[i] + b[i]), or affine(a[i] - b[i]) when subtract != 0 (add_pair, group_law.cuh); large batches
+// leave projective points in proj_out for affine_tail
+template <class F>
+__device__ __forceinline__ void add_batch(const uint8_t* __restrict__ a, const uint8_t* __restrict__ a_inf,
+                                          const uint8_t* __restrict__ b, const uint8_t* __restrict__ b_inf, size_t n,
+                                          int subtract, uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
+                                          uint8_t* __restrict__ proj_out) {
+  constexpr size_t W = sizeof(F);
+  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t i = i0 < n ? i0 : n - 1;  // the inversion of proj_to_affine is block-synchronised: every thread runs it
+  Proj<F> q = add_pair<F>(a, a_inf, b, b_inf, i, subtract);
+  if (proj_out) {
+    if (i0 >= n) return;
+    f_store_raw(proj_out + i * 3 * W, q.x);
+    f_store_raw(proj_out + i * 3 * W + W, q.y);
+    f_store_raw(proj_out + i * 3 * W + 2 * W, q.z);
+    return;
+  }
+  Affine<F> r = proj_to_affine(q);
+  if (i0 >= n) return;
+  f_store(out + i * 2 * W, r.x);
+  f_store(out + i * 2 * W + W, r.y);
+  if (out_inf) out_inf[i] = r.inf;
+}
+__global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
+k_g1_add(const uint8_t* __restrict__ a, const uint8_t* __restrict__ a_inf, const uint8_t* __restrict__ b,
+         const uint8_t* __restrict__ b_inf, size_t n, int subtract, uint8_t* __restrict__ out,
+         uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  add_batch<Fp>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj_out);
+}
+__global__ void __launch_bounds__(SY_G2_THREADS, SY_G2_MINB)
+k_g2_add(const uint8_t* __restrict__ a, const uint8_t* __restrict__ a_inf, const uint8_t* __restrict__ b,
+         const uint8_t* __restrict__ b_inf, size_t n, int subtract, uint8_t* __restrict__ out,
+         uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  add_batch<Fp2>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj_out);
+}
+
 // out[i] = affine(+-hash_to_curve(msg_i)); status[i] = 1 if the SvdW sqrt check failed
 __global__ void __launch_bounds__(SY_HASH_THREADS, SY_G1_MINB)
 k_hash_to_g1(const uint8_t* __restrict__ msgs, const uint64_t* __restrict__ offsets, size_t n,
@@ -387,15 +425,7 @@ __global__ void k_g1_validate(const uint8_t* __restrict__ g1, const uint8_t* __r
                               int8_t* __restrict__ status, int keep_errors) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  Fp xr = fp_load_raw(g1 + i * 64), yr = fp_load_raw(g1 + i * 64 + 32);
-  int8_t st = keep_errors ? status[i] : 0;
-  if (st == 0 && !(inf && inf[i])) {
-    if (!fp_raw_is_canonical(xr) || !fp_raw_is_canonical(yr))
-      st = SYLOW_B200_ERR_DECODE;
-    else if (!g1_on_curve(fp_to_mont(xr), fp_to_mont(yr)))
-      st = SYLOW_B200_ERR_NOT_ON_CURVE;
-  }
-  status[i] = st;
+  status[i] = g1_validate_item(g1, inf, status, i, keep_errors);
 }
 
 // + SYLOW_B200_ERR_NOT_IN_SUBGROUP: (x+1)Q + psi(xQ) + psi^2(xQ) != psi^3(2xQ)   (g2.rs:279-297, :460-525)
@@ -424,84 +454,13 @@ k_g2_validate(const uint8_t* __restrict__ g2, const uint8_t* __restrict__ inf, s
 }
 
 
-// ---- big-endian codecs (SURVEY.md 8f-2) -------------------------------------------------------------
-// 32 big-endian bytes -> Fp limbs (little-endian words), no reduction
-__device__ __forceinline__ Fp fp_from_be32(const uint8_t* b, uint32_t top_mask) {
-  Fp r;
-#pragma unroll
-  for (int i = 0; i < 8; i++) {
-    const uint8_t* q = b + 28 - 4 * i;
-    r.l[i] = ((uint32_t)q[0] << 24) | ((uint32_t)q[1] << 16) | ((uint32_t)q[2] << 8) | q[3];
-  }
-  r.l[7] &= top_mask;
-  return r;
-}
-__device__ __forceinline__ void fp_to_be32(uint8_t* b, const Fp& v) {
-#pragma unroll
-  for (int i = 0; i < 8; i++) {
-    uint8_t* q = b + 28 - 4 * i;
-    q[0] = (uint8_t)(v.l[i] >> 24);
-    q[1] = (uint8_t)(v.l[i] >> 16);
-    q[2] = (uint8_t)(v.l[i] >> 8);
-    q[3] = (uint8_t)v.l[i];
-  }
-}
-__device__ __forceinline__ bool fp_raw_is_u32(const Fp& a, uint32_t v) {
-  uint32_t o = a.l[0] ^ v;
-#pragma unroll
-  for (int i = 1; i < 8; i++) o |= a.l[i];
-  return o == 0;
-}
-// NF big-endian field elements per point (2 for G1, 4 for G2 with the imaginary parts first,
-// g2.rs:325-328) -> little-endian wire form + infinity flag + decode status.
-//   mode 0: sylow's codec (g1.rs:151-280, g2.rs:319-433): bit 7 of byte 0 flags infinity and must come
-//           with x = 0, y = 1;   mode 1: EIP-196/197: the all-zero encoding is the point at infinity
-//           (examples/reth_bn128.rs:118-126,187-194) and there is no flag bit.
+// ---- big-endian codecs (group_law.cuh) --------------------------------------------------------------
 template <int NF>
 __global__ void k_decode_be(const uint8_t* __restrict__ be, size_t stride, size_t n, int mode, uint8_t* __restrict__ out,
                             uint8_t* __restrict__ out_inf, int8_t* __restrict__ status) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const uint8_t* b = be + i * stride;
-  bool flag = mode == 0 && (b[0] >> 7);
-  Fp f[NF];
-  bool canon = true, all_zero = true;
-  for (int j = 0; j < NF; j++) {
-    f[j] = fp_from_be32(b + 32 * j, (mode == 0 && j == 0) ? 0x7fffffffu : 0xffffffffu);
-    canon &= fp_raw_is_canonical(f[j]);
-    all_zero &= fp_raw_is_u32(f[j], 0);
-  }
-  // wire order: G1 (x, y); G2 (x.c0, x.c1, y.c0, y.c1) from (x.c1, x.c0, y.c1, y.c0)
-  Fp w[NF];
-  if (NF == 2) {
-    w[0] = f[0];
-    w[1] = f[1];
-  } else {
-    w[0] = f[1];
-    w[1] = f[0];
-    w[2] = f[3];
-    w[3] = f[2];
-  }
-  bool x_zero = true, y_one = true;
-  for (int j = 0; j < NF / 2; j++) x_zero &= fp_raw_is_u32(w[j], 0);
-  for (int j = 0; j < NF / 2; j++) y_one &= fp_raw_is_u32(w[NF / 2 + j], j == 0 ? 1u : 0u);
-  int8_t st = canon ? 0 : SYLOW_B200_ERR_DECODE;
-  bool inf = false;
-  if (mode == 0) {
-    if (flag) {
-      inf = true;
-      if (st == 0 && !(x_zero && y_one)) st = SYLOW_B200_ERR_DECODE;
-    }
-  } else {
-    inf = all_zero;
-  }
-  if (inf || st != 0) {  // GroupAffine::zero(): (0, 1, infinity)
-    for (int j = 0; j < NF; j++) w[j] = fp_zero();
-    w[NF / 2].l[0] = 1;
-  }
-  for (int j = 0; j < NF; j++) fp_store_raw(out + i * (32 * NF) + 32 * j, w[j]);
-  out_inf[i] = inf ? 1 : 0;
-  status[i] = st;
+  decode_be_item<NF>(be + i * stride, mode, out + i * (32 * NF), out_inf + i, status + i);
 }
 
 // wire form -> big-endian (to_be_bytes / to_be_bytes_scrubbed, g1.rs:136-160, g2.rs:319-333)
@@ -528,6 +487,20 @@ __global__ void k_encode_be(const uint8_t* __restrict__ pts, const uint8_t* __re
     fp_to_be32(b + 96, w[2]);
   }
   if (is_inf && !scrub) b[0] |= 0x80;
+}
+
+// ecMul scalars: the 32 big-endian bytes at in + i * stride -> out[i], 32 bytes little-endian (k_g1_mul's form)
+__global__ void k_eip196_scalars(const uint8_t* __restrict__ in, size_t stride, size_t n, uint8_t* __restrict__ out) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) eip196_scalar_item(in + i * stride, out + i * 32);
+}
+// EIP-196 results: the statuses of each input's one (st_b null) or two points folded, and the 64-byte big-endian
+// point, all zero for infinity and for a failed input
+__global__ void k_eip196_finish(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ inf,
+                                const int8_t* __restrict__ st_a, const int8_t* __restrict__ st_b, size_t n,
+                                uint8_t* __restrict__ out, int8_t* __restrict__ status) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) eip196_finish_item(pts + i * 64, inf[i], st_a[i], st_b ? st_b[i] : 0, out + i * 64, status + i);
 }
 
 // per check: the first non-zero pair status wins and forces ok = 0
@@ -1469,9 +1442,20 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
 // ctx->proj and convert them to affine coordinates afterwards, with one inversion per SY_AFF_K points (affine_tail);
 // smaller ones convert each point in the kernel (*proj = null).
 #define SY_AFF_MIN_BATCH 32768
-static int affine_stage(sylow_b200_ctx* ctx, size_t n, size_t proj_bytes, uint8_t** proj) {
+// The pointwise additions (k_g1_add, k_g2_add) are short enough that below these sizes the launch of affine_tail and
+// its serial walk over SY_AFF_K points per thread cost more than an inversion in every thread; measured crossovers on
+// a B200 (DESIGN.md section 4, item 26): G1 between 2^15 and 2^16 points, G2 between 2^16 and 2^17.  The definitions
+// can be overridden only to build the variants tools/group_law_time.py times on both sides of them.
+#ifndef SY_G1_ADD_AFF_MIN_BATCH
+#define SY_G1_ADD_AFF_MIN_BATCH 65536
+#endif
+#ifndef SY_G2_ADD_AFF_MIN_BATCH
+#define SY_G2_ADD_AFF_MIN_BATCH 131072
+#endif
+static int affine_stage(sylow_b200_ctx* ctx, size_t n, size_t proj_bytes, uint8_t** proj,
+                        size_t min_batch = SY_AFF_MIN_BATCH) {
   *proj = nullptr;
-  if (n < SY_AFF_MIN_BATCH) return 0;
+  if (n < min_batch) return 0;
   CKS(reserve(ctx, ctx->proj, n * proj_bytes));
   *proj = ctx->proj.p;
   return 0;
@@ -1668,6 +1652,34 @@ int sylow_b200_g1_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_
 int sylow_b200_g2_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
                                           uint8_t* d_out_inf, void* stream) {
   return mul_gen_dev(ctx, 1, d_scalars, n, d_out, d_out_inf, stream);
+}
+
+// out[i] = affine(a[i] +- b[i]) in G1 (g2 = 0) or G2 (add_pair, group_law.cuh)
+static int add_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* a, const uint8_t* a_inf, const uint8_t* b,
+                   const uint8_t* b_inf, size_t n, int subtract, uint8_t* out, uint8_t* out_inf, void* stream) {
+  ENTER_DEV(ctx);
+  if (n && (!a || !b || !out)) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  cudaStream_t s = pick(ctx, stream);
+  uint8_t* proj;
+  CKS(affine_stage(ctx, n, g2 ? 192 : 96, &proj, g2 ? SY_G2_ADD_AFF_MIN_BATCH : SY_G1_ADD_AFF_MIN_BATCH));
+  if (g2)
+    k_g2_add<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj);
+  else
+    k_g1_add<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj);
+  LAUNCHED(ctx);
+  if (proj) CKS(affine_tail(ctx, g2, proj, n, 0, out, out_inf, s));
+  return 0;
+}
+int sylow_b200_g1_add_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_a, const uint8_t* d_a_inf, const uint8_t* d_b,
+                                const uint8_t* d_b_inf, size_t n, int subtract, uint8_t* d_out, uint8_t* d_out_inf,
+                                void* stream) {
+  return add_dev(ctx, 0, d_a, d_a_inf, d_b, d_b_inf, n, subtract, d_out, d_out_inf, stream);
+}
+int sylow_b200_g2_add_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_a, const uint8_t* d_a_inf, const uint8_t* d_b,
+                                const uint8_t* d_b_inf, size_t n, int subtract, uint8_t* d_out, uint8_t* d_out_inf,
+                                void* stream) {
+  return add_dev(ctx, 1, d_a, d_a_inf, d_b, d_b_inf, n, subtract, d_out, d_out_inf, stream);
 }
 
 // f[i] = miller(sig_i, G2gen) * miller(-H(m_i), pk_i) for every signature, Montgomery form, in scratch0:
@@ -2076,6 +2088,37 @@ int sylow_b200_g1_mul_generator_batch(sylow_b200_ctx* ctx, const uint8_t* scalar
 int sylow_b200_g2_mul_generator_batch(sylow_b200_ctx* ctx, const uint8_t* scalars, size_t n, uint8_t* out,
                                       uint8_t* out_inf) {
   return mul_host(ctx, 1, nullptr, nullptr, scalars, n, out, out_inf);
+}
+
+static int add_host(sylow_b200_ctx* ctx, int g2, const uint8_t* a, const uint8_t* a_inf, const uint8_t* b,
+                    const uint8_t* b_inf, size_t n, int subtract, uint8_t* out, uint8_t* out_inf) {
+  const size_t pb = g2 ? 128 : 64;
+  if (is_multi(ctx) && a && b && out) {
+    return multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t, size_t off, size_t m) {
+      return add_host(c, g2, a + off * pb, adv(a_inf, off), b + off * pb, adv(b_inf, off), m, subtract, out + off * pb,
+                      adv(out_inf, off));
+    });
+  }
+  ENTER(ctx);
+  if (n && (!a || !b || !out)) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  Staging io(ctx);
+  uint8_t* d_out = io.area(n * pb);
+  const uint8_t *da = io.up(a, n * pb), *db = io.up(b, n * pb), *dai = io.up(a_inf, n), *dbi = io.up(b_inf, n);
+  uint8_t* d_out_inf = io.area(n);
+  CKS(io.err);
+  CKS(add_dev(ctx, g2, da, dai, db, dbi, n, subtract, d_out, d_out_inf, nullptr));
+  io.down(out, d_out, n * pb);
+  if (out_inf) io.down(out_inf, d_out_inf, n);
+  return io.finish();
+}
+int sylow_b200_g1_add_batch(sylow_b200_ctx* ctx, const uint8_t* a, const uint8_t* a_inf, const uint8_t* b,
+                            const uint8_t* b_inf, size_t n, int subtract, uint8_t* out, uint8_t* out_inf) {
+  return add_host(ctx, 0, a, a_inf, b, b_inf, n, subtract, out, out_inf);
+}
+int sylow_b200_g2_add_batch(sylow_b200_ctx* ctx, const uint8_t* a, const uint8_t* a_inf, const uint8_t* b,
+                            const uint8_t* b_inf, size_t n, int subtract, uint8_t* out, uint8_t* out_inf) {
+  return add_host(ctx, 1, a, a_inf, b, b_inf, n, subtract, out, out_inf);
 }
 
 // the end of a hashing host form: finishes with the hash-to-curve failure flag, then CannotHashToGroup if it is set
@@ -2555,6 +2598,57 @@ int sylow_b200_eip197_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* in
   io.down(ok_out, d_ok, n_checks);
   io.down(status_out, d_st, n_checks);
   return io.finish();
+}
+
+// The EIP-196 ecAdd (mul = 0: x1 || y1 || x2 || y2, 128 B) and ecMul (mul = 1: x || y || s, 96 B) bodies over n
+// inputs: decode and validate the points, add or multiply, and encode.  A failed input's point decodes to (0, 1) or
+// stays off the curve; the group law runs on it as on any other (complete formulas, no memory it does not own) and
+// k_eip196_finish discards the result.
+static int eip196_host(sylow_b200_ctx* ctx, int mul, const uint8_t* input, size_t n, uint8_t* out, int8_t* status_out) {
+  const size_t stride = mul ? 96 : 128;
+  if (is_multi(ctx) && input && out && status_out) {
+    return multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t, size_t off, size_t m) {
+      return eip196_host(c, mul, input + off * stride, m, out + off * 64, status_out + off);
+    });
+  }
+  ENTER(ctx);
+  if (n && (!input || !out || !status_out)) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  Staging io(ctx);
+  const uint8_t* din = io.up(input, n * stride);
+  uint8_t *da = io.area(n * 64), *db = io.area(n * 64), *d_res = io.area(n * 64), *d_be = io.area(n * 64);
+  uint8_t* flags = io.area(6 * n);  // a_inf, b_inf, res_inf, then the int8 statuses of a, b and the result
+  CKS(io.err);
+  uint8_t *a_inf = flags, *b_inf = flags + n, *res_inf = flags + 2 * n;
+  int8_t* st_a = reinterpret_cast<int8_t*>(flags + 3 * n);
+  int8_t *st_b = mul ? nullptr : st_a + n, *st = st_a + 2 * n;
+  const unsigned blocks = nblocks(n, 128);
+  k_decode_be<2><<<blocks, 128, 0, ctx->stream>>>(din, stride, n, 1, da, a_inf, st_a);
+  LAUNCHED(ctx);
+  k_g1_validate<<<blocks, 128, 0, ctx->stream>>>(da, a_inf, n, st_a, 1);
+  LAUNCHED(ctx);
+  if (mul) {
+    k_eip196_scalars<<<blocks, 128, 0, ctx->stream>>>(din + 64, stride, n, db);
+    LAUNCHED(ctx);
+    CKS(sylow_b200_g1_mul_batch_dev(ctx, da, a_inf, db, n, d_res, res_inf, nullptr));
+  } else {
+    k_decode_be<2><<<blocks, 128, 0, ctx->stream>>>(din + 64, stride, n, 1, db, b_inf, st_b);
+    LAUNCHED(ctx);
+    k_g1_validate<<<blocks, 128, 0, ctx->stream>>>(db, b_inf, n, st_b, 1);
+    LAUNCHED(ctx);
+    CKS(add_dev(ctx, 0, da, a_inf, db, b_inf, n, 0, d_res, res_inf, nullptr));
+  }
+  k_eip196_finish<<<blocks, 128, 0, ctx->stream>>>(d_res, res_inf, st_a, st_b, n, d_be, st);
+  LAUNCHED(ctx);
+  io.down(out, d_be, n * 64);
+  io.down(status_out, st, n);
+  return io.finish();
+}
+int sylow_b200_eip196_add_batch(sylow_b200_ctx* ctx, const uint8_t* input, size_t n, uint8_t* out, int8_t* status_out) {
+  return eip196_host(ctx, 0, input, n, out, status_out);
+}
+int sylow_b200_eip196_mul_batch(sylow_b200_ctx* ctx, const uint8_t* input, size_t n, uint8_t* out, int8_t* status_out) {
+  return eip196_host(ctx, 1, input, n, out, status_out);
 }
 
 int sylow_b200_gt_mul_batch(sylow_b200_ctx* ctx, const uint8_t* gt, const uint8_t* scalars, size_t n, uint8_t* out) {

@@ -121,6 +121,18 @@ class G1Affine:
 
     __rmul__ = __mul__
 
+    def _add(self, other: "G1Affine", subtract: bool) -> "G1Affine":
+        """`&G1Projective + / - &G1Projective` (group.rs:528-624) followed by the affine conversion."""
+        out, inf = engine().g1_add_batch(_arr(self._b(), 64), _arr(other._b(), 64), [int(self.infinity)],
+                                         [int(other.infinity)], subtract)
+        return _g1_from(out[0], inf[0])
+
+    def __add__(self, other: "G1Affine") -> "G1Affine":
+        return self._add(other, False)
+
+    def __sub__(self, other: "G1Affine") -> "G1Affine":
+        return self._add(other, True)
+
     def to_be_bytes(self) -> bytes:
         return bytes(engine().g1_to_be_bytes_batch(_arr(self._b(), 64), [int(self.infinity)])[0])
 
@@ -186,6 +198,17 @@ class G2Affine:
         return _g2_from(out[0], inf[0])
 
     __rmul__ = __mul__
+
+    def _add(self, other: "G2Affine", subtract: bool) -> "G2Affine":
+        out, inf = engine().g2_add_batch(_arr(self._b(), 128), _arr(other._b(), 128), [int(self.infinity)],
+                                         [int(other.infinity)], subtract)
+        return _g2_from(out[0], inf[0])
+
+    def __add__(self, other: "G2Affine") -> "G2Affine":
+        return self._add(other, False)
+
+    def __sub__(self, other: "G2Affine") -> "G2Affine":
+        return self._add(other, True)
 
     @classmethod
     def rand(cls) -> "G2Affine":
