@@ -659,6 +659,85 @@ __device__ __forceinline__ void acc_lift_sub(uint32_t* A, const uint32_t* Lp, co
         "r"(T[10]), "r"(T[11]), "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]), "r"(Lp[0]), "r"(Lp[1]), "r"(Lp[2]),
         "r"(Lp[3]), "r"(Lp[4]), "r"(Lp[5]), "r"(Lp[6]), "r"(Lp[7]));
 }
+// A = C + T and A = C - T (mod 2^544) for a 17-limb constant C: the first term of an accumulator together with its
+// whole lift (a table of fp.cuh or tower.cuh)
+__device__ __forceinline__ void acc_const_add(uint32_t* A, const uint32_t* C, const uint32_t* T) {
+  asm("add.cc.u32 %0, %17, %34;\n\t"
+      "addc.cc.u32 %1, %18, %35;\n\t"
+      "addc.cc.u32 %2, %19, %36;\n\t"
+      "addc.cc.u32 %3, %20, %37;\n\t"
+      "addc.cc.u32 %4, %21, %38;\n\t"
+      "addc.cc.u32 %5, %22, %39;\n\t"
+      "addc.cc.u32 %6, %23, %40;\n\t"
+      "addc.cc.u32 %7, %24, %41;\n\t"
+      "addc.cc.u32 %8, %25, %42;\n\t"
+      "addc.cc.u32 %9, %26, %43;\n\t"
+      "addc.cc.u32 %10, %27, %44;\n\t"
+      "addc.cc.u32 %11, %28, %45;\n\t"
+      "addc.cc.u32 %12, %29, %46;\n\t"
+      "addc.cc.u32 %13, %30, %47;\n\t"
+      "addc.cc.u32 %14, %31, %48;\n\t"
+      "addc.cc.u32 %15, %32, %49;\n\t"
+      "addc.u32 %16, %33, 0;"
+      : "=r"(A[0]), "=r"(A[1]), "=r"(A[2]), "=r"(A[3]), "=r"(A[4]), "=r"(A[5]), "=r"(A[6]), "=r"(A[7]), "=r"(A[8]),
+        "=r"(A[9]), "=r"(A[10]), "=r"(A[11]), "=r"(A[12]), "=r"(A[13]), "=r"(A[14]), "=r"(A[15]), "=r"(A[16])
+      : "r"(C[0]), "r"(C[1]), "r"(C[2]), "r"(C[3]), "r"(C[4]), "r"(C[5]), "r"(C[6]), "r"(C[7]), "r"(C[8]), "r"(C[9]),
+        "r"(C[10]), "r"(C[11]), "r"(C[12]), "r"(C[13]), "r"(C[14]), "r"(C[15]), "r"(C[16]), "r"(T[0]), "r"(T[1]),
+        "r"(T[2]), "r"(T[3]), "r"(T[4]), "r"(T[5]), "r"(T[6]), "r"(T[7]), "r"(T[8]), "r"(T[9]), "r"(T[10]), "r"(T[11]),
+        "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]));
+  SY_ACC_TOP(A);
+}
+__device__ __forceinline__ void acc_const_sub(uint32_t* A, const uint32_t* C, const uint32_t* T) {
+  asm("sub.cc.u32 %0, %17, %34;\n\t"
+      "subc.cc.u32 %1, %18, %35;\n\t"
+      "subc.cc.u32 %2, %19, %36;\n\t"
+      "subc.cc.u32 %3, %20, %37;\n\t"
+      "subc.cc.u32 %4, %21, %38;\n\t"
+      "subc.cc.u32 %5, %22, %39;\n\t"
+      "subc.cc.u32 %6, %23, %40;\n\t"
+      "subc.cc.u32 %7, %24, %41;\n\t"
+      "subc.cc.u32 %8, %25, %42;\n\t"
+      "subc.cc.u32 %9, %26, %43;\n\t"
+      "subc.cc.u32 %10, %27, %44;\n\t"
+      "subc.cc.u32 %11, %28, %45;\n\t"
+      "subc.cc.u32 %12, %29, %46;\n\t"
+      "subc.cc.u32 %13, %30, %47;\n\t"
+      "subc.cc.u32 %14, %31, %48;\n\t"
+      "subc.cc.u32 %15, %32, %49;\n\t"
+      "subc.u32 %16, %33, 0;"
+      : "=r"(A[0]), "=r"(A[1]), "=r"(A[2]), "=r"(A[3]), "=r"(A[4]), "=r"(A[5]), "=r"(A[6]), "=r"(A[7]), "=r"(A[8]),
+        "=r"(A[9]), "=r"(A[10]), "=r"(A[11]), "=r"(A[12]), "=r"(A[13]), "=r"(A[14]), "=r"(A[15]), "=r"(A[16])
+      : "r"(C[0]), "r"(C[1]), "r"(C[2]), "r"(C[3]), "r"(C[4]), "r"(C[5]), "r"(C[6]), "r"(C[7]), "r"(C[8]), "r"(C[9]),
+        "r"(C[10]), "r"(C[11]), "r"(C[12]), "r"(C[13]), "r"(C[14]), "r"(C[15]), "r"(C[16]), "r"(T[0]), "r"(T[1]),
+        "r"(T[2]), "r"(T[3]), "r"(T[4]), "r"(T[5]), "r"(T[6]), "r"(T[7]), "r"(T[8]), "r"(T[9]), "r"(T[10]), "r"(T[11]),
+        "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]));
+  SY_ACC_TOP(A);
+}
+// A = -T mod 2^544 (17 limbs)
+__device__ __forceinline__ void acc_neg(uint32_t* A, const uint32_t* T) {
+  asm("sub.cc.u32 %0, 0, %17;\n\t"
+      "subc.cc.u32 %1, 0, %18;\n\t"
+      "subc.cc.u32 %2, 0, %19;\n\t"
+      "subc.cc.u32 %3, 0, %20;\n\t"
+      "subc.cc.u32 %4, 0, %21;\n\t"
+      "subc.cc.u32 %5, 0, %22;\n\t"
+      "subc.cc.u32 %6, 0, %23;\n\t"
+      "subc.cc.u32 %7, 0, %24;\n\t"
+      "subc.cc.u32 %8, 0, %25;\n\t"
+      "subc.cc.u32 %9, 0, %26;\n\t"
+      "subc.cc.u32 %10, 0, %27;\n\t"
+      "subc.cc.u32 %11, 0, %28;\n\t"
+      "subc.cc.u32 %12, 0, %29;\n\t"
+      "subc.cc.u32 %13, 0, %30;\n\t"
+      "subc.cc.u32 %14, 0, %31;\n\t"
+      "subc.cc.u32 %15, 0, %32;\n\t"
+      "subc.u32 %16, 0, %33;"
+      : "=r"(A[0]), "=r"(A[1]), "=r"(A[2]), "=r"(A[3]), "=r"(A[4]), "=r"(A[5]), "=r"(A[6]), "=r"(A[7]), "=r"(A[8]),
+        "=r"(A[9]), "=r"(A[10]), "=r"(A[11]), "=r"(A[12]), "=r"(A[13]), "=r"(A[14]), "=r"(A[15]), "=r"(A[16])
+      : "r"(T[0]), "r"(T[1]), "r"(T[2]), "r"(T[3]), "r"(T[4]), "r"(T[5]), "r"(T[6]), "r"(T[7]), "r"(T[8]), "r"(T[9]),
+        "r"(T[10]), "r"(T[11]), "r"(T[12]), "r"(T[13]), "r"(T[14]), "r"(T[15]), "r"(T[16]));
+  SY_ACC_TOP(A);
+}
 // A += T
 __device__ __forceinline__ void acc_add(uint32_t* A, const uint32_t* T) {
   asm("add.cc.u32 %0, %0, %17;\n\t"
@@ -852,6 +931,30 @@ inline void acc_lift_sub(uint32_t* A, const uint32_t* Lp, const uint32_t* T) {
     bw = d >> 32;
   }
   A[16] = 0;
+}
+inline void acc_const_add(uint32_t* A, const uint32_t* C, const uint32_t* T) {
+  uint64_t c = 0;
+  for (int i = 0; i < 17; i++) {
+    c += (uint64_t)C[i] + (i < 16 ? T[i] : 0u);
+    A[i] = (uint32_t)c;
+    c >>= 32;
+  }
+}
+inline void acc_const_sub(uint32_t* A, const uint32_t* C, const uint32_t* T) {
+  int64_t bw = 0;
+  for (int i = 0; i < 17; i++) {
+    int64_t d = (int64_t)C[i] - (int64_t)(i < 16 ? T[i] : 0u) + bw;
+    A[i] = (uint32_t)d;
+    bw = d >> 32;
+  }
+}
+inline void acc_neg(uint32_t* A, const uint32_t* T) {
+  int64_t bw = 0;
+  for (int i = 0; i < 17; i++) {
+    int64_t d = -(int64_t)T[i] + bw;
+    A[i] = (uint32_t)d;
+    bw = d >> 32;
+  }
 }
 inline void acc_add(uint32_t* A, const uint32_t* T) {
   uint64_t c = 0;
@@ -1081,6 +1184,30 @@ SY_HD void u9_add_shl(uint32_t* r, const uint32_t* a, const uint32_t* b, int s) 
     c += (uint64_t)a[i] + t[i];
     r[i] = (uint32_t)c;
     c >>= 32;
+  }
+#endif
+}
+// r = a - b mod 2^288 (9 limbs; the caller's final sum, not each step, lies in [0, 2^262))
+SY_HD void u9_sub(uint32_t* r, const uint32_t* a, const uint32_t* b) {
+#if defined(__CUDA_ARCH__)
+  asm("sub.cc.u32 %0, %9, %18;\n\t"
+      "subc.cc.u32 %1, %10, %19;\n\t"
+      "subc.cc.u32 %2, %11, %20;\n\t"
+      "subc.cc.u32 %3, %12, %21;\n\t"
+      "subc.cc.u32 %4, %13, %22;\n\t"
+      "subc.cc.u32 %5, %14, %23;\n\t"
+      "subc.cc.u32 %6, %15, %24;\n\t"
+      "subc.cc.u32 %7, %16, %25;\n\t"
+      "subc.u32 %8, %17, %26;"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(a[4]), "r"(a[5]), "r"(a[6]), "r"(a[7]), "r"(a[8]),
+        "r"(b[0]), "r"(b[1]), "r"(b[2]), "r"(b[3]), "r"(b[4]), "r"(b[5]), "r"(b[6]), "r"(b[7]), "r"(b[8]));
+#else
+  int64_t bw = 0;
+  for (int i = 0; i < 9; i++) {
+    int64_t d = (int64_t)a[i] - (int64_t)b[i] + bw;
+    r[i] = (uint32_t)d;
+    bw = d >> 32;
   }
 #endif
 }
