@@ -8,19 +8,16 @@
 
 namespace sylow {
 
-SY_HD Fp f_load(const uint8_t* p, const Fp*) { return fp_load(p); }
-SY_HD Fp2 f_load(const uint8_t* p, const Fp2*) { return fp2_load(p); }
-
 // a[i] + b[i], or a[i] - b[i] when subtract != 0, for canonical affine points (x || y, 2 sizeof(F) bytes each) with
 // optional infinity flags; projective, Montgomery form.  proj_add_mixed is complete for a = O, a = b and a = -b but
 // ignores b.inf, so an infinite b selects a.  No data-dependent branches.
 template <class F>
 SY_HD Proj<F> add_pair(const uint8_t* a, const uint8_t* a_inf, const uint8_t* b, const uint8_t* b_inf, size_t i,
                        int subtract) {
+  // the loads of affine_load written out: through the call, k_g1_add spills 16 more bytes (CUDA 12.9, sm_100a)
   constexpr size_t W = sizeof(F);
-  const F* tag = nullptr;
-  Affine<F> pa{f_load(a + i * 2 * W, tag), f_load(a + i * 2 * W + W, tag), a_inf && a_inf[i]};
-  Affine<F> pb{f_load(b + i * 2 * W, tag), f_load(b + i * 2 * W + W, tag), b_inf && b_inf[i]};
+  Affine<F> pa{f_load<F>(a + i * 2 * W), f_load<F>(a + i * 2 * W + W), a_inf && a_inf[i]};
+  Affine<F> pb{f_load<F>(b + i * 2 * W), f_load<F>(b + i * 2 * W + W), b_inf && b_inf[i]};
   pb.y = f_select(subtract && !pb.inf, f_neg(pb.y), pb.y);
   Proj<F> p = affine_to_proj(pa);
   Proj<F> s = proj_add_mixed(p, pb);

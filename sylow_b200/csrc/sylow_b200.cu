@@ -194,27 +194,15 @@ __global__ void k_gt_is_one(const uint8_t* gt, size_t n, uint8_t* ok) {
   ok[c] = d == 0 ? 1 : 0;
 }
 
-SY_HD void g1_store_proj(uint8_t* p, const G1Proj& q) {
-  fp_store_raw(p, q.x);
-  fp_store_raw(p + 32, q.y);
-  fp_store_raw(p + 64, q.z);
-}
 // Projective (Montgomery form) -> affine wire format for a whole batch with Montgomery's trick: thread t owns the
 // SY_AFF_K points t, t + T, t + 2T, ... (coalesced), multiplies their Z together, inverts ONCE and unwinds.  A point at
 // infinity (Z = 0) enters the product as 1 and is written as (0, 1) + flag, like GroupAffine::from (group.rs:475-495).
 // F = Fp: G1, 96-byte projective / 64-byte affine points; F = Fp2: G2, 192 / 128 bytes.
 #define SY_AFF_K 8
-SY_HD Fp f_load_raw(const uint8_t* p, const Fp*) { return fp_load_raw(p); }
-SY_HD Fp2 f_load_raw(const uint8_t* p, const Fp2*) { return fp2_load_raw(p); }
-SY_HD void f_store(uint8_t* p, const Fp& v) { fp_store(p, v); }
-SY_HD void f_store(uint8_t* p, const Fp2& v) { fp2_store(p, v); }
-SY_HD void f_store_raw(uint8_t* p, const Fp& v) { fp_store_raw(p, v); }
-SY_HD void f_store_raw(uint8_t* p, const Fp2& v) { fp2_store_raw(p, v); }
 template <class F>
 __device__ __forceinline__ void batch_affine(const uint8_t* __restrict__ proj, size_t n, int negate,
                                              uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf) {
   constexpr size_t W = sizeof(F);  // bytes per coordinate in both encodings
-  const F* tag = nullptr;
   F one;
   f_set_one(one);
   const size_t T = (n + SY_AFF_K - 1) / SY_AFF_K;
@@ -224,7 +212,7 @@ __device__ __forceinline__ void batch_affine(const uint8_t* __restrict__ proj, s
   F acc = one;
   for (int j = 0; j < SY_AFF_K; j++) {
     size_t i = t + (size_t)j * T;
-    F z = i < n ? f_load_raw(proj + i * 3 * W + 2 * W, tag) : one;
+    F z = i < n ? f_load_raw<F>(proj + i * 3 * W + 2 * W) : one;
     z = f_select(f_is_zero(z), one, z);
     acc = f_mul(acc, z);
     pre[j] = acc;
@@ -233,13 +221,13 @@ __device__ __forceinline__ void batch_affine(const uint8_t* __restrict__ proj, s
   for (int j = SY_AFF_K - 1; j >= 0; j--) {
     size_t i = t + (size_t)j * T;
     if (i >= n) continue;  // only the last stride can be short; its z entered the product as 1
-    F z = f_load_raw(proj + i * 3 * W + 2 * W, tag);
+    F z = f_load_raw<F>(proj + i * 3 * W + 2 * W);
     bool inf = f_is_zero(z);
     z = f_select(inf, one, z);
     F zi = j ? f_mul(inv, pre[j - 1]) : inv;
     inv = f_mul(inv, z);
     if (t0 >= T) continue;
-    F x = f_mul(f_load_raw(proj + i * 3 * W, tag), zi), y = f_mul(f_load_raw(proj + i * 3 * W + W, tag), zi);
+    F x = f_mul(f_load_raw<F>(proj + i * 3 * W), zi), y = f_mul(f_load_raw<F>(proj + i * 3 * W + W), zi);
     if (inf) {
       f_set_zero(x);
       y = one;
@@ -261,24 +249,53 @@ k_g2_batch_affine(const uint8_t* __restrict__ proj, size_t n, uint8_t* __restric
   batch_affine<Fp2>(proj, n, 0, out, out_inf);
 }
 
-__global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
-k_g1_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf,
-                     const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
-                     uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
-  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  size_t i = i0 < n ? i0 : n - 1;  // all threads run the (block-synchronised) loops; surplus is discarded
-  G1Aff a{fp_load(pts + i * 64), fp_load(pts + i * 64 + 32), pts_inf && pts_inf[i]};
-  Fp k = fp_load_raw(scalars + i * 32);
-  G1Proj q = proj_scalar_mul_glv(affine_to_proj(a), k.l);
-  if (proj_out) {  // large batches: k_g1_batch_affine shares one inversion between eight points
-    if (i0 < n) g1_store_proj(proj_out + i * 96, q);
+// The result q of item i = min(i0, n - 1) of a point-batch kernel, from thread i0, to its output:
+//  - every thread of the block calls it, surplus threads (i0 >= n) included: proj_to_affine's inversion ladder is
+//    block-synchronised; surplus threads store nothing;
+//  - with proj_out (large batches) the raw projective record for batch_affine, which shares one inversion between
+//    SY_AFF_K points and applies the negation;
+//  - otherwise the affine wire form and flag, y negated when negate is set and the point is finite.
+template <class F>
+__device__ __forceinline__ void put_point(const Proj<F>& q, size_t i0, size_t i, size_t n, int negate,
+                                          uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
+                                          uint8_t* __restrict__ proj_out) {
+  constexpr size_t W = sizeof(F);
+  if (proj_out) {
+    if (i0 < n) proj_store_raw(proj_out + i * 3 * W, q);
     return;
   }
-  G1Aff r = proj_to_affine(q);
+  Affine<F> r = proj_to_affine(q);
   if (i0 >= n) return;
-  fp_store(out + i * 64, r.x);
-  fp_store(out + i * 64 + 32, r.y);
+  if (negate && !r.inf) r.y = f_neg(r.y);
+  f_store(out + i * 2 * W, r.x);
+  f_store(out + i * 2 * W + W, r.y);
   if (out_inf) out_inf[i] = r.inf;
+}
+
+// the variable-base ladders: GLV on G1, GLS on G2
+SY_HD G1Proj scalar_mul(const G1Proj& p, const uint32_t* k) { return proj_scalar_mul_glv(p, k); }
+SY_HD G2Proj scalar_mul(const G2Proj& p, const uint32_t* k) { return g2_scalar_mul_gls(p, k); }
+
+// out[i] = affine(scalars[i] * pts[i]) for any 256-bit scalar
+template <class F>
+__device__ __forceinline__ void mul_batch(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf,
+                                          const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
+                                          uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t i = i0 < n ? i0 : n - 1;  // every thread runs the block-synchronised ladder
+  Affine<F> a = affine_load<F>(pts, pts_inf, i);
+  Fp k = fp_load_raw(scalars + i * 32);
+  put_point(scalar_mul(affine_to_proj(a), k.l), i0, i, n, 0, out, out_inf, proj_out);
+}
+__global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
+k_g1_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf, const uint8_t* __restrict__ scalars,
+         size_t n, uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  mul_batch<Fp>(pts, pts_inf, scalars, n, out, out_inf, proj_out);
+}
+__global__ void __launch_bounds__(SY_G2_THREADS, SY_G2_MINB)
+k_g2_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf, const uint8_t* __restrict__ scalars,
+         size_t n, uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
+  mul_batch<Fp2>(pts, pts_inf, scalars, n, out, out_inf, proj_out);
 }
 
 // proj_out[i] = r_i * pts[i] (projective, Montgomery form), r_i the weight of item first_index + i
@@ -287,9 +304,9 @@ k_g1_mul_weight(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts
                 uint64_t first_index, size_t n, uint8_t* __restrict__ proj_out) {
   size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   size_t i = i0 < n ? i0 : n - 1;
-  G1Aff a{fp_load(pts + i * 64), fp_load(pts + i * 64 + 32), pts_inf && pts_inf[i]};
+  G1Aff a = affine_load<Fp>(pts, pts_inf, i);
   G1Proj q = proj_scalar_mul_u64(affine_to_proj(a), batch_weight(seed, first_index + i));
-  if (i0 < n) g1_store_proj(proj_out + i * 96, q);
+  if (i0 < n) proj_store_raw(proj_out + i * 96, q);
 }
 // out[i] = the 64-bit weight of item first_index + i (tests)
 __global__ void k_batch_weights(const __grid_constant__ WeightSeed seed, uint64_t first_index, size_t n, uint64_t* out) {
@@ -297,53 +314,15 @@ __global__ void k_batch_weights(const __grid_constant__ WeightSeed seed, uint64_
   if (i < n) out[i] = batch_weight(seed, first_index + i);
 }
 
-__global__ void __launch_bounds__(SY_G2_THREADS, SY_G2_MINB)
-k_g2_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ pts_inf,
-                       const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
-                       uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
-  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  size_t i = i0 < n ? i0 : n - 1;
-  G2Aff a{fp2_load(pts + i * 128), fp2_load(pts + i * 128 + 64), pts_inf && pts_inf[i]};
-  Fp k = fp_load_raw(scalars + i * 32);
-  G2Proj q = g2_scalar_mul_gls(affine_to_proj(a), k.l);
-  if (proj_out) {
-    if (i0 < n) {
-      fp2_store_raw(proj_out + i * 192, q.x);
-      fp2_store_raw(proj_out + i * 192 + 64, q.y);
-      fp2_store_raw(proj_out + i * 192 + 128, q.z);
-    }
-    return;
-  }
-  G2Aff r = proj_to_affine(q);
-  if (i0 >= n) return;
-  fp2_store(out + i * 128, r.x);
-  fp2_store(out + i * 128 + 64, r.y);
-  if (out_inf) out_inf[i] = r.inf;
-}
-
-// out[i] = affine(scalars[i] * G) for the generator G of `table` (gen_scalar_mul; ensure_mul_table), any 256-bit
-// scalar; large batches leave projective points in proj_out for affine_tail, like k_g1_mul / k_g2_mul
+// out[i] = affine(scalars[i] * G) for the generator G of `table` (gen_scalar_mul; ensure_mul_table), any 256-bit scalar
 template <class F>
 __device__ __forceinline__ void mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n,
                                         uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
                                         uint8_t* __restrict__ proj_out) {
-  constexpr size_t W = sizeof(F);
   size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  size_t i = i0 < n ? i0 : n - 1;  // the inversion of proj_to_affine is block-synchronised: every thread runs it
+  size_t i = i0 < n ? i0 : n - 1;
   Fp k = fp_load_raw(scalars + i * 32);
-  Proj<F> q = gen_scalar_mul<F>(table, k.l);
-  if (proj_out) {
-    if (i0 >= n) return;
-    f_store_raw(proj_out + i * 3 * W, q.x);
-    f_store_raw(proj_out + i * 3 * W + W, q.y);
-    f_store_raw(proj_out + i * 3 * W + 2 * W, q.z);
-    return;
-  }
-  Affine<F> r = proj_to_affine(q);
-  if (i0 >= n) return;
-  f_store(out + i * 2 * W, r.x);
-  f_store(out + i * 2 * W + W, r.y);
-  if (out_inf) out_inf[i] = r.inf;
+  put_point(gen_scalar_mul<F>(table, k.l), i0, i, n, 0, out, out_inf, proj_out);
 }
 __global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
 k_g1_mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
@@ -356,29 +335,15 @@ k_g2_mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scal
   mul_gen<Fp2>(table, scalars, n, out, out_inf, proj_out);
 }
 
-// out[i] = affine(a[i] + b[i]), or affine(a[i] - b[i]) when subtract != 0 (add_pair, group_law.cuh); large batches
-// leave projective points in proj_out for affine_tail
+// out[i] = affine(a[i] + b[i]), or affine(a[i] - b[i]) when subtract != 0 (add_pair, group_law.cuh)
 template <class F>
 __device__ __forceinline__ void add_batch(const uint8_t* __restrict__ a, const uint8_t* __restrict__ a_inf,
                                           const uint8_t* __restrict__ b, const uint8_t* __restrict__ b_inf, size_t n,
                                           int subtract, uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
                                           uint8_t* __restrict__ proj_out) {
-  constexpr size_t W = sizeof(F);
   size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  size_t i = i0 < n ? i0 : n - 1;  // the inversion of proj_to_affine is block-synchronised: every thread runs it
-  Proj<F> q = add_pair<F>(a, a_inf, b, b_inf, i, subtract);
-  if (proj_out) {
-    if (i0 >= n) return;
-    f_store_raw(proj_out + i * 3 * W, q.x);
-    f_store_raw(proj_out + i * 3 * W + W, q.y);
-    f_store_raw(proj_out + i * 3 * W + 2 * W, q.z);
-    return;
-  }
-  Affine<F> r = proj_to_affine(q);
-  if (i0 >= n) return;
-  f_store(out + i * 2 * W, r.x);
-  f_store(out + i * 2 * W + W, r.y);
-  if (out_inf) out_inf[i] = r.inf;
+  size_t i = i0 < n ? i0 : n - 1;
+  put_point(add_pair<F>(a, a_inf, b, b_inf, i, subtract), i0, i, n, 0, out, out_inf, proj_out);
 }
 __global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
 k_g1_add(const uint8_t* __restrict__ a, const uint8_t* __restrict__ a_inf, const uint8_t* __restrict__ b,
@@ -393,7 +358,7 @@ k_g2_add(const uint8_t* __restrict__ a, const uint8_t* __restrict__ a_inf, const
   add_batch<Fp2>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj_out);
 }
 
-// out[i] = affine(+-hash_to_curve(msg_i)); status[i] = 1 if the SvdW sqrt check failed
+// out[i] = affine(+-hash_to_curve(msg_i)); *fail_flag = 1 if the SvdW sqrt check failed for any message
 __global__ void __launch_bounds__(SY_HASH_THREADS, SY_G1_MINB)
 k_hash_to_g1(const uint8_t* __restrict__ msgs, const uint64_t* __restrict__ offsets, size_t n,
              const __grid_constant__ DstPrime dst, int negate, uint8_t* __restrict__ out,
@@ -403,22 +368,9 @@ k_hash_to_g1(const uint8_t* __restrict__ msgs, const uint64_t* __restrict__ offs
   uint64_t o0 = offsets[i], o1 = offsets[i + 1];
   G1Proj p;
   bool ok = hash_to_g1(msgs + o0, (size_t)(o1 - o0), dst.b, dst.len, p, dst.hash_id);
-  if (proj_out) {  // large batches: affine conversion (and the negation) in k_g1_batch_affine
-    if (i0 < n) {
-      if (!ok) atomicExch(fail_flag, 1);
-      g1_store_proj(proj_out + i * 96, p);
-    }
-    return;
-  }
-  G1Aff r = proj_to_affine(p);
-  if (i0 >= n) return;
-  if (!ok) atomicExch(fail_flag, 1);
-  if (negate && !r.inf) r.y = fp_neg(r.y);
-  fp_store(out + i * 64, r.x);
-  fp_store(out + i * 64 + 32, r.y);
-  if (out_inf) out_inf[i] = r.inf;
+  put_point(p, i0, i, n, negate, out, out_inf, proj_out);
+  if (i0 < n && !ok) atomicExch(fail_flag, 1);
 }
-
 
 // status[i]: 0 ok, SYLOW_B200_ERR_DECODE (a coordinate >= p), SYLOW_B200_ERR_NOT_ON_CURVE   (g1.rs:111-132)
 __global__ void k_g1_validate(const uint8_t* __restrict__ g1, const uint8_t* __restrict__ inf, size_t n,
@@ -587,24 +539,19 @@ k_g1_sum_strided(const uint8_t* __restrict__ in, const uint8_t* __restrict__ in_
   G1Proj acc = proj_zero<Fp>();
   for (size_t i = t; i < n; i += T) {
     G1Proj v;
-    if (affine_in) {
-      G1Aff a{fp_load(in + i * 64), fp_load(in + i * 64 + 32), in_inf && in_inf[i]};
-      v = affine_to_proj(a);
-    } else {
-      v = G1Proj{fp_load_raw(in + i * 96), fp_load_raw(in + i * 96 + 32), fp_load_raw(in + i * 96 + 64)};
-    }
+    if (affine_in)
+      v = affine_to_proj(affine_load<Fp>(in, in_inf, i));
+    else
+      v = proj_load_raw<Fp>(in + i * 96);
     acc = proj_add(acc, v);
   }
-  fp_store_raw(out + t * 96, acc.x);
-  fp_store_raw(out + t * 96 + 32, acc.y);
-  fp_store_raw(out + t * 96 + 64, acc.z);
+  proj_store_raw(out + t * 96, acc);
 }
 // one projective point (Montgomery form) -> affine wire format + infinity flag, optionally negated
 __global__ void k_g1_finish_sum(const uint8_t* __restrict__ in, int negate, uint8_t* __restrict__ out,
                                 uint8_t* __restrict__ out_inf) {
   if (blockIdx.x || threadIdx.x) return;
-  G1Proj p{fp_load_raw(in), fp_load_raw(in + 32), fp_load_raw(in + 64)};
-  G1Aff r = proj_to_affine(p);
+  G1Aff r = proj_to_affine(proj_load_raw<Fp>(in));
   if (negate && !r.inf) r.y = fp_neg(r.y);
   fp_store(out, r.x);
   fp_store(out + 32, r.y);
@@ -632,12 +579,10 @@ k_lagrange_mul(const uint64_t* __restrict__ ids, const uint8_t* __restrict__ sig
   Fr lam = fr_lagrange_at_zero(ids + s * t, t, i);
   uint32_t w[8];
   fr_to_words(w, lam);
-  G1Aff a{fp_load(sigs + g * 64), fp_load(sigs + g * 64 + 32), sigs_inf && sigs_inf[g]};
+  G1Aff a = affine_load<Fp>(sigs, sigs_inf, g);
   G1Proj r = proj_scalar_mul_glv(affine_to_proj(a), w);
   if (g0 != g) return;
-  fp_store_raw(out + g * 96, r.x);
-  fp_store_raw(out + g * 96 + 32, r.y);
-  fp_store_raw(out + g * 96 + 64, r.z);
+  proj_store_raw(out + g * 96, r);
 }
 // One warp per set: sum of the set's t projective points, then affine wire format + infinity flag.
 __global__ void __launch_bounds__(128) k_g1_segment_sum(const uint8_t* __restrict__ in, size_t n_sets, size_t t,
@@ -647,10 +592,7 @@ __global__ void __launch_bounds__(128) k_g1_segment_sum(const uint8_t* __restric
   size_t s = s0 < n_sets ? s0 : n_sets - 1;
   unsigned lane = threadIdx.x & 31;
   G1Proj acc = proj_zero<Fp>();
-  for (size_t i = lane; i < t; i += 32) {
-    const uint8_t* p = in + (s * t + i) * 96;
-    acc = proj_add(acc, G1Proj{fp_load_raw(p), fp_load_raw(p + 32), fp_load_raw(p + 64)});
-  }
+  for (size_t i = lane; i < t; i += 32) acc = proj_add(acc, proj_load_raw<Fp>(in + (s * t + i) * 96));
   sh[threadIdx.x] = acc;
   __syncthreads();
   for (unsigned off = 16; off > 0; off >>= 1) {
@@ -736,7 +678,6 @@ __global__ void k_msm_scatter(const uint8_t* __restrict__ scalars, const uint8_t
     }
   }
 }
-SY_HD G1Proj g1_load_proj(const uint8_t* p) { return G1Proj{fp_load_raw(p), fp_load_raw(p + 32), fp_load_raw(p + 64)}; }
 __global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
 k_msm_item_sum(const uint8_t* __restrict__ pts, size_t n, int nw, size_t max_items,
                const uint32_t* __restrict__ item_start, const uint32_t* __restrict__ item_len,
@@ -752,7 +693,7 @@ k_msm_item_sum(const uint8_t* __restrict__ pts, size_t n, int nw, size_t max_ite
     const uint8_t* p = pts + (size_t)list[j] * 64;  // Montgomery form (converted once by k_fp_convert)
     acc = proj_add(acc, G1Proj{fp_load_raw(p), fp_load_raw(p + 32), fp_one()});
   }
-  g1_store_proj(item_sum + t * 96, acc);
+  proj_store_raw(item_sum + t * 96, acc);
 }
 __global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
 k_msm_bucket_sum(int c, int nw, size_t max_items, const uint32_t* __restrict__ count,
@@ -763,8 +704,9 @@ k_msm_bucket_sum(int c, int nw, size_t max_items, const uint32_t* __restrict__ c
   size_t w = b >> c;
   uint32_t items = (count[b] + SY_MSM_ITEM - 1) / SY_MSM_ITEM;
   G1Proj acc = proj_zero<Fp>();
-  for (uint32_t j = 0; j < items; j++) acc = proj_add(acc, g1_load_proj(item_sum + (w * max_items + item_first[b] + j) * 96));
-  g1_store_proj(buckets + b * 96, acc);
+  for (uint32_t j = 0; j < items; j++)
+    acc = proj_add(acc, proj_load_raw<Fp>(item_sum + (w * max_items + item_first[b] + j) * 96));
+  proj_store_raw(buckets + b * 96, acc);
 }
 // small multiple m * P, m < 2^16, double-and-add from the top bit
 SY_HD G1Proj g1_mul_small(const G1Proj& p, uint32_t m) {
@@ -787,20 +729,21 @@ __global__ void __launch_bounds__(64) k_msm_chunk_reduce(const uint8_t* __restri
   // to local weights 1 .. d1 - d0; digit 0 never holds points, the top digit 2^c - 1 is < 2^c = last d1
   G1Proj run = proj_zero<Fp>(), sum = proj_zero<Fp>();
   for (uint32_t d = d1; d > d0; d--) {
-    if (d < (1u << c)) run = proj_add(run, g1_load_proj(buckets + (((size_t)w << c) + d) * 96));
+    if (d < (1u << c)) run = proj_add(run, proj_load_raw<Fp>(buckets + (((size_t)w << c) + d) * 96));
     sum = proj_add(sum, run);
   }
   // sum = sum_{d in (d0, d1]} (d - d0) B_d, run = sum B_d; the window value needs d B_d = (d - d0) B_d + d0 B_d
   G1Proj r = proj_add(sum, g1_mul_small(run, d0));
-  g1_store_proj(partial + (size_t)t * 96, r);
+  proj_store_raw(partial + (size_t)t * 96, r);
 }
 // R_w = sum of the 64 chunk values of window w (one thread per window), written over the window's first partial
 __global__ void k_msm_window_sum(uint8_t* __restrict__ partial, int nw) {
   int w = blockIdx.x * blockDim.x + threadIdx.x;
   if (w >= nw) return;
   G1Proj r = proj_zero<Fp>();
-  for (int j = 0; j < SY_MSM_CHUNKS; j++) r = proj_add(r, g1_load_proj(partial + ((size_t)w * SY_MSM_CHUNKS + j) * 96));
-  g1_store_proj(partial + (size_t)w * SY_MSM_CHUNKS * 96, r);
+  for (int j = 0; j < SY_MSM_CHUNKS; j++)
+    r = proj_add(r, proj_load_raw<Fp>(partial + ((size_t)w * SY_MSM_CHUNKS + j) * 96));
+  proj_store_raw(partial + (size_t)w * SY_MSM_CHUNKS * 96, r);
 }
 // Horner over the windows: ((R_{nw-1} 2^c + R_{nw-2}) 2^c + ...) - 256 doublings, the only serial part
 __global__ void k_msm_window_final(const uint8_t* __restrict__ partial, int c, int nw, uint8_t* __restrict__ out_proj) {
@@ -808,9 +751,9 @@ __global__ void k_msm_window_final(const uint8_t* __restrict__ partial, int c, i
   G1Proj acc = proj_zero<Fp>();
   for (int w = nw - 1; w >= 0; w--) {
     for (int b = 0; b < c; b++) acc = proj_double(acc);
-    acc = proj_add(acc, g1_load_proj(partial + (size_t)w * SY_MSM_CHUNKS * 96));
+    acc = proj_add(acc, proj_load_raw<Fp>(partial + (size_t)w * SY_MSM_CHUNKS * 96));
   }
-  g1_store_proj(out_proj, acc);
+  proj_store_raw(out_proj, acc);
 }
 
 __global__ void k_fp_op(int op, const uint8_t* a, const uint8_t* b, size_t n, uint8_t* out) {
@@ -1226,6 +1169,44 @@ static int launch_miller_tables(sylow_b200_ctx* ctx, int m, const uint8_t* table
   return SYLOW_B200_ERR_ARG;
 }
 
+// Batches from SY_AFF_MIN_BATCH points on leave their results in projective form (Montgomery form) in ctx->proj and
+// convert them to affine coordinates afterwards, with one inversion per SY_AFF_K points (k_g1/g2_batch_affine); smaller
+// ones convert each point in the kernel.
+#define SY_AFF_MIN_BATCH 32768
+// The pointwise additions (k_g1_add, k_g2_add) are short enough that below these sizes the launch of
+// k_g*_batch_affine and its serial walk over SY_AFF_K points per thread cost more than an inversion in every
+// thread; measured crossovers on a B200 (DESIGN.md section 4, item 26): G1 between 2^15 and 2^16 points, G2
+// between 2^16 and 2^17.  The definitions can be overridden only to build the variants tools/group_law_time.py
+// times on both sides of them.
+#ifndef SY_G1_ADD_AFF_MIN_BATCH
+#define SY_G1_ADD_AFF_MIN_BATCH 65536
+#endif
+#ifndef SY_G2_ADD_AFF_MIN_BATCH
+#define SY_G2_ADD_AFF_MIN_BATCH 131072
+#endif
+// n points of G1 or G2 (g2) -> affine wire format + infinity flags at out / out_inf, G1 points negated when negate is
+// set: launch(proj) enqueues the point kernel on s with proj_out = proj, which is ctx->proj from min_batch points on
+// (followed by the batched conversion) and null below.
+template <class Launch>
+static int point_batch(sylow_b200_ctx* ctx, bool g2, size_t n, size_t min_batch, int negate, uint8_t* out,
+                       uint8_t* out_inf, cudaStream_t s, Launch launch) {
+  uint8_t* proj = nullptr;
+  if (n >= min_batch) {
+    CKS(reserve(ctx, ctx->proj, n * (g2 ? 192 : 96)));
+    proj = ctx->proj.p;
+  }
+  launch(proj);
+  LAUNCHED(ctx);
+  if (!proj) return 0;
+  const unsigned blocks = nblocks((n + SY_AFF_K - 1) / SY_AFF_K, SY_MUL_THREADS);
+  if (g2)
+    k_g2_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(proj, n, out, out_inf);
+  else
+    k_g1_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(proj, n, negate, out, out_inf);
+  LAUNCHED(ctx);
+  return 0;
+}
+
 extern "C" {
 
 int sylow_b200_create(sylow_b200_ctx** out, int device_id) {
@@ -1438,65 +1419,27 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
   return launch_check_products(ctx, ctx->scratch0.p, k_prod, n_checks, ok_out, s);
 }
 
-// Batches from SY_AFF_MIN_BATCH points on leave their results in projective form (proj_bytes per point, Montgomery form) in
-// ctx->proj and convert them to affine coordinates afterwards, with one inversion per SY_AFF_K points (affine_tail);
-// smaller ones convert each point in the kernel (*proj = null).
-#define SY_AFF_MIN_BATCH 32768
-// The pointwise additions (k_g1_add, k_g2_add) are short enough that below these sizes the launch of affine_tail and
-// its serial walk over SY_AFF_K points per thread cost more than an inversion in every thread; measured crossovers on
-// a B200 (DESIGN.md section 4, item 26): G1 between 2^15 and 2^16 points, G2 between 2^16 and 2^17.  The definitions
-// can be overridden only to build the variants tools/group_law_time.py times on both sides of them.
-#ifndef SY_G1_ADD_AFF_MIN_BATCH
-#define SY_G1_ADD_AFF_MIN_BATCH 65536
-#endif
-#ifndef SY_G2_ADD_AFF_MIN_BATCH
-#define SY_G2_ADD_AFF_MIN_BATCH 131072
-#endif
-static int affine_stage(sylow_b200_ctx* ctx, size_t n, size_t proj_bytes, uint8_t** proj,
-                        size_t min_batch = SY_AFF_MIN_BATCH) {
-  *proj = nullptr;
-  if (n < min_batch) return 0;
-  CKS(reserve(ctx, ctx->proj, n * proj_bytes));
-  *proj = ctx->proj.p;
-  return 0;
-}
-// n projective points at d_proj -> affine wire format + infinity flags; G1 points optionally negated
-static int affine_tail(sylow_b200_ctx* ctx, bool g2, const uint8_t* d_proj, size_t n, int negate, uint8_t* d_out,
-                       uint8_t* d_out_inf, cudaStream_t s) {
-  const unsigned blocks = nblocks((n + SY_AFF_K - 1) / SY_AFF_K, SY_MUL_THREADS);
-  if (g2)
-    k_g2_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(d_proj, n, d_out, d_out_inf);
-  else
-    k_g1_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(d_proj, n, negate, d_out, d_out_inf);
-  LAUNCHED(ctx);
-  return 0;
-}
-
-int sylow_b200_g1_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf,
-                                const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
+// out[i] = affine(scalars[i] * pts[i]) in G1 (g2 = 0) or G2
+static int mul_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
+                   size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
   ENTER_DEV(ctx);
   if (n && (!pts || !scalars || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   cudaStream_t s = pick(ctx, stream);
-  uint8_t* proj;
-  CKS(affine_stage(ctx, n, 96, &proj));
-  k_g1_mul<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(pts, pts_inf, scalars, n, out, out_inf, proj);
-  LAUNCHED(ctx);
-  if (proj) CKS(affine_tail(ctx, false, proj, n, 0, out, out_inf, s));
-  return 0;
+  return point_batch(ctx, g2, n, SY_AFF_MIN_BATCH, 0, out, out_inf, s, [&](uint8_t* proj) {
+    if (g2)
+      k_g2_mul<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(pts, pts_inf, scalars, n, out, out_inf, proj);
+    else
+      k_g1_mul<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(pts, pts_inf, scalars, n, out, out_inf, proj);
+  });
+}
+int sylow_b200_g1_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf,
+                                const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
+  return mul_dev(ctx, 0, pts, pts_inf, scalars, n, out, out_inf, stream);
 }
 int sylow_b200_g2_mul_batch_dev(sylow_b200_ctx* ctx, const uint8_t* pts, const uint8_t* pts_inf,
                                 const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
-  ENTER_DEV(ctx);
-  if (n && (!pts || !scalars || !out)) return SYLOW_B200_ERR_ARG;
-  if (!n) return 0;
-  cudaStream_t s = pick(ctx, stream);
-  uint8_t* proj;
-  CKS(affine_stage(ctx, n, 192, &proj));
-  k_g2_mul<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(pts, pts_inf, scalars, n, out, out_inf, proj);
-  LAUNCHED(ctx);
-  if (proj) CKS(affine_tail(ctx, true, proj, n, 0, out, out_inf, s));
-  return 0;
+  return mul_dev(ctx, 1, pts, pts_inf, scalars, n, out, out_inf, stream);
 }
 
 static int make_dst_prime(sylow_b200_ctx* ctx, const uint8_t* dst, size_t dst_len, int hash_id, DstPrime& dp) {
@@ -1531,14 +1474,11 @@ static int make_dst_prime(sylow_b200_ctx* ctx, const uint8_t* dst, size_t dst_le
 
 static int hash_launch(sylow_b200_ctx* ctx, const uint8_t* d_msgs, const uint64_t* d_offsets, size_t n,
                        const DstPrime& dp, int negate, uint8_t* d_out, uint8_t* d_out_inf, cudaStream_t s) {
-  uint8_t* proj;
-  CKS(affine_stage(ctx, n, 96, &proj));
   CK(cudaMemsetAsync(ctx->d_fail, 0, sizeof(int), s));  // the flag reports THIS call's hashes only
-  k_hash_to_g1<<<nblocks(n, SY_HASH_THREADS), SY_HASH_THREADS, 0, s>>>(d_msgs, d_offsets, n, dp, negate, d_out,
-                                                                     d_out_inf, ctx->d_fail, proj);
-  LAUNCHED(ctx);
-  if (proj) CKS(affine_tail(ctx, false, proj, n, negate, d_out, d_out_inf, s));
-  return 0;
+  return point_batch(ctx, false, n, SY_AFF_MIN_BATCH, negate, d_out, d_out_inf, s, [&](uint8_t* proj) {
+    k_hash_to_g1<<<nblocks(n, SY_HASH_THREADS), SY_HASH_THREADS, 0, s>>>(d_msgs, d_offsets, n, dp, negate, d_out,
+                                                                       d_out_inf, ctx->d_fail, proj);
+  });
 }
 
 int sylow_b200_hash_to_g1_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_msgs, const uint64_t* d_offsets, size_t n,
@@ -1585,7 +1525,7 @@ static int ensure_gen_table(sylow_b200_ctx* ctx, cudaStream_t s) {
 }
 
 // Fixed-base table of the G1 (g2 = 0) or G2 generator for gen_scalar_mul (curve.cuh), built on the device once per
-// context: the ladder of g1/g2_mul_batch_dev multiplies the generator by (j + 1) 2^(C w) mod r, and k_fp_convert takes
+// context: the ladder of mul_dev multiplies the generator by (j + 1) 2^(C w) mod r, and k_fp_convert takes
 // the affine results to Montgomery form, so every entry is the ladder's own point.  The field is set only after the
 // build has finished, like ensure_gen_table's.
 static int ensure_mul_table(sylow_b200_ctx* ctx, int g2, cudaStream_t s) {
@@ -1607,8 +1547,7 @@ static int ensure_mul_table(sylow_b200_ctx* ctx, int g2, cudaStream_t s) {
   int st = e == cudaSuccess ? 0 : fail_cuda(ctx, e);
   uint8_t* d_aff = d_in + in_bytes;
   if (!st)
-    st = (g2 ? sylow_b200_g2_mul_batch_dev : sylow_b200_g1_mul_batch_dev)(ctx, d_in + n * 32, nullptr, d_in, n, d_aff,
-                                                                           nullptr, s);
+    st = mul_dev(ctx, g2, d_in + n * 32, nullptr, d_in, n, d_aff, nullptr, s);
   if (!st) {
     k_fp_convert<<<nblocks(n * pb / 32, 128), 128, 0, s>>>(d_aff, n * pb / 32, d_tab, 1);
     ctx->launches++;
@@ -1625,7 +1564,7 @@ static int ensure_mul_table(sylow_b200_ctx* ctx, int g2, cudaStream_t s) {
   return 0;
 }
 
-// out[i] = affine(scalars[i] * G) for the G1 (g2 = 0) or G2 generator: the form of g1/g2_mul_batch_dev with the
+// out[i] = affine(scalars[i] * G) for the G1 (g2 = 0) or G2 generator: the form of mul_dev with the
 // fixed-base table in place of the ladder
 static int mul_gen_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* scalars, size_t n, uint8_t* out, uint8_t* out_inf,
                        void* stream) {
@@ -1634,16 +1573,14 @@ static int mul_gen_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* scalars, size
   if (!n) return 0;
   cudaStream_t s = pick(ctx, stream);
   CKS(ensure_mul_table(ctx, g2, s));
-  uint8_t* proj;
-  CKS(affine_stage(ctx, n, g2 ? 192 : 96, &proj));
-  if (g2)
-    k_g2_mul_gen<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(ctx->d_mul_table[1], scalars, n, out, out_inf, proj);
-  else
-    k_g1_mul_gen<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(ctx->d_mul_table[0], scalars, n, out, out_inf,
-                                                                        proj);
-  LAUNCHED(ctx);
-  if (proj) CKS(affine_tail(ctx, g2, proj, n, 0, out, out_inf, s));
-  return 0;
+  return point_batch(ctx, g2, n, SY_AFF_MIN_BATCH, 0, out, out_inf, s, [&](uint8_t* proj) {
+    if (g2)
+      k_g2_mul_gen<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(ctx->d_mul_table[1], scalars, n, out, out_inf,
+                                                                       proj);
+    else
+      k_g1_mul_gen<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(ctx->d_mul_table[0], scalars, n, out, out_inf,
+                                                                          proj);
+  });
 }
 int sylow_b200_g1_mul_generator_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_scalars, size_t n, uint8_t* d_out,
                                           uint8_t* d_out_inf, void* stream) {
@@ -1661,15 +1598,14 @@ static int add_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* a, const uint8_t*
   if (n && (!a || !b || !out)) return SYLOW_B200_ERR_ARG;
   if (!n) return 0;
   cudaStream_t s = pick(ctx, stream);
-  uint8_t* proj;
-  CKS(affine_stage(ctx, n, g2 ? 192 : 96, &proj, g2 ? SY_G2_ADD_AFF_MIN_BATCH : SY_G1_ADD_AFF_MIN_BATCH));
-  if (g2)
-    k_g2_add<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj);
-  else
-    k_g1_add<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj);
-  LAUNCHED(ctx);
-  if (proj) CKS(affine_tail(ctx, g2, proj, n, 0, out, out_inf, s));
-  return 0;
+  const size_t min_batch = g2 ? SY_G2_ADD_AFF_MIN_BATCH : SY_G1_ADD_AFF_MIN_BATCH;
+  return point_batch(ctx, g2, n, min_batch, 0, out, out_inf, s, [&](uint8_t* proj) {
+    if (g2)
+      k_g2_add<<<nblocks(n, SY_G2_THREADS), SY_G2_THREADS, 0, s>>>(a, a_inf, b, b_inf, n, subtract, out, out_inf, proj);
+    else
+      k_g1_add<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(a, a_inf, b, b_inf, n, subtract, out, out_inf,
+                                                                      proj);
+  });
 }
 int sylow_b200_g1_add_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_a, const uint8_t* d_a_inf, const uint8_t* d_b,
                                 const uint8_t* d_b_inf, size_t n, int subtract, uint8_t* d_out, uint8_t* d_out_inf,
@@ -1764,11 +1700,10 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
   uint8_t* d_sum_inf = d_sum + 64;
   CKS(hash_launch(ctx, d_msgs, d_offsets, n, dp, 1, d_hm, d_hm_inf, s));
   if (pairs_ready) CK(cudaStreamWaitEvent(s, pairs_ready, 0));
-  if (weighted) {
-    CKS(reserve(ctx, ctx->proj, n * 96));
-    k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_hm, d_hm_inf, ws, first_index, n, ctx->proj.p);
-    LAUNCHED(ctx);
-    CKS(affine_tail(ctx, false, ctx->proj.p, n, 0, d_hm, d_hm_inf, s));
+  if (weighted) {  // r_i H(m_i) in place; k_g1_mul_weight writes projective points only (min_batch 0)
+    CKS(point_batch(ctx, false, n, 0, 0, d_hm, d_hm_inf, s, [&](uint8_t* proj) {
+      k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_hm, d_hm_inf, ws, first_index, n, proj);
+    }));
   }
   // The n Miller loops (-r_i H(m_i), pk_i) only ever meet as a product, so 1, 2 or 4 signatures share one thread
   // and ONE Fp12 squaring per loop digit - what glued_miller_loop does for the whole batch in the reference
@@ -2063,10 +1998,8 @@ static int mul_host(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8
   CKS(io.err);
   if (!pts)
     CKS(mul_gen_dev(ctx, g2, dk, n, d_out, d_out_inf, nullptr));
-  else if (g2)
-    CKS(sylow_b200_g2_mul_batch_dev(ctx, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
   else
-    CKS(sylow_b200_g1_mul_batch_dev(ctx, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
+    CKS(mul_dev(ctx, g2, dp, dpi, dk, n, d_out, d_out_inf, nullptr));
   io.down(out, d_out, n * pb);
   if (out_inf) io.down(out_inf, d_out_inf, n);
   return io.finish();

@@ -43,6 +43,45 @@ SY_HD void fp2_store_raw(uint8_t* p, const Fp2& v) {
   fp_store_raw(p + 32, v.c1);
 }
 
+// ---- G1 (F = Fp) and G2 (F = Fp2) point records ----------------------------------------------------------------
+// A coordinate of either group, canonical (f_load / f_store) or Montgomery form (f_load_raw / f_store_raw).
+template <class F>
+SY_HD F f_load(const uint8_t* p);
+template <>
+SY_HD Fp f_load<Fp>(const uint8_t* p) { return fp_load(p); }
+template <>
+SY_HD Fp2 f_load<Fp2>(const uint8_t* p) { return fp2_load(p); }
+template <class F>
+SY_HD F f_load_raw(const uint8_t* p);
+template <>
+SY_HD Fp f_load_raw<Fp>(const uint8_t* p) { return fp_load_raw(p); }
+template <>
+SY_HD Fp2 f_load_raw<Fp2>(const uint8_t* p) { return fp2_load_raw(p); }
+SY_HD void f_store(uint8_t* p, const Fp& v) { fp_store(p, v); }
+SY_HD void f_store(uint8_t* p, const Fp2& v) { fp2_store(p, v); }
+SY_HD void f_store_raw(uint8_t* p, const Fp& v) { fp_store_raw(p, v); }
+SY_HD void f_store_raw(uint8_t* p, const Fp2& v) { fp2_store_raw(p, v); }
+
+// Point i of an affine wire array (x || y, 2 sizeof(F) bytes per point) with its flag from the optional array inf.
+template <class F>
+SY_HD Affine<F> affine_load(const uint8_t* pts, const uint8_t* inf, size_t i) {
+  constexpr size_t W = sizeof(F);
+  return Affine<F>{f_load<F>(pts + i * 2 * W), f_load<F>(pts + i * 2 * W + W), inf && inf[i]};
+}
+// The device-internal projective record: x || y || z in Montgomery form, 96 bytes for G1 and 192 for G2.
+template <class F>
+SY_HD Proj<F> proj_load_raw(const uint8_t* p) {
+  constexpr size_t W = sizeof(F);
+  return Proj<F>{f_load_raw<F>(p), f_load_raw<F>(p + W), f_load_raw<F>(p + 2 * W)};
+}
+template <class F>
+SY_HD void proj_store_raw(uint8_t* p, const Proj<F>& q) {
+  constexpr size_t W = sizeof(F);
+  f_store_raw(p, q.x);
+  f_store_raw(p + W, q.y);
+  f_store_raw(p + 2 * W, q.z);
+}
+
 // Fp12 in tower order.  *_raw keeps Montgomery form (device-internal intermediates).
 SY_HD Fp12 fp12_load(const uint8_t* p) {
   Fp12 r;

@@ -54,7 +54,8 @@ def _ladder(eng, g, k):
 @pytest.mark.parametrize("g", ["g1", "g2"])
 @pytest.mark.parametrize("n", [1, 7, 32767, 32768, (1 << 16) + 3])
 def test_matches_ladder_on_repeated_generator(eng, g, n):
-    """Straddles SY_AFF_MIN_BATCH (32 768): below it each thread converts its own point, from it affine_tail does."""
+    """Straddles SY_AFF_MIN_BATCH (32 768): below it each thread converts its own point, from it
+    k_g*_batch_affine does."""
     k = _scalars(n, n)
     out, inf = getattr(eng, g + "_mul_generator_batch")(k)
     ref, ref_inf = _ladder(eng, g, k)

@@ -79,7 +79,7 @@ def _read(g, row, inf):
 @pytest.mark.parametrize("sub", [False, True], ids=["add", "sub"])
 def test_against_python_oracle(eng, g, dn, sub):
     """n = 1, 7 and around SY_G*_ADD_AFF_MIN_BATCH = T: below it each thread converts its own point, from it
-    affine_tail does."""
+    k_g*_batch_affine does."""
     n = 1 if dn is None else dn if dn == 7 else T[g] + dn
     a, b, ai, bi = _operands(eng, g, n, 100 + n)
     out, inf = getattr(eng, g + "_add_batch")(a, b, ai, bi, subtract=sub)

@@ -4,7 +4,7 @@
 Three parts, each in its own process so that each loads one build of the library:
   shipped   the library as built, from 2^10 to 2^24 points, on both sides of SY_G1_ADD_AFF_MIN_BATCH and
             SY_G2_ADD_AFF_MIN_BATCH
-  always    a build with both thresholds 1: every batch writes projective points and affine_tail shares one
+  always    a build with both thresholds 1: every batch writes projective points and k_g*_batch_affine shares one
             inversion between SY_AFF_K points
   never     a build with both thresholds 2^62: every thread inverts its own point
 The last two run from 2^8 to 2^17 points and locate the crossovers the thresholds are set from.  The three
