@@ -109,7 +109,9 @@ int sylow_b200_fp12_product(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, uin
 
 /* n_checks independent product checks of pairs_per_check pairs each:
  * ok_out[c] = (glued_pairing(g1s_c, g2s_c) == Gt::identity())  (pairing.rs:1029-1037; the ecPairing
- * shape of examples/reth_bn128.rs:211-214).  Pair j of check c is element c*pairs_per_check + j. */
+ * shape of examples/reth_bn128.rs:211-214).  Pair j of check c is element c*pairs_per_check + j.
+ * pairs_per_check = 0: every check is the empty product, the identity, so every ok_out[c] is 1 (g1 and g2 may then be
+ * NULL; no kernel runs). */
 int sylow_b200_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                                    const uint8_t* g2_inf, size_t pairs_per_check, size_t n_checks, uint8_t* ok_out);
 

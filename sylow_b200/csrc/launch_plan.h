@@ -94,6 +94,15 @@ inline Segment check_products_segment(int sms, size_t n_checks, BlockShape fexp,
   return {0, n_checks, nblocks(n_checks, t), t, false};
 }
 
+// Whether pairing_check_batch runs each of n_checks checks of k pairs as ONE glued loop (k_glued<k, 0>, shape `glued`)
+// rather than k separate Miller loops multiplied by launch_check_products: 2- and 4-pair checks (ecPairing, Groth16
+// without fixed tables), once there are enough checks to fill the GPU - a whole glued wave of 2-pair checks, half of one
+// of 4-pair checks.
+inline bool glued_checks(int sms, size_t k, size_t n_checks, BlockShape glued) {
+  const size_t wave = wave_items(sms, glued);
+  return (k == 2 && n_checks >= wave) || (k == 4 && n_checks >= wave / 2);
+}
+
 // Pairs per thread (1, 2 or 4) for n >= 1 pairs whose Miller loops only meet as a product, glued into one loop per
 // thread (k_glued<M, 0>, k_miller_tables<M>, shape `glued`): the glue of fewest wave-times, i.e. whole waves of n / g
 // threads times the Fp multiplications of g glued pairs.  pair_cost is one pair's count (8 444 fused, 6 045 from a

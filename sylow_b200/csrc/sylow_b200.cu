@@ -1403,18 +1403,19 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
   size_t n = k * n_checks;
   if (n && (!g1 || !g2)) return SYLOW_B200_ERR_ARG;
   cudaStream_t s = pick(ctx, stream);
+  if (!k) {  // the product of no pairs is the identity: every check holds, and there is nothing to compute
+    CK(cudaMemsetAsync(ok_out, 1, n_checks, s));
+    return 0;
+  }
+  CKS(reserve(ctx, ctx->scratch0, n * 384));
   size_t k_prod = k;  // Miller values per check left for k_check_products to multiply
-  if (n) {
-    CKS(reserve(ctx, ctx->scratch0, n * 384));
-    // 2- and 4-pair checks (ecPairing, Groth16 without fixed tables) as ONE glued loop per check: one Fp12 squaring per
-    // digit for all pairs of the check, like glued_miller_loop (pairing.rs:970-1022); needs enough checks to fill the GPU
-    const size_t wave = wave_items(ctx->sms, kGluedShape);
-    if ((k == 2 && n_checks >= wave) || (k == 4 && n_checks >= wave / 2)) {
-      CKS(launch_glued(ctx, k, 0, g1, k, g1_inf, g2, g2_inf, nullptr, 0, nullptr, nullptr, n_checks, ctx->scratch0.p, s));
-      k_prod = 1;
-    } else {
-      CKS(launch_miller(ctx, g1, g1_inf, g2, g2_inf, n, ctx->scratch0.p, 1, s));
-    }
+  // 2- and 4-pair checks as ONE glued loop per check: one Fp12 squaring per digit for all pairs of the check, like
+  // glued_miller_loop (pairing.rs:970-1022)
+  if (glued_checks(ctx->sms, k, n_checks, kGluedShape)) {
+    CKS(launch_glued(ctx, k, 0, g1, k, g1_inf, g2, g2_inf, nullptr, 0, nullptr, nullptr, n_checks, ctx->scratch0.p, s));
+    k_prod = 1;
+  } else {
+    CKS(launch_miller(ctx, g1, g1_inf, g2, g2_inf, n, ctx->scratch0.p, 1, s));
   }
   return launch_check_products(ctx, ctx->scratch0.p, k_prod, n_checks, ok_out, s);
 }

@@ -36,4 +36,7 @@ void lp_check(int sms, uint64_t n_checks, int lanes_mode, uint64_t* out) {
 
 int lp_glue(int sms, uint64_t n, uint64_t pair_cost) { return glue_pairs(sms, n, pair_cost, kGlued); }
 
+// 1 if pairing_check_batch runs n_checks checks of k pairs as one glued loop per check
+int lp_check_glued(int sms, uint64_t k, uint64_t n_checks) { return glued_checks(sms, k, n_checks, kGlued); }
+
 }  // extern "C"

@@ -1,7 +1,7 @@
 """CPU tier: the launch policy of the batch kernels (sylow_b200/csrc/launch_plan.h), with the block shapes of
 csrc/kernels_pairing.cuh, compiled for the host (tests/hostsim/launch_plan.cu).  Pins the launches that launch_miller,
-launch_final_exp and launch_check_products make on 148 SMs (a B200) in the three SYLOW_B200_LANES modes, and
-glue_pairs' pairs per thread."""
+launch_final_exp and launch_check_products make on 148 SMs (a B200) in the three SYLOW_B200_LANES modes,
+glue_pairs' pairs per thread and the batch sizes from which pairing_check_batch glues each check into one loop."""
 import ctypes
 import os
 import subprocess
@@ -14,16 +14,22 @@ MILLER, FEXP = 0, 1
 NEVER, AUTO, ALWAYS = 0, 1, 2  # SYLOW_B200_LANES
 
 
-@pytest.fixture(scope="module")
-def lp(tmp_path_factory):
-    so = str(tmp_path_factory.mktemp("launch_plan") / "liblaunch_plan.so")
+def load_launch_plan(directory):
+    """tests/hostsim/launch_plan.cu compiled into `directory` and loaded (also used by test_gpu_verdict_seams.py)"""
+    so = os.path.join(str(directory), "liblaunch_plan.so")
     subprocess.check_call(["nvcc", "-x", "cu", "-O2", "-std=c++17", "-DSYLOW_HOSTSIM", "-shared", "-Xcompiler", "-fPIC",
                            "-w", "-o", so, os.path.join(HERE, "hostsim", "launch_plan.cu")])
     lib = ctypes.CDLL(so)
     lib.lp_batch.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_uint64, ctypes.c_int, ctypes.c_void_p]
     lib.lp_check.argtypes = [ctypes.c_int, ctypes.c_uint64, ctypes.c_int, ctypes.c_void_p]
     lib.lp_glue.argtypes = [ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64]
+    lib.lp_check_glued.argtypes = [ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64]
     return lib
+
+
+@pytest.fixture(scope="module")
+def lp(tmp_path_factory):
+    return load_launch_plan(tmp_path_factory.mktemp("launch_plan"))
 
 
 def _launches(lp, kernel, n, mode, sms=SMS):
@@ -83,6 +89,19 @@ def test_check_products_launch(lp, n_checks, mode, launch):
 @pytest.mark.parametrize("pair_cost", [8444, 6045])  # a fused pair, a pair against a precomputed table
 def test_glue_pairs(lp, n, glue, pair_cost):
     assert lp.lp_glue(SMS, n, pair_cost) == glue
+
+
+L, W = 148 * 64 * 2, 148 * 128 * 2  # one two-lane wave, one glued wave
+
+
+@pytest.mark.parametrize("k, n_checks, glued", [
+    # 2-pair checks from one whole glued wave of checks, 4-pair checks from half of one (= one two-lane wave)
+    (2, W - 1, False), (2, W, True), (4, L - 1, False), (4, L, True),
+    # other check sizes never run as one glued loop
+    (1, 1 << 20, False), (3, 1 << 20, False), (5, 1 << 20, False),
+])
+def test_glued_checks(lp, k, n_checks, glued):
+    assert bool(lp.lp_check_glued(SMS, k, n_checks)) is glued
 
 
 @pytest.mark.parametrize("sms", [1, 7, 132, 148])
