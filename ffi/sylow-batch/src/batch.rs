@@ -10,7 +10,8 @@
 //! pub use crate::batch::{final_exponentiation_batch, g1_add_batch, g1_generator_mul_batch, g1_mul_batch, g2_add_batch,
 //!                        g2_generator_mul_batch, g2_mul_batch, glued_miller_loop_batch,
 //!                        glued_miller_loop_precomputed_batch, glued_pairing_batch, pairing_batch, pairing_check_batch, sign_batch,
-//!                        threshold_aggregate_batch, verify_batch, verify_each, BatchError, Engine};
+//!                        threshold_aggregate_batch, verify_batch, verify_each, groth16_verify_each,
+//!                        groth16_verify_batch, Groth16Proof, Groth16VerifyingKey, BatchError, Engine};
 //! ```
 //!
 //! All slicing over GPUs, the per-GPU host threads and the combination of the 384-byte Miller partial products live
@@ -380,6 +381,77 @@ pub fn verify_batch(e: &mut Engine, pks: &[G2Projective], msgs: &[&[u8]], sigs: 
     e.check(unsafe {
         sys::sylow_b200_verify_batch(e.ctx, pk.as_ptr(), pki.as_ptr(), buf.as_ptr(), offs.as_ptr(), sg.as_ptr(), sgi.as_ptr(), n,
                                      crate::DST.as_ptr(), crate::DST.len(), sys::SYLOW_B200_HASH_KECCAK256, seed, &mut ok)
+    })?;
+    Ok(ok != 0)
+}
+
+/// A Groth16 verifying key over BN254: a proof (A, B, C) with public inputs x_1 .. x_l holds when
+/// e(A, B) e(-alpha, beta) e(-L, gamma) e(-C, delta) == 1 with L = ic[0] + sum_i x_i ic[i]; `ic` has l + 1 points.
+pub struct Groth16VerifyingKey {
+    pub alpha: G1Projective,
+    pub beta: G2Projective,
+    pub gamma: G2Projective,
+    pub delta: G2Projective,
+    pub ic: Vec<G1Projective>,
+}
+/// A Groth16 proof.  Its points are not validated here: decode untrusted proofs with the checked constructors.
+pub struct Groth16Proof {
+    pub a: G1Projective,
+    pub b: G2Projective,
+    pub c: G1Projective,
+}
+// key, proofs with their n x 3 infinity flags, and the public inputs (l canonical 32-byte little-endian Fr per proof) in
+// the wire form of include/sylow_b200.h; InvalidArgument if a proof does not carry l inputs
+fn marshal_groth16(vk: &Groth16VerifyingKey, proofs: &[Groth16Proof], inputs: &[&[[u8; 32]]])
+                   -> Result<(Vec<u8>, usize, Vec<u8>, Vec<u8>, Vec<u8>), BatchError> {
+    if vk.ic.is_empty() || same_len(proofs.len(), inputs.len()).is_err() {
+        return Err(BatchError::InvalidArgument);
+    }
+    let l = vk.ic.len() - 1;
+    let mut key = marshal_g1(core::slice::from_ref(&vk.alpha)).0;
+    key.extend(marshal_g2(&[vk.beta, vk.gamma, vk.delta]).0);
+    key.extend(marshal_g1(&vk.ic).0);
+    let (mut pr, mut inf, mut x) = (Vec::with_capacity(proofs.len() * 256), Vec::with_capacity(proofs.len() * 3),
+                                    Vec::with_capacity(proofs.len() * l * 32));
+    for (p, xs) in proofs.iter().zip(inputs) {
+        if xs.len() != l {
+            return Err(BatchError::InvalidArgument);
+        }
+        let (a, ai) = marshal_g1(core::slice::from_ref(&p.a));
+        let (b, bi) = marshal_g2(core::slice::from_ref(&p.b));
+        let (c, ci) = marshal_g1(core::slice::from_ref(&p.c));
+        pr.extend(a);
+        pr.extend(b);
+        pr.extend(c);
+        inf.extend([ai[0], bi[0], ci[0]]);
+        for v in xs.iter() {
+            x.extend_from_slice(v);
+        }
+    }
+    Ok((key, l, pr, inf, x))
+}
+
+/// One verdict per Groth16 proof under `vk`; `inputs[j]` are proof j's public inputs.  An input >= r fails its proof.
+pub fn groth16_verify_each(e: &mut Engine, vk: &Groth16VerifyingKey, proofs: &[Groth16Proof], inputs: &[&[[u8; 32]]])
+                           -> Result<Vec<bool>, BatchError> {
+    let (key, l, pr, inf, x) = marshal_groth16(vk, proofs, inputs)?;
+    let mut ok = vec![0u8; proofs.len()];
+    e.check(unsafe {
+        sys::sylow_b200_groth16_verify_each(e.ctx, key.as_ptr(), l, pr.as_ptr(), inf.as_ptr(), x.as_ptr(), proofs.len(),
+                                            ok.as_mut_ptr())
+    })?;
+    Ok(ok.into_iter().map(|b| b != 0).collect())
+}
+
+/// One verdict for a batch of Groth16 proofs under `vk`: prod_j check_j^{r_j} == 1 with random 64-bit weights from
+/// `weight_seed` (32 secret random bytes drawn after the batch is fixed) and ONE final exponentiation.
+pub fn groth16_verify_batch(e: &mut Engine, vk: &Groth16VerifyingKey, proofs: &[Groth16Proof], inputs: &[&[[u8; 32]]],
+                            weight_seed: &[u8; 32]) -> Result<bool, BatchError> {
+    let (key, l, pr, inf, x) = marshal_groth16(vk, proofs, inputs)?;
+    let mut ok = 0i32;
+    e.check(unsafe {
+        sys::sylow_b200_groth16_verify_batch(e.ctx, key.as_ptr(), l, pr.as_ptr(), inf.as_ptr(), x.as_ptr(), proofs.len(),
+                                             weight_seed.as_ptr(), &mut ok)
     })?;
     Ok(ok != 0)
 }

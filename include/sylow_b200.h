@@ -322,6 +322,53 @@ int sylow_b200_verify_batch_same_signer(sylow_b200_ctx* ctx, const uint8_t* pk /
                                         size_t n, const uint8_t* dst, size_t dst_len, int hash_id,
                                         const uint8_t* weight_seed /* 32 B or NULL */, int* ok);
 
+/* ---- Groth16 proof verification ------------------------------------------------------------------ */
+
+/* Verification of Groth16 proofs over BN254 under one verifying key with l = n_public public inputs (l may be 0):
+ *   e(A, B) e(-alpha, beta) e(-L, gamma) e(-C, delta) == 1,   L = IC_0 + sum_{i=1..l} x_i IC_i.
+ * Formats (wire form above, little-endian):
+ *   verifying key, host:  alpha (G1) || beta || gamma || delta (G2) || IC_0 .. IC_l (G1): 448 + 64 (l + 1) bytes.
+ *                         No point of the key can be infinite.
+ *   proof:                A (G1) || B (G2) || C (G1), 256 bytes.  proofs_inf: n x 3 flags (A, B, C) or NULL; a flagged
+ *                         A or B drops the pair e(A, B), a flagged C drops e(-C, delta).
+ *   public inputs:        n x l canonical Fr values, 32 bytes each (proof j's inputs at inputs + j*l*32).  An input >= r
+ *                         makes that proof INVALID; it is never reduced mod r (a reduced alias would let anyone change
+ *                         the public input without changing the proof; the snarkjs / Solidity verifiers reject it too).
+ *   prepared key, device: SYLOW_B200_GROTH16_VK_DEV_BYTES(l) bytes of caller-owned device memory (16-byte aligned):
+ *                         the beta, gamma, delta line tables in the device form of sylow_b200_tables_to_device
+ *                         (3 x 16704 B), -alpha (64 B, canonical affine), IC_0 (64 B), then one fixed-base table per
+ *                         IC_i, i = 1 .. l (32 windows x 128 affine multiples, Montgomery form: 262144 B each).
+ * Proof points are NOT validated, as in every pairing entry point: run sylow_b200_g1_validate_batch (A, C) and
+ * sylow_b200_g2_validate_batch (B) on untrusted proofs first.  The key is validated by prepare_vk and by the host forms.
+ * prepare_vk: validates the host key (G1 points on the curve, beta / gamma / delta on the curve and in the subgroup) and
+ *   returns the first failing status in key order (SYLOW_B200_ERR_DECODE, _NOT_ON_CURVE, _NOT_IN_SUBGROUP); otherwise
+ *   builds the device form at d_vk_out on the device.  Synchronous.
+ * verify_each: ok_out[j] = proof j verifies.  The host form prepares the key itself (on every device of a multi-device
+ *   context, which shards the proofs as usual).
+ * verify_batch: *ok = prod_j check_j^{r_j} == 1 with r_j = batch_weight(weight_seed, first_index + j) as for
+ *   sylow_b200_verify_batch: ONE final exponentiation, one fused Miller loop (r_j A_j, B_j) per proof and three table
+ *   pairs for the whole batch.  weight_seed (32 secret random bytes drawn after the batch is fixed) is REQUIRED: NULL
+ *   returns SYLOW_B200_ERR_ARG.  A batch with an invalid proof passes with probability <= 2^-63 (for validated points);
+ *   an input >= r always fails it.  n = 0 gives *ok = 1.
+ * verify_batch_partial_dev: the 384-byte share of a slice whose first proof has the global index first_index; combine
+ *   the shares with sylow_b200_verify_batch_finish.  An input >= r makes the share zero, so the batch fails. */
+#define SYLOW_B200_GROTH16_VK_DEV_BYTES(n_public) ((size_t)50240 + (size_t)(n_public) * (size_t)262144)
+int sylow_b200_groth16_prepare_vk(sylow_b200_ctx* ctx, const uint8_t* vk, size_t n_public, uint8_t* d_vk_out,
+                                  void* stream);
+int sylow_b200_groth16_verify_each(sylow_b200_ctx* ctx, const uint8_t* vk, size_t n_public, const uint8_t* proofs,
+                                   const uint8_t* proofs_inf, const uint8_t* inputs, size_t n, uint8_t* ok_out);
+int sylow_b200_groth16_verify_each_dev(sylow_b200_ctx* ctx, const uint8_t* d_vk, size_t n_public,
+                                       const uint8_t* d_proofs, const uint8_t* d_proofs_inf, const uint8_t* d_inputs,
+                                       size_t n, uint8_t* d_ok_out, void* stream);
+int sylow_b200_groth16_verify_batch(sylow_b200_ctx* ctx, const uint8_t* vk, size_t n_public, const uint8_t* proofs,
+                                    const uint8_t* proofs_inf, const uint8_t* inputs, size_t n,
+                                    const uint8_t* weight_seed /* 32 B, required */, int* ok);
+int sylow_b200_groth16_verify_batch_partial_dev(sylow_b200_ctx* ctx, const uint8_t* d_vk, size_t n_public,
+                                                const uint8_t* d_proofs, const uint8_t* d_proofs_inf,
+                                                const uint8_t* d_inputs, size_t n,
+                                                const uint8_t* weight_seed /* host, 32 B, required */,
+                                                uint64_t first_index, uint8_t* d_f_out /* 384 */, void* stream);
+
 /* ---- device-resident variants (DEVICE pointers, asynchronous on `stream`) ----------------------- */
 
 int sylow_b200_pairing_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_g1, const uint8_t* d_g1_inf,

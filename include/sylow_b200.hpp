@@ -35,6 +35,10 @@ struct G1Affine { Fp x, y; bool infinity = false; };   // groups/group.rs:174-18
 struct G2Affine { Fp2 x, y; bool infinity = false; };
 struct Gt { Fp12 v; bool operator==(const Gt& o) const { return v == o.v; } static Gt identity() { return Gt{Fp12::one()}; } };
 struct MillerLoopResult { Fp12 v; };
+// Groth16 (sylow_b200.h): e(A, B) e(-alpha, beta) e(-L, gamma) e(-C, delta) == 1, L = ic[0] + sum_i x_i ic[i]
+struct Groth16VerifyingKey { G1Affine alpha; G2Affine beta, gamma, delta; std::vector<G1Affine> ic; };
+struct Groth16Proof { G1Affine a; G2Affine b; G1Affine c; };
+using FrBytes = std::array<std::uint8_t, 32>;  // canonical little-endian public input
 
 static_assert(sizeof(Fp) == 32 && sizeof(Fp2) == 64 && sizeof(Fp12) == 384, "wire layout");
 
@@ -229,6 +233,26 @@ class Engine {
   }
   bool verify(const G2Affine& pk, const std::string& msg, const G1Affine& sig) { return verify_each({pk}, {msg}, {sig})[0]; }
 
+  // Groth16 verdicts under vk: inputs[j] holds proof j's vk.ic.size() - 1 public inputs; an input >= r fails its proof.
+  // Proof points are not validated (g1/g2_validate_batch first).
+  std::vector<bool> groth16_verify_each(const Groth16VerifyingKey& vk, const std::vector<Groth16Proof>& proofs,
+                                        const std::vector<std::vector<FrBytes>>& inputs) {
+    G16 g(vk, proofs, inputs);
+    std::vector<std::uint8_t> ok(proofs.size());
+    ck(sylow_b200_groth16_verify_each(ctx_, g.vk.data(), g.l, g.proofs.data(), g.inf.data(), g.x.data(), proofs.size(),
+                                      ok.data()), "groth16_verify_each");
+    return std::vector<bool>(ok.begin(), ok.end());
+  }
+  // one verdict for the batch, with random 64-bit weights from weight_seed (32 secret random bytes)
+  bool groth16_verify_batch(const Groth16VerifyingKey& vk, const std::vector<Groth16Proof>& proofs,
+                            const std::vector<std::vector<FrBytes>>& inputs, const std::array<std::uint8_t, 32>& weight_seed) {
+    G16 g(vk, proofs, inputs);
+    int ok = 0;
+    ck(sylow_b200_groth16_verify_batch(ctx_, g.vk.data(), g.l, g.proofs.data(), g.inf.data(), g.x.data(), proofs.size(),
+                                       weight_seed.data(), &ok), "groth16_verify_batch");
+    return ok != 0;
+  }
+
   sylow_b200_ctx* raw() { return ctx_; }
 
  private:
@@ -240,6 +264,32 @@ class Engine {
       offs.push_back(0);
       for (const auto& s : m) { buf.insert(buf.end(), s.begin(), s.end()); offs.push_back(buf.size()); }
       if (buf.empty()) buf.push_back(0);
+    }
+  };
+  // key, proofs, their n x 3 infinity flags and inputs in the wire form of sylow_b200.h
+  struct G16 {
+    std::vector<std::uint8_t> vk, proofs, inf, x;
+    size_t l;
+    G16(const Groth16VerifyingKey& k, const std::vector<Groth16Proof>& p, const std::vector<std::vector<FrBytes>>& in) {
+      if (k.ic.empty() || p.size() != in.size()) throw Error(SYLOW_B200_ERR_ARG, "groth16 arguments");
+      l = k.ic.size() - 1;
+      auto put = [](std::vector<std::uint8_t>& v, const void* a, size_t b) {
+        v.insert(v.end(), static_cast<const std::uint8_t*>(a), static_cast<const std::uint8_t*>(a) + b);
+      };
+      put(vk, &k.alpha.x, 64);
+      for (const G2Affine* q : {&k.beta, &k.gamma, &k.delta}) put(vk, &q->x, 128);
+      for (const G1Affine& q : k.ic) put(vk, &q.x, 64);
+      for (size_t j = 0; j < p.size(); j++) {
+        if (in[j].size() != l) throw Error(SYLOW_B200_ERR_ARG, "groth16 public inputs");
+        put(proofs, &p[j].a.x, 64);
+        put(proofs, &p[j].b.x, 128);
+        put(proofs, &p[j].c.x, 64);
+        inf.insert(inf.end(), {p[j].a.infinity, p[j].b.infinity, p[j].c.infinity});
+        for (const FrBytes& v : in[j]) put(x, v.data(), 32);
+      }
+      x.resize(x.size() + 16);  // a valid pointer for l = 0
+      proofs.resize(proofs.size() + 16);
+      inf.resize(inf.size() + 1);
     }
   };
   template <class P>

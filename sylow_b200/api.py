@@ -104,6 +104,33 @@ def _signed(pks, msgs, sigs, pks_inf, sigs_inf):
             _flags(sigs_inf, n, "sigs_inf"), n)
 
 
+def groth16_vk_dev_bytes(n_public: int) -> int:
+    """SYLOW_B200_GROTH16_VK_DEV_BYTES: bytes of a prepared Groth16 key in device memory."""
+    return 3 * TABLE + 128 + int(n_public) * 32 * 128 * 64
+
+
+def _vk(vk, n_public: int) -> np.ndarray:
+    """A Groth16 verifying key, alpha || beta || gamma || delta || IC_0 .. IC_n_public, as one row of bytes."""
+    if int(n_public) < 0:
+        raise ValueError("n_public must be >= 0")
+    return _rows(np.ascontiguousarray(vk, dtype=np.uint8).reshape(-1), 448 + 64 * (int(n_public) + 1), "vk", 1)
+
+
+def _groth16(vk, proofs, inputs, n_public: int, proofs_inf):
+    """(vk, n_public, proofs, proofs_inf, inputs, n) in the argument order of the Groth16 host entry points."""
+    l = int(n_public)
+    proofs = _rows(proofs, 256, "proofs")
+    n = proofs.shape[0]
+    if l:
+        inputs = np.ascontiguousarray(inputs, dtype=np.uint8)
+        if inputs.size != n * 32 * l:
+            raise ValueError("inputs must hold %d x %d x 32 bytes, got %d" % (n, l, inputs.size))
+        inputs = inputs.reshape(n, 32 * l)
+    else:
+        inputs = None
+    return _vk(vk, l), l, proofs, _flags(proofs_inf, 3 * n, "proofs_inf"), inputs, n
+
+
 def _ids(ids) -> np.ndarray:
     ids = np.ascontiguousarray(ids, dtype=np.uint64)
     if ids.ndim != 2:
@@ -509,6 +536,38 @@ class Engine:
         self._call("sylow_b200_verify_batch", *args, dst, len(dst), _lib.HASH_KECCAK256, _seed(weight_seed),
                    ctypes.byref(ok))
         return bool(ok.value)
+
+    # ------------------------------------------------------------------ Groth16
+    def groth16_prepare_vk(self, vk, n_public: int, d_vk_out):
+        """Validate the host key (448 + 64 (n_public + 1) bytes) and build its device form in d_vk_out, a torch CUDA
+        uint8 tensor of groth16_vk_dev_bytes(n_public) bytes; an invalid key raises with its status."""
+        self._call("sylow_b200_groth16_prepare_vk", _vk(vk, n_public), int(n_public), d_vk_out, self._stream())
+
+    def groth16_verify_each(self, vk, proofs, inputs, n_public: int, proofs_inf=None) -> np.ndarray:
+        """One verdict per proof: proofs (n, 256) A || B || C, inputs (n, n_public * 32) canonical Fr, proofs_inf
+        (n, 3) flags or None.  Proof points are not validated (g1/g2_validate_batch first)."""
+        args = _groth16(vk, proofs, inputs, n_public, proofs_inf)
+        ok = np.empty(args[-1], dtype=np.uint8)
+        self._call("sylow_b200_groth16_verify_each", *args, ok)
+        return ok.astype(bool)
+
+    def groth16_verify_batch(self, vk, proofs, inputs, n_public: int, weight_seed, proofs_inf=None) -> bool:
+        """One verdict for the batch, with random 64-bit weights from weight_seed (32 secret random bytes)."""
+        ok = ctypes.c_int(0)
+        self._call("sylow_b200_groth16_verify_batch", *_groth16(vk, proofs, inputs, n_public, proofs_inf),
+                   _seed(weight_seed), ctypes.byref(ok))
+        return bool(ok.value)
+
+    def groth16_verify_each_dev(self, d_vk, n_public: int, d_proofs, d_inputs, d_ok, d_proofs_inf=None):
+        self._call("sylow_b200_groth16_verify_each_dev", d_vk, int(n_public), d_proofs, d_proofs_inf, d_inputs,
+                   d_proofs.shape[0], d_ok, self._stream())
+
+    def groth16_verify_batch_partial_dev(self, d_vk, n_public: int, d_proofs, d_inputs, d_f_out, weight_seed,
+                                         first_index: int = 0, d_proofs_inf=None):
+        """The 384-byte share of the proofs d_proofs (global index of the first: first_index); combine the shares with
+        verify_batch_finish."""
+        self._call("sylow_b200_groth16_verify_batch_partial_dev", d_vk, int(n_public), d_proofs, d_proofs_inf,
+                   d_inputs, d_proofs.shape[0], _seed(weight_seed), int(first_index), d_f_out, self._stream())
 
     # ------------------------------------------------------------------ diagnostics
     def fp_op_batch(self, op: int, a, b) -> np.ndarray:

@@ -395,7 +395,7 @@ SY_HD_NOINLINE G2Proj g2_scalar_mul_gls(const G2Proj& p, const uint32_t* k) {
 // k G with a table of affine multiples of G: T[w][j] = (j + 1) 2^(C w) G, j < 2^(C-1), Montgomery form, x || y.
 // k mod r is recoded into W = ceil(254 / C) signed C-bit digits, least significant first, and the selected entries are
 // added up: W mixed additions and no doublings.  The table is built on the device from the variable-base ladder
-// (sylow_b200.cu: ensure_mul_table), so its entries are the ladder's own affine points.
+// (sylow_b200.cu: build_mul_tables), so its entries are the ladder's own affine points.
 #define SY_GEN_C 8
 #define SY_GEN_W ((254 + SY_GEN_C - 1) / SY_GEN_C)
 #define SY_GEN_E (1 << (SY_GEN_C - 1))  // entries per window
@@ -481,14 +481,14 @@ SY_HD void gen_entry_load(const uint8_t* p, Affine<Fp2>& e) {
   e.y = Fp2{b.x, b.y};
 }
 
-// k G over the table `tab` of G (SY_GEN_W x SY_GEN_E entries of 2 sizeof(F) bytes): the digit only selects an entry
-// and the sign of its y, a zero digit keeps the accumulator; no data-dependent branches.
+// acc + k G over the table `tab` of G (SY_GEN_W x SY_GEN_E entries of 2 sizeof(F) bytes): the digit only selects an entry
+// and the sign of its y, a zero digit keeps the accumulator; no data-dependent branches.  A non-zero start lets one
+// accumulator walk the tables of several bases (groth16.cuh: groth16_public_term).
 template <class F>
-SY_HD_NOINLINE Proj<F> gen_scalar_mul(const uint8_t* __restrict__ tab, const uint32_t* k_in) {
+SY_HD Proj<F> gen_scalar_mul_add(const uint8_t* __restrict__ tab, const uint32_t* k_in, Proj<F> acc) {
   uint32_t k[8];
   for (int i = 0; i < 8; i++) k[i] = k_in[i];
   scalar_reduce_r(k);
-  Proj<F> acc = proj_zero<F>();
   int carry = 0;
 #pragma unroll
   for (int w = 0; w < SY_GEN_W; w++) {
@@ -503,6 +503,11 @@ SY_HD_NOINLINE Proj<F> gen_scalar_mul(const uint8_t* __restrict__ tab, const uin
     acc.z = f_select(m != 0, s.z, acc.z);
   }
   return acc;
+}
+// k G (gen_scalar_mul_add from O)
+template <class F>
+SY_HD_NOINLINE Proj<F> gen_scalar_mul(const uint8_t* __restrict__ tab, const uint32_t* k_in) {
+  return gen_scalar_mul_add<F>(tab, k_in, proj_zero<F>());
 }
 
 // y^2 == x^3 + b

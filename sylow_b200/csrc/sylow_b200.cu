@@ -17,6 +17,7 @@
 #include "miller_tables.cuh"
 #include "group_law.cuh"
 #include "launch_plan.h"
+#include "groth16.cuh"
 
 using namespace sylow;
 
@@ -197,11 +198,13 @@ __global__ void k_gt_is_one(const uint8_t* gt, size_t n, uint8_t* ok) {
 // Projective (Montgomery form) -> affine wire format for a whole batch with Montgomery's trick: thread t owns the
 // SY_AFF_K points t, t + T, t + 2T, ... (coalesced), multiplies their Z together, inverts ONCE and unwinds.  A point at
 // infinity (Z = 0) enters the product as 1 and is written as (0, 1) + flag, like GroupAffine::from (group.rs:475-495).
-// F = Fp: G1, 96-byte projective / 64-byte affine points; F = Fp2: G2, 192 / 128 bytes.
+// F = Fp: G1, 96-byte projective / 64-byte affine points; F = Fp2: G2, 192 / 128 bytes.  Output i goes to record i of
+// `stride` points (and flags): stride 1 is a plain point array, 4 the 4-point records of the Groth16 check.
 #define SY_AFF_K 8
 template <class F>
 __device__ __forceinline__ void batch_affine(const uint8_t* __restrict__ proj, size_t n, int negate,
-                                             uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf) {
+                                             uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
+                                             size_t stride = 1) {
   constexpr size_t W = sizeof(F);  // bytes per coordinate in both encodings
   F one;
   f_set_one(one);
@@ -234,15 +237,15 @@ __device__ __forceinline__ void batch_affine(const uint8_t* __restrict__ proj, s
     } else if (negate) {
       y = f_neg(y);
     }
-    f_store(out + i * 2 * W, x);
-    f_store(out + i * 2 * W + W, y);
-    if (out_inf) out_inf[i] = inf;
+    f_store(out + i * stride * 2 * W, x);
+    f_store(out + i * stride * 2 * W + W, y);
+    if (out_inf) out_inf[i * stride] = inf;
   }
 }
 __global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
 k_g1_batch_affine(const uint8_t* __restrict__ proj, size_t n, int negate, uint8_t* __restrict__ out,
-                  uint8_t* __restrict__ out_inf) {
-  batch_affine<Fp>(proj, n, negate, out, out_inf);
+                  uint8_t* __restrict__ out_inf, size_t stride) {
+  batch_affine<Fp>(proj, n, negate, out, out_inf, stride);
 }
 __global__ void __launch_bounds__(SY_MUL_THREADS, 1)
 k_g2_batch_affine(const uint8_t* __restrict__ proj, size_t n, uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf) {
@@ -254,11 +257,12 @@ k_g2_batch_affine(const uint8_t* __restrict__ proj, size_t n, uint8_t* __restric
 //    block-synchronised; surplus threads store nothing;
 //  - with proj_out (large batches) the raw projective record for batch_affine, which shares one inversion between
 //    SY_AFF_K points and applies the negation;
-//  - otherwise the affine wire form and flag, y negated when negate is set and the point is finite.
+//  - otherwise the affine wire form and flag, y negated when negate is set and the point is finite, into record i of
+//    `stride` points (batch_affine's).
 template <class F>
 __device__ __forceinline__ void put_point(const Proj<F>& q, size_t i0, size_t i, size_t n, int negate,
                                           uint8_t* __restrict__ out, uint8_t* __restrict__ out_inf,
-                                          uint8_t* __restrict__ proj_out) {
+                                          uint8_t* __restrict__ proj_out, size_t stride = 1) {
   constexpr size_t W = sizeof(F);
   if (proj_out) {
     if (i0 < n) proj_store_raw(proj_out + i * 3 * W, q);
@@ -267,9 +271,9 @@ __device__ __forceinline__ void put_point(const Proj<F>& q, size_t i0, size_t i,
   Affine<F> r = proj_to_affine(q);
   if (i0 >= n) return;
   if (negate && !r.inf) r.y = f_neg(r.y);
-  f_store(out + i * 2 * W, r.x);
-  f_store(out + i * 2 * W + W, r.y);
-  if (out_inf) out_inf[i] = r.inf;
+  f_store(out + i * stride * 2 * W, r.x);
+  f_store(out + i * stride * 2 * W + W, r.y);
+  if (out_inf) out_inf[i * stride] = r.inf;
 }
 
 // the variable-base ladders: GLV on G1, GLS on G2
@@ -333,6 +337,113 @@ __global__ void __launch_bounds__(SY_G2_THREADS, SY_G2_MINB)
 k_g2_mul_gen(const uint8_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n, uint8_t* __restrict__ out,
              uint8_t* __restrict__ out_inf, uint8_t* __restrict__ proj_out) {
   mul_gen<Fp2>(table, scalars, n, out, out_inf, proj_out);
+}
+
+// ---- Groth16 (groth16.cuh) ----------------------------------------------------------------------------------------
+// Proof j (A || B || C, 256 B; flags A, B, C at proofs_inf[3 j ..]) against the prepared key vk -> the 4-point record
+// [A, -alpha, -L, -C] (rec, 256 B) with flags [A, 0, L, C] (rec_inf, 4 B) that k_glued<1, 3> reads with stride 4,
+// B_j to b (128 B) with its flag, in_range[j] = every public input of proof j is < r.  -L goes through put_point, so
+// from SY_AFF_MIN_BATCH proofs on batch_affine writes it with the same record stride.
+__global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
+k_groth16_assemble(const uint8_t* __restrict__ vk, size_t l, const uint8_t* __restrict__ proofs,
+                   const uint8_t* __restrict__ proofs_inf, const uint8_t* __restrict__ inputs, size_t n,
+                   uint8_t* __restrict__ rec, uint8_t* __restrict__ rec_inf, uint8_t* __restrict__ b,
+                   uint8_t* __restrict__ b_inf, uint8_t* __restrict__ in_range, uint8_t* __restrict__ proj_out) {
+  size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  size_t i = i0 < n ? i0 : n - 1;  // every thread reaches put_point's block-synchronised inversion
+  bool ok;
+  G1Proj L = groth16_public_term(vk, l, l ? inputs + i * l * 32 : nullptr, ok);
+  put_point(L, i0, i, n, 1, rec + 128, rec_inf + 2, proj_out, 4);
+  if (i0 >= n) return;
+  groth16_record(vk, proofs + i * 256, proofs_inf ? proofs_inf + 3 * i : nullptr, rec + i * 256, rec_inf + 4 * i,
+                 b + i * 128, b_inf + i);
+  in_range[i] = ok;
+}
+// a = the A, b = the B, c = the C of every proof as point arrays; inf = their flags, n A flags, then n B, then n C
+__global__ void k_groth16_split(const uint8_t* __restrict__ proofs, const uint8_t* __restrict__ proofs_inf, size_t n,
+                                uint8_t* __restrict__ a, uint8_t* __restrict__ b, uint8_t* __restrict__ c,
+                                uint8_t* __restrict__ inf) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint4* p = reinterpret_cast<const uint4*>(proofs + i * 256);
+  for (int k = 0; k < 4; k++) {
+    reinterpret_cast<uint4*>(a + i * 64)[k] = p[k];
+    reinterpret_cast<uint4*>(c + i * 64)[k] = p[12 + k];
+  }
+  for (int k = 0; k < 8; k++) reinterpret_cast<uint4*>(b + i * 128)[k] = p[4 + k];
+  for (int k = 0; k < 3; k++) inf[k * n + i] = proofs_inf ? proofs_inf[3 * i + k] : 0;
+}
+// The weighted Fr sums of the batch: column c = 0 is s_0 = sum_j r_j, column c = i >= 1 is s_i = sum_j r_j x_j(i-1).
+// Per-thread partial sums over a strided share of the proofs, a tree in shared memory per block (k_groth16_fr_partial,
+// one partial per block and column, scaled by 1/R: fr_weighted), then a tree over the block partials
+// (k_groth16_fr_final).  *bad = 1 if any input is >= r.
+#define SY_FR_THREADS 256
+__device__ __forceinline__ Fr fr_block_sum(Fr v) {  // to thread 0
+  __shared__ Fr sh[SY_FR_THREADS];
+  sh[threadIdx.x] = v;
+  __syncthreads();
+  for (unsigned off = SY_FR_THREADS / 2; off > 0; off >>= 1) {
+    if (threadIdx.x < off) sh[threadIdx.x] = fr_add(sh[threadIdx.x], sh[threadIdx.x + off]);
+    __syncthreads();
+  }
+  return sh[0];
+}
+__global__ void __launch_bounds__(SY_FR_THREADS)
+k_groth16_fr_partial(const uint8_t* __restrict__ inputs, size_t l, const uint64_t* __restrict__ w, size_t n,
+                     uint8_t* __restrict__ part, int* __restrict__ bad) {
+  const size_t c = blockIdx.y;
+  const uint32_t one[8] = {1, 0, 0, 0, 0, 0, 0, 0};
+  Fr acc{};
+  bool ok = true;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (size_t)gridDim.x * blockDim.x) {
+    if (c) {
+      const Fp x = fp_load_raw(inputs + (j * l + c - 1) * 32);
+      ok &= fr_words_canonical(x.l);
+      acc = fr_add(acc, fr_weighted(x.l, w[j]));
+    } else {
+      acc = fr_add(acc, fr_weighted(one, w[j]));
+    }
+  }
+  if (!ok) atomicExch(bad, 1);
+  const Fr s = fr_block_sum(acc);
+  if (threadIdx.x == 0)
+    for (int k = 0; k < 8; k++) reinterpret_cast<uint32_t*>(part + (c * gridDim.x + blockIdx.x) * 32)[k] = s.l[k];
+}
+// s_out = s_0 || s_0 || s_1 .. s_l, canonical 32-byte integers (s_0 twice: the scalars of the ladders over -alpha and
+// IC_0, which sit side by side in the prepared key)
+__global__ void __launch_bounds__(SY_FR_THREADS)
+k_groth16_fr_final(const uint8_t* __restrict__ part, size_t nb, uint8_t* __restrict__ s_out) {
+  const size_t c = blockIdx.x;
+  Fr acc{};
+  for (size_t k = threadIdx.x; k < nb; k += blockDim.x) {
+    Fr v;
+    for (int t = 0; t < 8; t++) v.l[t] = reinterpret_cast<const uint32_t*>(part + (c * nb + k) * 32)[t];
+    acc = fr_add(acc, v);
+  }
+  Fr s = fr_block_sum(acc);
+  if (threadIdx.x) return;
+  s = fr_unscale(s);
+  for (int t = 0; t < 8; t++) {
+    reinterpret_cast<uint32_t*>(s_out + (c + 1) * 32)[t] = s.l[t];
+    if (c == 0) reinterpret_cast<uint32_t*>(s_out)[t] = s.l[t];
+  }
+}
+// proj_out[i] = s[i] IC_(i+1) (projective, Montgomery form) over the prepared key's fixed-base tables, i < l
+__global__ void __launch_bounds__(SY_MUL_THREADS, SY_G1_MINB)
+k_groth16_ic_mul(const uint8_t* __restrict__ vk, const uint8_t* __restrict__ s, size_t l, uint8_t* __restrict__ proj_out) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= l) return;
+  const Fp k = fp_load_raw(s + i * 32);
+  proj_store_raw(proj_out + i * 96, gen_scalar_mul<Fp>(vk + kG16Tables + i * kG16IcTable, k.l));
+}
+// an input >= r: the partial becomes the Fp12 zero, whose final exponentiation is zero, never the identity (24 threads)
+__global__ void k_groth16_fail_closed(const int* __restrict__ bad, uint8_t* __restrict__ f) {
+  if (*bad) reinterpret_cast<uint4*>(f)[threadIdx.x] = make_uint4(0, 0, 0, 0);
+}
+// ok[i] &= flag[i]
+__global__ void k_and_flags(uint8_t* __restrict__ ok, const uint8_t* __restrict__ flag, size_t n) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) ok[i] &= flag[i];
 }
 
 // out[i] = affine(a[i] + b[i]), or affine(a[i] - b[i]) when subtract != 0 (add_pair, group_law.cuh)
@@ -1186,10 +1297,10 @@ static int launch_miller_tables(sylow_b200_ctx* ctx, int m, const uint8_t* table
 #endif
 // n points of G1 or G2 (g2) -> affine wire format + infinity flags at out / out_inf, G1 points negated when negate is
 // set: launch(proj) enqueues the point kernel on s with proj_out = proj, which is ctx->proj from min_batch points on
-// (followed by the batched conversion) and null below.
+// (followed by the batched conversion) and null below.  G1 points can land in records of `stride` points (put_point).
 template <class Launch>
 static int point_batch(sylow_b200_ctx* ctx, bool g2, size_t n, size_t min_batch, int negate, uint8_t* out,
-                       uint8_t* out_inf, cudaStream_t s, Launch launch) {
+                       uint8_t* out_inf, cudaStream_t s, Launch launch, size_t stride = 1) {
   uint8_t* proj = nullptr;
   if (n >= min_batch) {
     CKS(reserve(ctx, ctx->proj, n * (g2 ? 192 : 96)));
@@ -1202,7 +1313,7 @@ static int point_batch(sylow_b200_ctx* ctx, bool g2, size_t n, size_t min_batch,
   if (g2)
     k_g2_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(proj, n, out, out_inf);
   else
-    k_g1_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(proj, n, negate, out, out_inf);
+    k_g1_batch_affine<<<blocks, SY_MUL_THREADS, 0, s>>>(proj, n, negate, out, out_inf, stride);
   LAUNCHED(ctx);
   return 0;
 }
@@ -1525,40 +1636,55 @@ static int ensure_gen_table(sylow_b200_ctx* ctx, cudaStream_t s) {
   return 0;
 }
 
-// Fixed-base table of the G1 (g2 = 0) or G2 generator for gen_scalar_mul (curve.cuh), built on the device once per
-// context: the ladder of mul_dev multiplies the generator by (j + 1) 2^(C w) mod r, and k_fp_convert takes
-// the affine results to Montgomery form, so every entry is the ladder's own point.  The field is set only after the
-// build has finished, like ensure_gen_table's.
-static int ensure_mul_table(sylow_b200_ctx* ctx, int g2, cudaStream_t s) {
-  if (ctx->d_mul_table[g2]) return 0;
-  const size_t n = (size_t)SY_GEN_W * SY_GEN_E, pb = g2 ? 128 : 64, in_bytes = n * (32 + pb);
-  std::vector<uint8_t> in(in_bytes);  // n scalars, then the generator n times
-  Fr step{{1}};                       // 2^(C w) mod r
+// Fixed-base tables for gen_scalar_mul (curve.cuh) of k base points of G1 (g2 = 0) or G2, given in host wire form, to
+// d_tab (k tables of SY_GEN_W x SY_GEN_E entries, one after the other): the ladder of mul_dev multiplies each base by
+// (j + 1) 2^(C w) mod r, and k_fp_convert takes the affine results to Montgomery form, so every entry is the ladder's
+// own point.  All k tables come from one batch of ladders.  Synchronises s.
+static int build_mul_tables(sylow_b200_ctx* ctx, int g2, const uint8_t* bases, size_t k, uint8_t* d_tab, cudaStream_t s) {
+  const size_t e = (size_t)SY_GEN_W * SY_GEN_E, n = e * k, pb = g2 ? 128 : 64, in_bytes = n * (32 + pb);
+  std::vector<uint8_t> in;  // n scalars, then each base e times
+  try {
+    in.resize(in_bytes);
+  } catch (...) {
+    return SYLOW_B200_ERR_NOMEM;
+  }
+  Fr step{{1}};  // 2^(C w) mod r
   for (int w = 0; w < SY_GEN_W; w++) {
     Fr m = step;
     for (int j = 0; j < SY_GEN_E; j++, m = fr_add(m, step)) memcpy(&in[((size_t)w * SY_GEN_E + j) * 32], m.l, 32);
     for (int b = 0; b < SY_GEN_C; b++) step = fr_add(step, step);
   }
-  static const uint64_t kG1GenWords[8] = {1, 0, 0, 0, 2, 0, 0, 0};  // (1, 2)
-  for (size_t i = 0; i < n; i++) memcpy(&in[n * 32 + i * pb], g2 ? (const void*)kG2GenWords : kG1GenWords, pb);
-  uint8_t *d_in = nullptr, *d_tab = nullptr;
-  cudaError_t e = cudaMalloc(&d_in, in_bytes + n * pb);  // inputs, then the canonical affine points
-  if (e == cudaSuccess) e = cudaMalloc(&d_tab, n * pb);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d_in, in.data(), in_bytes, cudaMemcpyHostToDevice, s);
-  int st = e == cudaSuccess ? 0 : fail_cuda(ctx, e);
+  for (size_t t = 1; t < k; t++) memcpy(&in[t * e * 32], in.data(), e * 32);
+  for (size_t i = 0; i < n; i++) memcpy(&in[n * 32 + i * pb], bases + (i / e) * pb, pb);
+  uint8_t* d_in = nullptr;
+  cudaError_t err = cudaMalloc(&d_in, in_bytes + n * pb);  // inputs, then the canonical affine points
+  if (err == cudaSuccess) err = cudaMemcpyAsync(d_in, in.data(), in_bytes, cudaMemcpyHostToDevice, s);
+  int st = err == cudaSuccess ? 0 : fail_cuda(ctx, err);
   uint8_t* d_aff = d_in + in_bytes;
   if (!st)
     st = mul_dev(ctx, g2, d_in + n * 32, nullptr, d_in, n, d_aff, nullptr, s);
   if (!st) {
     k_fp_convert<<<nblocks(n * pb / 32, 128), 128, 0, s>>>(d_aff, n * pb / 32, d_tab, 1);
     ctx->launches++;
-    e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess) st = fail_cuda(ctx, e);
+    err = cudaGetLastError();
+    if (err == cudaSuccess) err = cudaStreamSynchronize(s);
+    if (err != cudaSuccess) st = fail_cuda(ctx, err);
   }
   if (d_in) cudaFree(d_in);
+  return st;
+}
+
+// Fixed-base table of the G1 (g2 = 0) or G2 generator, built on the device once per context.  The field is set only
+// after the build has finished, like ensure_gen_table's.
+static int ensure_mul_table(sylow_b200_ctx* ctx, int g2, cudaStream_t s) {
+  if (ctx->d_mul_table[g2]) return 0;
+  static const uint64_t kG1GenWords[8] = {1, 0, 0, 0, 2, 0, 0, 0};  // (1, 2)
+  uint8_t* d_tab = nullptr;
+  cudaError_t e = cudaMalloc(&d_tab, (size_t)SY_GEN_W * SY_GEN_E * (g2 ? 128 : 64));
+  if (e != cudaSuccess) return fail_cuda(ctx, e);
+  const int st = build_mul_tables(ctx, g2, reinterpret_cast<const uint8_t*>(g2 ? kG2GenWords : kG1GenWords), 1, d_tab, s);
   if (st) {
-    if (d_tab) cudaFree(d_tab);
+    cudaFree(d_tab);
     return st;
   }
   ctx->d_mul_table[g2] = d_tab;
@@ -1665,6 +1791,29 @@ static int g1_sum_reduce(sylow_b200_ctx* ctx, const uint8_t* d_pts, const uint8_
   return 0;
 }
 
+// The Miller values of n >= 1 fused pairs (g1[k], g2[k]) that only ever meet as a product, Montgomery form, to f;
+// *n_f = the number of values written.  1, 2 or 4 pairs share one thread and ONE Fp12 squaring per loop digit - what
+// glued_miller_loop does for the whole batch in the reference (pairing.rs:970-1022).  A thread's 2 / 4 pairs save
+// 63 x 36 of the 8 444 multiplications of every pair after its first.  The n % glue leftover pairs go through k_miller.
+// The glue is the one of fewest wave-times (glue_pairs).  Measured on verify_batch at 2^20 signatures
+// (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 / 163.3 ms for 1 / 2 / 4; at 2^13 the order reverses (9.3 / 12.4 /
+// 18.4 ms: a quarter of the threads, each four times as long).
+static int fused_product_values(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
+                                const uint8_t* g2_inf, size_t n, uint8_t* f, size_t* n_f, cudaStream_t s) {
+  const int glue = glue_pairs(ctx->sms, n, 8444, kGluedShape);
+  if (glue > 1 && n >= (size_t)glue) {
+    const size_t items = n / glue, done = items * glue;
+    CKS(launch_glued(ctx, glue, 0, g1, glue, g1_inf, g2, g2_inf, nullptr, 0, nullptr, nullptr, items, f, s));
+    if (done < n)
+      CKS(launch_miller(ctx, g1 + done * 64, adv(g1_inf, done), g2 + done * 128, adv(g2_inf, done), n - done,
+                        f + items * 384, 1, s));
+    *n_f = items + (n - done);
+    return 0;
+  }
+  *n_f = n;
+  return launch_miller(ctx, g1, g1_inf, g2, g2_inf, n, f, 1, s);
+}
+
 static bool load_seed(const uint8_t* weight_seed, WeightSeed& ws) {
   if (!weight_seed) return false;
   memcpy(ws.w, weight_seed, 32);
@@ -1706,26 +1855,8 @@ static int verify_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_pks, const 
       k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_hm, d_hm_inf, ws, first_index, n, proj);
     }));
   }
-  // The n Miller loops (-r_i H(m_i), pk_i) only ever meet as a product, so 1, 2 or 4 signatures share one thread
-  // and ONE Fp12 squaring per loop digit - what glued_miller_loop does for the whole batch in the reference
-  // (pairing.rs:970-1022).  A thread's 2 / 4 pairs save 63 x 36 of the 8 444 multiplications of every pair after its
-  // first.  The n % GLUE leftover pairs go through k_miller.
-  // The glue is the one of fewest wave-times (glue_pairs).  Measured at 2^20 signatures
-  // (profiles/r02_verify_glue.jsonl): 192.4 / 171.2 / 163.3 ms for 1 / 2 / 4; at 2^13 the order reverses (9.3 / 12.4 /
-  // 18.4 ms: a quarter of the threads, each four times as long).
-  const int glue = glue_pairs(ctx->sms, n, 8444, kGluedShape);
-  size_t n_f = n;  // Miller values in scratch0 before the signature pair's value is appended
-  if (glue > 1 && n >= (size_t)glue) {
-    const size_t items = n / glue, done = items * glue;
-    CKS(launch_glued(ctx, glue, 0, d_hm, glue, d_hm_inf, d_pks, d_pks_inf, nullptr, 0, nullptr, nullptr, items,
-                     ctx->scratch0.p, s));
-    if (done < n)
-      CKS(launch_miller(ctx, d_hm + done * 64, d_hm_inf + done, d_pks + done * 128, d_pks_inf ? d_pks_inf + done : nullptr,
-                        n - done, ctx->scratch0.p + items * 384, 1, s));
-    n_f = items + (n - done);
-  } else {
-    CKS(launch_miller(ctx, d_hm, d_hm_inf, d_pks, d_pks_inf, n, ctx->scratch0.p, 1, s));
-  }
+  size_t n_f;  // Miller values in scratch0 before the signature pair's value is appended
+  CKS(fused_product_values(ctx, d_hm, d_hm_inf, d_pks, d_pks_inf, n, ctx->scratch0.p, &n_f, s));
   if (weighted) {
     k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_sigs, d_sigs_inf, ws, first_index, n,
                                                                        ctx->proj.p);
@@ -2396,6 +2527,222 @@ int sylow_b200_miller_product_precomputed_dev(sylow_b200_ctx* ctx, const uint8_t
     return 0;
   }
   return miller_product_tables(ctx, d_tables, n_tables, d_table_idx, d_g1, d_g1_inf, n, d_f_out, s);
+}
+
+// ------------------------------------------------------------------------------- Groth16
+static_assert(kG16NegAlpha == 3 * SY_TABLE_BYTES && kG16IcTable == (size_t)SY_GEN_W * SY_GEN_E * 64 &&
+                  g16_vk_bytes(5) == SYLOW_B200_GROTH16_VK_DEV_BYTES(5),
+              "groth16.cuh's device key layout and the header's SYLOW_B200_GROTH16_VK_DEV_BYTES disagree");
+static constexpr size_t kG16VkHostBase = 448;  // alpha || beta || gamma || delta; IC_0 .. IC_l follow, 64 B each
+
+// Validates the host key vk of l public inputs and builds its device form at d_vk; io stages the key.  The first failing
+// status in key order (alpha, beta, gamma, delta, IC_0 .. IC_l) is returned and nothing is built.  The build runs on s
+// and is finished when this returns.
+static int groth16_prepare_core(Staging& io, const uint8_t* vk, size_t l, uint8_t* d_vk, cudaStream_t s) {
+  sylow_b200_ctx* ctx = io.ctx;
+  const size_t n_st = l + 5;
+  const uint8_t* dv = io.up(vk, kG16VkHostBase + 64 * (l + 1));
+  int8_t* d_st = reinterpret_cast<int8_t*>(io.area(n_st + 1));  // statuses, then -alpha's infinity flag
+  CKS(io.err);
+  k_g1_validate<<<1, 32, 0, ctx->stream>>>(dv, nullptr, 1, d_st, 0);
+  LAUNCHED(ctx);
+  k_g2_validate<<<1, SY_MUL_THREADS, 0, ctx->stream>>>(dv + 64, nullptr, 3, d_st + 1, 0);
+  LAUNCHED(ctx);
+  k_g1_validate<<<nblocks(l + 1, 128), 128, 0, ctx->stream>>>(dv + kG16VkHostBase, nullptr, l + 1, d_st + 4, 0);
+  LAUNCHED(ctx);
+  std::vector<int8_t> st(n_st);
+  io.down(st.data(), d_st, n_st);
+  CKS(io.err);
+  CK(cudaStreamSynchronize(ctx->stream));
+  for (int8_t v : st)
+    if (v) return v;
+  k_g2_precompute<<<1, 32, 0, s>>>(dv + 64, 3, d_vk, 1);  // beta, gamma, delta
+  LAUNCHED(ctx);
+  CKS(g1_sum_reduce(ctx, dv, nullptr, 1, 1, d_vk + kG16NegAlpha, reinterpret_cast<uint8_t*>(d_st) + n_st, s));
+  CK(cudaMemcpyAsync(d_vk + kG16Ic0, dv + kG16VkHostBase, 64, cudaMemcpyDeviceToDevice, s));
+  if (l) return build_mul_tables(ctx, 0, vk + kG16VkHostBase + 64, l, d_vk + kG16Tables, s);
+  CK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+// ok[j] = the Groth16 check of proof j against the prepared key d_vk: the records [A, -alpha, -L, -C] of
+// k_groth16_assemble, one k_glued<1, 3> per proof, launch_check_products, then the input range flags
+static int groth16_each_core(sylow_b200_ctx* ctx, const uint8_t* d_vk, size_t l, const uint8_t* proofs,
+                             const uint8_t* proofs_inf, const uint8_t* inputs, size_t n, uint8_t* ok, cudaStream_t s) {
+  CKS(reserve(ctx, ctx->scratch0, n * 384));
+  CKS(reserve(ctx, ctx->scratch2, n * (256 + 128 + 4 + 1 + 1)));
+  uint8_t* rec = ctx->scratch2.p;
+  uint8_t* b = rec + n * 256;
+  uint8_t* rec_inf = b + n * 128;
+  uint8_t* b_inf = rec_inf + n * 4;
+  uint8_t* in_range = b_inf + n;
+  CKS(point_batch(ctx, false, n, SY_AFF_MIN_BATCH, 1, rec + 128, rec_inf + 2, s, [&](uint8_t* proj) {
+    k_groth16_assemble<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(d_vk, l, proofs, proofs_inf, inputs, n, rec,
+                                                                          rec_inf, b, b_inf, in_range, proj);
+  }, 4));
+  CKS(launch_glued(ctx, 1, 3, rec, 4, rec_inf, b, b_inf, rec + 64, 4, rec_inf + 1, d_vk, n, ctx->scratch0.p, s));
+  CKS(launch_check_products(ctx, ctx->scratch0.p, 1, n, ok, s));
+  k_and_flags<<<nblocks(n, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(ok, in_range, n);
+  LAUNCHED(ctx);
+  return 0;
+}
+
+// d_f_out (384 B, canonical) = this slice's share of prod_j check_j^{r_j}, r_j = batch_weight(ws, first_index + j):
+// the n fused pairs (r_j A_j, B_j), glued like verify_batch's, times ONE k_glued<1, 3> item of the three table pairs
+// (-s_0 alpha, beta), (-(s_0 IC_0 + sum_i s_i IC_i), gamma), (-sum_j r_j C_j, delta) with its fused pair flagged away.
+// An input >= r makes the share the Fp12 zero (k_groth16_fail_closed).
+static int groth16_partial_core(sylow_b200_ctx* ctx, const uint8_t* d_vk, size_t l, const uint8_t* proofs,
+                                const uint8_t* proofs_inf, const uint8_t* inputs, size_t n, const WeightSeed& ws,
+                                uint64_t first_index, uint8_t* d_f_out, cudaStream_t s) {
+  if (!n) {
+    CK(cudaMemcpyAsync(d_f_out, kOneCanonical, 384, cudaMemcpyHostToDevice, s));
+    return 0;
+  }
+  const size_t cols = l + 1, nb = nblocks(n, SY_FR_THREADS) < 256 ? nblocks(n, SY_FR_THREADS) : 256;
+  auto up16 = [](size_t b) { return (b + 15) / 16 * 16; };
+  // scratch2: A (weighted in place), B, C, their flags, the weights, the Fr partials and sums, the ladder results, and
+  // the record of the table pairs: [unused, -s_0 alpha, -sum r L, -sum r C] + flags, an unused B + flag, the range flag
+  const size_t o_b = up16(n * 64), o_c = o_b + n * 128, o_inf = o_c + n * 64, o_w = up16(o_inf + 3 * n),
+               o_part = o_w + n * 8, o_s = up16(o_part + nb * cols * 32), o_lad = o_s + (cols + 1) * 32,
+               o_rec = o_lad + (cols + 1) * 96, o_b0 = o_rec + 256, o_rinf = o_b0 + 128, o_bad = o_rinf + 8,
+               total = o_bad + 16;
+  CKS(reserve(ctx, ctx->scratch0, (n + 1) * 384));
+  CKS(reserve(ctx, ctx->scratch1, ((n + 1) / 4 + 1) * 384));
+  CKS(reserve(ctx, ctx->scratch2, total));
+  uint8_t* x = ctx->scratch2.p;
+  uint8_t *a = x, *b = x + o_b, *c = x + o_c, *inf = x + o_inf, *part = x + o_part, *sv = x + o_s, *lad = x + o_lad;
+  uint8_t *rec = x + o_rec, *rinf = x + o_rinf;
+  uint64_t* w = reinterpret_cast<uint64_t*>(x + o_w);
+  int* bad = reinterpret_cast<int*>(x + o_bad);
+  CK(cudaMemsetAsync(rec, 0, total - o_rec, s));
+  CK(cudaMemsetAsync(rinf, 1, 1, s));      // the table item's fused pair: skipped on its G1 ...
+  CK(cudaMemsetAsync(rinf + 4, 1, 1, s));  // ... and its G2 side
+  k_groth16_split<<<nblocks(n, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(proofs, proofs_inf, n, a, b, c, inf);
+  LAUNCHED(ctx);
+  k_batch_weights<<<nblocks(n, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(ws, first_index, n, w);
+  LAUNCHED(ctx);
+  k_groth16_fr_partial<<<dim3((unsigned)nb, (unsigned)cols), SY_FR_THREADS, 0, s>>>(inputs, l, w, n, part, bad);
+  LAUNCHED(ctx);
+  k_groth16_fr_final<<<(unsigned)cols, SY_FR_THREADS, 0, s>>>(part, nb, sv);
+  LAUNCHED(ctx);
+  // r_j A_j in place; k_g1_mul_weight writes projective points only (min_batch 0)
+  CKS(point_batch(ctx, false, n, 0, 0, a, inf, s, [&](uint8_t* proj) {
+    k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(a, inf, ws, first_index, n, proj);
+  }));
+  size_t n_f;
+  CKS(fused_product_values(ctx, a, inf, b, inf + n, n, ctx->scratch0.p, &n_f, s));
+  k_g1_mul_weight<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, s>>>(c, inf + 2 * n, ws, first_index, n, ctx->proj.p);
+  LAUNCHED(ctx);
+  CKS(g1_sum_reduce(ctx, ctx->proj.p, nullptr, n, 1, rec + 192, rinf + 3, s, 0));
+  // s_0 (-alpha) and s_0 IC_0 by the variable-base ladder, s_i IC_i from the key's tables; then -(sum r L)
+  k_g1_mul<<<1, SY_MUL_THREADS, 0, s>>>(d_vk + kG16NegAlpha, nullptr, sv, 2, nullptr, nullptr, lad);
+  LAUNCHED(ctx);
+  if (l) {
+    k_groth16_ic_mul<<<nblocks(l, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(d_vk, sv + 64, l, lad + 192);
+    LAUNCHED(ctx);
+  }
+  CKS(g1_sum_reduce(ctx, lad + 96, nullptr, cols, 1, rec + 128, rinf + 2, s, 0));
+  k_g1_finish_sum<<<1, 1, 0, s>>>(lad, 0, rec + 64, rinf + 1);
+  LAUNCHED(ctx);
+  CKS(launch_glued(ctx, 1, 3, rec, 4, rinf, x + o_b0, rinf + 4, rec + 64, 4, rinf + 1, d_vk, 1,
+                   ctx->scratch0.p + n_f * 384, s));
+  CKS(product_reduce(ctx, ctx->scratch0.p, ctx->scratch1.p, n_f + 1, d_f_out, 0, s));
+  k_groth16_fail_closed<<<1, 24, 0, s>>>(bad, d_f_out);
+  LAUNCHED(ctx);
+  return 0;
+}
+
+int sylow_b200_groth16_prepare_vk(sylow_b200_ctx* ctx, const uint8_t* vk, size_t n_public, uint8_t* d_vk_out,
+                                  void* stream) {
+  ENTER_DEV(ctx);
+  if (!vk || !d_vk_out) return SYLOW_B200_ERR_ARG;
+  Staging io(ctx);
+  CKS(groth16_prepare_core(io, vk, n_public, d_vk_out, pick(ctx, stream)));
+  return io.finish();
+}
+
+int sylow_b200_groth16_verify_each_dev(sylow_b200_ctx* ctx, const uint8_t* d_vk, size_t n_public,
+                                       const uint8_t* d_proofs, const uint8_t* d_proofs_inf, const uint8_t* d_inputs,
+                                       size_t n, uint8_t* d_ok_out, void* stream) {
+  ENTER_DEV(ctx);
+  if (n && (!d_vk || !d_proofs || !d_ok_out || (n_public && !d_inputs))) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  return groth16_each_core(ctx, d_vk, n_public, d_proofs, d_proofs_inf, d_inputs, n, d_ok_out, pick(ctx, stream));
+}
+
+int sylow_b200_groth16_verify_batch_partial_dev(sylow_b200_ctx* ctx, const uint8_t* d_vk, size_t n_public,
+                                                const uint8_t* d_proofs, const uint8_t* d_proofs_inf,
+                                                const uint8_t* d_inputs, size_t n, const uint8_t* weight_seed,
+                                                uint64_t first_index, uint8_t* d_f_out, void* stream) {
+  ENTER_DEV(ctx);
+  WeightSeed ws;
+  if (!d_f_out || !load_seed(weight_seed, ws) || (n && (!d_vk || !d_proofs || (n_public && !d_inputs))))
+    return SYLOW_B200_ERR_ARG;
+  return groth16_partial_core(ctx, d_vk, n_public, d_proofs, d_proofs_inf, d_inputs, n, ws, first_index, d_f_out,
+                              pick(ctx, stream));
+}
+
+int sylow_b200_groth16_verify_each(sylow_b200_ctx* ctx, const uint8_t* vk, size_t n_public, const uint8_t* proofs,
+                                   const uint8_t* proofs_inf, const uint8_t* inputs, size_t n, uint8_t* ok_out) {
+  const bool args = vk && (!n || (proofs && ok_out && (inputs || !n_public)));
+  if (is_multi(ctx) && args)
+    return multi_slices(ctx, n, [=](sylow_b200_ctx* c, size_t, size_t off, size_t m) {
+      return sylow_b200_groth16_verify_each(c, vk, n_public, proofs + off * 256, adv(proofs_inf, off * 3),
+                                            adv(inputs, off * n_public * 32), m, ok_out + off);
+    });
+  ENTER(ctx);
+  if (!args) return SYLOW_B200_ERR_ARG;
+  if (!n) return 0;
+  Staging io(ctx);
+  uint8_t* d_vk = io.area(g16_vk_bytes(n_public));
+  CKS(groth16_prepare_core(io, vk, n_public, d_vk, ctx->stream));
+  const uint8_t *dp = io.up(proofs, n * 256), *dx = io.up(inputs, n * n_public * 32), *dpi = io.up(proofs_inf, n * 3);
+  uint8_t* d_ok = io.area(n);
+  CKS(io.err);
+  CKS(groth16_each_core(ctx, d_vk, n_public, dp, dpi, dx, n, d_ok, ctx->stream));
+  io.down(ok_out, d_ok, n);
+  return io.finish();
+}
+
+// one device's share of sylow_b200_groth16_verify_batch: the key prepared on that device, then groth16_partial_core
+static int groth16_partial_host(sylow_b200_ctx* ctx, const uint8_t* vk, size_t l, const uint8_t* proofs,
+                                const uint8_t* proofs_inf, const uint8_t* inputs, size_t n, const WeightSeed& ws,
+                                uint64_t first_index, uint8_t f_out[384]) {
+  ENTER(ctx);
+  Staging io(ctx);
+  uint8_t* d_vk = io.area(g16_vk_bytes(l));
+  CKS(groth16_prepare_core(io, vk, l, d_vk, ctx->stream));
+  const uint8_t *dp = io.up(proofs, n * 256), *dx = io.up(inputs, n * l * 32), *dpi = io.up(proofs_inf, n * 3);
+  uint8_t* d_f = io.area(384);
+  CKS(io.err);
+  CKS(groth16_partial_core(ctx, d_vk, l, dp, dpi, dx, n, ws, first_index, d_f, ctx->stream));
+  io.down(f_out, d_f, 384);
+  return io.finish();
+}
+
+int sylow_b200_groth16_verify_batch(sylow_b200_ctx* ctx, const uint8_t* vk, size_t n_public, const uint8_t* proofs,
+                                    const uint8_t* proofs_inf, const uint8_t* inputs, size_t n,
+                                    const uint8_t* weight_seed, int* ok) {
+  WeightSeed ws;
+  if (!ctx || !ok || !vk || !load_seed(weight_seed, ws) || (n && (!proofs || (n_public && !inputs))))
+    return SYLOW_B200_ERR_ARG;
+  if (!n) {
+    *ok = 1;
+    return 0;
+  }
+  // one partial per device over global proof indices, combined like verify_batch's
+  const size_t G = is_multi(ctx) ? ctx->children.size() : 1;
+  std::vector<uint8_t> part(G * 384, 0);
+  for (size_t g = 0; g < G; g++) part[g * 384] = 1;
+  uint8_t* pp = part.data();
+  if (G > 1)
+    CKS(multi_slices(ctx, n, [=, &ws](sylow_b200_ctx* c, size_t g, size_t off, size_t m) {
+      return groth16_partial_host(c, vk, n_public, proofs + off * 256, adv(proofs_inf, off * 3),
+                                  adv(inputs, off * n_public * 32), m, ws, off, pp + g * 384);
+    }));
+  else
+    CKS(groth16_partial_host(ctx, vk, n_public, proofs, proofs_inf, inputs, n, ws, 0, pp));
+  return sylow_b200_verify_batch_finish(ctx, pp, G, ok);
 }
 
 // ------------------------------------------------------------------------------- validation
