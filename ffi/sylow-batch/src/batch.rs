@@ -9,7 +9,8 @@
 //! mod batch;
 //! pub use crate::batch::{final_exponentiation_batch, g1_add_batch, g1_generator_mul_batch, g1_mul_batch, g2_add_batch,
 //!                        g2_generator_mul_batch, g2_mul_batch, glued_miller_loop_batch,
-//!                        glued_miller_loop_precomputed_batch, glued_pairing_batch, pairing_batch, pairing_check_batch, sign_batch,
+//!                        glued_miller_loop_precomputed_batch, glued_pairing_batch, pairing_batch, pairing_check_batch, pairing_check_ragged_batch,
+//!                        sign_batch,
 //!                        threshold_aggregate_batch, verify_batch, verify_each, groth16_verify_each,
 //!                        groth16_verify_batch, Groth16Proof, Groth16VerifyingKey, BatchError, Engine};
 //! ```
@@ -267,6 +268,24 @@ pub fn pairing_check_batch(e: &mut Engine, p: &[G1Projective], q: &[G2Projective
     e.check(unsafe {
         sys::sylow_b200_pairing_check_batch(e.ctx, g1.as_ptr(), g1i.as_ptr(), g2.as_ptr(), g2i.as_ptr(), pairs_per_check,
                                             n / pairs_per_check, ok.as_mut_ptr())
+    })?;
+    Ok(ok.into_iter().map(|b| b != 0).collect())
+}
+
+/// Checks with a pair count each: check c is `glued_pairing(p[o_c..o_{c+1}], q[o_c..o_{c+1}]) == Gt::identity()` with
+/// `o = offsets` (`offsets.len()` = checks + 1, non-decreasing, ending at `p.len()`); an empty check holds.  One call
+/// for a block's ecPairing inputs of every length.
+pub fn pairing_check_ragged_batch(e: &mut Engine, p: &[G1Projective], q: &[G2Projective], offsets: &[u64]) -> Result<Vec<bool>, BatchError> {
+    let n = same_len(p.len(), q.len())?;
+    if offsets.is_empty() || offsets[offsets.len() - 1] != n as u64 {
+        return Err(BatchError::InvalidArgument);
+    }
+    let (g1, g1i) = marshal_g1(p);
+    let (g2, g2i) = marshal_g2(q);
+    let mut ok = vec![0u8; offsets.len() - 1];
+    e.check(unsafe {
+        sys::sylow_b200_pairing_check_ragged_batch(e.ctx, g1.as_ptr(), g1i.as_ptr(), g2.as_ptr(), g2i.as_ptr(),
+                                                   offsets.as_ptr(), offsets.len() - 1, ok.as_mut_ptr())
     })?;
     Ok(ok.into_iter().map(|b| b != 0).collect())
 }

@@ -115,6 +115,19 @@ int sylow_b200_fp12_product(sylow_b200_ctx* ctx, const uint8_t* f, size_t n, uin
 int sylow_b200_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
                                    const uint8_t* g2_inf, size_t pairs_per_check, size_t n_checks, uint8_t* ok_out);
 
+/* Pairing checks with a pair count per check: ok_out[c] = (glued_pairing(pairs [offsets[c], offsets[c+1])) ==
+ * Gt::identity()).  offsets: n_checks + 1 non-decreasing uint64 values, as for the message offsets of the hashing calls
+ * (offsets[0] need not be 0; g1 / g2 / the flags hold offsets[n_checks] pairs).  An empty check is the identity
+ * (ok = 1).  Infinite pairs are skipped, as in pairing_check_batch.  Decreasing offsets: SYLOW_B200_ERR_ARG.
+ * One set of launches for the whole batch: each check of k pairs runs as k / G glued Miller loops of G = 1, 2 or 4
+ * pairs (G chosen once per batch from the total pair count, as for verify_batch) plus one 2-pair and / or one 1-pair
+ * loop for its remainder; the values of a check are multiplied in chunks of at most 32 per thread, level by level,
+ * then one final exponentiation per check.  A multi-device context cuts the batch at check boundaries into slices of
+ * about equal pair counts.  SYLOW_B200_RAGGED_GLUE (1, 2 or 4) fixes G for measurements. */
+int sylow_b200_pairing_check_ragged_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf,
+                                          const uint8_t* g2, const uint8_t* g2_inf, const uint64_t* offsets,
+                                          size_t n_checks, uint8_t* ok_out);
+
 /* ---- precomputed G2 (G2PreComputed) --------------------------------------------------------------- */
 
 /* coeffs_out[i] = G2Affine::precompute(g2[i]) (pairing.rs:676-708): the 87 line-coefficient triples
@@ -184,6 +197,13 @@ int sylow_b200_g2_to_be_bytes_batch(sylow_b200_ctx* ctx, const uint8_t* g2, cons
  * identity.  ok_out[c] = 1/0; status_out[c] = 0 or the first decode/validation error of input c (then ok = 0). */
 int sylow_b200_eip197_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* input, size_t k, size_t n_checks,
                                           uint8_t* ok_out, int8_t* status_out);
+/* EIP-197 over n_checks inputs of any length: input c = input[offsets[c] .. offsets[c+1]) (byte offsets, non-decreasing,
+ * offsets[0] need not be 0).  A length that is a multiple of 192: decode, validate and check, as in
+ * sylow_b200_eip197_pairing_check_batch; an empty input succeeds.  A length that is not: ok = 0 and status =
+ * SYLOW_B200_ERR_ARG, and none of its bytes are decoded.  The call itself returns 0 (SYLOW_B200_ERR_ARG for decreasing
+ * offsets).  Runs as sylow_b200_pairing_check_ragged_batch, sharded the same way on a multi-device context. */
+int sylow_b200_eip197_pairing_check_ragged_batch(sylow_b200_ctx* ctx, const uint8_t* input, const uint64_t* offsets,
+                                                 size_t n_checks, uint8_t* ok_out, int8_t* status_out);
 
 /* The EIP-196 precompile bodies (examples/reth_bn128.rs, the adapter ahead of the ecPairing body at :156-217) over
  * n fixed-size inputs.  The caller zero-pads short calldata and truncates long calldata, as the EVM does.
@@ -385,6 +405,13 @@ int sylow_b200_final_exp_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_f, size
 int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_g1, const uint8_t* d_g1_inf,
                                        const uint8_t* d_g2, const uint8_t* d_g2_inf, size_t pairs_per_check,
                                        size_t n_checks, uint8_t* d_ok_out, void* stream);
+/* Device points, flags and verdicts; offsets in HOST memory: the launch plan is built on the host from them.  The plan's
+ * device copy belongs to the call (a stream-ordered allocation freed on `stream` after its last kernel), so nothing of
+ * it is shared with the next call. */
+int sylow_b200_pairing_check_ragged_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_g1, const uint8_t* d_g1_inf,
+                                              const uint8_t* d_g2, const uint8_t* d_g2_inf,
+                                              const uint64_t* offsets /* host, n_checks + 1 */, size_t n_checks,
+                                              uint8_t* d_ok_out, void* stream);
 /* d_tables: k_fixed tables in the library's device form, produced by sylow_b200_tables_to_device. */
 int sylow_b200_pairing_check_fixed_batch_dev(sylow_b200_ctx* ctx, const uint8_t* d_g1, const uint8_t* d_g1_inf,
                                              const uint8_t* d_g2_var, const uint8_t* d_g2_var_inf, size_t k_var,

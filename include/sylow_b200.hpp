@@ -12,6 +12,7 @@
 #include <memory>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "sylow_b200.h"
@@ -100,6 +101,32 @@ class Engine {
     ck(sylow_b200_pairing_check_batch(ctx_, a.pts.data(), a.inf.data(), b.pts.data(), b.inf.data(), k, n / k, ok.data()),
        "pairing_check_batch");
     return std::vector<bool>(ok.begin(), ok.end());
+  }
+  // check c multiplies pairs [offsets[c], offsets[c+1]); offsets.size() = n_checks + 1, non-decreasing, ending at p.size()
+  std::vector<bool> pairing_check_ragged_batch(const std::vector<G1Affine>& p, const std::vector<G2Affine>& q,
+                                               const std::vector<std::uint64_t>& offsets) {
+    size_t n = same(p.size(), q.size());
+    if (offsets.empty() || offsets.back() != n) throw Error(SYLOW_B200_ERR_ARG, "pairing_check_ragged_batch");
+    Packed a = pack(p), b = pack(q);
+    std::vector<std::uint8_t> ok(offsets.size() - 1);
+    ck(sylow_b200_pairing_check_ragged_batch(ctx_, a.pts.data(), a.inf.data(), b.pts.data(), b.inf.data(), offsets.data(),
+                                             ok.size(), ok.data()),
+       "pairing_check_ragged_batch");
+    return std::vector<bool>(ok.begin(), ok.end());
+  }
+  // EIP-197 ecPairing bodies over calldata of any length: (ok, status) per input; see the C header
+  std::pair<std::vector<bool>, std::vector<std::int8_t>> eip197_pairing_check_ragged_batch(
+      const std::vector<std::vector<std::uint8_t>>& inputs) {
+    std::vector<std::uint64_t> offs(inputs.size() + 1, 0);
+    for (size_t i = 0; i < inputs.size(); i++) offs[i + 1] = offs[i] + inputs[i].size();
+    std::vector<std::uint8_t> buf;
+    buf.reserve(offs.back());
+    for (const auto& in : inputs) buf.insert(buf.end(), in.begin(), in.end());
+    std::vector<std::uint8_t> ok(inputs.size());
+    std::vector<std::int8_t> st(inputs.size());
+    ck(sylow_b200_eip197_pairing_check_ragged_batch(ctx_, buf.data(), offs.data(), inputs.size(), ok.data(), st.data()),
+       "eip197_pairing_check_ragged_batch");
+    return {std::vector<bool>(ok.begin(), ok.end()), st};
   }
 
   // &GroupProjective * &Fp (group.rs:639-667) + GroupAffine::from (:475-495)

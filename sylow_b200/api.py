@@ -82,6 +82,19 @@ def _seed(weight_seed) -> Optional[np.ndarray]:
     return seed
 
 
+def _offsets(offsets, n_items: Optional[int] = None, name: str = "offsets") -> np.ndarray:
+    """n + 1 non-decreasing uint64 offsets of n checks; n_items: the items the arrays hold, which offsets[-1] must equal
+    (the library reads offsets[-1] of them)."""
+    offs = np.ascontiguousarray(offsets, dtype=np.uint64).reshape(-1)
+    if offs.size == 0:
+        raise ValueError("%s of n checks must hold n + 1 entries" % name)
+    if (offs[1:] < offs[:-1]).any():
+        raise ValueError("%s must not decrease" % name)
+    if n_items is not None and int(offs[-1]) != n_items:
+        raise ValueError("%s end at %d, the arrays hold %d pairs" % (name, int(offs[-1]), n_items))
+    return offs
+
+
 def _pairs(g1, g2, g1_inf, g2_inf):
     """(g1, g1_inf, g2, g2_inf, n) of n pairs, in the argument order of the pairing entry points."""
     g1 = _rows(g1, 64, "g1")
@@ -229,6 +242,15 @@ class Engine:
         self._call("sylow_b200_pairing_check_batch", g1, g1_inf, g2, g2_inf, k, n // k, ok)
         return ok.astype(bool)
 
+    def pairing_check_ragged_batch(self, g1, g2, offsets, g1_inf=None, g2_inf=None) -> np.ndarray:
+        """Check c multiplies the pairs [offsets[c], offsets[c + 1]): n_checks + 1 non-decreasing offsets ending at the
+        number of pairs (offsets[0] may be above 0: the pairs before it are not read); an empty check holds."""
+        g1, g1_inf, g2, g2_inf, n = _pairs(g1, g2, g1_inf, g2_inf)
+        offs = _offsets(offsets, n)
+        ok = np.empty(offs.size - 1, dtype=np.uint8)
+        self._call("sylow_b200_pairing_check_ragged_batch", g1, g1_inf, g2, g2_inf, offs, offs.size - 1, ok)
+        return ok.astype(bool)
+
     # ------------------------------------------------------------------ precomputed G2
     def g2_precompute(self, g2) -> np.ndarray:
         """G2Affine::precompute: (n, 87, 3, 64) uint8 canonical line coefficients."""
@@ -335,6 +357,17 @@ class Engine:
         ok = np.empty(n, dtype=np.uint8)
         st = np.empty(n, dtype=np.int8)
         self._call("sylow_b200_eip197_pairing_check_batch", inputs, k, n, ok, st)
+        return ok.astype(bool), st
+
+    def eip197_pairing_check_ragged_batch(self, inputs):
+        """EIP-197 ecPairing bodies over inputs of any length: a list of bytes (or a packed (buffer, offsets) pair, as
+        for messages); returns (ok bool array, int8 status array).  A length that is not a multiple of 192 gives
+        ok = False and status ERR_ARG; an empty input succeeds."""
+        buf, offs, n = _msgs(inputs)
+        offs = _offsets(offs)
+        ok = np.empty(n, dtype=np.uint8)
+        st = np.empty(n, dtype=np.int8)
+        self._call("sylow_b200_eip197_pairing_check_ragged_batch", buf, offs, n, ok, st)
         return ok.astype(bool), st
 
     def _eip196(self, symbol, width, inputs):
@@ -627,6 +660,18 @@ class Engine:
     def pairing_check_batch_dev(self, d_g1, d_g2, pairs_per_check, d_ok, d_g1_inf=None, d_g2_inf=None):
         self._call("sylow_b200_pairing_check_batch_dev", d_g1, d_g1_inf, d_g2, d_g2_inf, pairs_per_check,
                    d_g1.shape[0] // pairs_per_check, d_ok, self._stream())
+
+    def pairing_check_ragged_batch_dev(self, d_g1, d_g2, offsets, d_ok, d_g1_inf=None, d_g2_inf=None):
+        """pairing_check_ragged_batch on torch CUDA tensors (d_g1 (n, 64), d_g2 (n, 128), flags (n,), d_ok (n_checks,)
+        uint8) with host (numpy) offsets; enqueued on torch's current stream."""
+        n = d_g1.shape[0]
+        offs = _offsets(offsets, n)
+        for t, name, want in ((d_g2, "d_g2", n), (d_g1_inf, "d_g1_inf", n), (d_g2_inf, "d_g2_inf", n),
+                              (d_ok, "d_ok", offs.size - 1)):
+            if t is not None and t.shape[0] != want:
+                raise ValueError("%s must have %d rows, got %d" % (name, want, t.shape[0]))
+        self._call("sylow_b200_pairing_check_ragged_batch_dev", d_g1, d_g1_inf, d_g2, d_g2_inf, offs, offs.size - 1,
+                   d_ok, self._stream())
 
     def g1_mul_batch_dev(self, d_pts, d_scalars, d_out, d_out_inf=None, d_pts_inf=None):
         self._call("sylow_b200_g1_mul_batch_dev", d_pts, d_pts_inf, d_scalars, d_pts.shape[0], d_out, d_out_inf,

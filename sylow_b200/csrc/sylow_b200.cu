@@ -17,6 +17,7 @@
 #include "miller_tables.cuh"
 #include "group_law.cuh"
 #include "launch_plan.h"
+#include "ragged_plan.h"
 #include "groth16.cuh"
 
 using namespace sylow;
@@ -566,18 +567,72 @@ __global__ void k_eip196_finish(const uint8_t* __restrict__ pts, const uint8_t* 
   if (i < n) eip196_finish_item(pts + i * 64, inf[i], st_a[i], st_b ? st_b[i] : 0, out + i * 64, status + i);
 }
 
-// per check: the first non-zero pair status wins and forces ok = 0
+// check c of the k pairs from `first`: the first non-zero pair status (G1 before G2 within a pair) wins and forces
+// ok = 0
+__device__ __forceinline__ void fold_status_item(const int8_t* __restrict__ st_g1, const int8_t* __restrict__ st_g2,
+                                                 size_t first, size_t k, size_t c, uint8_t* __restrict__ ok,
+                                                 int8_t* __restrict__ status) {
+  int8_t st = 0;
+  for (size_t j = 0; j < k && st == 0; j++) {
+    st = st_g1[first + j];
+    if (st == 0) st = st_g2[first + j];
+  }
+  if (st != 0) ok[c] = 0;
+  status[c] = st;
+}
 __global__ void k_fold_status(const int8_t* __restrict__ st_g1, const int8_t* __restrict__ st_g2, size_t k, size_t n_checks,
                               uint8_t* __restrict__ ok, int8_t* __restrict__ status) {
   size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= n_checks) return;
-  int8_t st = 0;
-  for (size_t j = 0; j < k && st == 0; j++) {
-    st = st_g1[c * k + j];
-    if (st == 0) st = st_g2[c * k + j];
+  fold_status_item(st_g1, st_g2, c * k, k, c, ok, status);
+}
+// the same per check of pairs [pair_off[c], pair_off[c + 1]) (pair_off[0] = 0)
+__global__ void k_fold_status_ragged(const int8_t* __restrict__ st_g1, const int8_t* __restrict__ st_g2,
+                                     const uint64_t* __restrict__ pair_off, size_t n_checks, uint8_t* __restrict__ ok,
+                                     int8_t* __restrict__ status) {
+  size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= n_checks) return;
+  fold_status_item(st_g1, st_g2, pair_off[c], pair_off[c + 1] - pair_off[c], c, ok, status);
+}
+
+// ---- ragged pairing checks (ragged_plan.h) ----------------------------------------------------------
+// position i of the gathered arrays <- pair src[i]: the G1 and G2 points and, where given, both infinity flags
+__global__ void k_gather_pairs(const uint8_t* __restrict__ g1, const uint8_t* __restrict__ g1_inf,
+                               const uint8_t* __restrict__ g2, const uint8_t* __restrict__ g2_inf,
+                               const uint32_t* __restrict__ src, size_t n, uint8_t* __restrict__ g1_out,
+                               uint8_t* __restrict__ g1_inf_out, uint8_t* __restrict__ g2_out,
+                               uint8_t* __restrict__ g2_inf_out) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const size_t s = src[i];
+  const uint4* a = reinterpret_cast<const uint4*>(g1 + s * 64);
+  const uint4* b = reinterpret_cast<const uint4*>(g2 + s * 128);
+  uint4* ao = reinterpret_cast<uint4*>(g1_out + i * 64);
+  uint4* bo = reinterpret_cast<uint4*>(g2_out + i * 128);
+#pragma unroll
+  for (int j = 0; j < 4; j++) ao[j] = a[j];
+#pragma unroll
+  for (int j = 0; j < 8; j++) bo[j] = b[j];
+  if (g1_inf) g1_inf_out[i] = g1_inf[s];
+  if (g2_inf) g2_inf_out[i] = g2_inf[s];
+}
+
+// One level of a ragged product: thread t multiplies the Montgomery-form values vals[idx[chunk[t]] .. idx[chunk[t+1]])
+// (at most kRaggedChunk of them; none gives 1) and writes the product to final slot dst & ~kRaggedFinal when
+// dst[t] has kRaggedFinal set, else to value dst[t] of vals.
+__global__ void __launch_bounds__(SY_SMALL_THREADS)
+k_fp12_segment_products(uint8_t* vals, const uint32_t* __restrict__ chunk, const uint32_t* __restrict__ dst,
+                        const uint32_t* __restrict__ idx, size_t n_chunks, uint8_t* final_out) {
+  size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_chunks) return;
+  const uint32_t b = chunk[t], e = chunk[t + 1];
+  Fp12 acc = fp12_one();
+  for (uint32_t j = b; j < e; j++) {
+    Fp12 v = fp12_load_raw(vals + (size_t)idx[j] * 384);
+    acc = j == b ? v : fp12_mul(acc, v);
   }
-  if (st != 0) ok[c] = 0;
-  status[c] = st;
+  const uint32_t d = dst[t];
+  fp12_store_raw((d & kRaggedFinal ? final_out : vals) + (size_t)(d & ~kRaggedFinal) * 384, acc);
 }
 
 
@@ -1531,6 +1586,89 @@ int sylow_b200_pairing_check_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, c
   return launch_check_products(ctx, ctx->scratch0.p, k_prod, n_checks, ok_out, s);
 }
 
+// SYLOW_B200_RAGGED_GLUE = 1, 2 or 4 fixes the pairs per glued item of the ragged checks in place of glue_pairs' choice,
+// for measurement (tools/ragged_check_time.py times what the gluing buys); read on every call.
+static int ragged_glue() {
+  const char* v = getenv("SYLOW_B200_RAGGED_GLUE");
+  const int g = v ? atoi(v) : 0;
+  return g == 1 || g == 2 || g == 4 ? g : 0;
+}
+
+// ok[c] = (the product of the pairs [offsets[c], offsets[c + 1]) == 1) for n_checks >= 1 checks with non-decreasing
+// host offsets; the pointers address pair offsets[0].  The plan (ragged_plan.h): gather the pairs into class order,
+// Miller values of the 4-pair, 2-pair and single items into one value array, chunk products level by level into one
+// Montgomery-form product per check, then the final exponentiation and the comparison with 1.
+static int ragged_check_core(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf, const uint8_t* g2,
+                             const uint8_t* g2_inf, const uint64_t* offsets, size_t n_checks, uint8_t* ok,
+                             cudaStream_t s) {
+  const size_t n = (size_t)(offsets[n_checks] - offsets[0]);
+  if (!n) {  // every check is the empty product, the identity
+    CK(cudaMemsetAsync(ok, 1, n_checks, s));
+    return 0;
+  }
+  // value indices and check slots share 32-bit words with the kRaggedFinal bit; 2^31 pairs would take 416 GB
+  if (n >= kRaggedFinal || n_checks >= kRaggedFinal) return SYLOW_B200_ERR_ARG;
+  RaggedPlan p;
+  try {
+    p = ragged_plan(ctx->sms, offsets, n_checks, kGluedShape, ragged_glue());
+  } catch (...) {
+    return SYLOW_B200_ERR_NOMEM;
+  }
+  const size_t n4 = p.n_items[0], n2 = p.n_items[1], n1 = p.n_items[2];
+  CKS(reserve(ctx, ctx->scratch0, p.n_values * 384));
+  CKS(reserve(ctx, ctx->scratch1, n * 194));
+  CKS(reserve(ctx, ctx->scratch2, n_checks * 384));
+  uint8_t *vals = ctx->scratch0.p, *fin = ctx->scratch2.p;
+  uint8_t *G1 = ctx->scratch1.p, *G2 = G1 + n * 64;
+  uint8_t *I1 = g1_inf ? G2 + n * 128 : nullptr, *I2 = g2_inf ? G2 + n * 129 : nullptr;
+  // The plan's device copy is a staging buffer of this call: a stream-ordered allocation on s, freed on s after the
+  // last kernel that reads it, so no later call, on any stream, overwrites it while these kernels run.  The copy comes
+  // from pageable memory, which cudaMemcpyAsync has read by the time it returns, so the host vector may go with p.
+  uint32_t* d_plan = nullptr;
+  CK(cudaMallocAsync((void**)&d_plan, p.words.size() * 4, s));
+  auto run = [&]() -> int {
+    CK(cudaMemcpyAsync(d_plan, p.words.data(), p.words.size() * 4, cudaMemcpyHostToDevice, s));
+    k_gather_pairs<<<nblocks(n, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(g1, g1_inf, g2, g2_inf, d_plan, n, G1, I1,
+                                                                            G2, I2);
+    LAUNCHED(ctx);
+    if (n4)
+      CKS(launch_glued(ctx, 4, 0, G1, 4, I1, G2, I2, nullptr, 0, nullptr, nullptr, n4, vals, s));
+    const size_t p2 = 4 * n4, p1 = p2 + 2 * n2;
+    if (n2)
+      CKS(launch_glued(ctx, 2, 0, G1 + p2 * 64, 2, adv(I1, p2), G2 + p2 * 128, adv(I2, p2), nullptr, 0, nullptr,
+                       nullptr, n2, vals + n4 * 384, s));
+    if (n1)
+      CKS(launch_miller(ctx, G1 + p1 * 64, adv(I1, p1), G2 + p1 * 128, adv(I2, p1), n1, vals + (n4 + n2) * 384, 1, s));
+    for (const RaggedLevel& l : p.levels) {
+      const uint32_t* chunk = d_plan + l.at;
+      k_fp12_segment_products<<<nblocks(l.n_chunks, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(
+          vals, chunk, chunk + l.n_chunks + 1, chunk + 2 * l.n_chunks + 1, l.n_chunks, fin);
+      LAUNCHED(ctx);
+    }
+    CKS(launch_final_exp(ctx, fin, 1, n_checks, fin, s));
+    k_gt_is_one<<<nblocks(n_checks, SY_SMALL_THREADS), SY_SMALL_THREADS, 0, s>>>(fin, n_checks, ok);
+    LAUNCHED(ctx);
+    return 0;
+  };
+  const int rc = run();
+  const cudaError_t e = cudaFreeAsync(d_plan, s);
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail_cuda(ctx, e);
+  return 0;
+}
+
+int sylow_b200_pairing_check_ragged_batch_dev(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf,
+                                              const uint8_t* g2, const uint8_t* g2_inf, const uint64_t* offsets,
+                                              size_t n_checks, uint8_t* ok_out, void* stream) {
+  ENTER_DEV(ctx);
+  if (!n_checks) return 0;
+  if (!offsets || !ok_out || !ragged_offsets_ok(offsets, n_checks)) return SYLOW_B200_ERR_ARG;
+  const uint64_t o0 = offsets[0];
+  if (offsets[n_checks] > o0 && (!g1 || !g2)) return SYLOW_B200_ERR_ARG;
+  return ragged_check_core(ctx, adv(g1, o0 * 64), adv(g1_inf, o0), adv(g2, o0 * 128), adv(g2_inf, o0), offsets,
+                           n_checks, ok_out, pick(ctx, stream));
+}
+
 // out[i] = affine(scalars[i] * pts[i]) in G1 (g2 = 0) or G2
 static int mul_dev(sylow_b200_ctx* ctx, int g2, const uint8_t* pts, const uint8_t* pts_inf, const uint8_t* scalars,
                    size_t n, uint8_t* out, uint8_t* out_inf, void* stream) {
@@ -1964,15 +2102,16 @@ static int pairing_host(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g
 // host thread per GPU driving that GPU's own single-device context (SURVEY.md 8e).  Per-item outputs land in the
 // caller's buffers directly; product forms combine the G 384-byte partials on the first device.  Nothing throws
 // across the ABI: thread creation failures come back as SYLOW_B200_ERR_NOMEM.
+// multi_cuts: the slices [cut[g], cut[g + 1]) of given cut points (cut[0] = 0, cut[G] = n, non-decreasing).
 template <class Fn>
-static int multi_slices(sylow_b200_ctx* ctx, size_t n, Fn fn) {
+static int multi_cuts(sylow_b200_ctx* ctx, const std::vector<size_t>& cut, Fn fn) {
   const size_t G = ctx->children.size();
   std::vector<int> rc(G, 0);
   try {
     std::vector<std::thread> th;
     th.reserve(G);
     for (size_t g = 0; g < G; g++) {
-      size_t off = g * n / G, m = (g + 1) * n / G - off;
+      size_t off = cut[g], m = cut[g + 1] - off;
       if (!m) continue;
       sylow_b200_ctx* c = ctx->children[g];
       th.emplace_back([&rc, &fn, c, g, off, m] { rc[g] = fn(c, g, off, m); });
@@ -1984,6 +2123,18 @@ static int multi_slices(sylow_b200_ctx* ctx, size_t n, Fn fn) {
   for (int r : rc)
     if (r) return r;
   return 0;
+}
+template <class Fn>
+static int multi_slices(sylow_b200_ctx* ctx, size_t n, Fn fn) {
+  const size_t G = ctx->children.size();
+  std::vector<size_t> cut;
+  try {
+    cut.resize(G + 1);
+  } catch (...) {
+    return SYLOW_B200_ERR_NOMEM;
+  }
+  for (size_t g = 0; g <= G; g++) cut[g] = g * n / G;
+  return multi_cuts(ctx, cut, fn);
 }
 // Product forms: fn(child, off, m, partial) writes the canonical product of its slice to `partial` (an empty slice
 // contributes 1), and the first device multiplies the G partials into f_out.
@@ -2105,6 +2256,38 @@ int sylow_b200_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const
   uint8_t* d_ok = io.area(n_checks);
   CKS(io.err);
   CKS(sylow_b200_pairing_check_batch_dev(ctx, d1, d1i, d2, d2i, k, n_checks, d_ok, nullptr));
+  io.down(ok_out, d_ok, n_checks);
+  return io.finish();
+}
+
+// Host form of the ragged checks.  A multi-device context cuts the batch at check boundaries into slices of about equal
+// pair counts (ragged_cuts); each slice is the same call on its device with offsets + cut (offsets[0] need not be 0).
+int sylow_b200_pairing_check_ragged_batch(sylow_b200_ctx* ctx, const uint8_t* g1, const uint8_t* g1_inf,
+                                          const uint8_t* g2, const uint8_t* g2_inf, const uint64_t* offsets,
+                                          size_t n_checks, uint8_t* ok_out) {
+  if (is_multi(ctx) && n_checks && offsets && ok_out && ragged_offsets_ok(offsets, n_checks)) {
+    std::vector<size_t> cut;
+    try {
+      cut = ragged_cuts(offsets, n_checks, ctx->children.size());
+    } catch (...) {
+      return SYLOW_B200_ERR_NOMEM;
+    }
+    return multi_cuts(ctx, cut, [=](sylow_b200_ctx* c, size_t, size_t first, size_t m) {
+      return sylow_b200_pairing_check_ragged_batch(c, g1, g1_inf, g2, g2_inf, offsets + first, m, ok_out + first);
+    });
+  }
+  ENTER(ctx);
+  if (!n_checks) return 0;
+  if (!offsets || !ok_out || !ragged_offsets_ok(offsets, n_checks)) return SYLOW_B200_ERR_ARG;
+  const uint64_t o0 = offsets[0];
+  const size_t n = (size_t)(offsets[n_checks] - o0);
+  if (n && (!g1 || !g2)) return SYLOW_B200_ERR_ARG;
+  Staging io(ctx);
+  const uint8_t *d2 = io.up(adv(g2, o0 * 128), n * 128), *d1 = io.up(adv(g1, o0 * 64), n * 64),
+                *d1i = io.up(adv(g1_inf, o0), n), *d2i = io.up(adv(g2_inf, o0), n);
+  uint8_t* d_ok = io.area(n_checks);
+  CKS(io.err);
+  CKS(ragged_check_core(ctx, d1, d1i, d2, d2i, offsets, n_checks, d_ok, ctx->stream));
   io.down(ok_out, d_ok, n_checks);
   return io.finish();
 }
@@ -2879,6 +3062,91 @@ int sylow_b200_eip197_pairing_check_batch(sylow_b200_ctx* ctx, const uint8_t* in
   io.down(ok_out, d_ok, n_checks);
   io.down(status_out, d_st, n_checks);
   return io.finish();
+}
+
+// EIP-197 over inputs of any length.  Only the well-formed inputs' bytes are staged, back to back (one copy per run of
+// inputs adjacent in the caller's buffer), so that the pairs sit at stride 192 for the decoders; a malformed input is an
+// empty check on the device and gets ok = 0, status = SYLOW_B200_ERR_ARG on the host.  A multi-device context cuts the
+// batch at input boundaries into slices of about equal pair counts.
+int sylow_b200_eip197_pairing_check_ragged_batch(sylow_b200_ctx* ctx, const uint8_t* input, const uint64_t* offsets,
+                                                 size_t n_checks, uint8_t* ok_out, int8_t* status_out) {
+  if (!ctx) return SYLOW_B200_ERR_ARG;
+  if (!n_checks) return 0;
+  if (!offsets || !ok_out || !status_out || !ragged_offsets_ok(offsets, n_checks)) return SYLOW_B200_ERR_ARG;
+  if (offsets[n_checks] > offsets[0] && !input) return SYLOW_B200_ERR_ARG;
+  // pair offsets of the staged inputs: a malformed input holds none
+  std::vector<uint64_t> po;
+  std::vector<size_t> cut;
+  try {
+    po.resize(n_checks + 1);
+    po[0] = 0;
+    for (size_t c = 0; c < n_checks; c++) {
+      const uint64_t len = offsets[c + 1] - offsets[c];
+      po[c + 1] = po[c] + (len % 192 ? 0 : len / 192);
+    }
+    if (is_multi(ctx)) cut = ragged_cuts(po.data(), n_checks, ctx->children.size());
+  } catch (...) {
+    return SYLOW_B200_ERR_NOMEM;
+  }
+  if (is_multi(ctx))
+    return multi_cuts(ctx, cut, [=](sylow_b200_ctx* c, size_t, size_t first, size_t m) {
+      return sylow_b200_eip197_pairing_check_ragged_batch(c, input, offsets + first, m, ok_out + first,
+                                                          status_out + first);
+    });
+  ENTER(ctx);
+  const size_t n = (size_t)po[n_checks];
+  Staging io(ctx);
+  uint8_t *din = io.area(n * 192), *d2 = io.area(n * 128), *d1 = io.area(n * 64), *flags = io.area(4 * n);
+  const uint64_t* d_po = reinterpret_cast<const uint64_t*>(io.up(po.data(), (n_checks + 1) * 8));
+  uint8_t* d_ok = io.area(2 * n_checks + 64);
+  uint8_t *d1i = flags, *d2i = flags + n;
+  int8_t* st1 = reinterpret_cast<int8_t*>(flags + 2 * n);  // per-pair decode status of G1, then of G2
+  int8_t* st2 = st1 + n;
+  uint64_t run_src = 0, run_len = 0, run_dst = 0;
+  auto flush = [&] {
+    if (run_len) io.check(cudaMemcpyAsync(din + run_dst, input + run_src, run_len, cudaMemcpyHostToDevice, ctx->stream));
+  };
+  for (size_t c = 0; c < n_checks && !io.err; c++) {
+    const uint64_t len = offsets[c + 1] - offsets[c];
+    if (!len || len % 192) continue;
+    if (run_len && offsets[c] == run_src + run_len) {
+      run_len += len;
+      continue;
+    }
+    flush();
+    run_src = offsets[c];
+    run_dst = po[c] * 192;
+    run_len = len;
+  }
+  flush();
+  CKS(io.err);
+  int8_t* d_st = reinterpret_cast<int8_t*>(d_ok + ((n_checks + 15) / 16) * 16);
+  if (n) {
+    k_decode_be<2><<<nblocks(n, 128), 128, 0, ctx->stream>>>(din, 192, n, 1, d1, d1i, st1);
+    LAUNCHED(ctx);
+    k_decode_be<4><<<nblocks(n, 128), 128, 0, ctx->stream>>>(din + 64, 192, n, 1, d2, d2i, st2);
+    LAUNCHED(ctx);
+    k_g1_validate<<<nblocks(n, 128), 128, 0, ctx->stream>>>(d1, d1i, n, st1, 1);
+    LAUNCHED(ctx);
+    k_g2_validate<<<nblocks(n, SY_MUL_THREADS), SY_MUL_THREADS, 0, ctx->stream>>>(d2, d2i, n, st2, 1);
+    LAUNCHED(ctx);
+  }
+  CKS(ragged_check_core(ctx, d1, d1i, d2, d2i, po.data(), n_checks, d_ok, ctx->stream));
+  if (n) {
+    k_fold_status_ragged<<<nblocks(n_checks, 128), 128, 0, ctx->stream>>>(st1, st2, d_po, n_checks, d_ok, d_st);
+    LAUNCHED(ctx);
+  } else {
+    CK(cudaMemsetAsync(d_st, 0, n_checks, ctx->stream));  // empty inputs only: success (reth_bn128.rs:173-175)
+  }
+  io.down(ok_out, d_ok, n_checks);
+  io.down(status_out, d_st, n_checks);
+  CKS(io.finish());
+  for (size_t c = 0; c < n_checks; c++)
+    if ((offsets[c + 1] - offsets[c]) % 192) {
+      ok_out[c] = 0;
+      status_out[c] = SYLOW_B200_ERR_ARG;
+    }
+  return 0;
 }
 
 // The EIP-196 ecAdd (mul = 0: x1 || y1 || x2 || y2, 128 B) and ecMul (mul = 1: x || y || s, 96 B) bodies over n
